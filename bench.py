@@ -2,7 +2,7 @@
 """bench.py -- GiNGR update() iterations/s on the BASELINE.json workload (C4: CPD, M = 20 000 moving points,
 N = 200 000 target points, rank-2000 GPMM, w = 0.1), synthetic seeded inputs (SURVEY.md 8d).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c4|c4_small|c3c|c1]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload c4|c4_small|c3c|c1] [--dump-outputs DIR]
 
 One "step" = one GingrAlgorithm.update + fit refresh (GingrGeneratorWrapper.propose) of ONE registration.
 With N > 1 (torchrun, one rank per GPU) the same registration is sharded over the ranks -- target points in the
@@ -22,6 +22,10 @@ library, so scaling is STRONG (total work fixed).  Prints one JSON line (rank 0)
             same workload (bounded sample = 1 iteration), N = 1 only.
   secondary the other named configurations of BASELINE.json (C1, C3, C5) and the ICP iteration at 200k points with the K2
             roofline (bench_secondary.py).
+
+--dump-outputs DIR writes the state the timed path computed in its last step (fit, shape coefficients, sigma2, scale,
+translation, Euler angles, iteration count) as DIR/<name>.npy in float64.  The inputs are seeded, so two builds run
+with the same arguments can be compared output for output.
 
 --impl reference times the CPU port as the main line (the JVM reference cannot run here: no JVM, scalismo /
 Breeze jars absent; DESIGN.md): real update() iterations of the oracle (oracle/fast.py: the algorithmic-minimum form,
@@ -90,6 +94,17 @@ def load_peaks():
             with open(p) as f:
                 peaks[fn] = json.load(f)
     return peaks
+
+
+def dump_outputs(out_dir: str, scale, translation, euler, shape, fit, sigma2, iteration):
+    """The registration state a caller receives after the last timed step, one float64 .npy file per field.  `iteration`
+    is the number of updates behind the state (warm-up included), so dumps of runs with different warm-up agree on which
+    step they describe."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"scale": scale, "translation": translation, "euler": euler, "shape": shape, "fit": fit, "sigma2": sigma2,
+              "iteration": iteration}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 class ClockSampler:
@@ -200,6 +215,9 @@ def run_reference(args):
     name = args.workload
     M, N, r, desc = WORKLOADS[name]
     secs, cores, note, st = cpu_oracle_chain(name, args.warmup, args.steps, budget_s=args.ref_budget_s)
+    if args.dump_outputs:
+        p = st.params
+        dump_outputs(args.dump_outputs, p.scale, p.translation, p.euler, p.shape, st.fit, st.sigma2, st.iteration)
     sec = statistics.mean(secs)
     v = 1.0 / sec
     line = {
@@ -313,6 +331,10 @@ def run_ours(args):
     barrier()
     launches = ctx.launch_count - l0
     ms_chain = e0.elapsed_time(e1)
+    if args.dump_outputs and rank == 0:
+        st = reg.downloadState()
+        p = st.modelParameters
+        dump_outputs(args.dump_outputs, p.scale, p.translation, p.euler, p.shape, st.fit, st.sigma2, st.iteration)
     reg.setProfiling(True)
     barrier()
     reg.updateChain(args.steps)
@@ -464,6 +486,8 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the C1 / C3 / C5 / ICP-200k entries")
     ap.add_argument("--ref-budget-s", type=float, default=900.0,
                     help="--impl reference: stop after this many seconds of iterations (the completed count is reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the state computed by the last timed step to DIR/<name>.npy (float64)")
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

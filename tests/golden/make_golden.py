@@ -1,16 +1,16 @@
 """Generate tests/golden/femur_golden.npz.
 
-INPUTS come from the reference's own example data (read here, in the build container, from
-/root/reference/examples/data/femur/{femur,femur_target}.stl and their landmark JSONs -- the data of
-examples/DemoICP.scala:11-17 and examples/DemoCPD.scala:11-17).  /root/reference does not exist on the GPU box, so the
-vertices / triangles / landmarks are committed in the fixture.
+INPUTS come from the reference's own example data, examples/data/femur/{femur,femur_target}.stl and their landmark
+JSONs in the GiNGR checkout that GINGR_REFERENCE names (the data of examples/DemoICP.scala:11-17 and
+examples/DemoCPD.scala:11-17).  The vertices / triangles / landmarks are committed in the fixture, so the tests that
+read it need no such checkout.
 
 OUTPUTS are those of the CPU oracle (oracle/) at the time of generation: the reference itself cannot run here (no
 JVM, scalismo and Breeze absent), so these are REGRESSION vectors on real data -- they pin the oracle and the CUDA
 path to each other across commits and machines; they are not outputs of the Scala code.  Parity stays "unpinned" in
 the sense of DESIGN.md.
 
-    python tests/golden/make_golden.py
+    GINGR_REFERENCE=<GiNGR checkout> python tests/golden/make_golden.py
 """
 import json
 import os
@@ -22,7 +22,6 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-DATA = "/root/reference/examples/data/femur"
 
 
 def read_binary_stl(path):
@@ -54,12 +53,15 @@ def femur_gpmm(ref, rank=50, seed=7):
 
 
 def main():
+    if not os.environ.get("GINGR_REFERENCE"):
+        sys.exit("make_golden.py: set GINGR_REFERENCE to a GiNGR checkout; its examples/data/femur holds the input meshes")
+    data = os.path.join(os.environ["GINGR_REFERENCE"], "examples", "data", "femur")
     from oracle import oracle
     oracle.build()
-    rv, rt = read_binary_stl(os.path.join(DATA, "femur.stl"))
-    tv, tt = read_binary_stl(os.path.join(DATA, "femur_target.stl"))
-    ids_r, lm_r = landmarks(os.path.join(DATA, "femur.json"))
-    ids_t, lm_t = landmarks(os.path.join(DATA, "femur_target.json"))
+    rv, rt = read_binary_stl(os.path.join(data, "femur.stl"))
+    tv, tt = read_binary_stl(os.path.join(data, "femur_target.stl"))
+    ids_r, lm_r = landmarks(os.path.join(data, "femur.json"))
+    ids_t, lm_t = landmarks(os.path.join(data, "femur_target.json"))
     common = [i for i in ids_r if i in ids_t]
     lm_r = np.array([lm_r[ids_r.index(i)] for i in common])
     lm_t = np.array([lm_t[ids_t.index(i)] for i in common])

@@ -9,8 +9,9 @@ import re
 import numpy as np
 import pytest
 
-REF = "/root/reference/src/main/scala/gingr"
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF), reason="reference sources not mounted (GPU box)")
+# GINGR_REFERENCE: a checkout of the Scala GiNGR project, the sources these defaults are checked against
+REF = os.path.join(os.environ["GINGR_REFERENCE"], "src", "main", "scala", "gingr") if os.environ.get("GINGR_REFERENCE") else ""
+needs_reference = pytest.mark.skipif(not os.path.isdir(REF), reason="GINGR_REFERENCE does not name a GiNGR checkout")
 
 
 def _case_class_defaults(path, name):

@@ -7,7 +7,8 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, os.path.join(ROOT, "examples"))
-REF_DATA = "/root/reference/examples/data"
+# GINGR_REFERENCE: a checkout of the Scala GiNGR project, whose example data files are read here
+REF_DATA = os.path.join(os.environ["GINGR_REFERENCE"], "examples", "data") if os.environ.get("GINGR_REFERENCE") else ""
 
 
 def test_demo_cli_and_synthetic_dataset(capsys):
@@ -24,7 +25,7 @@ def test_demo_cli_and_synthetic_dataset(capsys):
     assert np.allclose(b["target"][0], a["target"][0] @ R.T + [1.0, 2.0, 3.0])
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference examples not mounted (GPU box)")
+@pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="GINGR_REFERENCE does not name a GiNGR checkout")
 def test_demo_datasets_from_the_reference_files():
     import demos
     f = demos.load_dataset("femur", REF_DATA)

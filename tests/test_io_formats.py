@@ -8,8 +8,9 @@ import os
 import numpy as np
 import pytest
 
-REF_DATA = "/root/reference/examples/data"
-needs_reference = pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="reference examples not mounted (GPU box)")
+# GINGR_REFERENCE: a checkout of the Scala GiNGR project, whose example data files are read here
+REF_DATA = os.path.join(os.environ["GINGR_REFERENCE"], "examples", "data") if os.environ.get("GINGR_REFERENCE") else ""
+needs_reference = pytest.mark.skipif(not os.path.isdir(REF_DATA), reason="GINGR_REFERENCE does not name a GiNGR checkout")
 
 
 def _tetra():
