@@ -57,22 +57,20 @@ int32_t gingr_ctx_create(int32_t device, gingr_ctx** out) {
                       "gingr_ctx_create: no CUDA device (libgingr_cuda has no CPU fallback)");
   }
   if (device < 0 || device >= count) return gingr_fail(nullptr, GINGR_ERR_ARG, "gingr_ctx_create: bad device index");
-  gingr_ctx_full* ctx = new gingr_ctx_full();
+  std::unique_ptr<gingr_ctx, decltype(&gingr_ctx_destroy)> ctx(new gingr_ctx_full(), gingr_ctx_destroy);
   ctx->device = device;
   GINGR_CUDA_TRY(nullptr, cudaSetDevice(device));
   cudaDeviceProp prop;
   GINGR_CUDA_TRY(nullptr, cudaGetDeviceProperties(&prop, device));
-  if (prop.major < 10) {
-    delete ctx;
+  if (prop.major < 10)
     return gingr_fail(nullptr, GINGR_ERR_CUDA, "gingr_ctx_create: device is not sm_100 (Blackwell) -- unsupported");
-  }
   ctx->num_sms = prop.multiProcessorCount;
   int prio_lo = 0, prio_hi = 0;
   GINGR_CUDA_TRY(nullptr, cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
   GINGR_CUDA_TRY(nullptr, cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio_hi));
   GINGR_CUDA_TRY(nullptr, cudaStreamCreateWithPriority(&ctx->side_stream, cudaStreamNonBlocking, prio_lo));
   GINGR_CUDA_TRY(nullptr, cudaMallocHost((void**)&ctx->h_pinned, ctx->h_pinned_count * sizeof(double)));
-  *out = ctx;
+  *out = ctx.release();
   return GINGR_OK;
 }
 
@@ -80,20 +78,12 @@ int32_t gingr_ctx_destroy(gingr_ctx* ctx) {
   if (!ctx) return GINGR_OK;
   cudaSetDevice(ctx->device);
   cudaStreamSynchronize(ctx->stream);
-  CtxScratch* s = scratch_of(ctx);
-  s->estep.release();
-  s->a.release();
-  s->b.release();
-  s->c.release();
-  s->d.release();
-  s->ia.release();
-  s->ua.release();
   gingr::comm_destroy(ctx);
   if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
   for (auto& e : ctx->chol_events) cudaEventDestroy(e);
   if (ctx->side_stream) cudaStreamDestroy(ctx->side_stream);
-  cudaStreamDestroy(ctx->stream);
-  delete static_cast<gingr_ctx_full*>(ctx);
+  if (ctx->stream) cudaStreamDestroy(ctx->stream);
+  delete static_cast<gingr_ctx_full*>(ctx);   // frees the scratch buffers
   return GINGR_OK;
 }
 
@@ -116,8 +106,6 @@ int64_t gingr_ctx_launch_count(const gingr_ctx* ctx) { return ctx ? ctx->launche
 // ---------------------------------------------------------------------------------------------
 // uploads
 // ---------------------------------------------------------------------------------------------
-static int32_t target_upload_into(gingr_ctx* ctx, gingr_target* t, int32_t N, const double* pts, const int32_t* tri, int32_t T);
-
 int32_t gingr_target_upload(gingr_ctx* ctx, int32_t N, const double* pts, const int32_t* tri, int32_t T,
                             gingr_target** out) {
   if (!ctx || !out || !pts || N <= 0 || T < 0 || (T > 0 && !tri))
@@ -126,18 +114,8 @@ int32_t gingr_target_upload(gingr_ctx* ctx, int32_t N, const double* pts, const 
   if (T > 0)
     for (int k = 0; k < 3 * T; ++k)
       if (tri[k] < 0 || tri[k] >= N) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_target_upload: triangle index out of range");
-  gingr_target* t = new gingr_target();
+  std::unique_ptr<gingr_target> t(new gingr_target());
   t->ctx = ctx;
-  const int32_t rc = target_upload_into(ctx, t, N, pts, tri, T);
-  if (rc != GINGR_OK) {
-    gingr_target_destroy(t);   // releases whatever was allocated before the failure
-    return rc;
-  }
-  *out = t;
-  return GINGR_OK;
-}
-
-static int32_t target_upload_into(gingr_ctx* ctx, gingr_target* t, int32_t N, const double* pts, const int32_t* tri, int32_t T) {
   t->N_total = N;
   for (size_t k = 0; k < (size_t)3 * N; ++k) {
     if (!(fabs(pts[k]) < INFINITY)) { t->nonfinite = true; break; }
@@ -166,31 +144,24 @@ static int32_t target_upload_into(gingr_ctx* ctx, gingr_target* t, int32_t N, co
   if (gingr::grid_wanted(N) && !t->nonfinite) {
     gingr::VertexArray va;
     va.p = t->aos.p;
-    t->pgrid = new gingr::SpatialGrid();
+    t->pgrid = std::make_unique<gingr::SpatialGrid>();
     GINGR_TRY(t->pgrid->ensure(ctx, N, N, false));
     GINGR_TRY(gingr::grid_build_points_enqueue(ctx, *t->pgrid, N, va));
     if (T > 0) {
-      t->tgrid = new gingr::SpatialGrid();
+      t->tgrid = std::make_unique<gingr::SpatialGrid>();
       t->tgrid->entry_boxes = true;   // static grid, searched every iteration: boxes stored with the entries
       GINGR_TRY(t->tgrid->ensure(ctx, N, T, true));
       GINGR_TRY(gingr::grid_build_triangles_enqueue(ctx, *t->tgrid, N, va, T, t->tri.p));
     }
   }
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  *out = t.release();
   return GINGR_OK;
 }
 
 int32_t gingr_target_destroy(gingr_target* t) {
   if (!t) return GINGR_OK;
   cudaSetDevice(t->ctx->device);
-  t->soa.release();
-  t->verts.release();
-  t->aos.release();
-  t->tri.release();
-  t->normals.release();
-  t->boundary.release();
-  if (t->pgrid) { t->pgrid->release(); delete t->pgrid; }
-  if (t->tgrid) { t->tgrid->release(); delete t->tgrid; }
   delete t;
   return GINGR_OK;
 }
@@ -343,10 +314,6 @@ struct TemplateUpload {
   DevBuf<int32_t> tri, off, adj;
   DevBuf<uint8_t> boundary;
   gingr::SpatialGrid pgrid, tgrid;
-  void release() {
-    aos.release(); soa.release(); normals.release(); tri.release(); off.release(); adj.release(); boundary.release();
-    pgrid.release(); tgrid.release();
-  }
 };
 
 static int32_t upload_template(gingr_ctx* ctx, int M, const double* tpl, const int32_t* tpl_tri, int T, TemplateUpload* u,
@@ -408,8 +375,8 @@ static gingr::MeshView target_view(const gingr_target* t) {
   v.tri = t->tri.p;
   v.normals = t->normals.p;
   v.boundary = t->boundary.p;
-  v.pgrid = t->pgrid;
-  v.tgrid = t->tgrid;
+  v.pgrid = t->pgrid.get();
+  v.tgrid = t->tgrid.get();
   return v;
 }
 
@@ -422,23 +389,15 @@ int32_t gingr_icp_closest(gingr_ctx* ctx, const gingr_target* target, int32_t M,
   gingr::ClosestWorkspace ws;
   TemplateUpload up;
   gingr::MeshView tv;
-  int32_t rc = ws.ensure(ctx, M, target->N_total, target->T, T);
-  if (rc >= 0) rc = upload_template(ctx, M, tpl, tpl_tri, T, &up, &tv, false);
-  if (rc >= 0) rc = gingr::icp_correspondence_enqueue(ctx, ws, tv, target_view(target), method);
+  GINGR_TRY(ws.ensure(ctx, M, target->N_total, target->T, T));
+  GINGR_TRY(upload_template(ctx, M, tpl, tpl_tri, T, &up, &tv, false));
+  GINGR_TRY(gingr::icp_correspondence_enqueue(ctx, ws, tv, target_view(target), method));
   cudaStream_t st = ctx->stream;
-  cudaError_t e = cudaSuccess;
-  if (rc >= 0) {
-    if (idx && e == cudaSuccess) e = cudaMemcpyAsync(idx, ws.idx.p, sizeof(int32_t) * (size_t)M, cudaMemcpyDeviceToHost, st);
-    if (cp && e == cudaSuccess) e = cudaMemcpyAsync(cp, ws.cp.p, sizeof(double) * 3 * (size_t)M, cudaMemcpyDeviceToHost, st);
-    if (w && e == cudaSuccess) e = cudaMemcpyAsync(w, ws.w.p, (size_t)M, cudaMemcpyDeviceToHost, st);
-    if (mean_distance && e == cudaSuccess) e = cudaMemcpyAsync(mean_distance, ws.mean_dist.p, sizeof(double), cudaMemcpyDeviceToHost, st);
-  }
-  cudaError_t e2 = cudaStreamSynchronize(st);
-  if (e == cudaSuccess) e = e2;
-  ws.release();
-  up.release();
-  if (rc < 0) return rc;
-  GINGR_CUDA_TRY(ctx, e);
+  if (idx) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(idx, ws.idx.p, sizeof(int32_t) * (size_t)M, cudaMemcpyDeviceToHost, st));
+  if (cp) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(cp, ws.cp.p, sizeof(double) * 3 * (size_t)M, cudaMemcpyDeviceToHost, st));
+  if (w) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(w, ws.w.p, (size_t)M, cudaMemcpyDeviceToHost, st));
+  if (mean_distance) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mean_distance, ws.mean_dist.p, sizeof(double), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   return GINGR_OK;
 }
 
@@ -453,26 +412,18 @@ int32_t gingr_icp_closest_reversal(gingr_ctx* ctx, const gingr_target* target, i
   TemplateUpload up;
   gingr::MeshView tv;
   DevBuf<int32_t> tid;
-  int32_t rc = ws.ensure(ctx, N, M, T, target->T);
-  if (rc >= 0) rc = upload_template(ctx, M, tpl, tpl_tri, T, &up, &tv, true);
+  GINGR_TRY(ws.ensure(ctx, N, M, T, target->T));
+  GINGR_TRY(upload_template(ctx, M, tpl, tpl_tri, T, &up, &tv, true));
   // corr = closestPointCorrespondence(target, template): the roles are swapped (:38)
-  if (rc >= 0) rc = gingr::icp_correspondence_enqueue(ctx, ws, target_view(target), tv, method);
+  GINGR_TRY(gingr::icp_correspondence_enqueue(ctx, ws, target_view(target), tv, method));
   cudaStream_t st = ctx->stream;
-  cudaError_t e = tid.alloc((size_t)N);
+  GINGR_CUDA_TRY(ctx, tid.alloc((size_t)N));
   // templateId = template.pointSet.findClosestPoint(p).id for the corresponding point p (:40)
-  if (rc >= 0 && e == cudaSuccess) rc = gingr::nn_vertex_enqueue(ctx, ws, N, ws.cp.p, M, up.soa.p, ws.d2.p, tid.p, tv.pgrid, ws.qorder);
-  if (rc >= 0) {
-    if (tpl_id && e == cudaSuccess) e = cudaMemcpyAsync(tpl_id, tid.p, sizeof(int32_t) * (size_t)N, cudaMemcpyDeviceToHost, st);
-    if (w && e == cudaSuccess) e = cudaMemcpyAsync(w, ws.w.p, (size_t)N, cudaMemcpyDeviceToHost, st);
-    if (mean_distance && e == cudaSuccess) e = cudaMemcpyAsync(mean_distance, ws.mean_dist.p, sizeof(double), cudaMemcpyDeviceToHost, st);
-  }
-  cudaError_t e2 = cudaStreamSynchronize(st);
-  if (e == cudaSuccess) e = e2;
-  ws.release();
-  up.release();
-  tid.release();
-  if (rc < 0) return rc;
-  GINGR_CUDA_TRY(ctx, e);
+  GINGR_TRY(gingr::nn_vertex_enqueue(ctx, ws, N, ws.cp.p, M, up.soa.p, ws.d2.p, tid.p, tv.pgrid, ws.qorder.get()));
+  if (tpl_id) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(tpl_id, tid.p, sizeof(int32_t) * (size_t)N, cudaMemcpyDeviceToHost, st));
+  if (w) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(w, ws.w.p, (size_t)N, cudaMemcpyDeviceToHost, st));
+  if (mean_distance) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mean_distance, ws.mean_dist.p, sizeof(double), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   return GINGR_OK;
 }
 

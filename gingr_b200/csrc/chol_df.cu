@@ -551,13 +551,6 @@ int32_t CholWs::alloc(gingr_ctx* ctx, int n, int nrows) {
   return GINGR_OK;
 }
 
-void CholWs::release() {
-  sync.release();
-  linv.release();
-  bsync.release();
-  cap_n = cap_nrows = 0;
-}
-
 int32_t cholesky_df_enqueue(gingr_ctx* ctx, int n, int nrows, double* d_A, int ld, int* d_info, CholWs& ws) {
   static thread_local int attr_device = -1;
   if (attr_device != ctx->device) {

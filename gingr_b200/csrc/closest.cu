@@ -411,10 +411,6 @@ int32_t mesh_static_upload(gingr_ctx* ctx, int n, const double* verts_aos_host, 
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(boundary->p, flags.data(), (size_t)n, cudaMemcpyHostToDevice, st));
   GINGR_TRY(vertex_normals_enqueue(ctx, n, d_v.p, d_tri.p, d_off.p, d_adj.p, normals->p));
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-  d_off.release();
-  d_adj.release();
-  d_tri.release();
-  d_v.release();
   return GINGR_OK;
 }
 
@@ -447,25 +443,10 @@ int32_t ClosestWorkspace::ensure(gingr_ctx* ctx, int nq, int n_search, int T_sea
   GINGR_CUDA_TRY(ctx, mean_dist.alloc(1));
   GINGR_CUDA_TRY(ctx, mean_part.alloc(MEAN_BLOCKS));
   if (grid_wanted(std::max(n_search, std::max(T_search, T_query_mesh)))) {
-    if (!qorder) qorder = new SpatialGrid();
+    if (!qorder) qorder = std::make_unique<SpatialGrid>();
     GINGR_TRY(qorder->ensure(ctx, nq, nq, false));
   }
   return GINGR_OK;
-}
-
-void ClosestWorkspace::release() {
-  part_d2.release();
-  part_idx.release();
-  part_cp.release();
-  d2.release();
-  surf_d2.release();
-  idx.release();
-  cp.release();
-  w.release();
-  hit.release();
-  mean_dist.release();
-  mean_part.release();
-  if (qorder) { qorder->release(); delete qorder; qorder = nullptr; }
 }
 
 // Nearest vertex (of a SoA point set) of arbitrary query points (AoS, device).
@@ -510,7 +491,7 @@ int32_t icp_correspondence_enqueue(gingr_ctx* ctx, ClosestWorkspace& ws, const M
     VertexArray qa;
     qa.p = q_aos;
     GINGR_TRY(grid_build_points_enqueue(ctx, *ws.qorder, M, qa));
-    order = ws.qorder;
+    order = ws.qorder.get();
   }
   if (method == GINGR_POINTCLOUD_CLOSEST_POINT) {
     GINGR_TRY(nn_vertex_enqueue(ctx, ws, M, q_aos, N, tgt.soa, o_d2, o_idx, tgt.pgrid, order));

@@ -1,5 +1,6 @@
 // closest.cuh -- host-side interface of the K2 closest-point kernels (closest.cu).
 #pragma once
+#include <memory>
 #include <vector>
 
 #include "common.cuh"
@@ -38,10 +39,9 @@ struct ClosestWorkspace {
   DevBuf<uint8_t> hit;        // [nq]   along-normal: the line met the target
   DevBuf<double> mean_dist;   // [1]
   DevBuf<double> mean_part;   // [64] per-block partial sums of the mean distance
-  SpatialGrid* qorder = nullptr;  // point grid over the queries = their spatial sort (grid searches only)
+  std::unique_ptr<SpatialGrid> qorder;  // point grid over the queries = their spatial sort (grid searches only)
   // nq queries against a mesh of n_search vertices / T_search triangles; T_query_mesh triangles of the query mesh
   int32_t ensure(gingr_ctx* ctx, int nq, int n_search, int T_search, int T_query_mesh);
-  void release();
 };
 
 void build_vertex_adjacency(int n, int T, const int32_t* tri, std::vector<int32_t>* off, std::vector<int32_t>* adj);

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <memory>
 #include <string>
 #include <vector>
 
@@ -31,11 +32,27 @@ struct gingr_ctx {
   size_t h_pinned_count = 4096;
 };
 
-// Device-side buffer with RAII-less explicit free (handles own them).
+// Device buffer that owns its memory: freed when the owner goes away, moved but never copied.
 template <typename T>
 struct DevBuf {
   T* p = nullptr;
   size_t n = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), n(o.n) { o.p = nullptr; o.n = 0; }
+  DevBuf& operator=(DevBuf&& o) noexcept {
+    if (this != &o) {
+      if (p) cudaFree(p);
+      p = o.p; n = o.n;
+      o.p = nullptr; o.n = 0;
+    }
+    return *this;
+  }
+  ~DevBuf() {
+    if (p) cudaFree(p);
+  }
+  // grows only: keeps the block when it holds count elements, else frees it before allocating the larger one
   cudaError_t alloc(size_t count) {
     if (p && n >= count) return cudaSuccess;
     if (p) cudaFree(p);
@@ -45,10 +62,27 @@ struct DevBuf {
     if (e == cudaSuccess) n = count;
     return e;
   }
-  void release() {
-    if (p) cudaFree(p);
-    p = nullptr;
-    n = 0;
+};
+
+// Owner of an instantiated CUDA graph; reset() destroys it.
+struct GraphExec {
+  cudaGraphExec_t h = nullptr;
+  GraphExec() = default;
+  GraphExec(const GraphExec&) = delete;
+  GraphExec& operator=(const GraphExec&) = delete;
+  GraphExec(GraphExec&& o) noexcept : h(o.h) { o.h = nullptr; }
+  GraphExec& operator=(GraphExec&& o) noexcept {
+    if (this != &o) {
+      reset();
+      h = o.h;
+      o.h = nullptr;
+    }
+    return *this;
+  }
+  ~GraphExec() { reset(); }
+  void reset() {
+    if (h) cudaGraphExecDestroy(h);
+    h = nullptr;
   }
 };
 
@@ -67,8 +101,7 @@ struct gingr_target {
   DevBuf<double> normals;   // [3][N_total]
   DevBuf<uint8_t> boundary; // [N_total]
   // static uniform grids over the vertices / triangles (K2 at scale; null below the size where a scan wins)
-  gingr::SpatialGrid* pgrid = nullptr;
-  gingr::SpatialGrid* tgrid = nullptr;
+  std::unique_ptr<gingr::SpatialGrid> pgrid, tgrid;
 };
 
 struct gingr_model {

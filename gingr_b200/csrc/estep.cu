@@ -498,18 +498,6 @@ int32_t EstepWorkspace::ensure(gingr_ctx* ctx, int M, int N) {
   return GINGR_OK;
 }
 
-void EstepWorkspace::release() {
-  colpart.release();
-  pack.release();
-  pt1.release();
-  xpx_part.release();
-  rowpart.release();
-  rows.release();
-  fit_soa.release();
-  rowf.release();
-  scal.release();
-}
-
 // Enqueue the E-step on ctx->stream.  fit_soa / rowf (may be null) / scal must be set up by the caller:
 // scal[0] = sigma2, scal[1] = a, scal[2] = c.  Results: ws.pt1 [N], ws.rows [4][M], ws.xpx_part.
 int32_t estep_enqueue(gingr_ctx* ctx, EstepWorkspace& ws, int M, int N, const double* target_soa, bool use_rowf,

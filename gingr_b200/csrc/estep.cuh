@@ -22,7 +22,6 @@ struct EstepWorkspace {
   DevBuf<double> rowf;      // [M]      BCPD row factors
   DevBuf<double> scal;      // [16]     0 sigma2, 1 a, 2 c, 3 w, 4 M/N, 5 s, 6 1/N
   int32_t ensure(gingr_ctx* ctx, int M, int N);
-  void release();
 };
 
 void estep_plan(const gingr_ctx* ctx, int M, int N, EstepPlan* p);

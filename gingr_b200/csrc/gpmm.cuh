@@ -251,133 +251,132 @@ int32_t gingr_gpmm_gaussian_mixture(gingr_ctx* ctx, int32_t M, const double* ref
   // scalar columns that may be needed (6000: the previous columns' pivot row is staged in 48 KB of shared memory)
   const int kcap = (int)std::min<long long>(std::min<long long>((full_cap + 2) / 3, M), 6000);
   const int nb = std::min(128, ceil_div(M, 256));
-  DevBuf<double> pts, d, Ls, Lt, pmax, psum, dpiv, trace, norm2a, norm2b;
-  DevBuf<int> pidx, pivots, flag;
-  DevBuf<uint8_t> done;
-  DevBuf<GpmmColumn> dcols;
-  gingr_model* m = nullptr;
-  int32_t rc = GINGR_OK;
-  auto A = [&](cudaError_t e) { if (e != cudaSuccess && rc == GINGR_OK) { gingr_set_error(ctx, cudaGetErrorString(e)); rc = GINGR_ERR_CUDA; } };
-  auto cleanup = [&]() {
-    pts.release(); d.release(); Ls.release(); Lt.release(); pmax.release(); psum.release(); dpiv.release(); trace.release();
-    norm2a.release(); norm2b.release(); pidx.release(); pivots.release(); flag.release(); done.release(); dcols.release();
-  };
-  // the factor grows in chunks of columns so that a small rank does not allocate M x kcap
-  int kalloc = std::min(kcap, 256);
-  A(pts.alloc((size_t)3 * M)); A(d.alloc(M)); A(done.alloc(M)); A(Ls.alloc((size_t)kalloc * M));
-  A(pmax.alloc(nb)); A(psum.alloc(nb)); A(pidx.alloc(nb)); A(pivots.alloc(kcap + 1)); A(dpiv.alloc(kcap + 1));
-  A(trace.alloc(kcap + 2)); A(flag.alloc(4));
-  if (rc != GINGR_OK) { cleanup(); return rc; }
-  A(cudaMemcpyAsync(pts.p, ref_pts, sizeof(double) * 3 * (size_t)M, cudaMemcpyHostToDevice, st));
-  gpmm_init_diag_kernel<<<ceil_div(M, 256), 256, 0, st>>>(M, kp, d.p, done.p);
-  GINGR_LAUNCHED(ctx);
-  // ---- pivoted Cholesky: batches of steps, the trace history decides where the reference's loop would have stopped
-  std::vector<double> htrace;
-  int k = 0;            // scalar steps done
-  int rank = -1;        // full rank 3 kk + c once known
-  double tol = 0.0;
-  while (rc == GINGR_OK && rank < 0) {
-    const int batch = std::min(32, kcap - k);
-    if (k + batch > kalloc) {   // grow the factor
-      const int knew = std::min(kcap, std::max(kalloc * 2, k + batch));
-      DevBuf<double> bigger;
-      A(bigger.alloc((size_t)knew * M));
-      if (rc == GINGR_OK) A(cudaMemcpyAsync(bigger.p, Ls.p, sizeof(double) * (size_t)k * M, cudaMemcpyDeviceToDevice, st));
-      if (rc == GINGR_OK) A(cudaStreamSynchronize(st));
-      if (rc != GINGR_OK) { bigger.release(); break; }
-      Ls.release();
-      Ls = bigger;
-      kalloc = knew;
-    }
-    for (int s = 0; s < batch; ++s) {
-      gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, d.p, done.p, pmax.p, pidx.p, psum.p);
-      gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, k + s, pmax.p, pidx.p, psum.p, pivots.p, dpiv.p, trace.p);
-      gpmm_column_kernel<<<ceil_div(M, 256), 256, sizeof(double) * (size_t)std::max(k + s, 1), st>>>(M, k + s, kp, pts.p, pivots.p,
-                                                                                                    dpiv.p, Ls.p, d.p, done.p);
-      ctx->launches += 3;
-    }
-    k += batch;
-    // T(k) after the batch
-    gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, d.p, done.p, pmax.p, pidx.p, psum.p);
-    gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, k, pmax.p, pidx.p, psum.p, pivots.p, dpiv.p, trace.p);
-    ctx->launches += 2;
-    htrace.resize(k + 1);
-    A(cudaMemcpyAsync(htrace.data(), trace.p, sizeof(double) * (k + 1), cudaMemcpyDeviceToHost, st));
-    A(cudaStreamSynchronize(st));
-    A(cudaGetLastError());
-    if (rc != GINGR_OK) break;
-    tol = rel_tol * 3.0 * htrace[0];
-    // the reference's loop: while (cols < n && trace > tolerance) add a column
-    for (int kk = 0; kk < k && rank < 0; ++kk)
-      for (int c = 0; c < 3; ++c) {
-        const double tr_before = 3.0 * htrace[kk] - c * (htrace[kk] - htrace[kk + 1]);
-        const long long cols = 3LL * kk + c;
-        if (!(tr_before > tol) || cols >= full_cap) { rank = (int)cols; break; }
+  std::unique_ptr<gingr_model> m;
+  int r = 0;
+  {   // the factor and its scratch are freed before the regression constants are built
+    DevBuf<double> pts, d, Ls, Lt, pmax, psum, dpiv, trace, norm2a, norm2b;
+    DevBuf<int> pidx, pivots, flag;
+    DevBuf<uint8_t> done;
+    DevBuf<GpmmColumn> dcols;
+    // the factor grows in chunks of columns so that a small rank does not allocate M x kcap
+    int kalloc = std::min(kcap, 256);
+    GINGR_CUDA_TRY(ctx, pts.alloc((size_t)3 * M));
+    GINGR_CUDA_TRY(ctx, d.alloc(M));
+    GINGR_CUDA_TRY(ctx, done.alloc(M));
+    GINGR_CUDA_TRY(ctx, Ls.alloc((size_t)kalloc * M));
+    GINGR_CUDA_TRY(ctx, pmax.alloc(nb));
+    GINGR_CUDA_TRY(ctx, psum.alloc(nb));
+    GINGR_CUDA_TRY(ctx, pidx.alloc(nb));
+    GINGR_CUDA_TRY(ctx, pivots.alloc(kcap + 1));
+    GINGR_CUDA_TRY(ctx, dpiv.alloc(kcap + 1));
+    GINGR_CUDA_TRY(ctx, trace.alloc(kcap + 2));
+    GINGR_CUDA_TRY(ctx, flag.alloc(4));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(pts.p, ref_pts, sizeof(double) * 3 * (size_t)M, cudaMemcpyHostToDevice, st));
+    gpmm_init_diag_kernel<<<ceil_div(M, 256), 256, 0, st>>>(M, kp, d.p, done.p);
+    GINGR_LAUNCHED(ctx);
+    // ---- pivoted Cholesky: batches of steps, the trace history decides where the reference's loop would have stopped
+    std::vector<double> htrace;
+    int k = 0;            // scalar steps done
+    int rank = -1;        // full rank 3 kk + c once known
+    double tol = 0.0;
+    while (rank < 0) {
+      const int batch = std::min(32, kcap - k);
+      if (k + batch > kalloc) {   // grow the factor
+        const int knew = std::min(kcap, std::max(kalloc * 2, k + batch));
+        DevBuf<double> bigger;
+        GINGR_CUDA_TRY(ctx, bigger.alloc((size_t)knew * M));
+        GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(bigger.p, Ls.p, sizeof(double) * (size_t)k * M, cudaMemcpyDeviceToDevice, st));
+        GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+        Ls = std::move(bigger);
+        kalloc = knew;
       }
-    if (rank < 0 && (k >= kcap || !(3.0 * htrace[k] > tol))) rank = (int)std::min<long long>(3LL * k, full_cap);
-    if (rank < 0 && (long long)3 * k >= full_cap) rank = (int)full_cap;
-  }
-  if (rc == GINGR_OK && rank <= 0) rc = gingr_fail(ctx, GINGR_ERR_ARG, "gingr_gpmm_gaussian_mixture: the tolerance leaves an empty model");
-  if (rc != GINGR_OK) { cleanup(); return rc; }
-  // dims < c use k1 scalar columns, dims >= c use k1 - 1 (c == 0: all dims use rank / 3)
-  const int cpart = rank % 3;
-  const int k_hi = (rank + 2) / 3, k_lo = rank / 3;
-  // ---- KL basis: one-sided Jacobi on the factor (a second, truncated copy when the last triple is incomplete)
-  std::vector<double> n_hi, n_lo;
-  int sweeps = 0;
-  A(norm2a.alloc(std::max(k_hi, 1))); A(norm2b.alloc(std::max(k_lo, 1)));
-  if (cpart != 0 && k_lo > 0) {
-    A(Lt.alloc((size_t)k_lo * M));
-    if (rc == GINGR_OK) A(cudaMemcpyAsync(Lt.p, Ls.p, sizeof(double) * (size_t)k_lo * M, cudaMemcpyDeviceToDevice, st));
-  }
-  if (rc == GINGR_OK) rc = gpmm_jacobi(ctx, M, k_hi, Ls.p, flag.p, norm2a.p, &n_hi, &sweeps);
-  if (rc == GINGR_OK && cpart != 0 && k_lo > 0) rc = gpmm_jacobi(ctx, M, k_lo, Lt.p, flag.p, norm2b.p, &n_lo, nullptr);
-  if (rc != GINGR_OK) { cleanup(); return rc; }
-  // ---- columns of the model, sorted by variance (descending; ties: dimension, then scalar column)
-  std::vector<GpmmColumn> cols;
-  std::vector<double> lam;
-  for (int dd = 0; dd < 3; ++dd) {
-    const bool hi = cpart == 0 || dd < cpart;
-    const int kd = hi ? k_hi : k_lo;
-    for (int j = 0; j < kd; ++j) {
-      cols.push_back(GpmmColumn{hi ? 0 : 1, j, dd});
-      lam.push_back(hi ? n_hi[j] : n_lo[j]);
+      for (int s = 0; s < batch; ++s) {
+        gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, d.p, done.p, pmax.p, pidx.p, psum.p);
+        gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, k + s, pmax.p, pidx.p, psum.p, pivots.p, dpiv.p, trace.p);
+        gpmm_column_kernel<<<ceil_div(M, 256), 256, sizeof(double) * (size_t)std::max(k + s, 1), st>>>(M, k + s, kp, pts.p, pivots.p,
+                                                                                                      dpiv.p, Ls.p, d.p, done.p);
+        ctx->launches += 3;
+      }
+      k += batch;
+      // T(k) after the batch
+      gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, d.p, done.p, pmax.p, pidx.p, psum.p);
+      gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, k, pmax.p, pidx.p, psum.p, pivots.p, dpiv.p, trace.p);
+      ctx->launches += 2;
+      htrace.resize(k + 1);
+      GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(htrace.data(), trace.p, sizeof(double) * (k + 1), cudaMemcpyDeviceToHost, st));
+      GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+      GINGR_CUDA_TRY(ctx, cudaGetLastError());
+      tol = rel_tol * 3.0 * htrace[0];
+      // the reference's loop: while (cols < n && trace > tolerance) add a column
+      for (int kk = 0; kk < k && rank < 0; ++kk)
+        for (int c = 0; c < 3; ++c) {
+          const double tr_before = 3.0 * htrace[kk] - c * (htrace[kk] - htrace[kk + 1]);
+          const long long cols = 3LL * kk + c;
+          if (!(tr_before > tol) || cols >= full_cap) { rank = (int)cols; break; }
+        }
+      if (rank < 0 && (k >= kcap || !(3.0 * htrace[k] > tol))) rank = (int)std::min<long long>(3LL * k, full_cap);
+      if (rank < 0 && (long long)3 * k >= full_cap) rank = (int)full_cap;
     }
-  }
-  std::vector<int> order(cols.size());
-  for (size_t q = 0; q < order.size(); ++q) order[q] = (int)q;
-  std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return lam[x] > lam[y]; });
-  const int r = (int)cols.size();
-  std::vector<GpmmColumn> scols(r);
-  std::vector<double> var(r);
-  for (int q = 0; q < r; ++q) { scols[q] = cols[order[q]]; var[q] = lam[order[q]]; }
-  // ---- the model handle
-  m = new gingr_model();
-  m->ctx = ctx;
-  m->M = M; m->r = r; m->rp = (r + 7) / 8 * 8; m->m0 = 0; m->Ml = M;
-  A(m->ref.alloc((size_t)3 * M)); A(m->mean.alloc((size_t)3 * M)); A(m->sqrt_lambda.alloc(m->rp));
-  A(m->phi.alloc((size_t)3 * M * m->rp)); A(dcols.alloc(r));
-  if (rc == GINGR_OK) {
+    if (rank <= 0) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_gpmm_gaussian_mixture: the tolerance leaves an empty model");
+    // dims < c use k1 scalar columns, dims >= c use k1 - 1 (c == 0: all dims use rank / 3)
+    const int cpart = rank % 3;
+    const int k_hi = (rank + 2) / 3, k_lo = rank / 3;
+    // ---- KL basis: one-sided Jacobi on the factor (a second, truncated copy when the last triple is incomplete)
+    std::vector<double> n_hi, n_lo;
+    int sweeps = 0;
+    GINGR_CUDA_TRY(ctx, norm2a.alloc(std::max(k_hi, 1)));
+    GINGR_CUDA_TRY(ctx, norm2b.alloc(std::max(k_lo, 1)));
+    if (cpart != 0 && k_lo > 0) {
+      GINGR_CUDA_TRY(ctx, Lt.alloc((size_t)k_lo * M));
+      GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(Lt.p, Ls.p, sizeof(double) * (size_t)k_lo * M, cudaMemcpyDeviceToDevice, st));
+    }
+    GINGR_TRY(gpmm_jacobi(ctx, M, k_hi, Ls.p, flag.p, norm2a.p, &n_hi, &sweeps));
+    if (cpart != 0 && k_lo > 0) GINGR_TRY(gpmm_jacobi(ctx, M, k_lo, Lt.p, flag.p, norm2b.p, &n_lo, nullptr));
+    // ---- columns of the model, sorted by variance (descending; ties: dimension, then scalar column)
+    std::vector<GpmmColumn> cols;
+    std::vector<double> lam;
+    for (int dd = 0; dd < 3; ++dd) {
+      const bool hi = cpart == 0 || dd < cpart;
+      const int kd = hi ? k_hi : k_lo;
+      for (int j = 0; j < kd; ++j) {
+        cols.push_back(GpmmColumn{hi ? 0 : 1, j, dd});
+        lam.push_back(hi ? n_hi[j] : n_lo[j]);
+      }
+    }
+    std::vector<int> order(cols.size());
+    for (size_t q = 0; q < order.size(); ++q) order[q] = (int)q;
+    std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return lam[x] > lam[y]; });
+    r = (int)cols.size();
+    std::vector<GpmmColumn> scols(r);
+    std::vector<double> var(r);
+    for (int q = 0; q < r; ++q) { scols[q] = cols[order[q]]; var[q] = lam[order[q]]; }
+    // ---- the model handle
+    m.reset(new gingr_model());
+    m->ctx = ctx;
+    m->M = M; m->r = r; m->rp = (r + 7) / 8 * 8; m->m0 = 0; m->Ml = M;
+    GINGR_CUDA_TRY(ctx, m->ref.alloc((size_t)3 * M));
+    GINGR_CUDA_TRY(ctx, m->mean.alloc((size_t)3 * M));
+    GINGR_CUDA_TRY(ctx, m->sqrt_lambda.alloc(m->rp));
+    GINGR_CUDA_TRY(ctx, m->phi.alloc((size_t)3 * M * m->rp));
+    GINGR_CUDA_TRY(ctx, dcols.alloc(r));
     std::vector<double> sl(m->rp, 0.0);
     for (int q = 0; q < r; ++q) sl[q] = sqrt(var[q]);
-    A(cudaMemcpyAsync(m->ref.p, pts.p, sizeof(double) * 3 * (size_t)M, cudaMemcpyDeviceToDevice, st));
-    A(cudaMemsetAsync(m->mean.p, 0, sizeof(double) * 3 * (size_t)M, st));
-    A(cudaMemsetAsync(m->phi.p, 0, sizeof(double) * (size_t)3 * M * m->rp, st));
-    A(cudaMemcpyAsync(m->sqrt_lambda.p, sl.data(), sizeof(double) * m->rp, cudaMemcpyHostToDevice, st));
-    A(cudaMemcpyAsync(dcols.p, scols.data(), sizeof(GpmmColumn) * r, cudaMemcpyHostToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(m->ref.p, pts.p, sizeof(double) * 3 * (size_t)M, cudaMemcpyDeviceToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaMemsetAsync(m->mean.p, 0, sizeof(double) * 3 * (size_t)M, st));
+    GINGR_CUDA_TRY(ctx, cudaMemsetAsync(m->phi.p, 0, sizeof(double) * (size_t)3 * M * m->rp, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(m->sqrt_lambda.p, sl.data(), sizeof(double) * m->rp, cudaMemcpyHostToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(dcols.p, scols.data(), sizeof(GpmmColumn) * r, cudaMemcpyHostToDevice, st));
     gpmm_assemble_kernel<<<dim3(ceil_div(M, 256), r), 256, 0, st>>>(M, r, m->rp, dcols.p, Ls.p, norm2a.p, Lt.p ? Lt.p : Ls.p,
                                                                     norm2b.p, m->phi.p);
     GINGR_LAUNCHED(ctx);
-    A(cudaGetLastError());
-    A(cudaStreamSynchronize(st));   // sl / scols are host vectors
+    GINGR_CUDA_TRY(ctx, cudaGetLastError());
+    GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));   // sl / scols are host vectors
+    (void)sweeps;
   }
-  cleanup();
-  if (rc == GINGR_OK) rc = model_upload_topology(ctx, m, tri, T);
-  if (rc == GINGR_OK) rc = model_build_constants(ctx, m);
-  if (rc != GINGR_OK) { gingr_model_destroy(m); return rc; }
-  *out = m;
+  GINGR_TRY(model_upload_topology(ctx, m.get(), tri, T));
+  GINGR_TRY(model_build_constants(ctx, m.get()));
+  *out = m.release();
   if (rank_out) *rank_out = r;
-  (void)sweeps;
   return GINGR_OK;
 }
 

@@ -553,13 +553,6 @@ int32_t GramPlan::build(gingr_ctx* ctx, int rows_, int r_, int rp_, int max_cta)
   return GINGR_OK;
 }
 
-void GramPlan::release() {
-  d_segs.release();
-  d_seg_begin.release();
-  d_tile_first.release();
-  d_partial.release();
-}
-
 // partial tiles of G = Phi^T diag(wrow) Phi  (wrow may be null)
 bool gram_rhs_fusable(const GramPlan& plan) {
   static const int use_ws = [] { const char* e = getenv("GINGR_GRAM_WS"); return e ? atoi(e) : 1; }();

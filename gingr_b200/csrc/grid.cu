@@ -314,14 +314,6 @@ int32_t SpatialGrid::ensure(gingr_ctx* ctx, int nv, int items, bool tri) {
   return GINGR_OK;
 }
 
-void SpatialGrid::release() {
-  params.release(); cell_start.release(); fill.release(); entries.release(); pts.release(); bbox_part.release();
-  tri_box.release();
-  entry_box.release();
-  block_sums.release();
-  built = false;
-}
-
 bool grid_wanted(int n_search) {
   // read on every call (not cached) so that a test process can run both paths on the same inputs
   const char* e = getenv("GINGR_K2_GRID");

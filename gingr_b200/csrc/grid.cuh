@@ -40,7 +40,6 @@ struct SpatialGrid {
   DevBuf<int32_t> block_sums;  // scan scratch
   bool built = false;
   int32_t ensure(gingr_ctx* ctx, int n_vertices, int n_items, bool triangles);
-  void release();
 };
 
 // point i, coordinate d of a vertex array = p[i * stride_pt + d * stride_dim]  (AoS: 3, 1;  SoA: 1, n)

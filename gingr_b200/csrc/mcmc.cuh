@@ -377,17 +377,9 @@ struct McmcState {
   gingr::SpatialGrid fit_tgrid;
   bool use_fit_tgrid = false;
   bool primed = false;
-  cudaGraphExec_t graph_exec = nullptr;
+  GraphExec graph_exec;
   uint64_t graph_seed = 0;
   int64_t graph_launches = 0;
-  void release() {
-    model_ids.release(); target_ids.release(); s_ds.release(); s_alpha.release(); s_fit.release(); s_fac.release();
-    s_is.release(); raw_cur.release(); cm_cur.release(); cm_prop.release(); best_ds.release(); best_alpha.release();
-    best_fit.release(); best_is.release(); md.release(); mi.release(); sys.release(); vecs.release(); u3m.release();
-    inst.release(); q_pts.release(); target_sub.release(); ws_m2t.release(); ws_t2m.release(); fit_tgrid.release();
-    if (graph_exec) cudaGraphExecDestroy(graph_exec);
-    graph_exec = nullptr;
-  }
 };
 
 using namespace gingr;
@@ -395,9 +387,7 @@ using namespace gingr;
 static void mcmc_release(gingr_registration* g) {
   if (!g->mcmc) return;
   ++g_batch_epoch;   // a batched plan that names this chain is stale
-  g->mcmc->release();
-  delete g->mcmc;
-  g->mcmc = nullptr;
+  g->mcmc.reset();
 }
 
 // gingr_initialize_state / gingr_update / gingr_update_chain* / gingr_update_batch moved the device-resident state: the kept
@@ -406,12 +396,8 @@ static void mcmc_invalidate(gingr_registration* g) {
   if (g && g->mcmc) g->mcmc->primed = false;
 }
 
-static void mcmc_drop_graph(McmcState* mc) {
-  if (mc->graph_exec) cudaGraphExecDestroy(mc->graph_exec);
-  mc->graph_exec = nullptr;
-}
 static void mcmc_drop_chain_graph(gingr_registration* g) {
-  if (g && g->mcmc) mcmc_drop_graph(g->mcmc);
+  if (g && g->mcmc) g->mcmc->graph_exec.reset();
 }
 
 // EvaluatorWrapper.logValue pieces of the state in the working buffers (fit, alpha): out[0] = ModelEvaluator,
@@ -421,7 +407,7 @@ static void mcmc_drop_chain_graph(gingr_registration* g) {
 static int32_t enqueue_log_value(gingr_registration* g, const double* d_fit, const double* d_alpha, double* d_out,
                                  const double* d_surface_d2 = nullptr) {
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   const gingr_model* m = g->model;
   const gingr_target* tg = g->target;
   cudaStream_t st = ctx->stream;
@@ -443,7 +429,7 @@ static int32_t enqueue_log_value(gingr_registration* g, const double* d_fit, con
       d2 = d_surface_d2;
     } else {
       MeshView tv;
-      tv.n = N; tv.aos = tg->aos.p; tv.soa = tg->verts.p; tv.T = tg->T; tv.tri = tg->tri.p; tv.tgrid = tg->tgrid;
+      tv.n = N; tv.aos = tg->aos.p; tv.soa = tg->verts.p; tv.T = tg->T; tv.tri = tg->tri.p; tv.tgrid = tg->tgrid.get();
       GINGR_TRY(surface_distance_enqueue(ctx, mc->ws_m2t, nq, q, tv));
     }
     GINGR_LAUNCH(ctx, mcmc_distance_logpdf_kernel, 1, 256, 0, st, nq, d2, sd, mode == GINGR_EVAL_SYMMETRIC ? 0.5 : 1.0, acc,
@@ -479,7 +465,7 @@ static int32_t enqueue_log_value(gingr_registration* g, const double* d_fit, con
 static int32_t enqueue_log_transition(gingr_registration* g, const double* d_raw, const double* d_cmean, const double* d_from_ds,
                                       const int* d_from_is, const double* d_to_mesh, double* d_out) {
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   const gingr_model* m = g->model;
   const int M = m->M, r = m->r, rp = m->rp;
   cudaStream_t st = ctx->stream;
@@ -507,7 +493,7 @@ static int32_t enqueue_to_mesh(gingr_registration* g, double step_length, const 
                                const double* d_to_alpha, const double** out) {
   if (step_length == 1.0) { *out = d_from_fit; return GINGR_OK; }
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   const gingr_model* m = g->model;
   const int M = m->M, r = m->r, rp = m->rp;
   double* v = mc->vecs.p;
@@ -539,12 +525,12 @@ static const double* posterior_surface_d2(const gingr_registration* g) {
 // Posterior + evaluators of the device-resident state: the chain starts from it.
 static int32_t mcmc_prime(gingr_registration* g) {
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   const gingr_model* m = g->model;
   const int M = m->M, r = m->r, rp = m->rp;
   cudaStream_t st = ctx->stream;
   g->keep_raw = true;
-  mcmc_drop_graph(mc);   // the captured step bakes in the state's stepLength (toMesh of the transition density)
+  mc->graph_exec.reset();   // the captured step bakes in the state's stepLength (toMesh of the transition density)
   // a new chain: step counter (the Philox stream position) and statistics start at zero
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(mc->md.p, 0, sizeof(double) * MD_COUNT, st));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(mc->mi.p, 0, sizeof(int) * MI_COUNT, st));
@@ -573,7 +559,7 @@ static int32_t mcmc_prime(gingr_registration* g) {
 // One Metropolis-Hastings step on the working state (which holds the current state after its posterior phase).
 static int32_t enqueue_mcmc_step(gingr_registration* g, uint64_t seed) {
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   const gingr_model* m = g->model;
   const int M = m->M, r = m->r, rp = m->rp;
   cudaStream_t st = ctx->stream;
@@ -645,22 +631,9 @@ static int32_t enqueue_mcmc_step(gingr_registration* g, uint64_t seed) {
 }
 
 static int32_t mcmc_capture(gingr_registration* g, uint64_t seed) {
-  gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
-  if (mc->graph_exec && mc->graph_seed == seed) return GINGR_OK;
-  mcmc_drop_graph(mc);
-  const int64_t l0 = ctx->launches;
-  GINGR_CUDA_TRY(ctx, cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-  const int32_t rc = enqueue_mcmc_step(g, seed);
-  cudaGraph_t graph = nullptr;
-  const cudaError_t e = cudaStreamEndCapture(ctx->stream, &graph);
-  mc->graph_launches = ctx->launches - l0;
-  ctx->launches = l0;
-  if (rc < 0) { if (graph) cudaGraphDestroy(graph); return rc; }
-  GINGR_CUDA_TRY(ctx, e);
-  const cudaError_t e2 = cudaGraphInstantiate(&mc->graph_exec, graph, 0);
-  cudaGraphDestroy(graph);
-  GINGR_CUDA_TRY(ctx, e2);
+  McmcState* mc = g->mcmc.get();
+  if (mc->graph_exec.h && mc->graph_seed == seed) return GINGR_OK;
+  GINGR_TRY(capture_graph(g->ctx, mc->graph_exec, &mc->graph_launches, [&] { return enqueue_mcmc_step(g, seed); }));
   mc->graph_seed = seed;
   return GINGR_OK;
 }
@@ -700,8 +673,8 @@ int32_t gingr_mcmc_configure(gingr_registration* g, const gingr_mcmc_settings* s
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   mcmc_release(g);
-  McmcState* mc = new McmcState();
-  g->mcmc = mc;
+  g->mcmc = std::make_unique<McmcState>();
+  McmcState* mc = g->mcmc.get();
   mc->cfg = *s;
   mc->dev.rho = s->random_mixture;
   for (int k = 0; k < 3; ++k) { mc->dev.sd[k] = s->rot_sdev[k]; mc->dev.sd[3 + k] = s->trans_sdev[k]; mc->dev.sd[6 + k] = s->shape_sdev[k]; }
@@ -757,7 +730,7 @@ int32_t gingr_evaluate_log_value(gingr_registration* g, const gingr_state* s, co
   GINGR_TRY(mcmc_check(g, "gingr_evaluate_log_value: bad argument"));
   if (!s || !alpha || !out) return gingr_fail(g->ctx, GINGR_ERR_ARG, "gingr_evaluate_log_value: bad argument");
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   g->state_valid = false;
   mc->primed = false;
@@ -777,7 +750,7 @@ int32_t gingr_log_transition_probability(gingr_registration* g, const gingr_stat
   if (!from || !from_alpha || !to || !to_alpha || !out)
     return gingr_fail(g->ctx, GINGR_ERR_ARG, "gingr_log_transition_probability: bad argument");
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   const gingr_model* m = g->model;
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   g->state_valid = false;
@@ -801,7 +774,7 @@ int32_t gingr_log_transition_probability(gingr_registration* g, const gingr_stat
 int32_t gingr_mcmc_chain(gingr_registration* g, int32_t iters, uint64_t seed) {
   GINGR_TRY(mcmc_check(g, "gingr_mcmc_chain: bad argument"));
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   if (iters < 0) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_chain: bad argument");
   if (!g->state_valid) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_chain: no device-resident state (call gingr_initialize_state first)");
   g->host_mirror_current = false;
@@ -811,7 +784,7 @@ int32_t gingr_mcmc_chain(gingr_registration* g, int32_t iters, uint64_t seed) {
   if (graph) GINGR_TRY(mcmc_capture(g, seed));
   for (int k = 0; k < iters; ++k) {
     if (graph) {
-      GINGR_CUDA_TRY(ctx, cudaGraphLaunch(mc->graph_exec, ctx->stream));
+      GINGR_CUDA_TRY(ctx, cudaGraphLaunch(mc->graph_exec.h, ctx->stream));
       ctx->launches += mc->graph_launches;
     } else {
       GINGR_TRY(enqueue_mcmc_step(g, seed));
@@ -843,7 +816,7 @@ int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t iters, ui
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   static const int batched = [] { const char* e = getenv("GINGR_MCMC_BATCHED"); return e ? atoi(e) : 1; }();
   if (batched && n >= 2 && n <= 65535 && graphs_enabled(ctx)) {
-    static thread_local BatchPlan bp;
+    static thread_local BatchPlan& bp = *new BatchPlan();   // never deleted (BatchPlan)
     if (!batch_plan_current(bp, ctx, regs, n, seed, 2)) {
       const int32_t rc = mcmc_batch_plan_build(ctx, regs, n, seed, bp);
       if (rc < 0) { bp.drop(); return rc; }
@@ -851,7 +824,7 @@ int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t iters, ui
     if (!bp.unsupported) {
       for (int k = 0; k < n; ++k)
         if (!regs[k]->mcmc->primed) GINGR_TRY(mcmc_prime(regs[k]));
-      for (int it = 0; it < iters; ++it) GINGR_CUDA_TRY(ctx, cudaGraphLaunch(bp.exec, ctx->stream));
+      for (int it = 0; it < iters; ++it) GINGR_CUDA_TRY(ctx, cudaGraphLaunch(bp.exec.h, ctx->stream));
       ctx->launches += (int64_t)iters * bp.nlaunch;
       return GINGR_OK;
     }
@@ -862,7 +835,7 @@ int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t iters, ui
     if (!regs[k]->mcmc->primed) GINGR_TRY(mcmc_prime(regs[k]));
     GINGR_TRY(mcmc_capture(regs[k], seed + (uint64_t)k));
   }
-  GINGR_TRY(replay_chain_graphs(ctx, sp, n, iters, [&](int k) { return regs[k]->mcmc->graph_exec; }, [](int, cudaStream_t) {}));
+  GINGR_TRY(replay_chain_graphs(ctx, sp, n, iters, [&](int k) { return regs[k]->mcmc->graph_exec.h; }, [](int, cudaStream_t) {}));
   for (int k = 0; k < n; ++k) ctx->launches += (int64_t)iters * regs[k]->mcmc->graph_launches;
   GINGR_CUDA_TRY(ctx, cudaGetLastError());
   return GINGR_OK;
@@ -876,7 +849,7 @@ int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t iters, ui
 int32_t gingr_mcmc_stats(gingr_registration* g, double* values, int32_t* counts) {
   GINGR_TRY(mcmc_check(g, "gingr_mcmc_stats: bad argument"));
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   if (values) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(values, mc->md.p, sizeof(double) * MD_COUNT, cudaMemcpyDeviceToHost, ctx->stream));
   if (counts) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(counts, mc->mi.p, sizeof(int) * MI_COUNT, cudaMemcpyDeviceToHost, ctx->stream));
@@ -888,7 +861,7 @@ int32_t gingr_mcmc_stats(gingr_registration* g, double* values, int32_t* counts)
 int32_t gingr_mcmc_best(gingr_registration* g, gingr_state* out, double* alpha_out, double* fit_out) {
   GINGR_TRY(mcmc_check(g, "gingr_mcmc_best: bad argument"));
   gingr_ctx* ctx = g->ctx;
-  McmcState* mc = g->mcmc;
+  McmcState* mc = g->mcmc.get();
   const gingr_model* m = g->model;
   if (!out) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_best: bad argument");
   if (!mc->primed) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_best: the chain has not started");

@@ -14,7 +14,6 @@ struct GramPlan {
   DevBuf<double> d_partial;  // [nsegs][128][128]
   // max_cta > 0 caps the CTAs of the schedule (many chains batched in one launch: a chain's Gram on few CTAs, batch.cuh)
   int32_t build(gingr_ctx* ctx, int rows, int r, int rp, int max_cta = 0);
-  void release();
 };
 // d_resid (optional, needs gram_rhs_fusable): per-row residuals c_k; row r of the last tile row then comes out as
 // sum_k c_k w_k Phi[k][.] = Phi^T W c -- the right-hand side of the regression without a pass of its own over Phi
@@ -45,7 +44,6 @@ struct CholWs {
   DevBuf<double> linv;
   int cap_n = 0, cap_nrows = 0;
   int32_t alloc(gingr_ctx* ctx, int n, int nrows);
-  void release();
 };
 // ws == nullptr (or GINGR_CHOL_DF=0): the kernel-per-step form of chol.cu; else one persistent data-flow kernel.
 int32_t cholesky_enqueue(gingr_ctx* ctx, int n, int nrows, double* d_A, int ld, int* d_info, CholWs* ws = nullptr);

@@ -695,7 +695,7 @@ struct gingr_registration {
   bool keep_raw = false;
   bool skip_fit_refresh = false;        // MH step: the proposal's fit is evaluated after the random override
   const int* sample_counter = nullptr;  // device counter keyed into the posterior-sample stream (null: the iteration)
-  struct McmcState* mcmc = nullptr;  // Metropolis-Hastings chain state (mcmc.cuh), created by gingr_mcmc_configure
+  std::unique_ptr<struct McmcState> mcmc;  // Metropolis-Hastings chain state (mcmc.cuh), created by gingr_mcmc_configure
   DevBuf<unsigned long long> prep_sync;   // [2] cpd_prepare_kernel: running maximum and block ticket (self-resetting)
   DevBuf<double> wrow, u, resid, inst_a, inst_b, newshape, fit_local, gathered, fit;
   DevBuf<double> vec;          // 8 * rp scratch vectors
@@ -707,7 +707,7 @@ struct gingr_registration {
   int retry_counter = RETRY_COUNTER_INIT;  // mirror of the device counter, refreshed by download_state
   // One iteration captured as a CUDA graph: the ~100-launch sequence of a small registration (C1-C3 sizes) is
   // launch-latency bound, the graph replays it with one driver call.  Key = (probabilistic, seed).
-  cudaGraphExec_t graph_exec = nullptr;
+  GraphExec graph_exec;
   int graph_prob = -1;
   uint64_t graph_seed = 0;
   int64_t graph_launches = 0;
@@ -722,13 +722,13 @@ struct gingr_registration {
   static constexpr int EV_PER_ITER = 14, EV_MAX_ITERS = 256;
   cudaEvent_t* ev(int k) { return profiling && prof_iters < EV_MAX_ITERS ? &events[(size_t)prof_iters * EV_PER_ITER + k] : nullptr; }
   void rec(int k) { if (cudaEvent_t* e = ev(k)) cudaEventRecord(*e, ctx->stream); }
+  ~gingr_registration();   // defined behind mcmc.cuh, where McmcState is complete
 };
 
 static int32_t model_build_constants(gingr_ctx* ctx, gingr_model* m);
 static int32_t model_upload_topology(gingr_ctx* ctx, gingr_model* m, const int32_t* tri, int T);
 static void drop_graph(gingr_registration* g);
 static uint64_t g_batch_epoch = 1;   // bumped whenever a chain's captured sequence goes stale (drop_graph, mcmc_release): so are batched plans
-static void mcmc_release(gingr_registration* g);     // mcmc.cuh
 static void mcmc_invalidate(gingr_registration* g);  // mcmc.cuh: the device state changed outside the MH chain
 static void mcmc_drop_chain_graph(gingr_registration* g);   // mcmc.cuh: the captured MH step of the chain is stale
 
@@ -777,7 +777,7 @@ int32_t gingr_model_upload(gingr_ctx* ctx, int32_t M, int32_t r, const double* r
   for (int k = 0; k < r; ++k)
     if (!(variance[k] >= 0.0)) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_model_upload: negative or NaN variance");
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  gingr_model* m = new gingr_model();
+  std::unique_ptr<gingr_model> m(new gingr_model());
   m->ctx = ctx;
   m->M = M;
   m->r = r;
@@ -808,35 +808,17 @@ int32_t gingr_model_upload(gingr_ctx* ctx, int32_t M, int32_t r, const double* r
       GINGR_TRY(slab_transpose_enqueue(ctx, (int)rows, nc, tmp.p, m->phi.p + a0, m->rp));
     }
     GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    tmp.release();
   }
-  {
-    const int32_t rt = model_upload_topology(ctx, m, tri, T);
-    if (rt != GINGR_OK) { gingr_model_destroy(m); return rt; }
-  }
+  GINGR_TRY(model_upload_topology(ctx, m.get(), tri, T));
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-  int32_t rc = model_build_constants(ctx, m);
-  if (rc != GINGR_OK) {
-    gingr_model_destroy(m);
-    return rc;
-  }
-  *out = m;
+  GINGR_TRY(model_build_constants(ctx, m.get()));
+  *out = m.release();
   return GINGR_OK;
 }
 
 int32_t gingr_model_destroy(gingr_model* m) {
   if (!m) return GINGR_OK;
   cudaSetDevice(m->ctx->device);
-  m->ref.release();
-  m->mean.release();
-  m->phi.release();
-  m->sqrt_lambda.release();
-  m->tri.release();
-  m->adj_off.release();
-  m->adj.release();
-  m->boundary.release();
-  m->S.release();
-  m->W0.release();
   delete m;
   return GINGR_OK;
 }
@@ -853,42 +835,40 @@ int32_t gingr_model_new_reference(gingr_ctx* ctx, const gingr_model* model, int3
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const int M = model->M, r = model->r, rp = model->rp;
-  gingr_model* m = new gingr_model();
+  std::unique_ptr<gingr_model> m(new gingr_model());
   m->ctx = ctx;
   m->M = M2; m->r = r; m->rp = rp; m->m0 = 0; m->Ml = M2;
-  DevBuf<double> old_soa, d2;
-  DevBuf<int32_t> idx;
-  ClosestWorkspace ws;
-  SpatialGrid pgrid;
-  int32_t rc = GINGR_OK;
-  auto A = [&](cudaError_t e) { if (e != cudaSuccess && rc == GINGR_OK) { gingr_set_error(ctx, cudaGetErrorString(e)); rc = GINGR_ERR_CUDA; } };
-  A(m->ref.alloc((size_t)3 * M2)); A(m->mean.alloc((size_t)3 * M2)); A(m->sqrt_lambda.alloc((size_t)rp));
-  A(m->phi.alloc((size_t)3 * M2 * rp));
-  A(old_soa.alloc((size_t)3 * M)); A(d2.alloc((size_t)M2)); A(idx.alloc((size_t)M2));
-  if (rc == GINGR_OK) rc = ws.ensure(ctx, M2, M, 0, 0);
-  if (rc == GINGR_OK) {
-    A(cudaMemcpyAsync(m->ref.p, new_ref, sizeof(double) * 3 * (size_t)M2, cudaMemcpyHostToDevice, st));
-    A(cudaMemcpyAsync(m->sqrt_lambda.p, model->sqrt_lambda.p, sizeof(double) * rp, cudaMemcpyDeviceToDevice, st));
-  }
-  if (rc == GINGR_OK) rc = aos_to_soa_enqueue(ctx, M, model->ref.p, old_soa.p);
-  if (rc == GINGR_OK && grid_wanted(M)) {
-    VertexArray va;
-    va.p = model->ref.p;
-    rc = pgrid.ensure(ctx, M, M, false);
-    if (rc == GINGR_OK) rc = grid_build_points_enqueue(ctx, pgrid, M, va);
-  }
-  if (rc == GINGR_OK) rc = nn_vertex_enqueue(ctx, ws, M2, m->ref.p, M, old_soa.p, d2.p, idx.p, pgrid.built ? &pgrid : nullptr);
-  if (rc == GINGR_OK) {
+  GINGR_CUDA_TRY(ctx, m->ref.alloc((size_t)3 * M2));
+  GINGR_CUDA_TRY(ctx, m->mean.alloc((size_t)3 * M2));
+  GINGR_CUDA_TRY(ctx, m->sqrt_lambda.alloc((size_t)rp));
+  GINGR_CUDA_TRY(ctx, m->phi.alloc((size_t)3 * M2 * rp));
+  {   // the search scratch is freed before the regression constants are built
+    DevBuf<double> old_soa, d2;
+    DevBuf<int32_t> idx;
+    ClosestWorkspace ws;
+    SpatialGrid pgrid;
+    GINGR_CUDA_TRY(ctx, old_soa.alloc((size_t)3 * M));
+    GINGR_CUDA_TRY(ctx, d2.alloc((size_t)M2));
+    GINGR_CUDA_TRY(ctx, idx.alloc((size_t)M2));
+    GINGR_TRY(ws.ensure(ctx, M2, M, 0, 0));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(m->ref.p, new_ref, sizeof(double) * 3 * (size_t)M2, cudaMemcpyHostToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(m->sqrt_lambda.p, model->sqrt_lambda.p, sizeof(double) * rp, cudaMemcpyDeviceToDevice, st));
+    GINGR_TRY(aos_to_soa_enqueue(ctx, M, model->ref.p, old_soa.p));
+    if (grid_wanted(M)) {
+      VertexArray va;
+      va.p = model->ref.p;
+      GINGR_TRY(pgrid.ensure(ctx, M, M, false));
+      GINGR_TRY(grid_build_points_enqueue(ctx, pgrid, M, va));
+    }
+    GINGR_TRY(nn_vertex_enqueue(ctx, ws, M2, m->ref.p, M, old_soa.p, d2.p, idx.p, pgrid.built ? &pgrid : nullptr));
     rereference_rows_kernel<<<3 * M2, 128, 0, st>>>(M2, rp, idx.p, model->phi.p, model->mean.p, m->phi.p, m->mean.p);
     GINGR_LAUNCHED(ctx);
-    A(cudaGetLastError());
-    A(cudaStreamSynchronize(st));
+    GINGR_CUDA_TRY(ctx, cudaGetLastError());
+    GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   }
-  old_soa.release(); d2.release(); idx.release(); ws.release(); pgrid.release();
-  if (rc == GINGR_OK) rc = model_upload_topology(ctx, m, tri, T);
-  if (rc == GINGR_OK) rc = model_build_constants(ctx, m);
-  if (rc != GINGR_OK) { gingr_model_destroy(m); return rc; }
-  *out = m;
+  GINGR_TRY(model_upload_topology(ctx, m.get(), tri, T));
+  GINGR_TRY(model_build_constants(ctx, m.get()));
+  *out = m.release();
   return GINGR_OK;
 }
 
@@ -928,12 +908,6 @@ static int32_t model_build_constants(gingr_ctx* ctx, gingr_model* m) {
   int h_info = 0;
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(&h_info, info.p, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
-  plan.release();
-  plan2.release();
-  B.release();
-  Rt.release();
-  info.release();
-  cws.release();
   if (h_info != 0) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_model_upload: basis/variance not finite (1e-5 I + S not SPD)");
   m->has_regression_constants = true;
   return GINGR_OK;
@@ -973,11 +947,6 @@ struct PosteriorScratch {
   DevBuf<double> Mx, wrow, u, vec, gt_part, inst, fit_local, gathered, fit, ds;
   DevBuf<int> is, flags;
   gingr::CholWs cholws;
-  void release() {
-    gram.release(); cholws.release();
-    Mx.release(); wrow.release(); u.release(); vec.release(); gt_part.release(); inst.release();
-    fit_local.release(); gathered.release(); fit.release(); ds.release(); is.release(); flags.release();
-  }
 };
 
 namespace gingr {
@@ -1073,83 +1042,79 @@ static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const do
   if (bad) return GINGR_MODEL_FLEXIBILITY;
   const int L = (int)lpid.size();
   PosteriorScratch s;
-  auto fail = [&](int32_t rc) { cudaStreamSynchronize(ctx->stream); s.release(); return rc; };
-  int32_t rc;
-  if ((rc = s.gram.build(ctx, 3 * M, r, rp)) < 0) return fail(rc);
+  GINGR_TRY(s.gram.build(ctx, 3 * M, r, rp));
   cudaStream_t st = ctx->stream;
   DevBuf<int32_t> d_lpid;
   DevBuf<double> d_lpts, d_lcinv, d_lA, d_lrows;
-#define PM_TRY(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) { gingr_set_error(ctx, cudaGetErrorString(_e)); s.release(); d_lpid.release(); d_lpts.release(); d_lcinv.release(); d_lA.release(); d_lrows.release(); return GINGR_ERR_CUDA; } } while (0)
   const int xrows = cov_pts ? 3 * M : 0;       // rows of Q carried through the factorisation for the covariance
-  PM_TRY(s.Mx.alloc((size_t)(r + 8 + xrows) * rp));
-  PM_TRY(s.wrow.alloc((size_t)3 * M));
-  PM_TRY(s.u.alloc((size_t)3 * M));
-  PM_TRY(s.vec.alloc((size_t)8 * rp));
-  PM_TRY(s.gt_part.alloc((size_t)gemvT_splits(ctx, 3 * M) * rp));
-  PM_TRY(s.inst.alloc((size_t)3 * M));
-  PM_TRY(s.fit_local.alloc((size_t)3 * M));
-  PM_TRY(s.ds.alloc(DS_COUNT));
-  PM_TRY(s.is.alloc(IS_COUNT));
-  PM_TRY(s.flags.alloc(256));
-  if ((rc = s.cholws.alloc(ctx, r, r + 1 + xrows)) < 0) return fail(rc);
-  PM_TRY(cudaMemsetAsync(s.Mx.p, 0, sizeof(double) * (size_t)(r + 8) * rp, st));
-  PM_TRY(cudaMemsetAsync(s.is.p, 0, sizeof(int) * IS_COUNT, st));
-  PM_TRY(cudaMemcpyAsync(s.wrow.p, wrow.data(), sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
-  PM_TRY(cudaMemcpyAsync(s.u.p, u.data(), sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, s.Mx.alloc((size_t)(r + 8 + xrows) * rp));
+  GINGR_CUDA_TRY(ctx, s.wrow.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, s.u.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, s.vec.alloc((size_t)8 * rp));
+  GINGR_CUDA_TRY(ctx, s.gt_part.alloc((size_t)gemvT_splits(ctx, 3 * M) * rp));
+  GINGR_CUDA_TRY(ctx, s.inst.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, s.fit_local.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, s.ds.alloc(DS_COUNT));
+  GINGR_CUDA_TRY(ctx, s.is.alloc(IS_COUNT));
+  GINGR_CUDA_TRY(ctx, s.flags.alloc(256));
+  GINGR_TRY(s.cholws.alloc(ctx, r, r + 1 + xrows));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(s.Mx.p, 0, sizeof(double) * (size_t)(r + 8) * rp, st));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(s.is.p, 0, sizeof(int) * IS_COUNT, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s.wrow.p, wrow.data(), sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s.u.p, u.data(), sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
   double hds[DS_COUNT];
   memset(hds, 0, sizeof(hds));
   hds[DS_SCALE] = 1.0;
   for (int d = 0; d < 3; ++d) hds[DS_T + d] = t[d];
   for (int d = 0; d < 9; ++d) hds[DS_R + d] = R[d];
-  PM_TRY(cudaMemcpyAsync(s.ds.p, hds, sizeof(hds), cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s.ds.p, hds, sizeof(hds), cudaMemcpyHostToDevice, st));
   double* rhs = s.Mx.p + (size_t)r * rp;
-  if ((rc = gemvT_enqueue(ctx, 3 * M, r, rp, m->phi.p, s.u.p, m->sqrt_lambda.p, s.gt_part.p, rhs)) < 0) return fail(rc);
+  GINGR_TRY(gemvT_enqueue(ctx, 3 * M, r, rp, m->phi.p, s.u.p, m->sqrt_lambda.p, s.gt_part.p, rhs));
   if (L > 0) {
-    PM_TRY(d_lpid.alloc(L)); PM_TRY(d_lpts.alloc(3 * L)); PM_TRY(d_lcinv.alloc(9 * L)); PM_TRY(d_lA.alloc(9 * L));
-    PM_TRY(d_lrows.alloc((size_t)L * 3 * rp));
-    PM_TRY(cudaMemcpyAsync(d_lpid.p, lpid.data(), sizeof(int32_t) * L, cudaMemcpyHostToDevice, st));
-    PM_TRY(cudaMemcpyAsync(d_lpts.p, lpts.data(), sizeof(double) * 3 * L, cudaMemcpyHostToDevice, st));
-    PM_TRY(cudaMemcpyAsync(d_lcinv.p, lcinv.data(), sizeof(double) * 9 * L, cudaMemcpyHostToDevice, st));
+    GINGR_CUDA_TRY(ctx, d_lpid.alloc(L));
+    GINGR_CUDA_TRY(ctx, d_lpts.alloc(3 * L));
+    GINGR_CUDA_TRY(ctx, d_lcinv.alloc(9 * L));
+    GINGR_CUDA_TRY(ctx, d_lA.alloc(9 * L));
+    GINGR_CUDA_TRY(ctx, d_lrows.alloc((size_t)L * 3 * rp));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(d_lpid.p, lpid.data(), sizeof(int32_t) * L, cudaMemcpyHostToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(d_lpts.p, lpts.data(), sizeof(double) * 3 * L, cudaMemcpyHostToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(d_lcinv.p, lcinv.data(), sizeof(double) * 9 * L, cudaMemcpyHostToDevice, st));
     GINGR_LAUNCH(ctx, gather_rows_kernel, dim3(ceil_div(3 * rp, 256), L), 256, 0, st, L, rp, 0, d_lpid.p, m->phi.p, d_lrows.p);
     GINGR_LAUNCH(ctx, landmark_prepare_kernel, ceil_div(L, 64), 64, 0, st, L, d_lcinv.p, s.ds.p, d_lA.p);
     GINGR_LAUNCH(ctx, landmark_rhs_kernel, ceil_div(r, 256), 256, 0, st, r, rp, L, d_lpid.p, d_lpts.p, d_lA.p, d_lrows.p, m->ref.p,
                                                           m->mean.p, m->sqrt_lambda.p, s.ds.p, rhs);
     ctx->launches += 3;
   }
-  if ((rc = gram_partials_enqueue(ctx, s.gram, m->phi.p, s.wrow.p)) < 0) return fail(rc);
-  if ((rc = gram_finish_enqueue(ctx, s.gram, s.gram.d_partial.p, m->sqrt_lambda.p, 1.0, L, d_lrows.p, d_lA.p, rp, s.Mx.p, false, true)) < 0) return fail(rc);
+  GINGR_TRY(gram_partials_enqueue(ctx, s.gram, m->phi.p, s.wrow.p));
+  GINGR_TRY(gram_finish_enqueue(ctx, s.gram, s.gram.d_partial.p, m->sqrt_lambda.p, 1.0, L, d_lrows.p, d_lA.p, rp, s.Mx.p, false, true));
   if (xrows > 0) {
     gingr::posterior_cov_rows_kernel<<<dim3(ceil_div(rp, 256), xrows), 256, 0, st>>>(xrows, r, rp, m->phi.p, m->sqrt_lambda.p,
                                                                                  s.Mx.p + (size_t)(r + 1) * rp);
     GINGR_LAUNCHED(ctx);
   }
-  if ((rc = cholesky_enqueue(ctx, r, r + 1 + xrows, s.Mx.p, rp, s.is.p + IS_INFO, &s.cholws)) < 0) return fail(rc);
+  GINGR_TRY(cholesky_enqueue(ctx, r, r + 1 + xrows, s.Mx.p, rp, s.is.p + IS_INFO, &s.cholws));
   double* c = s.vec.p;
-  if ((rc = chol_backsolve_enqueue(ctx, r, s.Mx.p, rp, rhs, c, s.flags.p, &s.cholws)) < 0) return fail(rc);
+  GINGR_TRY(chol_backsolve_enqueue(ctx, r, s.Mx.p, rp, rhs, c, s.flags.p, &s.cholws));
   GINGR_LAUNCH(ctx, check_finite_kernel, ceil_div(r, 256), 256, 0, st, r, c, s.is.p + IS_FAIL_POST);
   GINGR_LAUNCHED(ctx);
   if (mean_pts) {
-    if ((rc = instance_rows(ctx, m, s.vec.p + 2 * rp, 1, c, nullptr, s.inst.p, nullptr)) < 0) return fail(rc);
+    GINGR_TRY(instance_rows(ctx, m, s.vec.p + 2 * rp, 1, c, nullptr, s.inst.p, nullptr));
     GINGR_LAUNCH(ctx, fit_from_instance_kernel, ceil_div(M, 256), 256, 0, st, 0, M, m->ref.p, m->mean.p, s.inst.p, s.ds.p, DS_SCALE, DS_T,
                                                                DS_R, s.fit_local.p);
     GINGR_LAUNCHED(ctx);
-    PM_TRY(cudaMemcpyAsync(mean_pts, s.fit_local.p, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mean_pts, s.fit_local.p, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
   }
   DevBuf<double> d_cov;
   if (cov_pts) {
-    if (d_cov.alloc((size_t)9 * M) != cudaSuccess) return fail(gingr_fail(ctx, GINGR_ERR_CUDA, "out of device memory"));
+    GINGR_CUDA_TRY(ctx, d_cov.alloc((size_t)9 * M));
     gingr::posterior_cov_kernel<<<ceil_div(M, 8), 256, 0, st>>>(M, r, rp, s.Mx.p + (size_t)(r + 1) * rp, s.ds.p, d_cov.p);
     GINGR_LAUNCHED(ctx);
-    cudaMemcpyAsync(cov_pts, d_cov.p, sizeof(double) * 9 * M, cudaMemcpyDeviceToHost, st);
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(cov_pts, d_cov.p, sizeof(double) * 9 * M, cudaMemcpyDeviceToHost, st));
   }
   int his[IS_COUNT];
-  if (coeffs) PM_TRY(cudaMemcpyAsync(coeffs, c, sizeof(double) * r, cudaMemcpyDeviceToHost, st));
-  PM_TRY(cudaMemcpyAsync(his, s.is.p, sizeof(int) * IS_COUNT, cudaMemcpyDeviceToHost, st));
-  PM_TRY(cudaStreamSynchronize(st));
-#undef PM_TRY
-  s.release();
-  d_cov.release();
-  d_lpid.release(); d_lpts.release(); d_lcinv.release(); d_lA.release(); d_lrows.release();
+  if (coeffs) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(coeffs, c, sizeof(double) * r, cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(his, s.is.p, sizeof(int) * IS_COUNT, cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   return (his[IS_INFO] || his[IS_FAIL_POST]) ? GINGR_MODEL_FLEXIBILITY : GINGR_OK;
 }
 
@@ -1180,30 +1145,29 @@ int32_t gingr_coefficients(gingr_ctx* ctx, const gingr_model* model, const doubl
   DevBuf<double> mesh, u, part, vec, ds;
   DevBuf<int> flag;
   cudaStream_t st = ctx->stream;
-  auto rel = [&]() { mesh.release(); u.release(); part.release(); vec.release(); ds.release(); flag.release(); };
-#define CO_TRY(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) { gingr_set_error(ctx, cudaGetErrorString(_e)); rel(); return GINGR_ERR_CUDA; } } while (0)
-  CO_TRY(mesh.alloc((size_t)3 * M)); CO_TRY(u.alloc((size_t)3 * M)); CO_TRY(vec.alloc((size_t)4 * rp));
-  CO_TRY(part.alloc((size_t)gemvT_splits(ctx, 3 * M) * rp)); CO_TRY(ds.alloc(DS_COUNT)); CO_TRY(flag.alloc(4));
+  GINGR_CUDA_TRY(ctx, mesh.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, u.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, vec.alloc((size_t)4 * rp));
+  GINGR_CUDA_TRY(ctx, part.alloc((size_t)gemvT_splits(ctx, 3 * M) * rp));
+  GINGR_CUDA_TRY(ctx, ds.alloc(DS_COUNT));
+  GINGR_CUDA_TRY(ctx, flag.alloc(4));
   double hds[DS_COUNT];
   memset(hds, 0, sizeof(hds));
   for (int d = 0; d < 3; ++d) hds[DS_NEW_T + d] = t[d];
   for (int d = 0; d < 9; ++d) hds[DS_R1 + d] = R[d];
-  CO_TRY(cudaMemcpyAsync(ds.p, hds, sizeof(hds), cudaMemcpyHostToDevice, st));
-  CO_TRY(cudaMemcpyAsync(mesh.p, mesh_pts, sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
-  CO_TRY(cudaMemsetAsync(flag.p, 0, sizeof(int) * 4, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(ds.p, hds, sizeof(hds), cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mesh.p, mesh_pts, sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(flag.p, 0, sizeof(int) * 4, st));
   GINGR_LAUNCH(ctx, coeff_residual_kernel, ceil_div(M, 256), 256, 0, st, 0, M, mesh.p, m->ref.p, m->mean.p, ds.p, u.p);
   GINGR_LAUNCHED(ctx);
-  int32_t rc = gemvT_enqueue(ctx, 3 * M, r, rp, m->phi.p, u.p, m->sqrt_lambda.p, part.p, vec.p);
-  if (rc >= 0) rc = dense_matvec_enqueue(ctx, r, m->W0.p, rp, vec.p, vec.p + rp);
-  if (rc < 0) { cudaStreamSynchronize(st); rel(); return rc; }
+  GINGR_TRY(gemvT_enqueue(ctx, 3 * M, r, rp, m->phi.p, u.p, m->sqrt_lambda.p, part.p, vec.p));
+  GINGR_TRY(dense_matvec_enqueue(ctx, r, m->W0.p, rp, vec.p, vec.p + rp));
   GINGR_LAUNCH(ctx, check_finite_kernel, ceil_div(r, 256), 256, 0, st, r, vec.p + rp, flag.p);
   GINGR_LAUNCHED(ctx);
   int hflag = 0;
-  CO_TRY(cudaMemcpyAsync(coeffs, vec.p + rp, sizeof(double) * r, cudaMemcpyDeviceToHost, st));
-  CO_TRY(cudaMemcpyAsync(&hflag, flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-  CO_TRY(cudaStreamSynchronize(st));
-#undef CO_TRY
-  rel();
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(coeffs, vec.p + rp, sizeof(double) * r, cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(&hflag, flag.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   return hflag ? GINGR_MODEL_FLEXIBILITY : GINGR_OK;
 }
 
@@ -1216,48 +1180,52 @@ int32_t gingr_spd_solve(gingr_ctx* ctx, int32_t n, const double* A, int32_t nrhs
   DevBuf<double> in, work, x;
   DevBuf<int> info, flags;
   CholWs ws;
-  cudaEvent_t e0 = nullptr, e1 = nullptr;
+  struct TimingEvents {   // destroyed on every exit
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    ~TimingEvents() {
+      if (e0) cudaEventDestroy(e0);
+      if (e1) cudaEventDestroy(e1);
+    }
+  } ev;
   cudaStream_t st = ctx->stream;
-  auto rel = [&]() { in.release(); work.release(); x.release(); info.release(); flags.release(); ws.release();
-                     if (e0) cudaEventDestroy(e0); if (e1) cudaEventDestroy(e1); };
-#define SS_TRY(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) { gingr_set_error(ctx, cudaGetErrorString(_e)); cudaStreamSynchronize(st); rel(); return GINGR_ERR_CUDA; } } while (0)
-  SS_TRY(in.alloc((size_t)nrows * np)); SS_TRY(work.alloc((size_t)(nrows + 8) * np)); SS_TRY(x.alloc(np));
-  SS_TRY(info.alloc(4)); SS_TRY(flags.alloc((size_t)ceil_div(n, 64) + 8));
-  int32_t rc = ws.alloc(ctx, n, nrows);
-  if (rc < 0) { rel(); return rc; }
-  SS_TRY(cudaEventCreate(&e0)); SS_TRY(cudaEventCreate(&e1));
-  SS_TRY(cudaMemsetAsync(in.p, 0, sizeof(double) * (size_t)nrows * np, st));
-  SS_TRY(cudaMemcpy2DAsync(in.p, sizeof(double) * np, A, sizeof(double) * n, sizeof(double) * n, n, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, in.alloc((size_t)nrows * np));
+  GINGR_CUDA_TRY(ctx, work.alloc((size_t)(nrows + 8) * np));
+  GINGR_CUDA_TRY(ctx, x.alloc(np));
+  GINGR_CUDA_TRY(ctx, info.alloc(4));
+  GINGR_CUDA_TRY(ctx, flags.alloc((size_t)ceil_div(n, 64) + 8));
+  GINGR_TRY(ws.alloc(ctx, n, nrows));
+  GINGR_CUDA_TRY(ctx, cudaEventCreate(&ev.e0));
+  GINGR_CUDA_TRY(ctx, cudaEventCreate(&ev.e1));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(in.p, 0, sizeof(double) * (size_t)nrows * np, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(in.p, sizeof(double) * np, A, sizeof(double) * n, sizeof(double) * n, n, cudaMemcpyHostToDevice, st));
   if (nrhs > 0)
-    SS_TRY(cudaMemcpy2DAsync(in.p + (size_t)n * np, sizeof(double) * np, B, sizeof(double) * n, sizeof(double) * n, nrhs,
-                             cudaMemcpyHostToDevice, st));
-  SS_TRY(cudaMemsetAsync(info.p, 0, sizeof(int) * 4, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(in.p + (size_t)n * np, sizeof(double) * np, B, sizeof(double) * n, sizeof(double) * n, nrhs,
+                                          cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(info.p, 0, sizeof(int) * 4, st));
   float ms_total = 0.f;
   for (int it = 0; it < reps; ++it) {
-    SS_TRY(cudaMemcpyAsync(work.p, in.p, sizeof(double) * (size_t)nrows * np, cudaMemcpyDeviceToDevice, st));
-    SS_TRY(cudaEventRecord(e0, st));
-    rc = cholesky_enqueue(ctx, n, nrows, work.p, np, info.p, &ws);
-    if (rc >= 0 && nrhs > 0) rc = chol_backsolve_enqueue(ctx, n, work.p, np, work.p + (size_t)n * np, x.p, flags.p, &ws);
-    if (rc < 0) { cudaStreamSynchronize(st); rel(); return rc; }
-    SS_TRY(cudaEventRecord(e1, st));
-    SS_TRY(cudaEventSynchronize(e1));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(work.p, in.p, sizeof(double) * (size_t)nrows * np, cudaMemcpyDeviceToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaEventRecord(ev.e0, st));
+    GINGR_TRY(cholesky_enqueue(ctx, n, nrows, work.p, np, info.p, &ws));
+    if (nrhs > 0) GINGR_TRY(chol_backsolve_enqueue(ctx, n, work.p, np, work.p + (size_t)n * np, x.p, flags.p, &ws));
+    GINGR_CUDA_TRY(ctx, cudaEventRecord(ev.e1, st));
+    GINGR_CUDA_TRY(ctx, cudaEventSynchronize(ev.e1));
     float ms = 0.f;
-    SS_TRY(cudaEventElapsedTime(&ms, e0, e1));
+    GINGR_CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ev.e0, ev.e1));
     ms_total += ms;
   }
   if (ms_out) *ms_out = (double)ms_total / reps;
   int h_info = 0;
-  SS_TRY(cudaMemcpyAsync(&h_info, info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(&h_info, info.p, sizeof(int), cudaMemcpyDeviceToHost, st));
   if (L_out) {
-    SS_TRY(cudaMemcpy2DAsync(L_out, sizeof(double) * n, work.p, sizeof(double) * np, sizeof(double) * n, n, cudaMemcpyDeviceToHost, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(L_out, sizeof(double) * n, work.p, sizeof(double) * np, sizeof(double) * n, n,
+                                          cudaMemcpyDeviceToHost, st));
   }
   if (Y_out && nrhs > 0)
-    SS_TRY(cudaMemcpy2DAsync(Y_out, sizeof(double) * n, work.p + (size_t)n * np, sizeof(double) * np, sizeof(double) * n, nrhs,
-                             cudaMemcpyDeviceToHost, st));
-  if (x_out) SS_TRY(cudaMemcpyAsync(x_out, x.p, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
-  SS_TRY(cudaStreamSynchronize(st));
-#undef SS_TRY
-  rel();
+    GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(Y_out, sizeof(double) * n, work.p + (size_t)n * np, sizeof(double) * np, sizeof(double) * n, nrhs,
+                                          cudaMemcpyDeviceToHost, st));
+  if (x_out) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(x_out, x.p, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   if (L_out)
     for (int i = 0; i < n; ++i)
       for (int k = i + 1; k < n; ++k) L_out[(size_t)i * n + k] = 0.0;
@@ -1277,27 +1245,25 @@ int32_t gingr_model_instance(gingr_ctx* ctx, const gingr_model* model, const gin
   DevBuf<double> vec, inst, out, ds;
   DevBuf<int> is;
   cudaStream_t st = ctx->stream;
-  auto rel = [&]() { vec.release(); inst.release(); out.release(); ds.release(); is.release(); };
-#define MI_TRY(x) do { cudaError_t _e = (x); if (_e != cudaSuccess) { gingr_set_error(ctx, cudaGetErrorString(_e)); rel(); return GINGR_ERR_CUDA; } } while (0)
-  MI_TRY(vec.alloc((size_t)4 * rp)); MI_TRY(inst.alloc((size_t)3 * M)); MI_TRY(out.alloc((size_t)3 * M));
-  MI_TRY(ds.alloc(DS_COUNT)); MI_TRY(is.alloc(IS_COUNT));
+  GINGR_CUDA_TRY(ctx, vec.alloc((size_t)4 * rp));
+  GINGR_CUDA_TRY(ctx, inst.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, out.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, ds.alloc(DS_COUNT));
+  GINGR_CUDA_TRY(ctx, is.alloc(IS_COUNT));
   double hds[DS_COUNT];
   memset(hds, 0, sizeof(hds));
   hds[DS_SCALE] = stt->scale;
   for (int d = 0; d < 3; ++d) { hds[DS_T + d] = stt->translation[d]; hds[DS_EULER + d] = stt->euler[d]; }
-  MI_TRY(cudaMemcpyAsync(ds.p, hds, sizeof(hds), cudaMemcpyHostToDevice, st));
-  MI_TRY(cudaMemcpyAsync(vec.p, alpha, sizeof(double) * r, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(ds.p, hds, sizeof(hds), cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(vec.p, alpha, sizeof(double) * r, cudaMemcpyHostToDevice, st));
   GINGR_LAUNCH(ctx, pose_kernel, 1, 1, 0, st, ds.p, is.p);
   GINGR_LAUNCHED(ctx);
-  int32_t rc = instance_rows(ctx, m, vec.p + rp, 1, vec.p, nullptr, inst.p, nullptr);
-  if (rc < 0) { cudaStreamSynchronize(st); rel(); return rc; }
+  GINGR_TRY(instance_rows(ctx, m, vec.p + rp, 1, vec.p, nullptr, inst.p, nullptr));
   GINGR_LAUNCH(ctx, fit_from_instance_kernel, ceil_div(M, 256), 256, 0, st, 0, M, m->ref.p, m->mean.p, inst.p, ds.p, DS_SCALE, DS_T, DS_R,
                                                              out.p);
   GINGR_LAUNCHED(ctx);
-  MI_TRY(cudaMemcpyAsync(fit, out.p, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
-  MI_TRY(cudaStreamSynchronize(st));
-#undef MI_TRY
-  rel();
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(fit, out.p, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   return GINGR_OK;
 }
 
@@ -1316,78 +1282,76 @@ int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, cons
       return gingr_fail(ctx, GINGR_ERR_ARG, "the mesh flavours of the ICP correspondence need model and target triangles");
   }
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  gingr_registration* g = new gingr_registration();
+  std::unique_ptr<gingr_registration> g(new gingr_registration());
   g->ctx = ctx;
   g->model = model;
   g->target = target;
   g->cfg = *cfg;
   const int M = model->M, r = model->r, rp = model->rp, Ml = model->Ml;
   const int Mmax = ceil_div(M, ctx->nranks);
-  int32_t rc = GINGR_OK;
-  auto A = [&](cudaError_t e) { if (e != cudaSuccess && rc == GINGR_OK) { gingr_set_error(ctx, cudaGetErrorString(e)); rc = GINGR_ERR_CUDA; } };
-  if (cfg->algorithm == GINGR_ALGO_CPD) { int32_t q = g->estep.ensure(ctx, M, std::max(target->N, 1)); if (q < 0) rc = q; }
-  else {
+  if (cfg->algorithm == GINGR_ALGO_CPD) {
+    GINGR_TRY(g->estep.ensure(ctx, M, std::max(target->N, 1)));
+  } else {
     const bool rev = cfg->reverse_correspondence_direction != 0;
-    int32_t q = rev ? g->closest.ensure(ctx, target->N_total, M, model->T, target->T)
-                    : g->closest.ensure(ctx, M, target->N_total, target->T, model->T);
-    if (q < 0) rc = q;
-    A(g->fit_normals.alloc((size_t)3 * M));
+    GINGR_TRY(rev ? g->closest.ensure(ctx, target->N_total, M, model->T, target->T)
+                  : g->closest.ensure(ctx, M, target->N_total, target->T, model->T));
+    GINGR_CUDA_TRY(ctx, g->fit_normals.alloc((size_t)3 * M));
     const bool mesh_flavour = cfg->correspondence_method != GINGR_POINTCLOUD_CLOSEST_POINT;
-    if (rc == GINGR_OK && grid_wanted(M)) {
+    if (grid_wanted(M)) {
       // the fit is scanned by the self-intersection test of the mesh flavours (both directions) and, in the
       // reversed direction, by the vertex / surface searches themselves
       if (mesh_flavour && model->T > 0) {
-        q = g->fit_tgrid.ensure(ctx, M, model->T, true);
-        if (q < 0) rc = q;
+        GINGR_TRY(g->fit_tgrid.ensure(ctx, M, model->T, true));
         g->use_fit_tgrid = true;
       }
-      if (rev && rc == GINGR_OK) {
-        q = g->fit_pgrid.ensure(ctx, M, M, false);
-        if (q < 0) rc = q;
+      if (rev) {
+        GINGR_TRY(g->fit_pgrid.ensure(ctx, M, M, false));
         g->use_fit_pgrid = true;
       }
     }
     if (rev) {
-      A(g->fit_soa.alloc((size_t)3 * M));
-      A(g->rev_tid.alloc((size_t)target->N_total));
-      A(g->rev_cp.alloc((size_t)3 * M));
-      A(g->rev_wcnt.alloc((size_t)M));
-      A(g->rev_scratch.alloc((size_t)3 * M + target->N_total + 1));
+      GINGR_CUDA_TRY(ctx, g->fit_soa.alloc((size_t)3 * M));
+      GINGR_CUDA_TRY(ctx, g->rev_tid.alloc((size_t)target->N_total));
+      GINGR_CUDA_TRY(ctx, g->rev_cp.alloc((size_t)3 * M));
+      GINGR_CUDA_TRY(ctx, g->rev_wcnt.alloc((size_t)M));
+      GINGR_CUDA_TRY(ctx, g->rev_scratch.alloc((size_t)3 * M + target->N_total + 1));
     }
   }
-  if (rc == GINGR_OK) { int32_t q = g->gram.build(ctx, 3 * Ml, r, rp); if (q < 0) rc = q; }
-  A(g->rows_ext.alloc((size_t)4 * M + 8));
-  A(g->Mx.alloc((size_t)(r + 8) * rp));
-  if (ctx->nranks > 1) A(g->Mx_packed.alloc(gram_packed_doubles(g->gram) + rp));
-  A(g->prep_sync.alloc(2)); A(cudaMemsetAsync(g->prep_sync.p, 0, 2 * sizeof(unsigned long long), ctx->stream));
-  A(g->wrow.alloc((size_t)3 * Mmax)); A(g->u.alloc((size_t)3 * Mmax)); A(g->resid.alloc((size_t)3 * Mmax));
-  A(g->inst_a.alloc((size_t)3 * Mmax)); A(g->inst_b.alloc((size_t)3 * Mmax));
-  A(g->newshape.alloc((size_t)3 * Mmax)); A(g->fit_local.alloc((size_t)3 * Mmax));
-  A(g->gathered.alloc((size_t)3 * Mmax * ctx->nranks)); A(g->fit.alloc((size_t)3 * M));
-  A(g->vec.alloc((size_t)8 * rp));
-  A(g->gt_part.alloc((size_t)gemvT_splits(ctx, 3 * Ml) * rp));
-  A(g->sums_part.alloc((size_t)3 * ceil_div(M, 256)));
-  A(g->pro_part.alloc((size_t)16 * ceil_div(std::max(Ml, 1), 256)));
-  A(g->pro_sums.alloc(32));
-  A(g->ds.alloc(DS_COUNT)); A(g->is.alloc(IS_COUNT)); A(g->flags.alloc(256));
-  if (rc == GINGR_OK) { int32_t q = g->cholws.alloc(ctx, r, r + 1); if (q < 0) rc = q; }
-  A(g->alpha.alloc((size_t)rp));
-  if (rc == GINGR_OK) {
-    A(cudaMemsetAsync(g->Mx.p, 0, sizeof(double) * (size_t)(r + 8) * rp, ctx->stream));
-    if (g->Mx_packed.p) A(cudaMemsetAsync(g->Mx_packed.p, 0, sizeof(double) * g->Mx_packed.n, ctx->stream));   // unused slots stay 0
-    A(cudaMemsetAsync(g->fit_local.p, 0, sizeof(double) * 3 * Mmax, ctx->stream));
-    A(cudaMemsetAsync(g->ds.p, 0, sizeof(double) * DS_COUNT, ctx->stream));
-    A(cudaMemsetAsync(g->is.p, 0, sizeof(int) * IS_COUNT, ctx->stream));
-    A(cudaMemcpyAsync(g->is.p + IS_RETRY, &g->retry_counter, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
-    A(cudaMemsetAsync(g->alpha.p, 0, sizeof(double) * rp, ctx->stream));
-    A(cudaMemsetAsync(g->rows_ext.p, 0, sizeof(double) * ((size_t)4 * M + 8), ctx->stream));
-    A(cudaStreamSynchronize(ctx->stream));
-  }
-  if (rc != GINGR_OK) {
-    gingr_registration_destroy(g);
-    return rc;
-  }
-  *out = g;
+  GINGR_TRY(g->gram.build(ctx, 3 * Ml, r, rp));
+  GINGR_CUDA_TRY(ctx, g->rows_ext.alloc((size_t)4 * M + 8));
+  GINGR_CUDA_TRY(ctx, g->Mx.alloc((size_t)(r + 8) * rp));
+  if (ctx->nranks > 1) GINGR_CUDA_TRY(ctx, g->Mx_packed.alloc(gram_packed_doubles(g->gram) + rp));
+  GINGR_CUDA_TRY(ctx, g->prep_sync.alloc(2));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->prep_sync.p, 0, 2 * sizeof(unsigned long long), ctx->stream));
+  GINGR_CUDA_TRY(ctx, g->wrow.alloc((size_t)3 * Mmax));
+  GINGR_CUDA_TRY(ctx, g->u.alloc((size_t)3 * Mmax));
+  GINGR_CUDA_TRY(ctx, g->resid.alloc((size_t)3 * Mmax));
+  GINGR_CUDA_TRY(ctx, g->inst_a.alloc((size_t)3 * Mmax));
+  GINGR_CUDA_TRY(ctx, g->inst_b.alloc((size_t)3 * Mmax));
+  GINGR_CUDA_TRY(ctx, g->newshape.alloc((size_t)3 * Mmax));
+  GINGR_CUDA_TRY(ctx, g->fit_local.alloc((size_t)3 * Mmax));
+  GINGR_CUDA_TRY(ctx, g->gathered.alloc((size_t)3 * Mmax * ctx->nranks));
+  GINGR_CUDA_TRY(ctx, g->fit.alloc((size_t)3 * M));
+  GINGR_CUDA_TRY(ctx, g->vec.alloc((size_t)8 * rp));
+  GINGR_CUDA_TRY(ctx, g->gt_part.alloc((size_t)gemvT_splits(ctx, 3 * Ml) * rp));
+  GINGR_CUDA_TRY(ctx, g->sums_part.alloc((size_t)3 * ceil_div(M, 256)));
+  GINGR_CUDA_TRY(ctx, g->pro_part.alloc((size_t)16 * ceil_div(std::max(Ml, 1), 256)));
+  GINGR_CUDA_TRY(ctx, g->pro_sums.alloc(32));
+  GINGR_CUDA_TRY(ctx, g->ds.alloc(DS_COUNT));
+  GINGR_CUDA_TRY(ctx, g->is.alloc(IS_COUNT));
+  GINGR_CUDA_TRY(ctx, g->flags.alloc(256));
+  GINGR_TRY(g->cholws.alloc(ctx, r, r + 1));
+  GINGR_CUDA_TRY(ctx, g->alpha.alloc((size_t)rp));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->Mx.p, 0, sizeof(double) * (size_t)(r + 8) * rp, ctx->stream));
+  if (g->Mx_packed.p) GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->Mx_packed.p, 0, sizeof(double) * g->Mx_packed.n, ctx->stream));   // unused slots stay 0
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->fit_local.p, 0, sizeof(double) * 3 * Mmax, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->ds.p, 0, sizeof(double) * DS_COUNT, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->is.p, 0, sizeof(int) * IS_COUNT, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(g->is.p + IS_RETRY, &g->retry_counter, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->alpha.p, 0, sizeof(double) * rp, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->rows_ext.p, 0, sizeof(double) * ((size_t)4 * M + 8), ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  *out = g.release();
   return GINGR_OK;
 }
 
@@ -1395,19 +1359,7 @@ int32_t gingr_registration_destroy(gingr_registration* g) {
   if (!g) return GINGR_OK;
   cudaSetDevice(g->ctx->device);
   cudaStreamSynchronize(g->ctx->stream);
-  drop_graph(g);
-  mcmc_release(g);
-  g->Mx_raw.release();
-  g->Mx_packed.release();
-  g->lm_pid.release(); g->lml_pid.release(); g->lml_pts.release(); g->lml_cinv.release(); g->lml_A.release();
-  g->lml_rows.release();
-  g->estep.release(); g->closest.release(); g->gram.release();
-  g->fit_pgrid.release(); g->fit_tgrid.release();
-  g->fit_normals.release(); g->fit_soa.release(); g->rev_tid.release(); g->rev_cp.release(); g->rev_wcnt.release(); g->rev_scratch.release();
-  g->prep_sync.release(); g->rows_ext.release(); g->Mx.release(); g->wrow.release(); g->u.release(); g->resid.release(); g->inst_a.release(); g->inst_b.release();
-  g->newshape.release(); g->fit_local.release(); g->gathered.release(); g->fit.release(); g->vec.release();
-  g->gt_part.release(); g->sums_part.release(); g->pro_part.release(); g->pro_sums.release();
-  g->ds.release(); g->is.release(); g->flags.release(); g->alpha.release(); g->cholws.release();
+  ++g_batch_epoch;   // a later registration can get this address: batched plans that name this one are stale
   for (auto& e : g->events) cudaEventDestroy(e);
   delete g;
   return GINGR_OK;
@@ -1562,7 +1514,7 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
     }
     tv.n = tg->N_total; tv.aos = tg->aos.p; tv.soa = tg->verts.p; tv.T = tg->T; tv.tri = tg->tri.p;
     tv.normals = tg->normals.p; tv.boundary = tg->boundary.p;
-    tv.pgrid = tg->pgrid; tv.tgrid = tg->tgrid;
+    tv.pgrid = tg->pgrid.get(); tv.tgrid = tg->tgrid.get();
     VertexArray fva;
     fva.p = g->fit.p;
     if (g->use_fit_tgrid) {
@@ -1588,7 +1540,7 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
       fv.soa = g->fit_soa.p;
       GINGR_TRY(icp_correspondence_enqueue(ctx, g->closest, tv, fv, cfg.correspondence_method));
       GINGR_TRY(nn_vertex_enqueue(ctx, g->closest, tg->N_total, g->closest.cp.p, M, g->fit_soa.p, g->closest.d2.p,
-                                  g->rev_tid.p, fv.pgrid, g->closest.qorder));
+                                  g->rev_tid.p, fv.pgrid, g->closest.qorder.get()));
       GINGR_TRY(reverse_fold_enqueue(ctx, M, tg->N_total, g->rev_tid.p, g->closest.w.p, tg->aos.p, g->rev_cp.p,
                                      g->rev_wcnt.p, g->rev_scratch.p));
       icp_cp = g->rev_cp.p;
@@ -1729,36 +1681,49 @@ static bool graphs_enabled(const gingr_ctx* ctx) {
 
 static void drop_graph(gingr_registration* g) {
   ++g_batch_epoch;
-  if (g->graph_exec) cudaGraphExecDestroy(g->graph_exec);
-  g->graph_exec = nullptr;
+  g->graph_exec.reset();
   g->graph_prob = -1;
+}
+
+// Captures into `exec` what enqueue() puts on the ctx stream.  *launches receives the launches enqueue() counted; nothing
+// ran yet, so they are taken off ctx->launches again, and every replay adds them.
+template <typename F>
+static int32_t capture_graph(gingr_ctx* ctx, GraphExec& exec, int64_t* launches, F&& enqueue) {
+  exec.reset();
+  const int64_t l0 = ctx->launches;
+  GINGR_CUDA_TRY(ctx, cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
+  const int32_t rc = enqueue();
+  cudaGraph_t graph = nullptr;
+  const cudaError_t e = cudaStreamEndCapture(ctx->stream, &graph);
+  *launches = ctx->launches - l0;
+  ctx->launches = l0;
+  if (rc < 0) {
+    if (graph) cudaGraphDestroy(graph);
+    return rc;
+  }
+  GINGR_CUDA_TRY(ctx, e);
+  const cudaError_t e2 = cudaGraphInstantiate(&exec.h, graph, 0);
+  cudaGraphDestroy(graph);
+  GINGR_CUDA_TRY(ctx, e2);
+  return GINGR_OK;
+}
+
+// The captured iteration of g for (probabilistic, seed); captured again when the key changed.
+static int32_t iteration_graph(gingr_registration* g, int probabilistic, uint64_t seed) {
+  if (g->graph_exec.h && g->graph_prob == probabilistic && (!probabilistic || g->graph_seed == seed)) return GINGR_OK;
+  drop_graph(g);
+  GINGR_TRY(capture_graph(g->ctx, g->graph_exec, &g->graph_launches, [&] { return enqueue_iteration(g, probabilistic, seed); }));
+  g->graph_prob = probabilistic;
+  g->graph_seed = seed;
+  return GINGR_OK;
 }
 
 // One iteration, through the captured graph when possible (not while profiling: the events live outside graphs).
 static int32_t run_iteration(gingr_registration* g, int probabilistic, uint64_t seed) {
   gingr_ctx* ctx = g->ctx;
   if (g->profiling || !graphs_enabled(ctx)) return enqueue_iteration(g, probabilistic, seed);
-  if (!g->graph_exec || g->graph_prob != probabilistic || (probabilistic && g->graph_seed != seed)) {
-    drop_graph(g);
-    const int64_t l0 = ctx->launches;
-    GINGR_CUDA_TRY(ctx, cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-    const int32_t rc = enqueue_iteration(g, probabilistic, seed);
-    cudaGraph_t graph = nullptr;
-    const cudaError_t e = cudaStreamEndCapture(ctx->stream, &graph);
-    g->graph_launches = ctx->launches - l0;
-    ctx->launches = l0;  // nothing ran yet
-    if (rc < 0) {
-      if (graph) cudaGraphDestroy(graph);
-      return rc;
-    }
-    GINGR_CUDA_TRY(ctx, e);
-    const cudaError_t e2 = cudaGraphInstantiate(&g->graph_exec, graph, 0);
-    cudaGraphDestroy(graph);
-    GINGR_CUDA_TRY(ctx, e2);
-    g->graph_prob = probabilistic;
-    g->graph_seed = seed;
-  }
-  GINGR_CUDA_TRY(ctx, cudaGraphLaunch(g->graph_exec, ctx->stream));
+  GINGR_TRY(iteration_graph(g, probabilistic, seed));
+  GINGR_CUDA_TRY(ctx, cudaGraphLaunch(g->graph_exec.h, ctx->stream));
   ctx->launches += g->graph_launches;
   return GINGR_OK;
 }
@@ -1844,7 +1809,9 @@ static int32_t replay_chain_graphs(gingr_ctx* ctx, ChainStreamPool* sp, int n, i
 // Every chain's step is recorded (arguments only, nothing is launched), the sequences are checked to be the same launch
 // for launch, the argument tuples go to the device as [launch][chain] arrays and the batched forms of the kernels are
 // captured as one graph: blockIdx.z = chain.  A plan is kept until the set of chains, the seed, the kind of step or a
-// chain's configuration changes.  Users: gingr_mcmc_batch (mcmc.cuh) and gingr_update_batch.
+// chain's configuration changes.  Users: gingr_mcmc_batch (mcmc.cuh) and gingr_update_batch.  Each keeps one plan per host
+// thread on the heap and never deletes it: a plan is never freed at thread or process exit, where the CUDA runtime may
+// already be shut down.
 struct BatchPlan {
   std::vector<gingr_registration*> regs;
   std::vector<double> step_lengths;
@@ -1853,10 +1820,9 @@ struct BatchPlan {
   bool unsupported = false;     // a launch / copy on the path is not batch-aware, or the chains differ: per-chain graphs
   int nlaunch = 0;
   DevBuf<unsigned char> d_args;
-  cudaGraphExec_t exec = nullptr;
+  GraphExec exec;
   void drop() {
-    if (exec) cudaGraphExecDestroy(exec);
-    exec = nullptr;
+    exec.reset();
     regs.clear();
     step_lengths.clear();
     unsupported = false;
@@ -1970,7 +1936,7 @@ static int32_t batch_plan_build(gingr_ctx* ctx, gingr_registration** regs, int n
     GINGR_CUDA_TRY(ctx, el);
     GINGR_CUDA_TRY(ctx, e2);
   }
-  const cudaError_t e3 = cudaGraphInstantiate(&bp.exec, graph, 0);
+  const cudaError_t e3 = cudaGraphInstantiate(&bp.exec.h, graph, 0);
   cudaGraphDestroy(graph);
   GINGR_CUDA_TRY(ctx, e3);
   bp.nlaunch = (int)r0.size();
@@ -1994,14 +1960,10 @@ int32_t gingr_initialize_state(gingr_registration* g, gingr_state* s, const doub
     GINGR_CUDA_TRY(ctx, mp.alloc((size_t)3 * m->M));
     GINGR_CUDA_TRY(ctx, outv.alloc(4));
     add_vectors_enqueue(ctx, 3 * m->M, m->ref.p, m->mean.p, mp.p);
-    int32_t rc = initial_sigma2_enqueue(ctx, m->M, mp.p, g->target->N_total, g->target->verts.p, outv.p);
+    GINGR_TRY(initial_sigma2_enqueue(ctx, m->M, mp.p, g->target->N_total, g->target->verts.p, outv.p));
     double v = 0.0;
-    cudaError_t e = cudaMemcpyAsync(&v, outv.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-    mp.release();
-    outv.release();
-    if (rc < 0) return rc;
-    GINGR_CUDA_TRY(ctx, e);
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(&v, outv.p, sizeof(double), cudaMemcpyDeviceToHost, ctx->stream));
+    GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
     s->sigma2 = v;
   }
   GINGR_TRY(upload_state(g, s, alpha));
@@ -2094,7 +2056,7 @@ int32_t gingr_update_batch(gingr_registration** regs, int32_t n, int32_t iters, 
   // (the ICP flavours on the scans; the CPD E-step is not: per-chain graphs), GINGR_UPDATE_BATCHED=0: always per-chain graphs
   static const int batched = [] { const char* e = getenv("GINGR_UPDATE_BATCHED"); return e ? atoi(e) : 1; }();
   if (batched && n >= 2 && n <= 65535 && graphs_enabled(ctx)) {
-    static thread_local BatchPlan bp;
+    static thread_local BatchPlan& bp = *new BatchPlan();   // never deleted (BatchPlan)
     const int kind = probabilistic ? 3 : 1;
     if (!batch_plan_current(bp, ctx, regs, n, seed, kind)) {
       int32_t rc = batch_cap_gram(ctx, regs, n);
@@ -2108,7 +2070,7 @@ int32_t gingr_update_batch(gingr_registration** regs, int32_t n, int32_t iters, 
       if (rc < 0) { bp.drop(); return rc; }
     }
     if (!bp.unsupported) {
-      for (int it = 0; it < iters; ++it) GINGR_CUDA_TRY(ctx, cudaGraphLaunch(bp.exec, ctx->stream));
+      for (int it = 0; it < iters; ++it) GINGR_CUDA_TRY(ctx, cudaGraphLaunch(bp.exec.h, ctx->stream));
       ctx->launches += (int64_t)iters * bp.nlaunch;
       return GINGR_OK;
     }
@@ -2116,28 +2078,8 @@ int32_t gingr_update_batch(gingr_registration** regs, int32_t n, int32_t iters, 
   ChainStreamPool* sp = nullptr;
   GINGR_TRY(chain_stream_pool(ctx, &sp));
   // capture (or re-key) every chain's graph on the ctx stream first: capture is not concurrent
-  for (int k = 0; k < n; ++k) {
-    gingr_registration* g = regs[k];
-    const uint64_t sk = seed + (uint64_t)k;
-    if (!g->graph_exec || g->graph_prob != (probabilistic != 0) || (probabilistic && g->graph_seed != sk)) {
-      drop_graph(g);
-      const int64_t l0 = ctx->launches;
-      GINGR_CUDA_TRY(ctx, cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal));
-      const int32_t rc = enqueue_iteration(g, probabilistic != 0, sk);
-      cudaGraph_t graph = nullptr;
-      const cudaError_t e = cudaStreamEndCapture(ctx->stream, &graph);
-      g->graph_launches = ctx->launches - l0;
-      ctx->launches = l0;
-      if (rc < 0) { if (graph) cudaGraphDestroy(graph); return rc; }
-      GINGR_CUDA_TRY(ctx, e);
-      const cudaError_t e2 = cudaGraphInstantiate(&g->graph_exec, graph, 0);
-      cudaGraphDestroy(graph);
-      GINGR_CUDA_TRY(ctx, e2);
-      g->graph_prob = probabilistic != 0;
-      g->graph_seed = sk;
-    }
-  }
-  GINGR_TRY(replay_chain_graphs(ctx, sp, n, iters, [&](int k) { return regs[k]->graph_exec; },
+  for (int k = 0; k < n; ++k) GINGR_TRY(iteration_graph(regs[k], probabilistic != 0, seed + (uint64_t)k));
+  GINGR_TRY(replay_chain_graphs(ctx, sp, n, iters, [&](int k) { return regs[k]->graph_exec.h; },
                                 [&](int k, cudaStream_t st) { GINGR_LAUNCH(ctx, bump_iteration_kernel, 1, 1, 0, st, regs[k]->is.p); }));
   for (int k = 0; k < n; ++k) ctx->launches += (int64_t)iters * (regs[k]->graph_launches + 1);
   GINGR_CUDA_TRY(ctx, cudaGetLastError());
@@ -2195,3 +2137,5 @@ int32_t gingr_state_download(gingr_registration* g, gingr_state* state_out, doub
 
 #include "mcmc.cuh"
 #include "gpmm.cuh"
+
+gingr_registration::~gingr_registration() = default;
