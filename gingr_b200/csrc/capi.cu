@@ -131,9 +131,20 @@ int32_t gingr_target_upload(gingr_ctx* ctx, int32_t N, const double* pts, const 
   GINGR_TRY(gingr::aos_to_soa_enqueue(ctx, N, s->a.p, t->verts.p));
   GINGR_CUDA_TRY(ctx, t->aos.alloc((size_t)3 * N));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(t->aos.p, s->a.p, sizeof(double) * 3 * (size_t)N, cudaMemcpyDeviceToDevice, ctx->stream));
+  std::vector<int32_t> perm;
+  std::vector<double> shard;
   if (t->N > 0) {
+    const double* p0 = pts + (size_t)3 * t->n0;
+    gingr::estep_target_order(p0, t->N, perm);
+    shard.resize((size_t)3 * t->N);
+    for (int j = 0; j < t->N; ++j)
+      for (int d = 0; d < 3; ++d) shard[(size_t)3 * j + d] = p0[(size_t)3 * perm[j] + d];
+    GINGR_CUDA_TRY(ctx, s->b.alloc((size_t)3 * t->N));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s->b.p, shard.data(), sizeof(double) * shard.size(), cudaMemcpyHostToDevice, ctx->stream));
     GINGR_CUDA_TRY(ctx, t->soa.alloc((size_t)3 * t->N));
-    GINGR_TRY(gingr::aos_to_soa_enqueue(ctx, t->N, s->a.p + (size_t)3 * t->n0, t->soa.p));
+    GINGR_TRY(gingr::aos_to_soa_enqueue(ctx, t->N, s->b.p, t->soa.p));
+    GINGR_CUDA_TRY(ctx, t->soa_perm.alloc((size_t)t->N));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(t->soa_perm.p, perm.data(), sizeof(int32_t) * perm.size(), cudaMemcpyHostToDevice, ctx->stream));
   }
   t->T = T;
   if (T > 0) {
@@ -188,14 +199,23 @@ static void fill_nan(double* p, size_t n) {
     for (size_t k = 0; k < n; ++k) p[k] = NAN;
 }
 
-static int32_t estep_common(gingr_ctx* ctx, const gingr_target* target, int32_t M, const double* fit,
+// ordered: fit_soa in the k-d order of the fit (CPD); otherwise in the caller's order, which the BCPD row factors share
+static int32_t estep_common(gingr_ctx* ctx, const gingr_target* target, int32_t M, const double* fit, bool ordered,
                             gingr::EstepWorkspace** ws_out) {
   CtxScratch* s = scratch_of(ctx);
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   GINGR_TRY(s->estep.ensure(ctx, M, target->N));
+  std::vector<int32_t> perm(M);
+  for (int i = 0; i < M; ++i) perm[i] = i;
+  if (ordered) gingr::estep_row_order(fit, M, perm);
+  std::vector<double> pf((size_t)3 * M);
+  for (int i = 0; i < M; ++i)
+    for (int d = 0; d < 3; ++d) pf[(size_t)3 * i + d] = fit[(size_t)3 * perm[i] + d];
+  GINGR_TRY(s->estep.set_row_order(ctx, M, perm.data()));
   GINGR_CUDA_TRY(ctx, s->a.alloc((size_t)3 * std::max(M, 1)));
-  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s->a.p, fit, sizeof(double) * 3 * (size_t)M, cudaMemcpyHostToDevice, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s->a.p, pf.data(), sizeof(double) * 3 * (size_t)M, cudaMemcpyHostToDevice, ctx->stream));
   GINGR_TRY(gingr::aos_to_soa_enqueue(ctx, M, s->a.p, s->estep.fit_soa.p));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));   // pf is a host vector
   *ws_out = &s->estep;
   return GINGR_OK;
 }
@@ -230,7 +250,7 @@ int32_t gingr_cpd_estep(gingr_ctx* ctx, const gingr_target* target, int32_t M, c
     return GINGR_OK;
   }
   gingr::EstepWorkspace* ws = nullptr;
-  GINGR_TRY(estep_common(ctx, target, M, fit, &ws));
+  GINGR_TRY(estep_common(ctx, target, M, fit, true, &ws));
   double* h = ctx->h_pinned;
   memset(h, 0, sizeof(double) * 16);
   h[0] = sigma2;
@@ -239,7 +259,7 @@ int32_t gingr_cpd_estep(gingr_ctx* ctx, const gingr_target* target, int32_t M, c
   h[7] = d2_bound(target, fit, (size_t)3 * M);
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(ws->scal.p, h, sizeof(double) * 16, cudaMemcpyHostToDevice, ctx->stream));
   GINGR_TRY(gingr::estep_cpd_scalars_enqueue(ctx, ws->scal.p));
-  if (target->N > 0) GINGR_TRY(gingr::estep_enqueue(ctx, *ws, M, target->N, target->soa.p, false));
+  if (target->N > 0) GINGR_TRY(gingr::estep_enqueue(ctx, *ws, M, target->N, target->soa.p, target->soa_perm.p, false));
   std::vector<double> rows;
   return estep_download(ctx, ws, M, target->N, P1, Pt1, PX, &rows);
 }
@@ -255,7 +275,7 @@ int32_t gingr_bcpd_estep(gingr_ctx* ctx, const gingr_target* target, int32_t M, 
     return GINGR_OK;
   }
   gingr::EstepWorkspace* ws = nullptr;
-  GINGR_TRY(estep_common(ctx, target, M, y, &ws));
+  GINGR_TRY(estep_common(ctx, target, M, y, false, &ws));
   CtxScratch* sc = scratch_of(ctx);
   GINGR_CUDA_TRY(ctx, sc->b.alloc((size_t)2 * M));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(sc->b.p, sigma_mm, sizeof(double) * (size_t)M, cudaMemcpyHostToDevice, ctx->stream));
@@ -269,7 +289,7 @@ int32_t gingr_bcpd_estep(gingr_ctx* ctx, const gingr_target* target, int32_t M, 
   h[7] = d2_bound(target, y, (size_t)3 * M);
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(ws->scal.p, h, sizeof(double) * 16, cudaMemcpyHostToDevice, ctx->stream));
   GINGR_TRY(gingr::estep_bcpd_rowf_enqueue(ctx, M, sc->b.p, sc->b.p + M, ws->scal.p, ws->rowf.p));
-  if (target->N > 0) GINGR_TRY(gingr::estep_enqueue(ctx, *ws, M, target->N, target->soa.p, true));
+  if (target->N > 0) GINGR_TRY(gingr::estep_enqueue(ctx, *ws, M, target->N, target->soa.p, target->soa_perm.p, true));
   std::vector<double> rows;
   std::vector<double> nup((size_t)target->N);
   std::vector<double> nuv((size_t)M), px((size_t)3 * M);

@@ -92,7 +92,8 @@ struct gingr_target {
   int n0 = 0, N = 0;    // this rank's shard [n0, n0 + N) for the E-step (== whole target when nranks == 1)
   double maxabs = 0.0;  // max |coordinate| (bounds the pair distances: gauss_exp2_tab<SAFE>)
   bool nonfinite = false;  // a NaN/Inf coordinate: every E-step on it fails like the reference's NaN-filled P
-  DevBuf<double> soa;   // E-step shard, SoA [3][N] (x[], y[], z[])
+  DevBuf<double> soa;   // E-step shard, SoA [3][N] (x[], y[], z[]) in the k-d order of gingr::estep_target_order
+  DevBuf<int32_t> soa_perm;  // [N] shard index (from n0) of soa position j
   // full mesh (ICP): vertices SoA [3][N_total], triangles, per-vertex normals and boundary flags
   DevBuf<double> verts; // [3][N_total]
   DevBuf<double> aos;   // [N_total][3] the same vertices, AoS (queries of the reversed ICP direction, line tests)

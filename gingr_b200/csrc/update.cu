@@ -118,11 +118,12 @@ __global__ void compact_gather_kernel(int M, int nranks, int Mmax, const double*
 
 // ---- CPD: fit and scalars for the E-step from the state block ----------------------------------
 // What the CPD E-step needs from the fit, in one pass and one launch (were four: two finite checks, the AoS -> SoA copy and a
-// one-block reduction): fit_soa, the failure flag for a non-finite fit / sigma2, and -- by the last block to finish, which
+// one-block reduction): fit_soa (row i of it is point perm[i], the E-step's k-d order), the failure flag for a non-finite fit / sigma2, and -- by the last block to finish, which
 // also resets the two words of `sync` for the next launch -- the scalars: scal[0] = sigma2, scal[1] = a = 1, scal[2] = c
 // (CPD.scala:69-70), scal[7] = bound of the pair distances from max |coordinate| of fit and target (gauss_exp2_tab<SAFE>).
 // The maximum is exact in any order, so the result does not depend on which block comes last.
-GINGR_KERNEL((256), cpd_prepare_kernel, int M, const double* __restrict__ fit /*AoS*/, double* __restrict__ fit_soa,
+GINGR_KERNEL((256), cpd_prepare_kernel, int M, const double* __restrict__ fit /*AoS*/, const int* __restrict__ perm,
+                                                          double* __restrict__ fit_soa,
                                                           const double* __restrict__ ds, double w, double ratio,
                                                           double target_maxabs, int* __restrict__ fail_flag,
                                                           unsigned long long* __restrict__ sync /*[2]: max bits, ticket*/,
@@ -132,7 +133,8 @@ GINGR_KERNEL((256), cpd_prepare_kernel, int M, const double* __restrict__ fit /*
   double m = 0.0;
   int bad = 0;
   if (i < M) {
-    const double x = fit[3 * i], y = fit[3 * i + 1], z = fit[3 * i + 2];
+    const size_t p = 3 * (size_t)perm[i];
+    const double x = fit[p], y = fit[p + 1], z = fit[p + 2];
     fit_soa[i] = x; fit_soa[M + i] = y; fit_soa[2 * (size_t)M + i] = z;
     bad = !(fabs(x) < INFINITY) || !(fabs(y) < INFINITY) || !(fabs(z) < INFINITY);
     m = fmax(fmax(fabs(x), fabs(y)), fabs(z));
@@ -1291,6 +1293,13 @@ int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, cons
   const int Mmax = ceil_div(M, ctx->nranks);
   if (cfg->algorithm == GINGR_ALGO_CPD) {
     GINGR_TRY(g->estep.ensure(ctx, M, std::max(target->N, 1)));
+    // the fit moves about the reference points, so their k-d order keeps the E-step's model tiles compact
+    std::vector<double> ref((size_t)3 * M);
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(ref.data(), model->ref.p, sizeof(double) * ref.size(), cudaMemcpyDeviceToHost, ctx->stream));
+    GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+    std::vector<int32_t> perm;
+    estep_row_order(ref.data(), M, perm);
+    GINGR_TRY(g->estep.set_row_order(ctx, M, perm.data()));
   } else {
     const bool rev = cfg->reverse_correspondence_direction != 0;
     GINGR_TRY(rev ? g->closest.ensure(ctx, target->N_total, M, model->T, target->T)
@@ -1487,7 +1496,7 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
   if (cfg.algorithm == GINGR_ALGO_CPD) {
     // non-finite fit / sigma2 / target: the reference's P is all NaN and the posterior fails
     if (tg->nonfinite) GINGR_TRY(validate_finite_enqueue(ctx, 3 * tg->N_total, tg->verts.p, g->is.p + IS_FAIL_POST));
-    GINGR_LAUNCH(ctx, cpd_prepare_kernel, ceil_div(M, 256), 256, 0, st, M, g->fit.p, g->estep.fit_soa.p, g->ds.p, cfg.w,
+    GINGR_LAUNCH(ctx, cpd_prepare_kernel, ceil_div(M, 256), 256, 0, st, M, g->fit.p, g->estep.row_perm.p, g->estep.fit_soa.p, g->ds.p, cfg.w,
                                                          (double)M / (double)tg->N_total, tg->maxabs, g->is.p + IS_FAIL_POST,
                                                          g->prep_sync.p, g->estep.scal.p);
     GINGR_LAUNCHED(ctx);
@@ -1495,7 +1504,7 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
       EstepEvents ee;
       const bool pe = g->ev(2) != nullptr;
       if (pe) { ee.a0 = *g->ev(2); ee.a1 = *g->ev(3); ee.b0 = *g->ev(4); ee.b1 = *g->ev(5); }
-      GINGR_TRY(estep_enqueue(ctx, g->estep, M, tg->N, tg->soa.p, false, pe ? &ee : nullptr));
+      GINGR_TRY(estep_enqueue(ctx, g->estep, M, tg->N, tg->soa.p, tg->soa_perm.p, false, pe ? &ee : nullptr));
       GINGR_CUDA_TRY(ctx, gingr_copy_d2d(ctx, g->rows_ext.p, g->estep.rows.p, sizeof(double) * 4 * (size_t)M, st));
       GINGR_LAUNCH(ctx, xpx_total_kernel, 1, 256, 0, st, g->estep.plan.den_blocks, g->estep.xpx_part.p, g->rows_ext.p + (size_t)4 * M);
       GINGR_LAUNCHED(ctx);
@@ -2097,6 +2106,7 @@ int32_t gingr_registration_set_profiling(gingr_registration* g, int32_t enable) 
   }
   g->profiling = enable != 0;
   g->prof_iters = 0;
+  if (g->estep.live.p) GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->estep.live.p, 0, 2 * sizeof(unsigned long long), ctx->stream));
   return GINGR_OK;
 }
 
@@ -2115,6 +2125,16 @@ int32_t gingr_registration_get_profile(gingr_registration* g, double* ms, int32_
     ms[2] += el(6, 7);
     ms[3] += el(8, 9);
     ms[4] += el(0, 1);
+  }
+  if (cpd) {
+    const EstepPlan& p = g->estep.plan;
+    unsigned long long live[2] = {0, 0};
+    if (p.cull) {
+      GINGR_CUDA_TRY(ctx, cudaMemcpy(live, g->estep.live.p, sizeof(live), cudaMemcpyDeviceToHost));
+      GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->estep.live.p, 0, sizeof(live), ctx->stream));
+    }
+    ms[6] = p.cull ? (double)live[0] / ((double)p.col_blocks * p.nsub) : g->prof_iters;
+    ms[7] = p.cull ? (double)live[1] / ((double)p.row_blocks * p.ntt) : g->prof_iters;
   }
   *iterations = g->prof_iters;
   g->prof_iters = 0;

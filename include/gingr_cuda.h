@@ -327,8 +327,9 @@ GINGR_API int32_t gingr_mcmc_best(gingr_registration* reg, gingr_state* state_ou
 
 /* ---- measurement hooks (new; used by bench.py for the roofline numbers) ------------------------ */
 /* Per-phase device timing with CUDA events recorded on the ctx stream around the kernels of gingr_update /
- * gingr_update_chain.  ms[8]: 0 = E-step sweep A kernel, 1 = E-step sweep B kernel, 2 = Gram (DMMA) kernel,
- * 3 = Cholesky + back substitution, 4 = whole iteration, 5 = closest-point search (ICP), 6 and 7 = unused.  Values are sums over `iterations` iterations since the last
+ * gingr_update_chain.  ms[8]: 0 = E-step sweep A kernels, 1 = E-step sweep B kernels (each with its cull kernels), 2 = Gram (DMMA) kernel,
+ * 3 = Cholesky + back substitution, 4 = whole iteration, 5 = closest-point search (ICP), 6 and 7 = CPD: live fraction
+ * of the tile pairs of sweep A / B (1 when nothing was culled; not a time).  Values are sums over `iterations` iterations since the last
  * call (the call synchronises the stream and resets the counters). */
 GINGR_API int32_t gingr_registration_set_profiling(gingr_registration* reg, int32_t enable);
 GINGR_API int32_t gingr_registration_get_profile(gingr_registration* reg, double* ms /*[8]*/, int32_t* iterations);
