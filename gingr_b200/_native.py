@@ -105,6 +105,8 @@ SIGNATURES = {
     "gingr_icp_closest_reversal": (c_int32, [c_void_p, c_void_p, c_int32, dp, ip, c_int32, c_int32, ip, bp, dp]),
     "gingr_posterior_mean": (c_int32, [c_void_p, c_void_p, dp, dp, c_int32, ip, dp, c_int32, dp, dp, dp]),
     "gingr_posterior_covariance": (c_int32, [c_void_p, c_void_p, dp, dp, c_int32, ip, dp, c_int32, dp, dp]),
+    "gingr_model_posterior": (c_int32, [c_void_p, c_void_p, dp, dp, c_int32, ip, dp, c_int32, dp, vpp]),
+    "gingr_posterior_model_profile": (c_int32, [c_void_p, dp, ip]),
     "gingr_coefficients": (c_int32, [c_void_p, c_void_p, dp, dp, dp, dp]),
     "gingr_spd_solve": (c_int32, [c_void_p, c_int32, dp, c_int32, dp, dp, dp, dp, c_int32, dp]),
     "gingr_model_instance": (c_int32, [c_void_p, c_void_p, POINTER(GingrState), dp, dp]),
@@ -117,6 +119,7 @@ SIGNATURES = {
     "gingr_update_chain_sampled": (c_int32, [c_void_p, c_int32, c_uint64]),
     "gingr_update_batch": (c_int32, [POINTER(c_void_p), c_int32, c_int32, c_int32, c_uint64]),
     "gingr_state_download": (c_int32, [c_void_p, POINTER(GingrState), dp, dp]),
+    "gingr_registration_posterior_model": (c_int32, [c_void_p, POINTER(GingrState), dp, vpp]),
     "gingr_mcmc_configure": (c_int32, [c_void_p, POINTER(GingrMcmcSettings), ip, c_int32, ip, c_int32]),
     "gingr_evaluate_log_value": (c_int32, [c_void_p, POINTER(GingrState), dp, dp]),
     "gingr_log_transition_probability": (c_int32, [c_void_p, POINTER(GingrState), dp, POINTER(GingrState), dp, dp]),

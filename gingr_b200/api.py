@@ -174,6 +174,16 @@ class Model:
                                                           basis.ctypes.data_as(nat.dp), 3 * self.M, nat.as_dp(var)))
         return ref, mean, basis, var
 
+    @staticmethod
+    def _from_handle(ctx: Context, h, M: int, rank: int, triangles) -> "Model":
+        """A model the library built: its host copy of the reference points is read back from the device."""
+        m = Model.__new__(Model)
+        m.ctx, m.M, m.rank, m.handle, m.triangles = ctx, M, rank, h, triangles
+        m.T = 0 if triangles is None else triangles.shape[0]
+        m.reference = np.empty((M, 3))
+        ctx.check(ctx._lib.gingr_model_download(ctx.handle, h, None, None, nat.as_dp(m.reference), None, None, 0, None))
+        return m
+
     def newReference(self, ref_points, triangles=None) -> "Model":
         """model.newReference(newRef, NearestNeighborInterpolator()) (SimpleRegistrator.scala:90-92) on the device: the
         new model's rows are gathered from the resident basis at the nearest old reference points."""
@@ -382,6 +392,38 @@ def posterior_covariance(ctx: Context, model: Model, R, t, pids, points, noise) 
     if code == nat.GINGR_MODEL_FLEXIBILITY:
         raise FloatingPointError("posterior failed (ModelFlexibilityError)")
     return cov
+
+
+def posterior_model(ctx: Context, model: Model, R, t, pids, points, noise) -> Model:
+    """model.transform(R, t).posterior(obs) as a new device model (scalismo PointDistributionModel.posterior, SURVEY A3;
+    GingrAlgorithm.scala:299-300): reference R ref + t, mean R (mean + basis D c), basis (I (x) R) basis U, variance s
+    (descending) with U diag(s) U^T = D Mx^-1 D.  Arguments as posterior_mean; raises FloatingPointError where the
+    posterior fails (ModelFlexibilityError)."""
+    R = nat.f64(R).reshape(3, 3)
+    t = nat.f64(t).reshape(3)
+    pids = nat.i32(pids)
+    pts = nat.f64(points).reshape(-1, 3)
+    noise = nat.f64(noise)
+    n = pids.shape[0]
+    if pids.ndim != 1 or pts.shape[0] != n:
+        raise ValueError(f"{n} point ids but {pts.shape[0]} points")
+    if noise.shape not in ((n,), (n, 3, 3)):
+        raise ValueError(f"noise must have shape ({n},) or ({n}, 3, 3), got {noise.shape}")
+    h = ctypes.c_void_p()
+    code = ctx.check(ctx._lib.gingr_model_posterior(ctx.handle, model.handle, nat.as_dp(R), nat.as_dp(t), n, nat.as_ip(pids),
+                                                    nat.as_dp(pts), 0 if noise.ndim == 1 else 1, nat.as_dp(noise), ctypes.byref(h)))
+    if code == nat.GINGR_MODEL_FLEXIBILITY:
+        raise FloatingPointError("posterior failed (ModelFlexibilityError)")
+    return Model._from_handle(ctx, h, model.M, model.rank, model.triangles)
+
+
+def posterior_model_profile(ctx: Context):
+    """Device times (ms) of the last posterior model built on ctx: dict(system, jacobi, gemm, constants, total, sweeps)."""
+    ms = np.zeros(5)
+    sweeps = ctypes.c_int32()
+    ctx.check(ctx._lib.gingr_posterior_model_profile(ctx.handle, nat.as_dp(ms), ctypes.byref(sweeps)))
+    return dict(system=float(ms[0]), jacobi=float(ms[1]), gemm=float(ms[2]), constants=float(ms[3]), total=float(ms[4]),
+                sweeps=int(sweeps.value))
 
 
 def spd_solve(ctx: Context, A, B=None, reps: int = 1):
@@ -645,6 +687,18 @@ class GingrAlgorithm:
         if st.status == STATUS_NONE:
             st = dataclasses.replace(st, status=final)
         return st
+
+    def computePosterior(self, current: GeneralRegistrationState) -> Model:
+        """GingrAlgorithm.computePosterior(current) (:281-302): the posterior model of the configuration's correspondences
+        and uncertainties (and landmarks) at `current`.  Raises FloatingPointError where the posterior fails.  The device-resident
+        state is replaced; the next update uploads its own."""
+        st, alpha = current.to_pod()
+        h = ctypes.c_void_p()
+        code = self.ctx.check(self.ctx._lib.gingr_registration_posterior_model(self.handle, ctypes.byref(st), nat.as_dp(alpha),
+                                                                               ctypes.byref(h)))
+        if code == nat.GINGR_MODEL_FLEXIBILITY:
+            raise FloatingPointError("posterior failed (ModelFlexibilityError)")
+        return Model._from_handle(self.ctx, h, self.model.M, self.model.rank, self.model.triangles)
 
     # device-resident chaining (throughput runs)
     def updateChain(self, iters: int):

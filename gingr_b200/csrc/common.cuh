@@ -30,6 +30,9 @@ struct gingr_ctx {
   // small pinned staging buffer for scalars
   double* h_pinned = nullptr;  // 4096 doubles
   size_t h_pinned_count = 4096;
+  // phase times (ms) and Jacobi sweeps of the last posterior model built on this ctx (gingr_posterior_model_profile)
+  double posterior_model_ms[5] = {0, 0, 0, 0, 0};
+  int posterior_model_sweeps = 0;
 };
 
 // Device buffer that owns its memory: freed when the owner goes away, moved but never copied.

@@ -26,6 +26,7 @@
 #include <vector>
 
 #include "batch.cuh"
+#include "dmma.cuh"
 #include "posterior.cuh"
 
 namespace gingr {
@@ -41,24 +42,6 @@ constexpr int GRAM_THREADS = GRAM_WARPS_M * 4 * 32;
 constexpr int WTM = BT / GRAM_WARPS_M;   // warp tile rows
 constexpr int MI = WTM / 8;              // 8-row DMMA fragments per warp tile
 constexpr size_t GRAM_SMEM = (size_t)STAGES * (2 * BK * PITCH + BK) * sizeof(double);
-
-__device__ __forceinline__ void cp_async16(void* smem, const void* gmem, int src_bytes) {
-  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(s), "l"(gmem), "r"(src_bytes));
-}
-__device__ __forceinline__ void cp_async8(void* smem, const void* gmem, int src_bytes) {
-  const unsigned s = (unsigned)__cvta_generic_to_shared(smem);
-  asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;\n" ::"r"(s), "l"(gmem), "r"(src_bytes));
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;\n" ::); }
-template <int N>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;\n" ::"n"(N)); }
-
-__device__ __forceinline__ void dmma884(double& c0, double& c1, double a, double b) {
-  asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n"
-               : "+d"(c0), "+d"(c1)
-               : "d"(a), "d"(b));
-}
 
 // segment of work of one CTA: tile (ta >= tb), chunk range [c0, c1), output slot
 struct GramSegment {

@@ -55,6 +55,12 @@ int32_t chol_backsolve_enqueue(gingr_ctx* ctx, int n, const double* d_L, int ld,
                                int* d_flags, CholWs* ws = nullptr);
 int32_t chol_backsolve_z_enqueue(gingr_ctx* ctx, int n, const double* d_L, int ld, const double* d_z, double* d_c, CholWs& ws);
 
+// ---- basis_rotate.cu -----------------------------------------------------------------------------
+// out[3i + d][j] = scale[j] * sum_e R[d][e] (Phi U)[3i + e][j]  on DMMA: Phi, out [rows][rp], U [rp][rp] (all row-major,
+// zero padded), scale [rp], d_R: 9 doubles (row-major rotation) on the device.  rows a multiple of 3, rp of 8.
+int32_t basis_rotate_enqueue(gingr_ctx* ctx, int rows, int rp, const double* d_phi, const double* d_U, const double* d_scale,
+                             const double* d_R, double* d_out);
+
 // ---- vecops.cu -----------------------------------------------------------------------------------
 // out_q[k] = sum_a phi[k][a] v_q[a],  q < nvec (1 or 2), k < rows
 // d_scale (optional): the vectors are multiplied elementwise by it while they are staged (instance(alpha) = Phi (sqrt(lambda) alpha))

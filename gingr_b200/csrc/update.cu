@@ -960,6 +960,12 @@ __global__ void posterior_cov_rows_kernel(int rows, int r, int rp, const double*
   for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < rp; c += gridDim.x * blockDim.x)
     out[(size_t)k * rp + c] = c < r ? phi[(size_t)k * rp + c] * sqrt_lambda[c] : 0.0;
 }
+// rows r + 1 + k of the system <- sqrt(lambda_k) e_k: they come out as the rows of B = D L^-T, B B^T = D Mx^-1 D
+__global__ void posterior_model_rows_kernel(int r, int rp, const double* __restrict__ sqrt_lambda, double* __restrict__ out) {
+  const int k = blockIdx.y;
+  for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < rp; c += gridDim.x * blockDim.x)
+    out[(size_t)k * rp + c] = c == k ? sqrt_lambda[k] : 0.0;
+}
 // cov_i = R (X_i X_i^T) R^T with X_i the three solved rows of vertex i; one warp per vertex
 __global__ void __launch_bounds__(256) posterior_cov_kernel(int M, int r, int rp, const double* __restrict__ X,
                                                             const double* __restrict__ ds, double* __restrict__ cov) {
@@ -989,18 +995,44 @@ __global__ void __launch_bounds__(256) posterior_cov_kernel(int M, int r, int rp
         cov[(size_t)9 * i + 3 * a + b] = T[3 * a] * R[3 * b] + T[3 * a + 1] * R[3 * b + 1] + T[3 * a + 2] * R[3 * b + 2];
   }
 }
+
+// CUDA events at the phase boundaries of a posterior-model build (gingr_posterior_model_profile); destroyed on every exit
+struct PosteriorModelEvents {
+  cudaEvent_t e[5] = {};
+  ~PosteriorModelEvents() {
+    for (cudaEvent_t x : e)
+      if (x) cudaEventDestroy(x);
+  }
+  int32_t create(gingr_ctx* ctx) {
+    for (cudaEvent_t& x : e) GINGR_CUDA_TRY(ctx, cudaEventCreate(&x));
+    return GINGR_OK;
+  }
+  int32_t record(gingr_ctx* ctx, int k) {
+    GINGR_CUDA_TRY(ctx, cudaEventRecord(e[k], ctx->stream));
+    return GINGR_OK;
+  }
+};
 }  // namespace gingr
+// posterior_model.cuh: the model from the factorised system (rows B = D L^-T behind the rhs row), c and the pose in d_ds
+static int32_t posterior_model_finish(gingr_ctx* ctx, const gingr_model* m, const double* d_B, const double* d_c,
+                                      const double* d_ds, gingr::PosteriorModelEvents& ev, gingr_model** out);
 
 // the regression of model.transform(R, t).posterior(obs): coefficients, mean mesh and (optionally) the covariance blocks
+// or the posterior model itself
 static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const double* R, const double* t, int32_t n,
                               const int32_t* pid, const double* points, int32_t noise_kind, const double* noise,
-                              double* coeffs, double* mean_pts, double* cov_pts) {
+                              double* coeffs, double* mean_pts, double* cov_pts, gingr_model** model_out = nullptr) {
   if (!ctx || !model || !R || !t || n < 0 || (n > 0 && (!pid || !points || !noise)) || noise_kind < 0 || noise_kind > 1)
     return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_posterior_mean: bad argument");
   if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_posterior_mean: single-GPU entry point");
   const gingr_model* m = model;
   const int M = m->M, r = m->r, rp = m->rp;
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  gingr::PosteriorModelEvents ev;
+  if (model_out) {
+    GINGR_TRY(ev.create(ctx));
+    GINGR_TRY(ev.record(ctx, 0));
+  }
   // Host-side marshalling of the observation list into per-vertex weights / residuals.  Isotropic
   // observations of the same vertex add up (W = sum 1/var, W y = sum y/var); full-covariance ones become
   // "landmark" blocks.
@@ -1048,7 +1080,8 @@ static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const do
   cudaStream_t st = ctx->stream;
   DevBuf<int32_t> d_lpid;
   DevBuf<double> d_lpts, d_lcinv, d_lA, d_lrows;
-  const int xrows = cov_pts ? 3 * M : 0;       // rows of Q carried through the factorisation for the covariance
+  // rows carried through the factorisation: Q for the covariance, D for the posterior model
+  const int xrows = cov_pts ? 3 * M : (model_out ? r : 0);
   GINGR_CUDA_TRY(ctx, s.Mx.alloc((size_t)(r + 8 + xrows) * rp));
   GINGR_CUDA_TRY(ctx, s.wrow.alloc((size_t)3 * M));
   GINGR_CUDA_TRY(ctx, s.u.alloc((size_t)3 * M));
@@ -1089,9 +1122,12 @@ static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const do
   }
   GINGR_TRY(gram_partials_enqueue(ctx, s.gram, m->phi.p, s.wrow.p));
   GINGR_TRY(gram_finish_enqueue(ctx, s.gram, s.gram.d_partial.p, m->sqrt_lambda.p, 1.0, L, d_lrows.p, d_lA.p, rp, s.Mx.p, false, true));
-  if (xrows > 0) {
+  if (cov_pts) {
     gingr::posterior_cov_rows_kernel<<<dim3(ceil_div(rp, 256), xrows), 256, 0, st>>>(xrows, r, rp, m->phi.p, m->sqrt_lambda.p,
                                                                                  s.Mx.p + (size_t)(r + 1) * rp);
+    GINGR_LAUNCHED(ctx);
+  } else if (model_out) {
+    gingr::posterior_model_rows_kernel<<<dim3(ceil_div(rp, 256), r), 256, 0, st>>>(r, rp, m->sqrt_lambda.p, s.Mx.p + (size_t)(r + 1) * rp);
     GINGR_LAUNCHED(ctx);
   }
   GINGR_TRY(cholesky_enqueue(ctx, r, r + 1 + xrows, s.Mx.p, rp, s.is.p + IS_INFO, &s.cholws));
@@ -1099,6 +1135,7 @@ static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const do
   GINGR_TRY(chol_backsolve_enqueue(ctx, r, s.Mx.p, rp, rhs, c, s.flags.p, &s.cholws));
   GINGR_LAUNCH(ctx, check_finite_kernel, ceil_div(r, 256), 256, 0, st, r, c, s.is.p + IS_FAIL_POST);
   GINGR_LAUNCHED(ctx);
+  if (model_out) GINGR_TRY(ev.record(ctx, 1));
   if (mean_pts) {
     GINGR_TRY(instance_rows(ctx, m, s.vec.p + 2 * rp, 1, c, nullptr, s.inst.p, nullptr));
     GINGR_LAUNCH(ctx, fit_from_instance_kernel, ceil_div(M, 256), 256, 0, st, 0, M, m->ref.p, m->mean.p, s.inst.p, s.ds.p, DS_SCALE, DS_T,
@@ -1117,7 +1154,9 @@ static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const do
   if (coeffs) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(coeffs, c, sizeof(double) * r, cudaMemcpyDeviceToHost, st));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(his, s.is.p, sizeof(int) * IS_COUNT, cudaMemcpyDeviceToHost, st));
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-  return (his[IS_INFO] || his[IS_FAIL_POST]) ? GINGR_MODEL_FLEXIBILITY : GINGR_OK;
+  if (his[IS_INFO] || his[IS_FAIL_POST]) return GINGR_MODEL_FLEXIBILITY;
+  if (model_out) return posterior_model_finish(ctx, m, s.Mx.p + (size_t)(r + 1) * rp, c, s.ds.p, ev, model_out);
+  return GINGR_OK;
 }
 
 extern "C" {
@@ -1127,6 +1166,14 @@ int32_t gingr_posterior_mean(gingr_ctx* ctx, const gingr_model* model, const dou
                              const int32_t* pid, const double* points, int32_t noise_kind, const double* noise,
                              double* coeffs, double* mean_pts) {
   return posterior_core(ctx, model, R, t, n, pid, points, noise_kind, noise, coeffs, mean_pts, nullptr);
+}
+
+int32_t gingr_model_posterior(gingr_ctx* ctx, const gingr_model* model, const double* R, const double* t, int32_t n,
+                              const int32_t* pid, const double* points, int32_t noise_kind, const double* noise,
+                              gingr_model** out) {
+  if (!out) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_model_posterior: bad argument");
+  *out = nullptr;
+  return posterior_core(ctx, model, R, t, n, pid, points, noise_kind, noise, nullptr, nullptr, nullptr, out);
 }
 
 int32_t gingr_posterior_covariance(gingr_ctx* ctx, const gingr_model* model, const double* R, const double* t, int32_t n,
@@ -2157,5 +2204,6 @@ int32_t gingr_state_download(gingr_registration* g, gingr_state* state_out, doub
 
 #include "mcmc.cuh"
 #include "gpmm.cuh"
+#include "posterior_model.cuh"
 
 gingr_registration::~gingr_registration() = default;

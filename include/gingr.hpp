@@ -204,6 +204,9 @@ struct ProbabilisticSettings {
   }
 };
 
+template <class Config>
+class GingrAlgorithm;
+
 // scalismo PointDistributionModel on the device
 class Model {
  public:
@@ -234,6 +237,21 @@ class Model {
     m.r_ = r_;
     return m;
   }
+  // model.transform(R, t).posterior(trainingData) as a new model (GingrAlgorithm.scala:299-300; scalismo, SURVEY.md A3).
+  // R row-major [9], t [3]; noiseKind 0: noise[n] isotropic variances, 1: noise[9n] covariances.  Throws Error with code
+  // GINGR_MODEL_FLEXIBILITY where the posterior fails.
+  Model posterior(const std::array<double, 9>& R, const std::array<double, 3>& t, const std::vector<int32_t>& pid,
+                  const std::vector<double>& points, int noiseKind, const std::vector<double>& noise) const {
+    const size_t n = pid.size();
+    if (points.size() != 3 * n || noise.size() != (noiseKind == 0 ? n : 9 * n)) throw Error(GINGR_ERR_ARG, "observation array sizes");
+    Model m(*ctx_);
+    if (ctx_->check(gingr_model_posterior(ctx_->handle(), h_, R.data(), t.data(), static_cast<int32_t>(n), pid.data(), points.data(),
+                                          noiseKind, noise.data(), &m.h_)) == GINGR_MODEL_FLEXIBILITY)
+      throw Error(GINGR_MODEL_FLEXIBILITY, "posterior failed (ModelFlexibilityError)");
+    m.M_ = M_;
+    m.r_ = r_;
+    return m;
+  }
   // ModelFittingParameters.modelInstanceShapePoseScale, api/ModelFittingParameters.scala:130-143
   std::vector<double> instance(const ModelFittingParameters& p) const {
     GeneralRegistrationState s;
@@ -252,6 +270,8 @@ class Model {
   int rank() const { return r_; }
 
  private:
+  template <class Config>
+  friend class GingrAlgorithm;
   explicit Model(const Context& ctx) : ctx_(&ctx) {}
   const Context* ctx_;
   gingr_model* h_ = nullptr;
@@ -328,6 +348,18 @@ class GingrAlgorithm {
     next.fromPod(out);
     next.modelParameters.shape = std::move(alpha);
     return next;
+  }
+
+  // GingrAlgorithm.computePosterior(current) (:281-302): the posterior model of the configuration's correspondences,
+  // uncertainties and landmarks at `current`.  Throws Error with code GINGR_MODEL_FLEXIBILITY where the posterior fails.
+  Model computePosterior(const State& current) const {
+    const gingr_state in = current.toPod();
+    Model m(*ctx_);
+    if (ctx_->check(gingr_registration_posterior_model(h_, &in, current.modelParameters.shape.data(), &m.h_)) == GINGR_MODEL_FLEXIBILITY)
+      throw Error(GINGR_MODEL_FLEXIBILITY, "posterior failed (ModelFlexibilityError)");
+    m.M_ = model_->points();
+    m.r_ = model_->rank();
+    return m;
   }
 
   // GingrGeneratorWrapper.propose (GingrGeneratorWrapper.scala:28-39): update, refreshed fit, iteration + 1, generatedBy

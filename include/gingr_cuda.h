@@ -215,6 +215,20 @@ GINGR_API int32_t gingr_posterior_mean(gingr_ctx* ctx, const gingr_model* model,
 GINGR_API int32_t gingr_posterior_covariance(gingr_ctx* ctx, const gingr_model* model, const double* R, const double* t,
                                              int32_t n, const int32_t* pid, const double* points /*[3n]*/,
                                              int32_t noise_kind, const double* noise, double* cov_pts /*[9M]*/);
+/* scalismo model.transform(R, t).posterior(trainingData) (SURVEY.md A3; call site GingrAlgorithm.scala:299-300) as a
+ * new model handle.  Observation arguments exactly as gingr_posterior_mean.  The new model: reference R ref_i + t with the
+ * source model's triangles, mean R (mean_i + Phi_i D c) (c: the coefficients of gingr_posterior_mean, D = diag(sqrt(lambda))),
+ * basis (I (x) R) Phi U, variance s in descending order (stable) with U diag(s) U^T = D Mx^-1 D.  Indices with variance 0 in
+ * the source model keep the unit vector e_k and variance 0.  The basis is unique up to rotations inside degenerate
+ * eigenspaces.  Returns GINGR_MODEL_FLEXIBILITY with *out = NULL for non-finite noise or a failed factorisation.
+ * Single-GPU contexts only. */
+GINGR_API int32_t gingr_model_posterior(gingr_ctx* ctx, const gingr_model* model, const double* R, const double* t,
+                                        int32_t n, const int32_t* pid, const double* points /*[3n]*/, int32_t noise_kind,
+                                        const double* noise, gingr_model** out);
+/* Device times of the last posterior model built on the ctx (gingr_model_posterior, gingr_registration_posterior_model),
+ * CUDA events in ms: [0] observations, system assembly and factorisation, [1] eigenpairs (Jacobi), [2] basis product,
+ * [3] mean, reference and regression constants, [4] the whole call.  sweeps (may be NULL): Jacobi sweeps. */
+GINGR_API int32_t gingr_posterior_model_profile(const gingr_ctx* ctx, double* ms /*[5]*/, int32_t* sweeps);
 /* Replaces model.transform(rigid).coefficients(mesh) (GingrAlgorithm.scala:215, :236): regression on
  * all M points with noise 1e-5 * I3. */
 GINGR_API int32_t gingr_coefficients(gingr_ctx* ctx, const gingr_model* model, const double* R, const double* t,
@@ -278,6 +292,12 @@ GINGR_API int32_t gingr_update_batch(gingr_registration** regs, int32_t n, int32
 /* Read back the device-resident state after gingr_update_chain / gingr_update_batch. */
 GINGR_API int32_t gingr_state_download(gingr_registration* reg, gingr_state* state_out, double* alpha_out,
                                        double* fit_out);
+
+/* GingrAlgorithm.computePosterior(current) (GingrAlgorithm.scala:281-302): the correspondences and uncertainties of the
+ * registration's configuration (CPD E-step / ICP flavours, landmarks) at `state`, then the posterior model as
+ * gingr_model_posterior builds it.  The device-resident state is replaced (the next gingr_update uploads its own). */
+GINGR_API int32_t gingr_registration_posterior_model(gingr_registration* reg, const gingr_state* state,
+                                                     const double* alpha /*[r]*/, gingr_model** out);
 
 /* ---- probabilistic registration: Metropolis-Hastings with the informed GiNGR proposal (SURVEY.md 8f item 1) ---- */
 /* sampling/evaluators/IndependentPointDistanceEvaluator.scala:26-32 EvaluationMode */

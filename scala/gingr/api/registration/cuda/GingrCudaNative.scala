@@ -112,6 +112,11 @@ object GingrCudaNative {
   // per-vertex 3 x 3 covariance of the same posterior (what PosteriorHelper colour-maps)
   val posteriorCov   = fn("gingr_posterior_covariance", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT,
                           ADDRESS, ADDRESS)
+  // GingrAlgorithm.scala:299-300 model.transform(rigid).posterior(trainingData) as a new model handle, :281-302 computePosterior
+  val modelPosterior = fn("gingr_model_posterior", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT,
+                          ADDRESS, ADDRESS)
+  val registrationPosteriorModel = fn("gingr_registration_posterior_model", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS)
+  val posteriorModelProfile = fn("gingr_posterior_model_profile", JAVA_INT, ADDRESS, ADDRESS, ADDRESS)
   val coefficients   = fn("gingr_coefficients", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS)
   // the r x r solve of the regression alone (pinv(Mx) * rhs as a Cholesky solve): A, nrhs rows of B -> L, L^-1 B^T rows, A^-1 b_0
   val spdSolve       = fn("gingr_spd_solve", JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_INT,
