@@ -132,16 +132,30 @@ class Model:
                         maxRank: int = 0) -> "Model":
         """GPMMTriangleMesh3D(reference, relativeTolerance).GaussianMixture(pars) (api/gpmm/GPMMHelper.scala:117-121;
         .Gaussian(sigma, scaling) is the one-kernel case, :100-103) built on the device."""
+        return Model._build_gpmm(ctx, "gingr_gpmm_gaussian_mixture", ref_points, triangles, sigmas, scalings, relativeTolerance, maxRank)
+
+    @staticmethod
+    def gaussianSymmetric(ctx: Context, ref_points, triangles, sigmas, scalings, relativeTolerance: float = 0.01,
+                          maxRank: int = 0) -> "Model":
+        """The mirror-symmetric Gaussian (mixture) model about the plane x = 0, built on the device: scalismo's
+        symmetrised kernel K(x, y) = diag(k(x, y) - k(Sx, y), k(x, y) + k(Sx, y), k(x, y) + k(Sx, y)), S = diag(-1, 1, 1),
+        k = sum_q scaling_q exp(-|x - y|^2 / sigma_q^2).  Left and right halves deform as mirror images; the caller centres
+        the template on the plane x = 0.  Arguments and stopping rule as gaussianMixture."""
+        return Model._build_gpmm(ctx, "gingr_gpmm_gaussian_symmetric", ref_points, triangles, sigmas, scalings, relativeTolerance, maxRank)
+
+    @staticmethod
+    def _build_gpmm(ctx: Context, entry: str, ref_points, triangles, sigmas, scalings, relativeTolerance, maxRank) -> "Model":
+        """A model from one of the device GPMM builders, which share their arguments."""
         ref = nat.f64(ref_points).reshape(-1, 3)
         tri = None if triangles is None else nat.i32(triangles).reshape(-1, 3)
         sg, sc = nat.f64(np.atleast_1d(sigmas)), nat.f64(np.atleast_1d(scalings))
         if sg.shape != sc.shape or sg.ndim != 1:
-            raise ValueError("gaussianMixture: one scaling per sigma")
+            raise ValueError(f"{entry}: one scaling per sigma")
+        build = getattr(ctx._lib, entry)
         h = ctypes.c_void_p()
         rank = ctypes.c_int32()
-        ctx.check(ctx._lib.gingr_gpmm_gaussian_mixture(ctx.handle, ref.shape[0], nat.as_dp(ref), nat.as_ip(tri),
-                                                       0 if tri is None else tri.shape[0], len(sg), nat.as_dp(sg), nat.as_dp(sc),
-                                                       float(relativeTolerance), int(maxRank), ctypes.byref(h), ctypes.byref(rank)))
+        ctx.check(build(ctx.handle, ref.shape[0], nat.as_dp(ref), nat.as_ip(tri), 0 if tri is None else tri.shape[0], len(sg),
+                        nat.as_dp(sg), nat.as_dp(sc), float(relativeTolerance), int(maxRank), ctypes.byref(h), ctypes.byref(rank)))
         m = Model.__new__(Model)
         m.ctx, m.M, m.rank, m.T, m.handle, m.triangles = ctx, ref.shape[0], int(rank.value), 0 if tri is None else tri.shape[0], h, tri
         m.reference = ref.copy()
@@ -899,6 +913,20 @@ class GaussKernel:
 
 
 @dataclass(frozen=True)
+class GaussSymKernel:
+    """The mirror-symmetric Gaussian kernel about x = 0 (Model.gaussianSymmetric) with one (scaling, sigma).  The
+    reference's own name for this selector is not known here: the name "GaussSym", and with it the cache file name
+    <name>_dec-<d>_GaussSym_<scaling>_<sigma>.h5.json, are this project's."""
+    scaling: float
+    sigma: float
+    name = "GaussSym"
+
+    @property
+    def printpars(self) -> str:
+        return _scala_double(self.scaling) + "_" + _scala_double(self.sigma)
+
+
+@dataclass(frozen=True)
 class GaussMixKernel:
     """simple/SimpleModels.scala:41-44 (AutomaticGaussian)."""
     name = "GaussMix"
@@ -907,17 +935,21 @@ class GaussMixKernel:
 
 class SimpleTriangleModels3D:
     """simple/SimpleModels.scala:54-77 for the Gaussian families (the kernels the demos load: femur Gauss(50, 70), bunny
-    Gauss(20, 40), DemoDatasetLoader.scala:113-114, :146-147).  The Laplacian, dot-product and mirror kernels are not
-    on the path SURVEY.md 8 scopes and are refused rather than approximated."""
+    Gauss(20, 40), DemoDatasetLoader.scala:113-114, :146-147) and the mirror-symmetric Gaussian kernel (GaussSymKernel).
+    The Laplacian and dot-product kernels are not on the path SURVEY.md 8 scopes and are refused rather than
+    approximated."""
 
     @staticmethod
     def create(ctx: Context, reference_points, triangles, kernelSelect, relativeTolerance: float = 0.01) -> Model:
         if isinstance(kernelSelect, GaussKernel):
             return Model.gaussianMixture(ctx, reference_points, triangles, [kernelSelect.sigma], [kernelSelect.scaling],
                                          relativeTolerance)
+        if isinstance(kernelSelect, GaussSymKernel):
+            return Model.gaussianSymmetric(ctx, reference_points, triangles, [kernelSelect.sigma], [kernelSelect.scaling],
+                                           relativeTolerance)
         if isinstance(kernelSelect, GaussMixKernel):
             return Model.automaticGaussian(ctx, reference_points, triangles, relativeTolerance)
-        raise NotImplementedError(f"kernel {type(kernelSelect).__name__} is outside the device GPMM builder (Gaussian families only)")
+        raise NotImplementedError(f"kernel {type(kernelSelect).__name__} is outside the device GPMM builder (Gaussian families and their mirror-symmetric form only)")
 
 
 class SimpleRegistrator:

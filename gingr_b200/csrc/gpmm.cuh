@@ -10,6 +10,9 @@
 // residual diagonal of (p, 1), (p, 2) untouched and maximal, so the columns come in triples of the same point, and after
 // c columns of triple k the trace is 3 T(k) - c (T(k) - T(k+1)) with T the scalar traces -- which also reproduces a rank
 // that is not a multiple of three (tests/test_oracle_gpmm.py proves this against the literal 3M x 3M algorithm).
+// The mirror-symmetric kernel (scalismo's symmetrised kernel about x = 0, gingr_gpmm_gaussian_symmetric) is diagonal
+// too, with two distinct blocks: ks - ks_m for dimension 0 and ks + ks_m for dimensions 1 and 2, ks_m(x, y) = ks(S x, y).
+// Both cases are one loop (gpmm_build): a scalar factorisation per block, merged on the host in the literal order.
 //   pivoted Cholesky   one column per step: argmax of the residual diagonal (lowest index on ties), the kernel column
 //                      minus the projection on the previous columns, diagonal update; all scalars stay on the device,
 //                      the host looks at the trace history once per batch of steps
@@ -35,10 +38,30 @@ __device__ __forceinline__ double gpmm_kernel(const GaussKernelDev& kp, double d
   return s;
 }
 
-__global__ void gpmm_init_diag_kernel(int M, GaussKernelDev kp, double* __restrict__ d, uint8_t* __restrict__ done) {
+// The scalar M x M block a factorisation works on: GPMM_PLAIN is ks itself; GPMM_MINUS / GPMM_PLUS are ks(x, y) -/+ ks(S x, y)
+// with the mirror S = diag(-1, 1, 1) about the plane x = 0 (the blocks of the mirror-symmetric kernel, see
+// gingr_gpmm_gaussian_symmetric).
+enum GpmmBlockKind { GPMM_PLAIN = 0, GPMM_MINUS = 1, GPMM_PLUS = 2 };
+
+template <int KIND>
+__device__ __forceinline__ double gpmm_entry(const GaussKernelDev& kp, const double* __restrict__ pts, int i, int p) {
+  if constexpr (KIND == GPMM_PLAIN) {
+    return gpmm_kernel(kp, pts[3 * i] - pts[3 * p], pts[3 * i + 1] - pts[3 * p + 1], pts[3 * i + 2] - pts[3 * p + 2]);
+  } else {
+    const double dy = pts[3 * i + 1] - pts[3 * p + 1], dz = pts[3 * i + 2] - pts[3 * p + 2];
+    const double k = gpmm_kernel(kp, pts[3 * i] - pts[3 * p], dy, dz);
+    const double km = gpmm_kernel(kp, -pts[3 * i] - pts[3 * p], dy, dz);   // S x_i - x_p
+    return KIND == GPMM_MINUS ? k - km : k + km;
+  }
+}
+
+template <int KIND>
+__global__ void gpmm_init_diag_kernel(int M, GaussKernelDev kp, const double* __restrict__ pts, double* __restrict__ d,
+                                      uint8_t* __restrict__ done) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= M) return;
-  d[i] = gpmm_kernel(kp, 0.0, 0.0, 0.0);
+  if constexpr (KIND == GPMM_PLAIN) d[i] = gpmm_kernel(kp, 0.0, 0.0, 0.0);
+  else d[i] = gpmm_entry<KIND>(kp, pts, i, i);
   done[i] = 0;
 }
 
@@ -86,8 +109,9 @@ __global__ void gpmm_argmax_final_kernel(int nb, int k, const double* __restrict
   trace[k] = sum;
 }
 
-// column k of the scalar factor (column-major Ls[k][M]): (ks(x_i, x_p) - sum_{j<k} Ls[j][i] Ls[j][p]) / sqrt(d_p) for the
+// column k of the scalar factor (column-major Ls[k][M]): (block(x_i, x_p) - sum_{j<k} Ls[j][i] Ls[j][p]) / sqrt(d_p) for the
 // points not yet chosen, sqrt(d_p) at the pivot, 0 at earlier pivots; residual diagonal updated
+template <int KIND>
 __global__ void __launch_bounds__(256) gpmm_column_kernel(int M, int k, GaussKernelDev kp, const double* __restrict__ pts /*AoS*/,
                                                           const int* __restrict__ pivots, const double* __restrict__ dpiv,
                                                           double* __restrict__ Ls, double* __restrict__ d,
@@ -105,7 +129,7 @@ __global__ void __launch_bounds__(256) gpmm_column_kernel(int M, int k, GaussKer
     if (i == p) {
       out = piv;
     } else if (!done[i]) {
-      double v = gpmm_kernel(kp, pts[3 * i] - pts[3 * p], pts[3 * i + 1] - pts[3 * p + 1], pts[3 * i + 2] - pts[3 * p + 2]);
+      double v = gpmm_entry<KIND>(kp, pts, i, p);
       for (int j = 0; j < k; ++j) v -= Ls[(size_t)j * M + i] * lp[j];
       out = v / piv;
       d[i] -= out * out;
@@ -185,13 +209,13 @@ __global__ void __launch_bounds__(256) gpmm_colnorm_kernel(int M, const double* 
 struct GpmmColumn { int set, j, d; };
 __global__ void gpmm_assemble_kernel(int M, int r, int rp, const GpmmColumn* __restrict__ cols, const double* __restrict__ A0,
                                      const double* __restrict__ n0, const double* __restrict__ A1, const double* __restrict__ n1,
-                                     double* __restrict__ phi) {
+                                     const double* __restrict__ A2, const double* __restrict__ n2, double* __restrict__ phi) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   const int c = blockIdx.y;
   if (i >= M || c >= r) return;
   const GpmmColumn col = cols[c];
-  const double* A = col.set == 0 ? A0 : A1;
-  const double* nn = col.set == 0 ? n0 : n1;
+  const double* A = col.set == 0 ? A0 : col.set == 1 ? A1 : A2;
+  const double* nn = col.set == 0 ? n0 : col.set == 1 ? n1 : n2;
   phi[((size_t)3 * i + col.d) * rp + c] = A[(size_t)col.j * M + i] / sqrt(nn[col.j]);
 }
 
@@ -229,128 +253,221 @@ static int32_t gpmm_jacobi(gingr_ctx* ctx, int M, int n, double* d_A, int* d_fla
   return GINGR_OK;
 }
 
-extern "C" {
+namespace {
 
-int32_t gingr_gpmm_gaussian_mixture(gingr_ctx* ctx, int32_t M, const double* ref_pts, const int32_t* tri, int32_t T,
-                                    int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol,
-                                    int32_t max_rank, gingr_model** out, int32_t* rank_out) {
+// One scalar pivoted Cholesky of an M x M block of K, run in batches of steps.  Its host history as of the last batch:
+// htrace[k] = residual trace before step k, hdpiv[k] / hpiv[k] = pivot value / point of step k, for k <= steps done.
+struct GpmmBlock {
+  int kind = GPMM_PLAIN;
+  int ncoord = 0;   // coordinates d of the 3M x 3M factor (rows 3 i + d) whose columns come from this block
+  int kcap = 0;     // scalar columns it may compute
+  int k = 0;        // scalar steps done
+  int kalloc = 0;   // columns allocated in Ls
+  DevBuf<double> d, Ls, dpiv, trace;
+  DevBuf<int> pivots;
+  DevBuf<uint8_t> done;
+  std::vector<double> htrace, hdpiv;
+  std::vector<int> hpiv;
+};
+
+using GpmmInitFn = void (*)(int, GaussKernelDev, const double*, double*, uint8_t*);
+using GpmmColumnFn = void (*)(int, int, GaussKernelDev, const double*, const int*, const double*, double*, double*, uint8_t*);
+
+void gpmm_kernels_of(int kind, GpmmInitFn* init, GpmmColumnFn* column) {
+  *init = kind == GPMM_MINUS ? gpmm_init_diag_kernel<GPMM_MINUS> : kind == GPMM_PLUS ? gpmm_init_diag_kernel<GPMM_PLUS>
+                                                                                     : gpmm_init_diag_kernel<GPMM_PLAIN>;
+  *column = kind == GPMM_MINUS ? gpmm_column_kernel<GPMM_MINUS> : kind == GPMM_PLUS ? gpmm_column_kernel<GPMM_PLUS>
+                                                                                     : gpmm_column_kernel<GPMM_PLAIN>;
+}
+
+int32_t gpmm_block_init(gingr_ctx* ctx, int M, int kind, int ncoord, int kcap, const GaussKernelDev& kp, const double* pts,
+                        GpmmBlock& b) {
+  b.kind = kind; b.ncoord = ncoord; b.kcap = kcap;
+  // the factor grows in chunks of columns so that a small rank does not allocate M x kcap
+  b.kalloc = std::min(kcap, 256);
+  GINGR_CUDA_TRY(ctx, b.d.alloc(M));
+  GINGR_CUDA_TRY(ctx, b.done.alloc(M));
+  GINGR_CUDA_TRY(ctx, b.Ls.alloc((size_t)b.kalloc * M));
+  GINGR_CUDA_TRY(ctx, b.pivots.alloc(kcap + 1));
+  GINGR_CUDA_TRY(ctx, b.dpiv.alloc(kcap + 1));
+  GINGR_CUDA_TRY(ctx, b.trace.alloc(kcap + 2));
+  GpmmInitFn init;
+  GpmmColumnFn column;
+  gpmm_kernels_of(kind, &init, &column);
+  init<<<ceil_div(M, 256), 256, 0, ctx->stream>>>(M, kp, pts, b.d.p, b.done.p);
+  GINGR_LAUNCHED(ctx);
+  return GINGR_OK;
+}
+
+// the block's next batch of steps (at most 32, never past kcap), then the pivot and trace of the step after it; the
+// history is copied back
+int32_t gpmm_block_batch(gingr_ctx* ctx, int M, int nb, const GaussKernelDev& kp, const double* pts, double* pmax, int* pidx,
+                         double* psum, GpmmBlock& b) {
+  cudaStream_t st = ctx->stream;
+  const int batch = std::min(32, b.kcap - b.k);
+  if (b.k + batch > b.kalloc) {   // grow the factor
+    const int knew = std::min(b.kcap, std::max(b.kalloc * 2, b.k + batch));
+    DevBuf<double> bigger;
+    GINGR_CUDA_TRY(ctx, bigger.alloc((size_t)knew * M));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(bigger.p, b.Ls.p, sizeof(double) * (size_t)b.k * M, cudaMemcpyDeviceToDevice, st));
+    GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    b.Ls = std::move(bigger);
+    b.kalloc = knew;
+  }
+  GpmmInitFn init;
+  GpmmColumnFn column;
+  gpmm_kernels_of(b.kind, &init, &column);
+  for (int s = 0; s < batch; ++s) {
+    const int k = b.k + s;
+    gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, b.d.p, b.done.p, pmax, pidx, psum);
+    gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, k, pmax, pidx, psum, b.pivots.p, b.dpiv.p, b.trace.p);
+    column<<<ceil_div(M, 256), 256, sizeof(double) * (size_t)std::max(k, 1), st>>>(M, k, kp, pts, b.pivots.p, b.dpiv.p, b.Ls.p,
+                                                                                  b.d.p, b.done.p);
+    ctx->launches += 3;
+  }
+  b.k += batch;
+  gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, b.d.p, b.done.p, pmax, pidx, psum);
+  gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, b.k, pmax, pidx, psum, b.pivots.p, b.dpiv.p, b.trace.p);
+  ctx->launches += 2;
+  b.htrace.resize(b.k + 1);
+  b.hdpiv.resize(b.k + 1);
+  b.hpiv.resize(b.k + 1);
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(b.htrace.data(), b.trace.p, sizeof(double) * (b.k + 1), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(b.hdpiv.data(), b.dpiv.p, sizeof(double) * (b.k + 1), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(b.hpiv.data(), b.pivots.p, sizeof(int) * (b.k + 1), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  GINGR_CUDA_TRY(ctx, cudaGetLastError());
+  return GINGR_OK;
+}
+
+// scalismo's approximateGPCholesky for a kernel that is diagonal in the coordinate index, with coordinate d taking the
+// scalar block blk[g[d]] (rows 3 i + d of the 3M x 3M matrix).  The 3M x 3M algorithm picks the first maximal residual
+// diagonal; a pivot in one coordinate leaves the others' residuals untouched and each block's pivot values never increase,
+// so its column sequence is the merge of the blocks' scalar sequences: at each step the coordinate whose next pivot value
+// is largest, ties to the lowest index 3 i + d.  Coordinates that share a block are at most one scalar step apart (on a
+// tie the lagging one's pivot point has the lower index), which gives the residual trace before a step as, per block,
+// n T(k) - c (T(k) - T(k + 1)) with k the lagging step and c the coordinates one step ahead.  The loop stops where the
+// reference's does -- trace <= relTol * trace(K), or max_rank columns -- or where a block would need a column past kcap.
+int32_t gpmm_build(gingr_ctx* ctx, const char* fn, bool symmetric, int32_t M, const double* ref_pts, const int32_t* tri,
+                   int32_t T, int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol, int32_t max_rank,
+                   gingr_model** out, int32_t* rank_out) {
   if (!ctx || !ref_pts || !out || M <= 0 || T < 0 || (T > 0 && !tri) || n_kernels <= 0 || n_kernels > 8 || !sigma || !scaling ||
       !(rel_tol >= 0.0) || max_rank < 0)
-    return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_gpmm_gaussian_mixture: bad argument (1..8 kernels, relTol >= 0)");
-  if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_gpmm_gaussian_mixture: single-GPU entry point (build before sharding)");
+    return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": bad argument (1..8 kernels, relTol >= 0)").c_str());
+  if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, (std::string(fn) + ": single-GPU entry point (build before sharding)").c_str());
   GaussKernelDev kp;
   kp.n = n_kernels;
   for (int q = 0; q < n_kernels; ++q) {
-    if (!(sigma[q] > 0.0) || !(scaling[q] > 0.0)) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_gpmm_gaussian_mixture: sigma and scaling must be positive");
+    if (!(sigma[q] > 0.0) || !(scaling[q] > 0.0)) return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": sigma and scaling must be positive").c_str());
     kp.inv_sigma2[q] = 1.0 / (sigma[q] * sigma[q]);
     kp.scaling[q] = scaling[q];
   }
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const long long full_cap = max_rank > 0 ? std::min<long long>(max_rank, 3LL * M) : 3LL * M;
-  // scalar columns that may be needed (6000: the previous columns' pivot row is staged in 48 KB of shared memory)
-  const int kcap = (int)std::min<long long>(std::min<long long>((full_cap + 2) / 3, M), 6000);
+  const int nblk = symmetric ? 2 : 1;
+  const int g[3] = {0, symmetric ? 1 : 0, symmetric ? 1 : 0};
   const int nb = std::min(128, ceil_div(M, 256));
   std::unique_ptr<gingr_model> m;
   int r = 0;
-  {   // the factor and its scratch are freed before the regression constants are built
-    DevBuf<double> pts, d, Ls, Lt, pmax, psum, dpiv, trace, norm2a, norm2b;
-    DevBuf<int> pidx, pivots, flag;
-    DevBuf<uint8_t> done;
-    DevBuf<GpmmColumn> dcols;
-    // the factor grows in chunks of columns so that a small rank does not allocate M x kcap
-    int kalloc = std::min(kcap, 256);
+  {   // the factors and their scratch are freed before the regression constants are built
+    DevBuf<double> pts, pmax, psum;
+    DevBuf<int> pidx, flag;
+    GpmmBlock blk[2];
     GINGR_CUDA_TRY(ctx, pts.alloc((size_t)3 * M));
-    GINGR_CUDA_TRY(ctx, d.alloc(M));
-    GINGR_CUDA_TRY(ctx, done.alloc(M));
-    GINGR_CUDA_TRY(ctx, Ls.alloc((size_t)kalloc * M));
     GINGR_CUDA_TRY(ctx, pmax.alloc(nb));
     GINGR_CUDA_TRY(ctx, psum.alloc(nb));
     GINGR_CUDA_TRY(ctx, pidx.alloc(nb));
-    GINGR_CUDA_TRY(ctx, pivots.alloc(kcap + 1));
-    GINGR_CUDA_TRY(ctx, dpiv.alloc(kcap + 1));
-    GINGR_CUDA_TRY(ctx, trace.alloc(kcap + 2));
     GINGR_CUDA_TRY(ctx, flag.alloc(4));
     GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(pts.p, ref_pts, sizeof(double) * 3 * (size_t)M, cudaMemcpyHostToDevice, st));
-    gpmm_init_diag_kernel<<<ceil_div(M, 256), 256, 0, st>>>(M, kp, d.p, done.p);
-    GINGR_LAUNCHED(ctx);
-    // ---- pivoted Cholesky: batches of steps, the trace history decides where the reference's loop would have stopped
-    std::vector<double> htrace;
-    int k = 0;            // scalar steps done
-    int rank = -1;        // full rank 3 kk + c once known
+    for (int b = 0; b < nblk; ++b) {
+      const int ncoord = symmetric ? (b == 0 ? 1 : 2) : 3;
+      const int kind = symmetric ? (b == 0 ? GPMM_MINUS : GPMM_PLUS) : GPMM_PLAIN;
+      // scalar columns that may be needed (6000: the previous columns' pivot row is staged in 48 KB of shared memory)
+      const int kcap = (int)std::min<long long>(std::min<long long>((full_cap + ncoord - 1) / ncoord, M), 6000);
+      GINGR_TRY(gpmm_block_init(ctx, M, kind, ncoord, kcap, kp, pts.p, blk[b]));
+    }
+    for (int b = 0; b < nblk; ++b) GINGR_TRY(gpmm_block_batch(ctx, M, nb, kp, pts.p, pmax.p, pidx.p, psum.p, blk[b]));
+    // ---- the merge, batch by batch: a block runs its next batch when the merged sequence takes its first column not yet computed
     double tol = 0.0;
-    while (rank < 0) {
-      const int batch = std::min(32, kcap - k);
-      if (k + batch > kalloc) {   // grow the factor
-        const int knew = std::min(kcap, std::max(kalloc * 2, k + batch));
-        DevBuf<double> bigger;
-        GINGR_CUDA_TRY(ctx, bigger.alloc((size_t)knew * M));
-        GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(bigger.p, Ls.p, sizeof(double) * (size_t)k * M, cudaMemcpyDeviceToDevice, st));
-        GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-        Ls = std::move(bigger);
-        kalloc = knew;
+    for (int b = 0; b < nblk; ++b) tol += rel_tol * blk[b].ncoord * blk[b].htrace[0];
+    int kd[3] = {0, 0, 0};   // scalar columns coordinate d has taken
+    long long cols = 0;
+    for (;;) {
+      if (cols >= full_cap) break;
+      double tr = 0.0;
+      for (int b = 0; b < nblk; ++b) {
+        int klag = M, ahead = 0;
+        for (int dd = 0; dd < 3; ++dd)
+          if (g[dd] == b) klag = std::min(klag, kd[dd]);
+        for (int dd = 0; dd < 3; ++dd) ahead += g[dd] == b && kd[dd] > klag;
+        const std::vector<double>& h = blk[b].htrace;
+        tr += ahead ? blk[b].ncoord * h[klag] - ahead * (h[klag] - h[klag + 1]) : blk[b].ncoord * h[klag];
       }
-      for (int s = 0; s < batch; ++s) {
-        gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, d.p, done.p, pmax.p, pidx.p, psum.p);
-        gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, k + s, pmax.p, pidx.p, psum.p, pivots.p, dpiv.p, trace.p);
-        gpmm_column_kernel<<<ceil_div(M, 256), 256, sizeof(double) * (size_t)std::max(k + s, 1), st>>>(M, k + s, kp, pts.p, pivots.p,
-                                                                                                      dpiv.p, Ls.p, d.p, done.p);
-        ctx->launches += 3;
+      if (!(tr > tol)) break;
+      int dn = -1;
+      for (int dd = 0; dd < 3; ++dd) {
+        if (kd[dd] >= M) continue;   // every point of this coordinate is a pivot
+        if (dn < 0) { dn = dd; continue; }
+        const GpmmBlock &a = blk[g[dd]], &c = blk[g[dn]];
+        const double va = a.hdpiv[kd[dd]], vc = c.hdpiv[kd[dn]];
+        if (va > vc || (va == vc && 3LL * a.hpiv[kd[dd]] + dd < 3LL * c.hpiv[kd[dn]] + dn)) dn = dd;
       }
-      k += batch;
-      // T(k) after the batch
-      gpmm_argmax_partial_kernel<<<nb, 256, 0, st>>>(M, d.p, done.p, pmax.p, pidx.p, psum.p);
-      gpmm_argmax_final_kernel<<<1, 32, 0, st>>>(nb, k, pmax.p, pidx.p, psum.p, pivots.p, dpiv.p, trace.p);
-      ctx->launches += 2;
-      htrace.resize(k + 1);
-      GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(htrace.data(), trace.p, sizeof(double) * (k + 1), cudaMemcpyDeviceToHost, st));
-      GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
-      GINGR_CUDA_TRY(ctx, cudaGetLastError());
-      tol = rel_tol * 3.0 * htrace[0];
-      // the reference's loop: while (cols < n && trace > tolerance) add a column
-      for (int kk = 0; kk < k && rank < 0; ++kk)
-        for (int c = 0; c < 3; ++c) {
-          const double tr_before = 3.0 * htrace[kk] - c * (htrace[kk] - htrace[kk + 1]);
-          const long long cols = 3LL * kk + c;
-          if (!(tr_before > tol) || cols >= full_cap) { rank = (int)cols; break; }
-        }
-      if (rank < 0 && (k >= kcap || !(3.0 * htrace[k] > tol))) rank = (int)std::min<long long>(3LL * k, full_cap);
-      if (rank < 0 && (long long)3 * k >= full_cap) rank = (int)full_cap;
+      if (dn < 0) break;
+      GpmmBlock& b = blk[g[dn]];
+      if (kd[dn] >= b.k) {
+        if (b.k >= b.kcap) break;
+        GINGR_TRY(gpmm_block_batch(ctx, M, nb, kp, pts.p, pmax.p, pidx.p, psum.p, b));
+      }
+      ++kd[dn];
+      ++cols;
     }
-    if (rank <= 0) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_gpmm_gaussian_mixture: the tolerance leaves an empty model");
-    // dims < c use k1 scalar columns, dims >= c use k1 - 1 (c == 0: all dims use rank / 3)
-    const int cpart = rank % 3;
-    const int k_hi = (rank + 2) / 3, k_lo = rank / 3;
-    // ---- KL basis: one-sided Jacobi on the factor (a second, truncated copy when the last triple is incomplete)
-    std::vector<double> n_hi, n_lo;
-    int sweeps = 0;
-    GINGR_CUDA_TRY(ctx, norm2a.alloc(std::max(k_hi, 1)));
-    GINGR_CUDA_TRY(ctx, norm2b.alloc(std::max(k_lo, 1)));
-    if (cpart != 0 && k_lo > 0) {
-      GINGR_CUDA_TRY(ctx, Lt.alloc((size_t)k_lo * M));
-      GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(Lt.p, Ls.p, sizeof(double) * (size_t)k_lo * M, cudaMemcpyDeviceToDevice, st));
+    const int rank = (int)cols;
+    if (rank <= 0) return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": the tolerance leaves an empty model").c_str());
+    // ---- KL basis: one-sided Jacobi on each block's factor; where the block's coordinates took different column counts
+    // the lower count gets a truncated copy, rotated on its own
+    DevBuf<double> Lt[2], norm2[3];
+    std::vector<double> n2[3];
+    const double* setA[3] = {nullptr, nullptr, nullptr};
+    int set_of[3] = {0, 0, 0};
+    int nset = 0;
+    for (int b = 0; b < nblk; ++b) {
+      int hi = 0, lo = M;
+      for (int dd = 0; dd < 3; ++dd)
+        if (g[dd] == b) { hi = std::max(hi, kd[dd]); lo = std::min(lo, kd[dd]); }
+      const int shi = nset++;
+      const int slo = lo < hi && lo > 0 ? nset++ : shi;
+      for (int dd = 0; dd < 3; ++dd)
+        if (g[dd] == b) set_of[dd] = kd[dd] == hi ? shi : slo;
+      GINGR_CUDA_TRY(ctx, norm2[shi].alloc(std::max(hi, 1)));
+      setA[shi] = blk[b].Ls.p;
+      if (slo != shi) {
+        GINGR_CUDA_TRY(ctx, norm2[slo].alloc(lo));
+        GINGR_CUDA_TRY(ctx, Lt[b].alloc((size_t)lo * M));
+        GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(Lt[b].p, blk[b].Ls.p, sizeof(double) * (size_t)lo * M, cudaMemcpyDeviceToDevice, st));
+        setA[slo] = Lt[b].p;
+      }
+      if (hi > 0) GINGR_TRY(gpmm_jacobi(ctx, M, hi, blk[b].Ls.p, flag.p, norm2[shi].p, &n2[shi], nullptr));
+      if (slo != shi) GINGR_TRY(gpmm_jacobi(ctx, M, lo, Lt[b].p, flag.p, norm2[slo].p, &n2[slo], nullptr));
     }
-    GINGR_TRY(gpmm_jacobi(ctx, M, k_hi, Ls.p, flag.p, norm2a.p, &n_hi, &sweeps));
-    if (cpart != 0 && k_lo > 0) GINGR_TRY(gpmm_jacobi(ctx, M, k_lo, Lt.p, flag.p, norm2b.p, &n_lo, nullptr));
+    for (int q = nset; q < 3; ++q) setA[q] = setA[0];
     // ---- columns of the model, sorted by variance (descending; ties: dimension, then scalar column)
-    std::vector<GpmmColumn> cols;
+    std::vector<GpmmColumn> cols_v;
     std::vector<double> lam;
-    for (int dd = 0; dd < 3; ++dd) {
-      const bool hi = cpart == 0 || dd < cpart;
-      const int kd = hi ? k_hi : k_lo;
-      for (int j = 0; j < kd; ++j) {
-        cols.push_back(GpmmColumn{hi ? 0 : 1, j, dd});
-        lam.push_back(hi ? n_hi[j] : n_lo[j]);
+    for (int dd = 0; dd < 3; ++dd)
+      for (int j = 0; j < kd[dd]; ++j) {
+        cols_v.push_back(GpmmColumn{set_of[dd], j, dd});
+        lam.push_back(n2[set_of[dd]][j]);
       }
-    }
-    std::vector<int> order(cols.size());
+    std::vector<int> order(cols_v.size());
     for (size_t q = 0; q < order.size(); ++q) order[q] = (int)q;
     std::stable_sort(order.begin(), order.end(), [&](int x, int y) { return lam[x] > lam[y]; });
-    r = (int)cols.size();
+    r = (int)cols_v.size();
     std::vector<GpmmColumn> scols(r);
     std::vector<double> var(r);
-    for (int q = 0; q < r; ++q) { scols[q] = cols[order[q]]; var[q] = lam[order[q]]; }
+    for (int q = 0; q < r; ++q) { scols[q] = cols_v[order[q]]; var[q] = lam[order[q]]; }
     // ---- the model handle
+    DevBuf<GpmmColumn> dcols;
     m.reset(new gingr_model());
     m->ctx = ctx;
     m->M = M; m->r = r; m->rp = (r + 7) / 8 * 8; m->m0 = 0; m->Ml = M;
@@ -366,18 +483,37 @@ int32_t gingr_gpmm_gaussian_mixture(gingr_ctx* ctx, int32_t M, const double* ref
     GINGR_CUDA_TRY(ctx, cudaMemsetAsync(m->phi.p, 0, sizeof(double) * (size_t)3 * M * m->rp, st));
     GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(m->sqrt_lambda.p, sl.data(), sizeof(double) * m->rp, cudaMemcpyHostToDevice, st));
     GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(dcols.p, scols.data(), sizeof(GpmmColumn) * r, cudaMemcpyHostToDevice, st));
-    gpmm_assemble_kernel<<<dim3(ceil_div(M, 256), r), 256, 0, st>>>(M, r, m->rp, dcols.p, Ls.p, norm2a.p, Lt.p ? Lt.p : Ls.p,
-                                                                    norm2b.p, m->phi.p);
+    const double* setn[3];
+    for (int q = 0; q < 3; ++q) setn[q] = q < nset ? norm2[q].p : norm2[0].p;
+    gpmm_assemble_kernel<<<dim3(ceil_div(M, 256), r), 256, 0, st>>>(M, r, m->rp, dcols.p, setA[0], setn[0], setA[1], setn[1],
+                                                                    setA[2], setn[2], m->phi.p);
     GINGR_LAUNCHED(ctx);
     GINGR_CUDA_TRY(ctx, cudaGetLastError());
     GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));   // sl / scols are host vectors
-    (void)sweeps;
   }
   GINGR_TRY(model_upload_topology(ctx, m.get(), tri, T));
   GINGR_TRY(model_build_constants(ctx, m.get()));
   *out = m.release();
   if (rank_out) *rank_out = r;
   return GINGR_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int32_t gingr_gpmm_gaussian_mixture(gingr_ctx* ctx, int32_t M, const double* ref_pts, const int32_t* tri, int32_t T,
+                                    int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol,
+                                    int32_t max_rank, gingr_model** out, int32_t* rank_out) {
+  return gpmm_build(ctx, "gingr_gpmm_gaussian_mixture", false, M, ref_pts, tri, T, n_kernels, sigma, scaling, rel_tol, max_rank,
+                    out, rank_out);
+}
+
+int32_t gingr_gpmm_gaussian_symmetric(gingr_ctx* ctx, int32_t M, const double* ref_pts, const int32_t* tri, int32_t T,
+                                      int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol,
+                                      int32_t max_rank, gingr_model** out, int32_t* rank_out) {
+  return gpmm_build(ctx, "gingr_gpmm_gaussian_symmetric", true, M, ref_pts, tri, T, n_kernels, sigma, scaling, rel_tol, max_rank,
+                    out, rank_out);
 }
 
 // The model as scalismo stores it (SURVEY.md A1): meanVector [3M], basisMatrix column-major [3M x r] (leading dimension

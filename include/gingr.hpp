@@ -229,6 +229,20 @@ class Model {
     m.r_ = rank;
     return m;
   }
+  // the mirror-symmetric Gaussian (mixture) kernel about the plane x = 0 (gingr_gpmm_gaussian_symmetric), on the device;
+  // the caller centres the template on that plane
+  static Model gaussianSymmetric(const Context& ctx, int M, const double* ref, const int32_t* tri, int T,
+                                 const std::vector<double>& sigma, const std::vector<double>& scaling,
+                                 double relativeTolerance = 0.01, int maxRank = 0) {
+    if (sigma.size() != scaling.size() || sigma.empty()) throw Error(GINGR_ERR_ARG, "one scaling per sigma");
+    Model m(ctx);
+    int32_t rank = 0;
+    ctx.check(gingr_gpmm_gaussian_symmetric(ctx.handle(), M, ref, tri, T, static_cast<int32_t>(sigma.size()), sigma.data(),
+                                            scaling.data(), relativeTolerance, maxRank, &m.h_, &rank));
+    m.M_ = M;
+    m.r_ = rank;
+    return m;
+  }
   // model.newReference(newRef, NearestNeighborInterpolator()), registration/SimpleRegistrator.scala:90-92
   Model newReference(int M2, const double* ref, const int32_t* tri = nullptr, int T = 0) const {
     Model m(*ctx_);

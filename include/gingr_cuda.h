@@ -154,6 +154,17 @@ GINGR_API int32_t gingr_gpmm_gaussian_mixture(gingr_ctx* ctx, int32_t M, const d
                                               const int32_t* tri /*[3T]*/, int32_t T, int32_t n_kernels,
                                               const double* sigma /*[n]*/, const double* scaling /*[n]*/, double rel_tol,
                                               int32_t max_rank, gingr_model** out, int32_t* rank_out);
+/* The mirror-symmetric Gaussian (mixture) model: scalismo's symmetrised kernel about the plane x = 0 (the tutorial's
+ * "XmirroredKernel"), with S = diag(-1, 1, 1), k the scalar mixture above and k_m(x, y) = k(S x, y):
+ *   K(x, y) = DiagonalKernel(k, 3) + DiagonalKernel(-k_m, k_m, k_m)
+ *           = diag(k(x, y) - k(S x, y),  k(x, y) + k(S x, y),  k(x, y) + k(S x, y)).
+ * Left and right halves of the template deform as mirror images, and points on the plane do not move off it (their
+ * x rows of the basis are exactly zero).  The plane is fixed at x = 0: the caller centres the template on it.
+ * Arguments, validation, stopping rule and outputs are those of gingr_gpmm_gaussian_mixture. */
+GINGR_API int32_t gingr_gpmm_gaussian_symmetric(gingr_ctx* ctx, int32_t M, const double* ref_pts /*[3M]*/,
+                                                const int32_t* tri /*[3T]*/, int32_t T, int32_t n_kernels,
+                                                const double* sigma /*[n]*/, const double* scaling /*[n]*/, double rel_tol,
+                                                int32_t max_rank, gingr_model** out, int32_t* rank_out);
 /* The model as scalismo stores it (SURVEY.md A1): meanVector, basisMatrix column-major with leading dimension ld_basis,
  * variance.  Any output may be NULL (M_out / r_out give the sizes to allocate). */
 GINGR_API int32_t gingr_model_download(gingr_ctx* ctx, const gingr_model* model, int32_t* M_out, int32_t* r_out,

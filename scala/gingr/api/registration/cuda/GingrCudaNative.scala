@@ -88,6 +88,9 @@ object GingrCudaNative {
   // GPMM construction on the device (api/gpmm/GPMMHelper.scala:99-129) and the way back into scalismo's storage
   val gpmmGaussianMixture = fn("gingr_gpmm_gaussian_mixture", JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT,
                                ADDRESS, ADDRESS, JAVA_DOUBLE, JAVA_INT, ADDRESS, ADDRESS)
+  // the mirror-symmetric kernel about x = 0 (scalismo's symmetrised Gaussian kernel), same arguments
+  val gpmmGaussianSymmetric = fn("gingr_gpmm_gaussian_symmetric", JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT,
+                                 ADDRESS, ADDRESS, JAVA_DOUBLE, JAVA_INT, ADDRESS, ADDRESS)
   val modelDownload  = fn("gingr_model_download", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS)
 
   // the remaining entry points of include/gingr_cuda.h (every exported function has a handle here; tests/test_scala_shim.py
