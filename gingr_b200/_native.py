@@ -95,6 +95,7 @@ SIGNATURES = {
     "gingr_model_new_reference": (c_int32, [c_void_p, c_void_p, c_int32, dp, ip, c_int32, vpp]),
     "gingr_gpmm_gaussian_mixture": (c_int32, [c_void_p, c_int32, dp, ip, c_int32, c_int32, dp, dp, c_double, c_int32, vpp, ip]),
     "gingr_gpmm_gaussian_symmetric": (c_int32, [c_void_p, c_int32, dp, ip, c_int32, c_int32, dp, dp, c_double, c_int32, vpp, ip]),
+    "gingr_gpmm_inverse_laplacian": (c_int32, [c_void_p, c_int32, dp, ip, c_int32, c_double, c_double, c_double, c_int32, vpp, ip]),
     "gingr_model_download": (c_int32, [c_void_p, c_void_p, ip, ip, dp, dp, dp, c_int64, dp]),
     "gingr_target_upload": (c_int32, [c_void_p, c_int32, dp, ip, c_int32, vpp]),
     "gingr_target_destroy": (c_int32, [c_void_p]),

@@ -144,6 +144,34 @@ class Model:
         return Model._build_gpmm(ctx, "gingr_gpmm_gaussian_symmetric", ref_points, triangles, sigmas, scalings, relativeTolerance, maxRank)
 
     @staticmethod
+    def inverseLaplacian(ctx: Context, ref_points, triangles, scaling: float, gamma: float, relativeTolerance: float = 0.01,
+                         maxRank: int = 0) -> "Model":
+        """The inverse-Laplacian model (the model chooser's look-up kernel, api/gpmm LaplacianHelper.scala:26-55 with
+        MatrixHelper.pinv :23-26), built on the device: vertices close on the triangle graph move together, vertices merely
+        close in space (fingers, the lips of a jaw) do not.  This project's reading of the kernel: L = D - A, the graph
+        Laplacian of the triangle edges with unit weights; Ks = scaling (L + gamma I)^-1, or scaling pinv(L) for gamma = 0;
+        K = Ks (x) I3; then approximateGPCholesky with the stopping rule of gaussianMixture.  Needs triangles and at most 6000
+        vertices.  The models are nearly full rank (about 0.97-0.99 of 3M at relativeTolerance 0.01); the registrations take
+        a rank of at most 9472, so above about 3200 vertices pass maxRank.  With gamma = 0 the kernel has rank
+        3 (M - #components); at relativeTolerance 0 the factorisation would go on to take noise columns from the
+        rounding-level residual of the null space, so a full-rank gamma = 0 model wants a small positive tolerance (1e-12
+        suffices).  Raises FloatingPointError when L + gamma I is not numerically positive definite."""
+        ref = nat.f64(ref_points).reshape(-1, 3)
+        tri = None if triangles is None else nat.i32(triangles).reshape(-1, 3)
+        h = ctypes.c_void_p()
+        rank = ctypes.c_int32()
+        code = ctx.check(ctx._lib.gingr_gpmm_inverse_laplacian(ctx.handle, ref.shape[0], nat.as_dp(ref), nat.as_ip(tri),
+                                                               0 if tri is None else tri.shape[0], float(scaling), float(gamma),
+                                                               float(relativeTolerance), int(maxRank), ctypes.byref(h),
+                                                               ctypes.byref(rank)))
+        if code == nat.GINGR_MODEL_FLEXIBILITY:
+            raise FloatingPointError("inverseLaplacian: L + gamma I is not numerically positive definite (ModelFlexibilityError)")
+        m = Model.__new__(Model)
+        m.ctx, m.M, m.rank, m.T, m.handle, m.triangles = ctx, ref.shape[0], int(rank.value), tri.shape[0], h, tri
+        m.reference = ref.copy()
+        return m
+
+    @staticmethod
     def _build_gpmm(ctx: Context, entry: str, ref_points, triangles, sigmas, scalings, relativeTolerance, maxRank) -> "Model":
         """A model from one of the device GPMM builders, which share their arguments."""
         ref = nat.f64(ref_points).reshape(-1, 3)
@@ -927,6 +955,19 @@ class GaussSymKernel:
 
 
 @dataclass(frozen=True)
+class InvLapKernel:
+    """The inverse-Laplacian look-up kernel (Model.inverseLaplacian) with its (scaling, gamma).  The name "InvLap", and
+    with it the cache file name <name>_dec-<d>_InvLap_<scaling>_<gamma>.h5.json, are this project's."""
+    scaling: float
+    gamma: float
+    name = "InvLap"
+
+    @property
+    def printpars(self) -> str:
+        return _scala_double(self.scaling) + "_" + _scala_double(self.gamma)
+
+
+@dataclass(frozen=True)
 class GaussMixKernel:
     """simple/SimpleModels.scala:41-44 (AutomaticGaussian)."""
     name = "GaussMix"
@@ -935,9 +976,9 @@ class GaussMixKernel:
 
 class SimpleTriangleModels3D:
     """simple/SimpleModels.scala:54-77 for the Gaussian families (the kernels the demos load: femur Gauss(50, 70), bunny
-    Gauss(20, 40), DemoDatasetLoader.scala:113-114, :146-147) and the mirror-symmetric Gaussian kernel (GaussSymKernel).
-    The Laplacian and dot-product kernels are not on the path SURVEY.md 8 scopes and are refused rather than
-    approximated."""
+    Gauss(20, 40), DemoDatasetLoader.scala:113-114, :146-147), the mirror-symmetric Gaussian kernel (GaussSymKernel) and
+    the inverse-Laplacian look-up kernel (InvLapKernel).  The dot-product kernels are not on the path SURVEY.md 8 scopes
+    and are refused rather than approximated."""
 
     @staticmethod
     def create(ctx: Context, reference_points, triangles, kernelSelect, relativeTolerance: float = 0.01) -> Model:
@@ -947,9 +988,13 @@ class SimpleTriangleModels3D:
         if isinstance(kernelSelect, GaussSymKernel):
             return Model.gaussianSymmetric(ctx, reference_points, triangles, [kernelSelect.sigma], [kernelSelect.scaling],
                                            relativeTolerance)
+        if isinstance(kernelSelect, InvLapKernel):
+            return Model.inverseLaplacian(ctx, reference_points, triangles, kernelSelect.scaling, kernelSelect.gamma,
+                                          relativeTolerance)
         if isinstance(kernelSelect, GaussMixKernel):
             return Model.automaticGaussian(ctx, reference_points, triangles, relativeTolerance)
-        raise NotImplementedError(f"kernel {type(kernelSelect).__name__} is outside the device GPMM builder (Gaussian families and their mirror-symmetric form only)")
+        raise NotImplementedError(f"kernel {type(kernelSelect).__name__} is outside the device GPMM builder (Gaussian families, "
+                                  "their mirror-symmetric form and the inverse Laplacian only)")
 
 
 class SimpleRegistrator:

@@ -12,7 +12,9 @@
 // that is not a multiple of three (tests/test_oracle_gpmm.py proves this against the literal 3M x 3M algorithm).
 // The mirror-symmetric kernel (scalismo's symmetrised kernel about x = 0, gingr_gpmm_gaussian_symmetric) is diagonal
 // too, with two distinct blocks: ks - ks_m for dimension 0 and ks + ks_m for dimensions 1 and 2, ks_m(x, y) = ks(S x, y).
-// Both cases are one loop (gpmm_build): a scalar factorisation per block, merged on the host in the literal order.
+// The inverse-Laplacian kernel (gingr_gpmm_inverse_laplacian) is Ks (x) I3 with Ks a dense M x M matrix computed up
+// front (Laplacian assembly, data-flow Cholesky with the identity riding along, DMMA Gram); its block reads Ks.
+// All cases are one loop (gpmm_build): a scalar factorisation per block, merged on the host in the literal order.
 //   pivoted Cholesky   one column per step: argmax of the residual diagonal (lowest index on ties), the kernel column
 //                      minus the projection on the previous columns, diagonal update; all scalars stay on the device,
 //                      the host looks at the trace history once per batch of steps
@@ -40,12 +42,15 @@ __device__ __forceinline__ double gpmm_kernel(const GaussKernelDev& kp, double d
 
 // The scalar M x M block a factorisation works on: GPMM_PLAIN is ks itself; GPMM_MINUS / GPMM_PLUS are ks(x, y) -/+ ks(S x, y)
 // with the mirror S = diag(-1, 1, 1) about the plane x = 0 (the blocks of the mirror-symmetric kernel, see
-// gingr_gpmm_gaussian_symmetric).
-enum GpmmBlockKind { GPMM_PLAIN = 0, GPMM_MINUS = 1, GPMM_PLUS = 2 };
+// gingr_gpmm_gaussian_symmetric); GPMM_LOOKUP reads a dense symmetric M x M matrix (pitch M) passed in place of the points
+// (the inverse-Laplacian kernel, gingr_gpmm_inverse_laplacian).
+enum GpmmBlockKind { GPMM_PLAIN = 0, GPMM_MINUS = 1, GPMM_PLUS = 2, GPMM_LOOKUP = 3 };
 
 template <int KIND>
-__device__ __forceinline__ double gpmm_entry(const GaussKernelDev& kp, const double* __restrict__ pts, int i, int p) {
-  if constexpr (KIND == GPMM_PLAIN) {
+__device__ __forceinline__ double gpmm_entry(const GaussKernelDev& kp, const double* __restrict__ pts, int M, int i, int p) {
+  if constexpr (KIND == GPMM_LOOKUP) {
+    return pts[(size_t)p * M + i];   // row p = column p: coalesced over i
+  } else if constexpr (KIND == GPMM_PLAIN) {
     return gpmm_kernel(kp, pts[3 * i] - pts[3 * p], pts[3 * i + 1] - pts[3 * p + 1], pts[3 * i + 2] - pts[3 * p + 2]);
   } else {
     const double dy = pts[3 * i + 1] - pts[3 * p + 1], dz = pts[3 * i + 2] - pts[3 * p + 2];
@@ -61,7 +66,7 @@ __global__ void gpmm_init_diag_kernel(int M, GaussKernelDev kp, const double* __
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= M) return;
   if constexpr (KIND == GPMM_PLAIN) d[i] = gpmm_kernel(kp, 0.0, 0.0, 0.0);
-  else d[i] = gpmm_entry<KIND>(kp, pts, i, i);
+  else d[i] = gpmm_entry<KIND>(kp, pts, M, i, i);
   done[i] = 0;
 }
 
@@ -129,7 +134,7 @@ __global__ void __launch_bounds__(256) gpmm_column_kernel(int M, int k, GaussKer
     if (i == p) {
       out = piv;
     } else if (!done[i]) {
-      double v = gpmm_entry<KIND>(kp, pts, i, p);
+      double v = gpmm_entry<KIND>(kp, pts, M, i, p);
       for (int j = 0; j < k; ++j) v -= Ls[(size_t)j * M + i] * lp[j];
       out = v / piv;
       d[i] -= out * out;
@@ -219,6 +224,59 @@ __global__ void gpmm_assemble_kernel(int M, int r, int rp, const GpmmColumn* __r
   phi[((size_t)3 * i + col.d) * rp + c] = A[(size_t)col.j * M + i] / sqrt(nn[col.j]);
 }
 
+// ---- the inverse-Laplacian kernel: the system [L + gamma I (or L + P); I] for the data-flow Cholesky --------------------
+// each edge of each triangle marks A[a][b] = A[b][a] = -1: one value stored, so duplicated edges and the triangle order do
+// not change the result; self-edges of degenerate triangles are skipped
+__global__ void lap_edges_kernel(int T, const int32_t* __restrict__ tri, int ld, double* __restrict__ A) {
+  const int t = blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= T) return;
+  const int v[3] = {tri[3 * t], tri[3 * t + 1], tri[3 * t + 2]};
+  for (int e = 0; e < 3; ++e) {
+    const int a = v[e], b = v[(e + 1) % 3];
+    if (a == b) continue;
+    A[(size_t)a * ld + b] = -1.0;
+    A[(size_t)b * ld + a] = -1.0;
+  }
+}
+
+// row i: the degree (the marks of the row) + gamma on the diagonal; with project, P = sum_c 1_c 1_c^T / |c| added
+// (comp: component of each vertex, inv_size: 1 / |c|); the identity row M + i rides along below the square part
+__global__ void __launch_bounds__(256) lap_rows_kernel(int M, int ld, double gamma, int project, const int* __restrict__ comp,
+                                                       const double* __restrict__ inv_size, double* __restrict__ A) {
+  __shared__ int red[256];
+  const int i = blockIdx.x;
+  double* row = A + (size_t)i * ld;
+  int deg = 0;
+  for (int j = threadIdx.x; j < M; j += 256) deg += row[j] != 0.0;
+  red[threadIdx.x] = deg;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  deg = red[0];
+  const int ci = project ? comp[i] : 0;
+  for (int j = threadIdx.x; j < M; j += 256) {
+    double v = j == i ? deg + gamma : row[j];
+    if (project && comp[j] == ci) v += inv_size[ci];
+    row[j] = v;
+  }
+  if (threadIdx.x == 0) A[(size_t)(M + i) * ld + i] = 1.0;
+}
+
+// Ks = s (G - P) from G = A^-1 (pitch ld) into K (pitch M); *bad = 1 for a non-finite entry
+__global__ void lap_scale_kernel(int M, int ld, double s, int project, const int* __restrict__ comp,
+                                 const double* __restrict__ inv_size, const double* __restrict__ G, double* __restrict__ K,
+                                 int* __restrict__ bad) {
+  const int j = blockIdx.x * blockDim.x + threadIdx.x, i = blockIdx.y;
+  if (j >= M) return;
+  double g = G[(size_t)i * ld + j];
+  if (project && comp[i] == comp[j]) g -= inv_size[comp[i]];
+  const double v = s * g;
+  K[(size_t)i * M + j] = v;
+  if (!isfinite(v)) *bad = 1;
+}
+
 }  // namespace gingr
 
 using namespace gingr;
@@ -275,9 +333,9 @@ using GpmmColumnFn = void (*)(int, int, GaussKernelDev, const double*, const int
 
 void gpmm_kernels_of(int kind, GpmmInitFn* init, GpmmColumnFn* column) {
   *init = kind == GPMM_MINUS ? gpmm_init_diag_kernel<GPMM_MINUS> : kind == GPMM_PLUS ? gpmm_init_diag_kernel<GPMM_PLUS>
-                                                                                     : gpmm_init_diag_kernel<GPMM_PLAIN>;
+         : kind == GPMM_LOOKUP ? gpmm_init_diag_kernel<GPMM_LOOKUP> : gpmm_init_diag_kernel<GPMM_PLAIN>;
   *column = kind == GPMM_MINUS ? gpmm_column_kernel<GPMM_MINUS> : kind == GPMM_PLUS ? gpmm_column_kernel<GPMM_PLUS>
-                                                                                     : gpmm_column_kernel<GPMM_PLAIN>;
+           : kind == GPMM_LOOKUP ? gpmm_column_kernel<GPMM_LOOKUP> : gpmm_column_kernel<GPMM_PLAIN>;
 }
 
 int32_t gpmm_block_init(gingr_ctx* ctx, int M, int kind, int ncoord, int kcap, const GaussKernelDev& kp, const double* pts,
@@ -348,20 +406,11 @@ int32_t gpmm_block_batch(gingr_ctx* ctx, int M, int nb, const GaussKernelDev& kp
 // tie the lagging one's pivot point has the lower index), which gives the residual trace before a step as, per block,
 // n T(k) - c (T(k) - T(k + 1)) with k the lagging step and c the coordinates one step ahead.  The loop stops where the
 // reference's does -- trace <= relTol * trace(K), or max_rank columns -- or where a block would need a column past kcap.
+// The arguments are checked by the callers.  lookup (device, M x M, pitch M) non-null: the one block is that matrix
+// (GPMM_LOOKUP) instead of the Gaussian kp.
 int32_t gpmm_build(gingr_ctx* ctx, const char* fn, bool symmetric, int32_t M, const double* ref_pts, const int32_t* tri,
-                   int32_t T, int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol, int32_t max_rank,
+                   int32_t T, const GaussKernelDev& kp, const double* lookup, double rel_tol, int32_t max_rank,
                    gingr_model** out, int32_t* rank_out) {
-  if (!ctx || !ref_pts || !out || M <= 0 || T < 0 || (T > 0 && !tri) || n_kernels <= 0 || n_kernels > 8 || !sigma || !scaling ||
-      !(rel_tol >= 0.0) || max_rank < 0)
-    return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": bad argument (1..8 kernels, relTol >= 0)").c_str());
-  if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, (std::string(fn) + ": single-GPU entry point (build before sharding)").c_str());
-  GaussKernelDev kp;
-  kp.n = n_kernels;
-  for (int q = 0; q < n_kernels; ++q) {
-    if (!(sigma[q] > 0.0) || !(scaling[q] > 0.0)) return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": sigma and scaling must be positive").c_str());
-    kp.inv_sigma2[q] = 1.0 / (sigma[q] * sigma[q]);
-    kp.scaling[q] = scaling[q];
-  }
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const long long full_cap = max_rank > 0 ? std::min<long long>(max_rank, 3LL * M) : 3LL * M;
@@ -380,14 +429,15 @@ int32_t gpmm_build(gingr_ctx* ctx, const char* fn, bool symmetric, int32_t M, co
     GINGR_CUDA_TRY(ctx, pidx.alloc(nb));
     GINGR_CUDA_TRY(ctx, flag.alloc(4));
     GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(pts.p, ref_pts, sizeof(double) * 3 * (size_t)M, cudaMemcpyHostToDevice, st));
+    const double* src = lookup ? lookup : pts.p;   // what the blocks' entries are computed from
     for (int b = 0; b < nblk; ++b) {
       const int ncoord = symmetric ? (b == 0 ? 1 : 2) : 3;
-      const int kind = symmetric ? (b == 0 ? GPMM_MINUS : GPMM_PLUS) : GPMM_PLAIN;
+      const int kind = symmetric ? (b == 0 ? GPMM_MINUS : GPMM_PLUS) : lookup ? GPMM_LOOKUP : GPMM_PLAIN;
       // scalar columns that may be needed (6000: the previous columns' pivot row is staged in 48 KB of shared memory)
       const int kcap = (int)std::min<long long>(std::min<long long>((full_cap + ncoord - 1) / ncoord, M), 6000);
-      GINGR_TRY(gpmm_block_init(ctx, M, kind, ncoord, kcap, kp, pts.p, blk[b]));
+      GINGR_TRY(gpmm_block_init(ctx, M, kind, ncoord, kcap, kp, src, blk[b]));
     }
-    for (int b = 0; b < nblk; ++b) GINGR_TRY(gpmm_block_batch(ctx, M, nb, kp, pts.p, pmax.p, pidx.p, psum.p, blk[b]));
+    for (int b = 0; b < nblk; ++b) GINGR_TRY(gpmm_block_batch(ctx, M, nb, kp, src, pmax.p, pidx.p, psum.p, blk[b]));
     // ---- the merge, batch by batch: a block runs its next batch when the merged sequence takes its first column not yet computed
     double tol = 0.0;
     for (int b = 0; b < nblk; ++b) tol += rel_tol * blk[b].ncoord * blk[b].htrace[0];
@@ -417,7 +467,7 @@ int32_t gpmm_build(gingr_ctx* ctx, const char* fn, bool symmetric, int32_t M, co
       GpmmBlock& b = blk[g[dn]];
       if (kd[dn] >= b.k) {
         if (b.k >= b.kcap) break;
-        GINGR_TRY(gpmm_block_batch(ctx, M, nb, kp, pts.p, pmax.p, pidx.p, psum.p, b));
+        GINGR_TRY(gpmm_block_batch(ctx, M, nb, kp, src, pmax.p, pidx.p, psum.p, b));
       }
       ++kd[dn];
       ++cols;
@@ -498,6 +548,104 @@ int32_t gpmm_build(gingr_ctx* ctx, const char* fn, bool symmetric, int32_t M, co
   return GINGR_OK;
 }
 
+int32_t gpmm_build_gaussian(gingr_ctx* ctx, const char* fn, bool symmetric, int32_t M, const double* ref_pts, const int32_t* tri,
+                            int32_t T, int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol,
+                            int32_t max_rank, gingr_model** out, int32_t* rank_out) {
+  if (!ctx || !ref_pts || !out || M <= 0 || T < 0 || (T > 0 && !tri) || n_kernels <= 0 || n_kernels > 8 || !sigma || !scaling ||
+      !(rel_tol >= 0.0) || max_rank < 0)
+    return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": bad argument (1..8 kernels, relTol >= 0)").c_str());
+  if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, (std::string(fn) + ": single-GPU entry point (build before sharding)").c_str());
+  GaussKernelDev kp;
+  kp.n = n_kernels;
+  for (int q = 0; q < n_kernels; ++q) {
+    if (!(sigma[q] > 0.0) || !(scaling[q] > 0.0)) return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": sigma and scaling must be positive").c_str());
+    kp.inv_sigma2[q] = 1.0 / (sigma[q] * sigma[q]);
+    kp.scaling[q] = scaling[q];
+  }
+  return gpmm_build(ctx, fn, symmetric, M, ref_pts, tri, T, kp, nullptr, rel_tol, max_rank, out, rank_out);
+}
+
+// The largest template of the inverse-Laplacian builder: its models are nearly full rank, and the pivoted Cholesky computes
+// at most 6000 scalar columns (gpmm_build's kcap).
+constexpr int LAP_MAX_M = 6000;
+
+// Ks = scaling (L + gamma I)^-1, or for gamma = 0 scaling L^+ = scaling ((L + P)^-1 - P), into K (device, M x M, pitch M).
+// The components behind P come from a union-find over the triangles on the host (O(T)); a vertex in no triangle is a
+// component of its own.  The system [A; I] is factorised by the data-flow Cholesky, the identity rows come out as
+// Y = L_A^-T, and A^-1 = Y Y^T is the DMMA Gram of Y^T.  *failed: A not numerically positive definite, or Ks not finite.
+int32_t laplacian_inverse(gingr_ctx* ctx, int M, const int32_t* tri, int T, double scaling, double gamma, DevBuf<double>& K,
+                          bool* failed) {
+  cudaStream_t st = ctx->stream;
+  const bool project = gamma == 0.0;
+  std::vector<int> comp(M, 0);
+  std::vector<double> inv_size(1, 0.0);
+  if (project) {
+    std::vector<int> parent(M);
+    for (int i = 0; i < M; ++i) parent[i] = i;
+    auto find = [&](int x) {
+      while (parent[x] != x) x = parent[x] = parent[parent[x]];
+      return x;
+    };
+    for (int t = 0; t < T; ++t)
+      for (int e = 0; e < 3; ++e) {
+        const int a = find(tri[3 * t + e]), b = find(tri[3 * t + (e + 1) % 3]);
+        if (a != b) parent[std::max(a, b)] = std::min(a, b);
+      }
+    std::vector<int> label(M, -1), size;
+    for (int i = 0; i < M; ++i) {
+      const int root = find(i);
+      if (label[root] < 0) { label[root] = (int)size.size(); size.push_back(0); }
+      comp[i] = label[root];
+      ++size[comp[i]];
+    }
+    inv_size.resize(size.size());
+    for (size_t c = 0; c < size.size(); ++c) inv_size[c] = 1.0 / size[c];
+  }
+  const int ld = (M + 7) / 8 * 8;   // even pitch, 16-byte rows (chol_df), rp of the Gram
+  DevBuf<double> G;
+  DevBuf<int32_t> dtri, dcomp;
+  DevBuf<double> dinv;
+  DevBuf<int> info;
+  GINGR_CUDA_TRY(ctx, dtri.alloc((size_t)3 * T));
+  GINGR_CUDA_TRY(ctx, dcomp.alloc(M));
+  GINGR_CUDA_TRY(ctx, dinv.alloc(inv_size.size()));
+  GINGR_CUDA_TRY(ctx, info.alloc(4));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(dtri.p, tri, sizeof(int32_t) * 3 * (size_t)T, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(dcomp.p, comp.data(), sizeof(int) * (size_t)M, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(dinv.p, inv_size.data(), sizeof(double) * inv_size.size(), cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(info.p, 0, sizeof(int) * 4, st));
+  {
+    DevBuf<double> sys, Yt;
+    CholWs cws;
+    GramPlan plan;
+    GINGR_CUDA_TRY(ctx, sys.alloc((size_t)(2 * M + 8) * ld));
+    GINGR_CUDA_TRY(ctx, Yt.alloc((size_t)M * ld));
+    GINGR_CUDA_TRY(ctx, G.alloc((size_t)M * ld));
+    GINGR_TRY(cws.alloc(ctx, M, 2 * M));
+    GINGR_CUDA_TRY(ctx, cudaMemsetAsync(sys.p, 0, sizeof(double) * (size_t)(2 * M + 8) * ld, st));
+    GINGR_CUDA_TRY(ctx, cudaMemsetAsync(Yt.p, 0, sizeof(double) * (size_t)M * ld, st));
+    lap_edges_kernel<<<ceil_div(T, 256), 256, 0, st>>>(T, dtri.p, ld, sys.p);
+    GINGR_LAUNCHED(ctx);
+    lap_rows_kernel<<<M, 256, 0, st>>>(M, ld, gamma, project ? 1 : 0, dcomp.p, dinv.p, sys.p);
+    GINGR_LAUNCHED(ctx);
+    GINGR_TRY(cholesky_df_enqueue(ctx, M, 2 * M, sys.p, ld, info.p, cws));
+    GINGR_TRY(transpose_enqueue(ctx, M, sys.p + (size_t)M * ld, ld, Yt.p, ld));   // Y^T = L_A^-1, lower triangular
+    GINGR_TRY(plan.build(ctx, M, M, ld));
+    GINGR_TRY(gram_partials_enqueue(ctx, plan, Yt.p, nullptr));
+    GINGR_TRY(gram_finish_enqueue(ctx, plan, plan.d_partial.p, nullptr, 0.0, 0, nullptr, nullptr, ld, G.p));
+    GINGR_CUDA_TRY(ctx, K.alloc((size_t)M * M));
+    lap_scale_kernel<<<dim3(ceil_div(M, 256), M), 256, 0, st>>>(M, ld, scaling, project ? 1 : 0, dcomp.p, dinv.p, G.p, K.p,
+                                                                 info.p + 1);
+    GINGR_LAUNCHED(ctx);
+    GINGR_CUDA_TRY(ctx, cudaGetLastError());
+    int h[2] = {0, 0};
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(h, info.p, sizeof(int) * 2, cudaMemcpyDeviceToHost, st));
+    GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));   // also: the host vectors above were copied
+    *failed = h[0] != 0 || h[1] != 0;
+  }
+  return GINGR_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -505,15 +653,40 @@ extern "C" {
 int32_t gingr_gpmm_gaussian_mixture(gingr_ctx* ctx, int32_t M, const double* ref_pts, const int32_t* tri, int32_t T,
                                     int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol,
                                     int32_t max_rank, gingr_model** out, int32_t* rank_out) {
-  return gpmm_build(ctx, "gingr_gpmm_gaussian_mixture", false, M, ref_pts, tri, T, n_kernels, sigma, scaling, rel_tol, max_rank,
-                    out, rank_out);
+  return gpmm_build_gaussian(ctx, "gingr_gpmm_gaussian_mixture", false, M, ref_pts, tri, T, n_kernels, sigma, scaling, rel_tol,
+                             max_rank, out, rank_out);
 }
 
 int32_t gingr_gpmm_gaussian_symmetric(gingr_ctx* ctx, int32_t M, const double* ref_pts, const int32_t* tri, int32_t T,
                                       int32_t n_kernels, const double* sigma, const double* scaling, double rel_tol,
                                       int32_t max_rank, gingr_model** out, int32_t* rank_out) {
-  return gpmm_build(ctx, "gingr_gpmm_gaussian_symmetric", true, M, ref_pts, tri, T, n_kernels, sigma, scaling, rel_tol, max_rank,
-                    out, rank_out);
+  return gpmm_build_gaussian(ctx, "gingr_gpmm_gaussian_symmetric", true, M, ref_pts, tri, T, n_kernels, sigma, scaling, rel_tol,
+                             max_rank, out, rank_out);
+}
+
+int32_t gingr_gpmm_inverse_laplacian(gingr_ctx* ctx, int32_t M, const double* ref_pts, const int32_t* tri, int32_t T,
+                                     double scaling, double gamma, double rel_tol, int32_t max_rank, gingr_model** out,
+                                     int32_t* rank_out) {
+  const char* fn = "gingr_gpmm_inverse_laplacian";
+  if (out) *out = nullptr;
+  if (!ctx || !ref_pts || !out || M <= 0 || T <= 0 || !tri || !(scaling > 0.0) || !std::isfinite(scaling) || !(gamma >= 0.0) ||
+      !std::isfinite(gamma) || !(rel_tol >= 0.0) || max_rank < 0)
+    return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": bad argument (T > 0, scaling > 0 and gamma >= 0 finite, relTol >= 0, "
+                                                             "maxRank >= 0)").c_str());
+  for (int64_t q = 0; q < 3 * (int64_t)T; ++q)
+    if (tri[q] < 0 || tri[q] >= M) return gingr_fail(ctx, GINGR_ERR_ARG, (std::string(fn) + ": triangle index outside [0, M)").c_str());
+  if (M > LAP_MAX_M)
+    return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, (std::string(fn) + ": at most 6000 vertices (a dense, nearly full-rank model); "
+                                                                     "decimate the template first").c_str());
+  if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, (std::string(fn) + ": single-GPU entry point (build before sharding)").c_str());
+  GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  DevBuf<double> K;
+  bool failed = false;
+  GINGR_TRY(laplacian_inverse(ctx, M, tri, T, scaling, gamma, K, &failed));
+  if (failed) return gingr_fail(ctx, GINGR_MODEL_FLEXIBILITY, (std::string(fn) + ": L + gamma I is not numerically positive definite "
+                                                                                 "or the kernel is not finite").c_str());
+  GaussKernelDev kp{};
+  return gpmm_build(ctx, fn, false, M, ref_pts, tri, T, kp, K.p, rel_tol, max_rank, out, rank_out);
 }
 
 // The model as scalismo stores it (SURVEY.md A1): meanVector [3M], basisMatrix column-major [3M x r] (leading dimension

@@ -510,7 +510,7 @@ def load_or_create_model(ctx, directory: str, name: str, reference_points, trian
                          decimate: Optional[int] = None, relativeTolerance: float = 0.01):
     """DataSetLoader.model(decimate, kernelSelect, ...) (DemoDatasetLoader.scala:40-53): read the cached model when its
     file exists, else build it ON THE DEVICE (api.SimpleTriangleModels3D.create) and write the file.  The caller passes
-    the (already decimated) reference; kernelSelect is api.GaussKernel / api.GaussSymKernel / api.GaussMixKernel; -> gingr_b200.api.Model."""
+    the (already decimated) reference; kernelSelect is api.GaussKernel / api.GaussSymKernel / api.InvLapKernel / api.GaussMixKernel; -> gingr_b200.api.Model."""
     import os
     from . import api
     path = os.path.join(directory, model_file_name(name, decimate, kernelSelect.name, kernelSelect.printpars))

@@ -26,6 +26,56 @@ def sphere_mesh(n: int, radius: float = 100.0):
     return pts, tri
 
 
+def icosphere(subdivisions: int, radius: float = 100.0):
+    """Icosahedron with every triangle split in four, `subdivisions` times: 10 4^s + 2 vertices (642 for s = 3)."""
+    t = (1.0 + 5.0 ** 0.5) / 2.0
+    verts = [(-1, t, 0), (1, t, 0), (-1, -t, 0), (1, -t, 0), (0, -1, t), (0, 1, t), (0, -1, -t), (0, 1, -t), (t, 0, -1),
+             (t, 0, 1), (-t, 0, -1), (-t, 0, 1)]
+    tri = [(0, 11, 5), (0, 5, 1), (0, 1, 7), (0, 7, 10), (0, 10, 11), (1, 5, 9), (5, 11, 4), (11, 10, 2), (10, 7, 6), (7, 1, 8),
+           (3, 9, 4), (3, 4, 2), (3, 2, 6), (3, 6, 8), (3, 8, 9), (4, 9, 5), (2, 4, 11), (6, 2, 10), (8, 6, 7), (9, 8, 1)]
+    v = [np.asarray(p, float) / np.linalg.norm(p) for p in verts]
+    for _ in range(subdivisions):
+        mid, nxt = {}, []
+
+        def m(a, b):
+            k = (min(a, b), max(a, b))
+            if k not in mid:
+                p = v[a] + v[b]
+                v.append(p / np.linalg.norm(p))
+                mid[k] = len(v) - 1
+            return mid[k]
+        for a, b, c in tri:
+            ab, bc, ca = m(a, b), m(b, c), m(c, a)
+            nxt += [(a, ab, ca), (b, bc, ab), (c, ca, bc), (ab, bc, ca)]
+        tri = nxt
+    return radius * np.array(v), np.array(tri, dtype=np.int32)
+
+
+def grid_patch(n: int, spacing: float = 1.0):
+    """Open n x n vertex grid in the plane z = 0, two triangles per cell (a surface with a boundary)."""
+    y, x = np.mgrid[0:n, 0:n]
+    pts = spacing * np.stack([x.ravel(), y.ravel(), np.zeros(n * n)], axis=1).astype(float)
+    i = (np.arange(n - 1)[:, None] * n + np.arange(n - 1)[None, :]).ravel()
+    tri = np.concatenate([np.stack([i, i + 1, i + n + 1], 1), np.stack([i, i + n + 1, i + n], 1)]).astype(np.int32)
+    return pts, tri
+
+
+def random_sphere_mesh(n: int, seed: int, radius: float = 100.0):
+    """Convex hull of n random points on a sphere: a closed mesh whose graph has no symmetry (unlike the icosphere's,
+    where pivot values of a graph kernel tie exactly)."""
+    from scipy.spatial import ConvexHull
+    p = np.random.default_rng(seed).normal(size=(n, 3))
+    p = radius * p / np.linalg.norm(p, axis=1)[:, None]
+    return p, ConvexHull(p).simplices.astype(np.int32)
+
+
+def random_patch(n: int, seed: int, size: float = 100.0):
+    """Delaunay triangulation of n random points in a square in the plane z = 0: an open mesh without symmetry."""
+    from scipy.spatial import Delaunay
+    q = np.random.default_rng(seed).uniform(0.0, size, size=(n, 2))
+    return np.hstack([q, np.zeros((n, 1))]), Delaunay(q).simplices.astype(np.int32)
+
+
 def euler_matrix(phi, theta, psi):
     from .rotation import euler_to_matrix
     return euler_to_matrix(phi, theta, psi)

@@ -243,6 +243,19 @@ class Model {
     m.r_ = rank;
     return m;
   }
+  // the inverse-Laplacian look-up kernel scaling (L + gamma I)^-1 (pinv for gamma = 0) of the triangle graph
+  // (gingr_gpmm_inverse_laplacian), on the device; at most 6000 vertices
+  static Model inverseLaplacian(const Context& ctx, int M, const double* ref, const int32_t* tri, int T, double scaling,
+                                double gamma, double relativeTolerance = 0.01, int maxRank = 0) {
+    Model m(ctx);
+    int32_t rank = 0;
+    if (ctx.check(gingr_gpmm_inverse_laplacian(ctx.handle(), M, ref, tri, T, scaling, gamma, relativeTolerance, maxRank, &m.h_,
+                                               &rank)) == GINGR_MODEL_FLEXIBILITY)
+      throw Error(GINGR_MODEL_FLEXIBILITY, "L + gamma I is not numerically positive definite");
+    m.M_ = M;
+    m.r_ = rank;
+    return m;
+  }
   // model.newReference(newRef, NearestNeighborInterpolator()), registration/SimpleRegistrator.scala:90-92
   Model newReference(int M2, const double* ref, const int32_t* tri = nullptr, int T = 0) const {
     Model m(*ctx_);

@@ -165,6 +165,27 @@ GINGR_API int32_t gingr_gpmm_gaussian_symmetric(gingr_ctx* ctx, int32_t M, const
                                                 const int32_t* tri /*[3T]*/, int32_t T, int32_t n_kernels,
                                                 const double* sigma /*[n]*/, const double* scaling /*[n]*/, double rel_tol,
                                                 int32_t max_rank, gingr_model** out, int32_t* rank_out);
+/* The inverse-Laplacian model: the look-up kernel of the model chooser (api/gpmm LaplacianHelper.scala:26-55 with
+ * MatrixHelper.pinv :23-26), the GP form of a mesh-graph stiffness term -- vertices close on the triangle graph move
+ * together, vertices merely close in space do not.  This project's reading of that kernel (unit weights, the role of
+ * gamma and the parameter names are not verified against the reference):
+ *   L = D - A, the combinatorial graph Laplacian of the triangle edges (unit weights, each undirected edge once however
+ *       many triangles share it, self-edges of degenerate triangles ignored);
+ *   Ks = scaling (L + gamma I)^-1 for gamma > 0, and for gamma = 0 the pseudo-inverse scaling L^+ = scaling ((L + P)^-1 - P),
+ *       P = sum_c 1_c 1_c^T / |c| over the connected components c of the edge graph (a vertex in no triangle is a component
+ *       of its own);
+ *   K = DiagonalKernel(Ks, 3) = Ks (x) I3, then approximateGPCholesky with the stopping rule and outputs of
+ *       gingr_gpmm_gaussian_mixture; the mean is zero.
+ * Ks is formed densely on the device, so M <= 6000 (GINGR_ERR_UNSUPPORTED above).  Its spectrum decays like 1/k: at
+ * rel_tol 0.01 the rank is about 0.97-0.99 of 3M, and the registrations take rank <= 9472 (about M <= 3200 at rel_tol 0.01):
+ * larger templates want max_rank.  With gamma = 0 the kernel has rank 3 (M - #components): at rel_tol = 0 the
+ * factorisation goes on past that rank and takes up to 3 * #components more columns from the rounding-level residual of
+ * the null space, so a full-rank gamma = 0 model wants a small positive rel_tol (1e-12 suffices).  Requires T > 0,
+ * indices in [0, M), scaling > 0 and gamma >= 0 finite, rel_tol >= 0, max_rank >= 0 and a single-GPU context.  Returns GINGR_MODEL_FLEXIBILITY with *out = NULL when L + gamma I is not
+ * numerically positive definite (a gamma far below the rounding of L) or Ks is not finite. */
+GINGR_API int32_t gingr_gpmm_inverse_laplacian(gingr_ctx* ctx, int32_t M, const double* ref_pts /*[3M]*/,
+                                               const int32_t* tri /*[3T]*/, int32_t T, double scaling, double gamma,
+                                               double rel_tol, int32_t max_rank, gingr_model** out, int32_t* rank_out);
 /* The model as scalismo stores it (SURVEY.md A1): meanVector, basisMatrix column-major with leading dimension ld_basis,
  * variance.  Any output may be NULL (M_out / r_out give the sizes to allocate). */
 GINGR_API int32_t gingr_model_download(gingr_ctx* ctx, const gingr_model* model, int32_t* M_out, int32_t* r_out,

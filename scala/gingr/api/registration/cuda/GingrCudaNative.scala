@@ -91,6 +91,9 @@ object GingrCudaNative {
   // the mirror-symmetric kernel about x = 0 (scalismo's symmetrised Gaussian kernel), same arguments
   val gpmmGaussianSymmetric = fn("gingr_gpmm_gaussian_symmetric", JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT,
                                  ADDRESS, ADDRESS, JAVA_DOUBLE, JAVA_INT, ADDRESS, ADDRESS)
+  // the inverse-Laplacian look-up kernel of the triangle graph (LaplacianHelper.scala:26-55)
+  val gpmmInverseLaplacian = fn("gingr_gpmm_inverse_laplacian", JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_DOUBLE,
+                                JAVA_DOUBLE, JAVA_DOUBLE, JAVA_INT, ADDRESS, ADDRESS)
   val modelDownload  = fn("gingr_model_download", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, ADDRESS, JAVA_LONG, ADDRESS)
 
   // the remaining entry points of include/gingr_cuda.h (every exported function has a handle here; tests/test_scala_shim.py
