@@ -187,6 +187,56 @@ int32_t gingr_registration_posterior_model(gingr_registration* g, const gingr_st
   return posterior_model_finish(ctx, m, sys.p + (size_t)(r + 1) * rp, c.p, g->ds.p, ev, out);
 }
 
+// Test window on the iteration's posterior system (not in gingr_cuda.h): the same posterior phase as above at the given
+// state, then sys [(r + 1) x r] = the kept raw system unpadded (rows 0 .. r-1 the full symmetric Mx as the MH chain reads
+// it, row r the rhs) and, if non-null, wrow / u [3M] as obs_kernel wrote them.  max_cta > 0 schedules the Gram of this
+// call on at most that many CTAs; the plan is rebuilt as it was afterwards and whatever captured the old plan is dropped.
+GINGR_API int32_t gingr_debug_posterior_system(gingr_registration* g, const gingr_state* state, const double* alpha,
+                                               int32_t max_cta, double* sys, double* wrow, double* u) {
+  if (!g || !state || !alpha || !sys || max_cta < 0)
+    return gingr_fail(g ? g->ctx : nullptr, GINGR_ERR_ARG, "gingr_debug_posterior_system: bad argument");
+  gingr_ctx* ctx = g->ctx;
+  if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_debug_posterior_system: single-GPU entry point");
+  const gingr_model* m = g->model;
+  const int r = m->r, rp = m->rp, M = m->M;
+  GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  const int prev_cta = g->gram.ncta;
+  if (max_cta > 0) {
+    drop_graph(g);
+    mcmc_invalidate(g);
+    mcmc_drop_chain_graph(g);
+    GINGR_TRY(g->gram.build(ctx, g->gram.rows, r, rp, max_cta));
+  }
+  static_assert(IS_FAIL_POST == IS_INFO + 1, "the posterior flags are copied as one pair");
+  int hflags[2] = {0, 0};
+  int32_t rc = [&]() -> int32_t {
+    mcmc_invalidate(g);
+    g->state_valid = false;
+    GINGR_TRY(upload_state(g, state, alpha));
+    GINGR_TRY(evaluate_fit(g, DS_SCALE, DS_T, DS_R));
+    GINGR_CUDA_TRY(ctx, g->Mx_raw.alloc((size_t)(r + 1) * rp));
+    const bool keep_raw = g->keep_raw;
+    g->keep_raw = true;
+    const int32_t rc_post = enqueue_posterior_phase(g);
+    g->keep_raw = keep_raw;
+    GINGR_TRY(rc_post);
+    cudaStream_t st = ctx->stream;
+    GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(sys, sizeof(double) * r, g->Mx_raw.p, sizeof(double) * rp, sizeof(double) * r, r + 1,
+                                          cudaMemcpyDeviceToHost, st));
+    if (wrow) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(wrow, g->wrow.p, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
+    if (u) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(u, g->u.p, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
+    GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(hflags, g->is.p + IS_INFO, sizeof(int) * 2, cudaMemcpyDeviceToHost, st));
+    GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    return GINGR_OK;
+  }();
+  if (max_cta > 0) {   // the plan of the registration back, also after a failure
+    const int32_t rb = g->gram.build(ctx, g->gram.rows, r, rp, prev_cta);
+    if (rc >= 0) rc = rb;
+  }
+  GINGR_TRY(rc);
+  return hflags[0] || hflags[1] ? GINGR_MODEL_FLEXIBILITY : GINGR_OK;
+}
+
 int32_t gingr_posterior_model_profile(const gingr_ctx* ctx, double* ms, int32_t* sweeps) {
   if (!ctx || !ms) return gingr_fail(nullptr, GINGR_ERR_ARG, "gingr_posterior_model_profile: bad argument");
   for (int k = 0; k < 5; ++k) ms[k] = ctx->posterior_model_ms[k];
