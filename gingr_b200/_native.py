@@ -22,7 +22,7 @@ GINGR_ERR_ARG, GINGR_ERR_CUDA, GINGR_ERR_NCCL, GINGR_ERR_UNSUPPORTED = -1, -2, -
 STATUS_NONE, STATUS_MAX_ITERATION, STATUS_CONVERGED, STATUS_MODEL_FLEXIBILITY_ERROR = 0, 1, 2, 3
 SIMILARITY_TRANSFORMS, RIGID_TRANSFORMS, NO_TRANSFORMS = 0, 1, 2
 TRIANGULAR_CLOSEST_POINT, ALONG_NORMAL_CLOSEST_POINT, POINTCLOUD_CLOSEST_POINT = 0, 1, 2
-ALGO_CPD, ALGO_ICP = 0, 1
+ALGO_CPD, ALGO_ICP, ALGO_BCPD = 0, 1, 2
 
 
 class GingrState(ctypes.Structure):
@@ -121,6 +121,8 @@ SIGNATURES = {
     "gingr_update_chain_sampled": (c_int32, [c_void_p, c_int32, c_uint64]),
     "gingr_update_batch": (c_int32, [POINTER(c_void_p), c_int32, c_int32, c_int32, c_uint64]),
     "gingr_state_download": (c_int32, [c_void_p, POINTER(GingrState), dp, dp]),
+    "gingr_registration_set_bcpd": (c_int32, [c_void_p, c_double]),
+    "gingr_bcpd_state_download": (c_int32, [c_void_p, dp, dp]),
     "gingr_registration_posterior_model": (c_int32, [c_void_p, POINTER(GingrState), dp, vpp]),
     "gingr_mcmc_configure": (c_int32, [c_void_p, POINTER(GingrMcmcSettings), ip, c_int32, ip, c_int32]),
     "gingr_evaluate_log_value": (c_int32, [c_void_p, POINTER(GingrState), dp, dp]),

@@ -19,7 +19,7 @@ from typing import Callable, Optional, Sequence, Tuple
 import numpy as np
 
 from . import _native as nat
-from ._native import (ALGO_CPD, ALGO_ICP, NO_TRANSFORMS, POINTCLOUD_CLOSEST_POINT, RIGID_TRANSFORMS,
+from ._native import (ALGO_BCPD, ALGO_CPD, ALGO_ICP, NO_TRANSFORMS, POINTCLOUD_CLOSEST_POINT, RIGID_TRANSFORMS,
                       SIMILARITY_TRANSFORMS, STATUS_CONVERGED, STATUS_MAX_ITERATION,
                       STATUS_MODEL_FLEXIBILITY_ERROR, STATUS_NONE, TRIANGULAR_CLOSEST_POINT,
                       ALONG_NORMAL_CLOSEST_POINT, EVAL_MODEL_TO_TARGET, EVAL_SYMMETRIC, EVAL_TARGET_TO_MODEL,
@@ -635,6 +635,31 @@ class IcpConfiguration:
         return c
 
 
+@dataclass
+class BcpdConfiguration:
+    """The BCPD configuration of GingrAlgorithm (include/gingr_cuda.h GINGR_ALGO_BCPD; this project's reading of
+    other/algorithms/cpd/BCPD.scala on GiNGR's hooks).  Every field but `kappa` means what it means for CPD; `kappa` is the
+    Dirichlet concentration of the mixing-weight update alpha_m = exp(psi(kappa + nu_m) - psi(kappa M + Nhat)).
+
+    Scale: the E-step's outlier term is w / N, literally as in BCPD.scala, against Gaussians of height (2 pi sigma2)^-3/2.
+    With w > 0 on data whose initial sigma2 is large (coordinates of hundreds of units) it outweighs every Gaussian, Nhat
+    becomes tiny and sigma2 grows without bound; use w = 0 there, or scale the coordinates down."""
+    maxIterations: int = 100
+    threshold: float = 1e-10
+    converged: Callable = lambda last, cur, thr: abs(last.sigma2 - cur.sigma2) < thr
+    useLandmarkCorrespondence: bool = True
+    initialSigma: Optional[float] = None
+    w: float = 0.0
+    lambda_: float = 1.0
+    kappa: float = 1.0
+
+    def to_pod(self) -> GingrConfig:
+        c = CpdConfiguration(self.maxIterations, self.threshold, self.converged, self.useLandmarkCorrespondence,
+                             self.initialSigma, self.w, self.lambda_).to_pod()
+        c.algorithm = ALGO_BCPD
+        return c
+
+
 class GingrAlgorithm:
     """api/GingrAlgorithm.scala:65-303 with `update` (:192-254) executed on the device."""
     name = "Gingr"
@@ -1136,3 +1161,21 @@ class IcpRegistration(GingrAlgorithm):
 
     def __init__(self, ctx, model, target, config: Optional[IcpConfiguration] = None):
         super().__init__(ctx, model, target, config or IcpConfiguration())
+
+
+class BcpdRegistration(GingrAlgorithm):
+    """GingrAlgorithm with BCPD correspondences (BcpdConfiguration).  Besides the GeneralRegistrationState the registration
+    keeps per-vertex mixing weights and posterior variances on the device: creation and initializeState set them to 1 / M
+    and the prior variance, every committed update advances them (bcpdState() reads them back).  Deterministic updates on one GPU
+    only: the probabilistic calls raise GingrError with GINGR_ERR_UNSUPPORTED."""
+    name = "BCPD"
+
+    def __init__(self, ctx, model, target, config: Optional[BcpdConfiguration] = None):
+        super().__init__(ctx, model, target, config or BcpdConfiguration())
+        self.ctx.check(self.ctx._lib.gingr_registration_set_bcpd(self.handle, float(self.config.kappa)))
+
+    def bcpdState(self) -> Tuple[np.ndarray, np.ndarray]:
+        """(alpha[M], Sigma[M]): the mixing weights and per-vertex posterior variances the next update's E-step uses."""
+        alpha, sigma = np.empty(self.model.M), np.empty(self.model.M)
+        self.ctx.check(self.ctx._lib.gingr_bcpd_state_download(self.handle, nat.as_dp(alpha), nat.as_dp(sigma)))
+        return alpha, sigma

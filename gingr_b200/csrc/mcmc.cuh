@@ -653,6 +653,7 @@ int32_t gingr_mcmc_configure(gingr_registration* g, const gingr_mcmc_settings* s
     return gingr_fail(g ? g->ctx : nullptr, GINGR_ERR_ARG, "gingr_mcmc_configure: bad argument");
   gingr_ctx* ctx = g->ctx;
   if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_mcmc_configure: single-GPU chains only");
+  if (g->cfg.algorithm == GINGR_ALGO_BCPD) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_mcmc_configure: BCPD registrations are deterministic");
   if (!(s->random_mixture >= 0.0 && s->random_mixture <= 1.0) || !(s->uncertainty > 0.0) || s->evaluation_mode < 0 ||
       s->evaluation_mode > 2)
     return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_configure: randomMixture in [0, 1], uncertainty > 0, mode 0..2");

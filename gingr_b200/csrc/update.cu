@@ -9,6 +9,7 @@
 //
 //   pose_kernel            R = Rz(phi) Ry(theta) Rx(psi) from the Euler angles of the state
 //   [CPD] E-step (estep.cu) on this rank's target shard  -> P1, PX, Pt1 ; all-reduce over ranks
+//   [BCPD] BCPD E-step (estep.cu) with row factors from alpha, Sigma -> nu, PX, nu'  (see "BCPD" below)
 //   [ICP] closest point (closest.cu)                     -> cp, 0/1 weights
 //   obs_kernel             correspondence point, observation weight 1/var, residual u = w R^T (y - m'),
 //                          per-row weights; sums for the sigma2 update (pre-update fit, CPD.scala:133-147)
@@ -22,6 +23,19 @@
 //   gemvT + W0             alpha_new = transformedModel.coefficients(newshape)                    (:234-237)
 //   finalize               new state or ModelFlexibilityError, sigma2 hook                        (:239-251)
 //   gemv_rows + pose       fit = s (R instance(alpha_new) + t)            (ModelFittingParameters.scala:130-143)
+//
+// BCPD (GINGR_ALGO_BCPD) is this project's reading of the textbook BCPD (other/algorithms/cpd/BCPD.scala) on GiNGR's three
+// hooks; the reference ships no BCPD configuration.  Next to the state block the registration keeps alpha[M] (mixing
+// weights) and Sigma[M] (per-vertex posterior variance).  One iteration is the CPD one with:
+//   E-step        the BCPD E-step, row factors f_m = (1 - w) (2 pi sigma2)^-3/2 exp(-s / (2 sigma2) 3 Sigma_m) alpha_m formed
+//                 on the device from the state block (s: the state's scale, not s^2, as in BCPD.scala) -> nu, nu', xhat
+//   observations  xhat_m with noise sigma2 lambda / nu_m I3 (CPD.scala:125 with P1 -> nu)
+//   sigma2 hook   (sXX - 2 sXY + sYY + sigma2 sigma2bar) / (3 Nhat) on the pre-update fit, sigma2bar = sum nu_m Sigma_m / Nhat
+//                 (the textbook's sC = sigma2 sigma2bar kept literally); Nhat = sum nu_m (= sum nu'_n)
+//   next state    alpha_m = exp(psi(kappa + nu_m) - psi(kappa M + Nhat)) (BCPD.scala:218) and Sigma_m = tr(cov_m) / 3 with
+//                 cov_m the posterior covariance at vertex m of this iteration's system: the 3M rows of Q = Phi D ride
+//                 through the factorisation (3M x rp doubles more, about 1 GB at M = 20 000, r = 2000), as in
+//                 gingr_posterior_covariance; committed only together with the rest of the state
 #include <math.h>
 #include <stdlib.h>
 #include <string.h>
@@ -43,7 +57,7 @@ enum {
   DS_SCALE = 0, DS_T = 1, DS_EULER = 4, DS_CENTER = 7, DS_SIGMA2 = 10, DS_STEP = 11, DS_R = 12,
   DS_NEW_SCALE = 24, DS_NEW_T = 25, DS_NEW_EULER = 28, DS_R1 = 31, DS_R2 = 40,
   DS_NEW_SIGMA2 = 50, DS_NP = 51, DS_XPX = 52, DS_YPY = 53, DS_TRPXY = 54,
-  DS_MUX = 56, DS_MUY = 59, DS_S2X = 62, DS_SXY = 63, DS_COUNT = 80
+  DS_MUX = 56, DS_MUY = 59, DS_S2X = 62, DS_SXY = 63, DS_S2BAR = 72, DS_COUNT = 80
 };
 enum { IS_GT = 0, IS_ITER = 1, IS_STATUS = 2, IS_INFO = 3, IS_FAIL_POST = 4, IS_FAIL_COEF = 5, IS_RETRY = 6, IS_COUNT = 16 };
 constexpr int RETRY_COUNTER_INIT = 10;  // GingrAlgorithm.scala:69-70
@@ -283,6 +297,214 @@ GINGR_KERNEL_NB(sigma2_kernel, int algo, int nblocks, const double* __restrict__
     }
   } else if (lane == 0) {
     ds[DS_NEW_SIGMA2] = fmax(ds[DS_SIGMA2] - sigma_step, end_sigma);
+  }
+}
+
+// ---- BCPD ------------------------------------------------------------------------------------------
+// What the BCPD E-step needs from the state block, in one launch: fit_soa in the caller's order (the row factors share it;
+// the registration's row_perm is the identity), the row factors, the failure flag for a non-finite fit / alpha / Sigma /
+// sigma2 and -- by the last block, as in cpd_prepare_kernel -- the scalars: scal[0] = sigma2, scal[1] = a = 1 - w,
+// scal[2] = c = w / N, scal[3] = w, scal[5] = s, scal[6] = 1 / N, scal[7] = bound of the pair distances.  The row factor is
+// the expression of estep_bcpd_rowf_kernel (gingr_bcpd_estep), so both E-steps see the same bits.
+GINGR_KERNEL((256), bcpd_prepare_kernel, int M, const double* __restrict__ fit /*AoS*/, double* __restrict__ fit_soa,
+                                                           const double* __restrict__ sigma_mm, const double* __restrict__ alpha,
+                                                           double* __restrict__ rowf, const double* __restrict__ ds, double w,
+                                                           double inv_n, double target_maxabs, int* __restrict__ fail_flag,
+                                                           unsigned long long* __restrict__ sync /*[2]: max bits, ticket*/,
+                                                           double* __restrict__ scal) {
+  __shared__ double red[8];
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  const double sigma2 = ds[DS_SIGMA2], s = ds[DS_SCALE];
+  double m = 0.0;
+  int bad = 0;
+  if (i < M) {
+    const double x = fit[3 * i], y = fit[3 * i + 1], z = fit[3 * i + 2];
+    fit_soa[i] = x; fit_soa[M + i] = y; fit_soa[2 * (size_t)M + i] = z;
+    const double t = 2.0 * 3.14159265358979323846 * sigma2;
+    const double norm = 1.0 / (t * sqrt(t));
+    rowf[i] = (1.0 - w) * norm * exp(-s / (2.0 * sigma2) * (3.0 * sigma_mm[i])) * alpha[i];
+    bad = !(fabs(x) < INFINITY) || !(fabs(y) < INFINITY) || !(fabs(z) < INFINITY) || !(fabs(sigma_mm[i]) < INFINITY) ||
+          !(fabs(alpha[i]) < INFINITY);
+    m = fmax(fmax(fabs(x), fabs(y)), fabs(z));
+  }
+  bad = __syncthreads_or(bad);
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) m = fmax(m, __shfl_xor_sync(0xffffffffu, m, o));
+  if ((threadIdx.x & 31) == 0) red[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x != 0) return;
+  for (int k = 1; k < 8; ++k) m = fmax(m, red[k]);
+  if (bad) *fail_flag = 1;
+  atomicMax(sync, (unsigned long long)__double_as_longlong(m));   // non-negative doubles order like their bit patterns
+  __threadfence();
+  if (atomicAdd(sync + 1, 1ULL) != (unsigned long long)gridDim.x - 1) return;
+  __threadfence();
+  const double fmaxabs = __longlong_as_double((long long)atomicExch(sync, 0ULL));
+  sync[1] = 0ULL;
+  if (!(fabs(sigma2) < INFINITY)) *fail_flag = 1;
+  scal[0] = sigma2;
+  scal[1] = 1.0 - w;
+  scal[2] = w * inv_n;
+  scal[3] = w;
+  scal[5] = s;
+  scal[6] = inv_n;
+  const double s2 = fmaxabs + target_maxabs;
+  scal[7] = 3.0 * s2 * s2;
+}
+
+// BCPD observations: the CPD branch of obs_kernel with P1 -> nu (point xhat_m = PX_m / nu_m, variance sigma2 lambda / nu_m),
+// and a fourth block sum for the sigma2 hook: per block nu, nu |fit|^2, fit . PX, nu Sigma.
+GINGR_KERNEL((256), bcpd_obs_kernel, const ObsArgs& a, const double* __restrict__ rows /*[4][M]*/,
+                                                       const double* __restrict__ sigma_mm, const double* __restrict__ fit,
+                                                       const double* __restrict__ ref, const double* __restrict__ mean,
+                                                       const int32_t* __restrict__ lm_pid, const double* __restrict__ ds,
+                                                       int* __restrict__ is, double* __restrict__ wrow, double* __restrict__ u,
+                                                       double* __restrict__ sums_part /*[blocks][4]*/,
+                                                       double* __restrict__ resid /*[3 Ml], may be null*/) {
+  __shared__ double red[4][8];
+  const int i = blockIdx.x * 256 + threadIdx.x;
+  double v[4] = {0.0, 0.0, 0.0, 0.0};
+  if (i < a.M) {
+    const double sigma2 = ds[DS_SIGMA2];
+    const double nu = rows[i];
+    const double X = rows[(size_t)a.M + i], Y = rows[(size_t)2 * a.M + i], Z = rows[(size_t)3 * a.M + i];
+    const double inv = 1.0 / nu;
+    const double px = X * inv, py = Y * inv, pz = Z * inv;
+    const double var = sigma2 * a.lambda * inv;
+    double wt = 1.0 / var;
+    if (!(var < INFINITY) || !(var > 0.0) || !(wt < INFINITY)) is[IS_FAIL_POST] = 1;
+    const double fx = fit[3 * i], fy = fit[3 * i + 1], fz = fit[3 * i + 2];
+    v[0] = nu;
+    v[1] = nu * (fx * fx + fy * fy + fz * fz);
+    v[2] = fx * X + fy * Y + fz * Z;
+    v[3] = nu * sigma_mm[i];
+    if (a.use_lm)
+      for (int l = 0; l < a.L; ++l)
+        if (lm_pid[l] == i) wt = 0.0;  // correspondences at landmark ids are replaced (GingrAlgorithm.scala:288-296)
+    const int li = i - a.m0;
+    if (li >= 0 && li < a.Ml) {
+      const double* R = ds + DS_R;
+      const double bx = ref[3 * i] + mean[3 * i], by = ref[3 * i + 1] + mean[3 * i + 1], bz = ref[3 * i + 2] + mean[3 * i + 2];
+      double rx = px - (R[0] * bx + R[1] * by + R[2] * bz + ds[DS_T]);
+      double ry = py - (R[3] * bx + R[4] * by + R[5] * bz + ds[DS_T + 1]);
+      double rz = pz - (R[6] * bx + R[7] * by + R[8] * bz + ds[DS_T + 2]);
+      if (wt == 0.0) { rx = ry = rz = 0.0; }
+      wrow[3 * li] = wrow[3 * li + 1] = wrow[3 * li + 2] = wt;
+      const double q0 = R[0] * rx + R[3] * ry + R[6] * rz, q1 = R[1] * rx + R[4] * ry + R[7] * rz,
+                   q2 = R[2] * rx + R[5] * ry + R[8] * rz;
+      u[3 * li] = wt * q0;
+      u[3 * li + 1] = wt * q1;
+      u[3 * li + 2] = wt * q2;
+      if (resid) { resid[3 * li] = q0; resid[3 * li + 1] = q1; resid[3 * li + 2] = q2; }
+    }
+  }
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_down_sync(0xffffffffu, v[q], o);
+    if ((threadIdx.x & 31) == 0) red[q][threadIdx.x >> 5] = v[q];
+  }
+  __syncthreads();
+  if (threadIdx.x < 4) {
+    double s = 0.0;
+    for (int k = 0; k < 8; ++k) s += red[threadIdx.x][k];
+    sums_part[blockIdx.x * 4 + threadIdx.x] = s;
+  }
+}
+
+// BCPD sigma2 hook (one warp, fixed order as sigma2_kernel): Nhat = sum nu, sYY, sXY, sigma2bar = sum nu Sigma / Nhat,
+// sXX from the E-step; new sigma2 = (sXX - 2 sXY + sYY + sigma2 sigma2bar) / (3 Nhat)
+GINGR_KERNEL_NB(bcpd_sigma2_kernel, int nblocks, const double* __restrict__ sums_part, const double* __restrict__ xpx,
+                                   double* __restrict__ ds) {
+  const int lane = threadIdx.x;
+  double v[4] = {0.0, 0.0, 0.0, 0.0};
+  for (int k = lane; k < nblocks; k += 32)
+    for (int q = 0; q < 4; ++q) v[q] += sums_part[4 * k + q];
+#pragma unroll
+  for (int q = 0; q < 4; ++q)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) v[q] += __shfl_xor_sync(0xffffffffu, v[q], o);
+  if (lane == 0) {
+    const double nhat = v[0], s2bar = v[3] / nhat;
+    ds[DS_NP] = nhat; ds[DS_XPX] = xpx[0]; ds[DS_YPY] = v[1]; ds[DS_TRPXY] = v[2]; ds[DS_S2BAR] = s2bar;
+    ds[DS_NEW_SIGMA2] = (xpx[0] - 2.0 * v[2] + v[1] + ds[DS_SIGMA2] * s2bar) / (nhat * 3.0);
+  }
+}
+
+// rows r + 1 + k of the system <- row k of Q = Phi D (as posterior_cov_rows_kernel); the factorisation turns them into
+// Q_k L^-T, whose squared norms summed over a vertex's three rows are tr(cov_m)
+GINGR_KERNEL_NB(bcpd_var_rows_kernel, int rows, int r, int rp, const double* __restrict__ phi,
+                                     const double* __restrict__ sqrt_lambda, double* __restrict__ out) {
+  for (int k = blockIdx.y; k < rows; k += gridDim.y)   // rows may exceed the 65535 of a grid's y extent
+    for (int c = blockIdx.x * blockDim.x + threadIdx.x; c < rp; c += gridDim.x * blockDim.x)
+      out[(size_t)k * rp + c] = c < r ? phi[(size_t)k * rp + c] * sqrt_lambda[c] : 0.0;
+}
+
+// psi(x) for x > 0: the recurrence psi(x) = psi(x + 1) - 1 / x up to x >= 6, then the asymptotic series
+// ln x - 1/(2x) - sum_k B_2k / (2k x^2k) through k = 13 (first omitted term < 2e-16 at x = 6)
+__device__ double digamma_dev(double x) {
+  if (!(x > 0.0)) return x == 0.0 ? -INFINITY : NAN;   // the recurrence would not end; BCPD's arguments are > 0
+  double acc = 0.0;
+  while (x < 6.0) {
+    acc -= 1.0 / x;
+    x += 1.0;
+  }
+  const double f = 1.0 / (x * x);
+  const double t =
+      f * (1.0 / 12 - f * (1.0 / 120 - f * (1.0 / 252 - f * (1.0 / 240 - f * (1.0 / 132 - f * (691.0 / 32760 - f * (1.0 / 12 -
+      f * (3617.0 / 8160 - f * (43867.0 / 14364 - f * (174611.0 / 6600 - f * (854513.0 / 3036 - f * (236364091.0 / 65520 -
+      f * (8553103.0 / 156)))))))))))));
+  return acc + (log(x) - 0.5 / x - t);
+}
+
+GINGR_KERNEL_NB(digamma_kernel, int n, const double* __restrict__ x, double* __restrict__ out) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i < n) out[i] = digamma_dev(x[i]);
+}
+
+// prior state (gingr_initialize_state): alpha_m = 1 / M, Sigma_m = tr(Phi_m Lambda Phi_m^T) / 3, the posterior variance
+// without observations (the textbook starts from Sigma = I, which has no meaning in a GPMM's units).  One warp per vertex.
+GINGR_KERNEL((256), bcpd_prior_kernel, int M, int r, int rp, const double* __restrict__ phi, const double* __restrict__ sl,
+                                                         double* __restrict__ alpha, double* __restrict__ sigma) {
+  const int i = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (i >= M) return;
+  const double* x = phi + (size_t)(3 * i) * rp;
+  double s = 0.0;
+  for (int d = 0; d < 3; ++d)
+    for (int c = lane; c < r; c += 32) {
+      const double q = x[(size_t)d * rp + c] * sl[c];
+      s = fma(q, q, s);
+    }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) {
+    alpha[i] = 1.0 / M;
+    sigma[i] = s / 3.0;
+  }
+}
+
+// next BCPD state, after finalize_kernel: Sigma_m = tr(cov_m) / 3 from the three solved rows X of vertex m (rotation
+// invariant) and alpha_m = exp(psi(kappa + nu_m) - psi(kappa M + Nhat)); written only where finalize_kernel committed the
+// iteration (no posterior / coefficients failure), so a ModelFlexibilityError leaves them as they were.  One warp per vertex.
+GINGR_KERNEL((256), bcpd_state_kernel, int M, int r, int rp, double kappa, const double* __restrict__ X,
+                                                         const double* __restrict__ nu, const double* __restrict__ ds,
+                                                         const int* __restrict__ is, double* __restrict__ alpha,
+                                                         double* __restrict__ sigma) {
+  const int i = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  if (i >= M) return;
+  if (is[IS_INFO] != 0 || is[IS_FAIL_POST] != 0 || is[IS_FAIL_COEF] != 0) return;
+  const double* x = X + (size_t)(3 * i) * rp;
+  double s = 0.0;
+  for (int d = 0; d < 3; ++d)
+    for (int c = lane; c < r; c += 32) {
+      const double q = x[(size_t)d * rp + c];
+      s = fma(q, q, s);
+    }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
+  if (lane == 0) {
+    sigma[i] = s / 3.0;
+    alpha[i] = exp(digamma_dev(kappa + nu[i]) - digamma_dev(kappa * M + ds[DS_NP]));
   }
 }
 
@@ -706,6 +928,11 @@ struct gingr_registration {
   DevBuf<int> is, flags;
   CholWs cholws;               // tickets / flags / diagonal-block inverses of the data-flow Cholesky (chol_df.cu)
   DevBuf<double> alpha;
+  // BCPD: Dirichlet concentration kappa (gingr_registration_set_bcpd), mixing weights and per-vertex posterior variances
+  // [M] (set to the prior at creation and by gingr_initialize_state, advanced by every committed iteration; the iteration's
+  // Mx carries 3 M more rows)
+  double bcpd_kappa = 1.0;
+  DevBuf<double> bcpd_alpha, bcpd_sigma;
   int retry_counter = RETRY_COUNTER_INIT;  // mirror of the device counter, refreshed by download_state
   // One iteration captured as a CUDA graph: the ~100-launch sequence of a small registration (C1-C3 sizes) is
   // launch-latency bound, the graph replays it with one driver call.  Key = (probabilistic, seed).
@@ -1320,10 +1547,15 @@ int32_t gingr_model_instance(gingr_ctx* ctx, const gingr_model* model, const gin
 int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, const gingr_target* target,
                                   const gingr_config* cfg, gingr_registration** out) {
   if (!ctx || !model || !target || !cfg || !out) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_registration_create: bad argument");
-  if (cfg->algorithm != GINGR_ALGO_CPD && cfg->algorithm != GINGR_ALGO_ICP)
+  if (cfg->algorithm != GINGR_ALGO_CPD && cfg->algorithm != GINGR_ALGO_ICP && cfg->algorithm != GINGR_ALGO_BCPD)
     return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_registration_create: unknown algorithm");
   if (cfg->algorithm == GINGR_ALGO_CPD && !(cfg->w >= 0.0 && cfg->w < 1.0))
     return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_registration_create: CPD w must be in [0, 1)");
+  const bool bcpd = cfg->algorithm == GINGR_ALGO_BCPD;
+  if (bcpd && !(cfg->w >= 0.0 && cfg->w < 1.0))
+    return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_registration_create: BCPD w must be in [0, 1)");
+  if (bcpd && ctx->nranks != 1)
+    return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_registration_create: BCPD registrations run on one GPU");
   if (cfg->algorithm == GINGR_ALGO_ICP) {
     if (cfg->correspondence_method < GINGR_TRIANGULAR_CLOSEST_POINT || cfg->correspondence_method > GINGR_POINTCLOUD_CLOSEST_POINT)
       return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_registration_create: unknown correspondence method");
@@ -1347,6 +1579,18 @@ int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, cons
     std::vector<int32_t> perm;
     estep_row_order(ref.data(), M, perm);
     GINGR_TRY(g->estep.set_row_order(ctx, M, perm.data()));
+  } else if (bcpd) {
+    // the rows stay in the caller's order, as in gingr_bcpd_estep (the E-step is not culled with row factors)
+    GINGR_TRY(g->estep.ensure(ctx, M, std::max(target->N, 1)));
+    std::vector<int32_t> perm((size_t)M);
+    for (int i = 0; i < M; ++i) perm[i] = i;
+    GINGR_TRY(g->estep.set_row_order(ctx, M, perm.data()));
+    GINGR_CUDA_TRY(ctx, g->bcpd_alpha.alloc((size_t)M));
+    GINGR_CUDA_TRY(ctx, g->bcpd_sigma.alloc((size_t)M));
+    // the prior state from the start, so that an update on a caller-built state (no gingr_initialize_state) is defined
+    GINGR_LAUNCH(ctx, bcpd_prior_kernel, ceil_div(M, 8), 256, 0, ctx->stream, M, r, rp, model->phi.p, model->sqrt_lambda.p,
+                 g->bcpd_alpha.p, g->bcpd_sigma.p);
+    GINGR_LAUNCHED(ctx);
   } else {
     const bool rev = cfg->reverse_correspondence_direction != 0;
     GINGR_TRY(rev ? g->closest.ensure(ctx, target->N_total, M, model->T, target->T)
@@ -1375,7 +1619,9 @@ int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, cons
   }
   GINGR_TRY(g->gram.build(ctx, 3 * Ml, r, rp));
   GINGR_CUDA_TRY(ctx, g->rows_ext.alloc((size_t)4 * M + 8));
-  GINGR_CUDA_TRY(ctx, g->Mx.alloc((size_t)(r + 8) * rp));
+  // BCPD: the 3 M rows of Q ride behind the rhs row through the factorisation (bcpd_var_rows_kernel)
+  const int xrows = bcpd ? 3 * M : 0;
+  GINGR_CUDA_TRY(ctx, g->Mx.alloc((size_t)(r + 8 + xrows) * rp));
   if (ctx->nranks > 1) GINGR_CUDA_TRY(ctx, g->Mx_packed.alloc(gram_packed_doubles(g->gram) + rp));
   GINGR_CUDA_TRY(ctx, g->prep_sync.alloc(2));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->prep_sync.p, 0, 2 * sizeof(unsigned long long), ctx->stream));
@@ -1390,13 +1636,13 @@ int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, cons
   GINGR_CUDA_TRY(ctx, g->fit.alloc((size_t)3 * M));
   GINGR_CUDA_TRY(ctx, g->vec.alloc((size_t)8 * rp));
   GINGR_CUDA_TRY(ctx, g->gt_part.alloc((size_t)gemvT_splits(ctx, 3 * Ml) * rp));
-  GINGR_CUDA_TRY(ctx, g->sums_part.alloc((size_t)3 * ceil_div(M, 256)));
+  GINGR_CUDA_TRY(ctx, g->sums_part.alloc((size_t)(bcpd ? 4 : 3) * ceil_div(M, 256)));
   GINGR_CUDA_TRY(ctx, g->pro_part.alloc((size_t)16 * ceil_div(std::max(Ml, 1), 256)));
   GINGR_CUDA_TRY(ctx, g->pro_sums.alloc(32));
   GINGR_CUDA_TRY(ctx, g->ds.alloc(DS_COUNT));
   GINGR_CUDA_TRY(ctx, g->is.alloc(IS_COUNT));
   GINGR_CUDA_TRY(ctx, g->flags.alloc(256));
-  GINGR_TRY(g->cholws.alloc(ctx, r, r + 1));
+  GINGR_TRY(g->cholws.alloc(ctx, r, r + 1 + xrows));
   GINGR_CUDA_TRY(ctx, g->alpha.alloc((size_t)rp));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->Mx.p, 0, sizeof(double) * (size_t)(r + 8) * rp, ctx->stream));
   if (g->Mx_packed.p) GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->Mx_packed.p, 0, sizeof(double) * g->Mx_packed.n, ctx->stream));   // unused slots stay 0
@@ -1540,18 +1786,25 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
   // ---- correspondence -------------------------------------------------------------------------------
   const double* icp_cp = nullptr;
   const double* icp_wcnt = nullptr;
-  if (cfg.algorithm == GINGR_ALGO_CPD) {
+  const bool bcpd = cfg.algorithm == GINGR_ALGO_BCPD;
+  if (cfg.algorithm == GINGR_ALGO_CPD || bcpd) {
     // non-finite fit / sigma2 / target: the reference's P is all NaN and the posterior fails
     if (tg->nonfinite) GINGR_TRY(validate_finite_enqueue(ctx, 3 * tg->N_total, tg->verts.p, g->is.p + IS_FAIL_POST));
-    GINGR_LAUNCH(ctx, cpd_prepare_kernel, ceil_div(M, 256), 256, 0, st, M, g->fit.p, g->estep.row_perm.p, g->estep.fit_soa.p, g->ds.p, cfg.w,
-                                                         (double)M / (double)tg->N_total, tg->maxabs, g->is.p + IS_FAIL_POST,
-                                                         g->prep_sync.p, g->estep.scal.p);
+    if (bcpd) {
+      GINGR_LAUNCH(ctx, bcpd_prepare_kernel, ceil_div(M, 256), 256, 0, st, M, g->fit.p, g->estep.fit_soa.p, g->bcpd_sigma.p, g->bcpd_alpha.p,
+                                                            g->estep.rowf.p, g->ds.p, cfg.w, 1.0 / (double)tg->N_total, tg->maxabs,
+                                                            g->is.p + IS_FAIL_POST, g->prep_sync.p, g->estep.scal.p);
+    } else {
+      GINGR_LAUNCH(ctx, cpd_prepare_kernel, ceil_div(M, 256), 256, 0, st, M, g->fit.p, g->estep.row_perm.p, g->estep.fit_soa.p, g->ds.p, cfg.w,
+                                                           (double)M / (double)tg->N_total, tg->maxabs, g->is.p + IS_FAIL_POST,
+                                                           g->prep_sync.p, g->estep.scal.p);
+    }
     GINGR_LAUNCHED(ctx);
     if (tg->N > 0) {
       EstepEvents ee;
       const bool pe = g->ev(2) != nullptr;
       if (pe) { ee.a0 = *g->ev(2); ee.a1 = *g->ev(3); ee.b0 = *g->ev(4); ee.b1 = *g->ev(5); }
-      GINGR_TRY(estep_enqueue(ctx, g->estep, M, tg->N, tg->soa.p, tg->soa_perm.p, false, pe ? &ee : nullptr));
+      GINGR_TRY(estep_enqueue(ctx, g->estep, M, tg->N, tg->soa.p, tg->soa_perm.p, bcpd, pe ? &ee : nullptr));
       GINGR_CUDA_TRY(ctx, gingr_copy_d2d(ctx, g->rows_ext.p, g->estep.rows.p, sizeof(double) * 4 * (size_t)M, st));
       GINGR_LAUNCH(ctx, xpx_total_kernel, 1, 256, 0, st, g->estep.plan.den_blocks, g->estep.xpx_part.p, g->rows_ext.p + (size_t)4 * M);
       GINGR_LAUNCHED(ctx);
@@ -1614,14 +1867,22 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
   const bool use_lm = cfg.use_landmark_correspondence && g->Ll > 0;
   const bool any_lm = cfg.use_landmark_correspondence && g->L > 0;
   const bool rhs_fused = !any_lm && gram_rhs_fusable(g->gram);
-  GINGR_LAUNCH(ctx, obs_kernel, oblocks, 256, 0, st, oa, g->rows_ext.p, icp_cp, g->closest.w.p, icp_wcnt, g->fit.p, m->ref.p, m->mean.p,
-                                      g->lm_pid.p, g->ds.p, g->is.p, g->wrow.p, g->u.p, g->sums_part.p,
-                                      rhs_fused ? g->resid.p : nullptr);
-  GINGR_LAUNCHED(ctx);
-  const double sigma_step = cfg.algorithm == GINGR_ALGO_ICP ? (cfg.initial_sigma - cfg.end_sigma) / (double)cfg.max_iterations : 0.0;
-  GINGR_LAUNCH(ctx, sigma2_kernel, 1, 32, 0, st, cfg.algorithm, oblocks, g->sums_part.p, g->rows_ext.p + (size_t)4 * M, sigma_step,
-                                 cfg.end_sigma, g->ds.p);
-  GINGR_LAUNCHED(ctx);
+  if (bcpd) {
+    GINGR_LAUNCH(ctx, bcpd_obs_kernel, oblocks, 256, 0, st, oa, g->rows_ext.p, g->bcpd_sigma.p, g->fit.p, m->ref.p, m->mean.p, g->lm_pid.p,
+                                             g->ds.p, g->is.p, g->wrow.p, g->u.p, g->sums_part.p, rhs_fused ? g->resid.p : nullptr);
+    GINGR_LAUNCHED(ctx);
+    GINGR_LAUNCH(ctx, bcpd_sigma2_kernel, 1, 32, 0, st, oblocks, g->sums_part.p, g->rows_ext.p + (size_t)4 * M, g->ds.p);
+    GINGR_LAUNCHED(ctx);
+  } else {
+    GINGR_LAUNCH(ctx, obs_kernel, oblocks, 256, 0, st, oa, g->rows_ext.p, icp_cp, g->closest.w.p, icp_wcnt, g->fit.p, m->ref.p, m->mean.p,
+                                        g->lm_pid.p, g->ds.p, g->is.p, g->wrow.p, g->u.p, g->sums_part.p,
+                                        rhs_fused ? g->resid.p : nullptr);
+    GINGR_LAUNCHED(ctx);
+    const double sigma_step = cfg.algorithm == GINGR_ALGO_ICP ? (cfg.initial_sigma - cfg.end_sigma) / (double)cfg.max_iterations : 0.0;
+    GINGR_LAUNCH(ctx, sigma2_kernel, 1, 32, 0, st, cfg.algorithm, oblocks, g->sums_part.p, g->rows_ext.p + (size_t)4 * M, sigma_step,
+                                   cfg.end_sigma, g->ds.p);
+    GINGR_LAUNCHED(ctx);
+  }
   // ---- posterior: rhs, Gram, Cholesky --------------------------------------------------------------------
   // several ranks: the partial matrix is written as packed lower tiles with the rhs behind them, so that ONE all-reduce of
   // half the bytes of the (r + 1) x rp rectangle combines both; it is unpacked into g->Mx afterwards
@@ -1651,8 +1912,15 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
   }
   if (g->keep_raw)
     GINGR_CUDA_TRY(ctx, gingr_copy_d2d(ctx, g->Mx_raw.p, g->Mx.p, sizeof(double) * (size_t)(r + 1) * rp, st));
+  int xrows = 0;
+  if (bcpd) {
+    xrows = 3 * M;
+    GINGR_LAUNCH(ctx, bcpd_var_rows_kernel, dim3(ceil_div(rp, 256), std::min(xrows, 65535)), 256, 0, st, xrows, r, rp, m->phi.p,
+                 m->sqrt_lambda.p, g->Mx.p + (size_t)(r + 1) * rp);
+    GINGR_LAUNCHED(ctx);
+  }
   g->rec(8);
-  GINGR_TRY(cholesky_enqueue(ctx, r, r + 1, g->Mx.p, rp, g->is.p + IS_INFO, &g->cholws));
+  GINGR_TRY(cholesky_enqueue(ctx, r, r + 1 + xrows, g->Mx.p, rp, g->is.p + IS_INFO, &g->cholws));
   return GINGR_OK;
 }
 
@@ -1716,6 +1984,11 @@ static int32_t enqueue_update_phase(gingr_registration* g, int probabilistic, ui
   // ---- commit, refresh the fit ------------------------------------------------------------------------------------------
   GINGR_LAUNCH(ctx, finalize_kernel, 1, 256, 0, st, r, probabilistic, vec + 5 * rp, g->alpha.p, g->ds.p, g->is.p);
   GINGR_LAUNCHED(ctx);
+  if (cfg.algorithm == GINGR_ALGO_BCPD) {
+    GINGR_LAUNCH(ctx, bcpd_state_kernel, ceil_div(M, 8), 256, 0, st, M, r, rp, g->bcpd_kappa, g->Mx.p + (size_t)(r + 1) * rp, g->rows_ext.p,
+                 g->ds.p, g->is.p, g->bcpd_alpha.p, g->bcpd_sigma.p);
+    GINGR_LAUNCHED(ctx);
+  }
   if (!g->skip_fit_refresh) GINGR_TRY(evaluate_fit(g, DS_SCALE, DS_T, DS_R2));
   g->rec(1);
   if (g->profiling && g->prof_iters < gingr_registration::EV_MAX_ITERS) g->prof_iters++;
@@ -2008,6 +2281,11 @@ int32_t gingr_initialize_state(gingr_registration* g, gingr_state* s, const doub
   const gingr_model* m = g->model;
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   s->rank = m->r;
+  if (g->cfg.algorithm == GINGR_ALGO_BCPD) {
+    GINGR_LAUNCH(ctx, bcpd_prior_kernel, ceil_div(m->M, 8), 256, 0, ctx->stream, m->M, m->r, m->rp, m->phi.p, m->sqrt_lambda.p,
+                 g->bcpd_alpha.p, g->bcpd_sigma.p);
+    GINGR_LAUNCHED(ctx);
+  }
   if (g->cfg.algorithm == GINGR_ALGO_ICP || g->cfg.has_initial_sigma) {
     s->sigma2 = g->cfg.initial_sigma;  // ICP.scala:74-78 ; CPD.scala:94 (initialSigma given)
   } else {
@@ -2037,8 +2315,10 @@ int32_t gingr_update(gingr_registration* g, const gingr_state* state_in, const d
                      uint64_t seed, gingr_state* state_out, double* alpha_out, double* fit_out) {
   if (!g || !state_in || !alpha_in || !state_out || !alpha_out)
     return gingr_fail(g ? g->ctx : nullptr, GINGR_ERR_ARG, "gingr_update: bad argument");
-  mcmc_invalidate(g);
   gingr_ctx* ctx = g->ctx;
+  if (probabilistic && g->cfg.algorithm == GINGR_ALGO_BCPD)
+    return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_update: BCPD registrations are deterministic");
+  mcmc_invalidate(g);
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const gingr_model* m = g->model;
   // Re-seed the device state unless the caller hands back exactly what the previous call returned
@@ -2080,6 +2360,8 @@ int32_t gingr_update_chain(gingr_registration* g, int32_t iters) {
 int32_t gingr_update_chain_sampled(gingr_registration* g, int32_t iters, uint64_t seed) {
   if (!g || iters < 0) return gingr_fail(g ? g->ctx : nullptr, GINGR_ERR_ARG, "gingr_update_chain_sampled: bad argument");
   gingr_ctx* ctx = g->ctx;
+  if (g->cfg.algorithm == GINGR_ALGO_BCPD)
+    return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_update_chain_sampled: BCPD registrations are deterministic");
   if (!g->state_valid) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_update_chain_sampled: no device-resident state");
   mcmc_invalidate(g);
   g->host_mirror_current = false;
@@ -2103,6 +2385,10 @@ int32_t gingr_update_batch(gingr_registration** regs, int32_t n, int32_t iters, 
     if (!regs[k] || regs[k]->ctx != ctx) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_update_batch: chains must share one ctx");
     if (!regs[k]->state_valid) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_update_batch: chain without device-resident state");
     if (regs[k]->profiling) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_update_batch: profiling is per registration");
+    if (probabilistic && regs[k]->cfg.algorithm == GINGR_ALGO_BCPD)
+      return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_update_batch: BCPD registrations are deterministic");
+  }
+  for (int k = 0; k < n; ++k) {
     mcmc_invalidate(regs[k]);
     regs[k]->host_mirror_current = false;
   }
@@ -2163,7 +2449,8 @@ int32_t gingr_registration_get_profile(gingr_registration* g, double* ms, int32_
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   for (int k = 0; k < 8; ++k) ms[k] = 0.0;
-  const bool cpd = g->cfg.algorithm == GINGR_ALGO_CPD && g->target->N > 0;
+  const bool bcpd = g->cfg.algorithm == GINGR_ALGO_BCPD && g->target->N > 0;   // E-step sweeps as CPD, never culled
+  const bool cpd = (g->cfg.algorithm == GINGR_ALGO_CPD && g->target->N > 0) || bcpd;
   for (int it = 0; it < g->prof_iters; ++it) {
     cudaEvent_t* e = &g->events[(size_t)it * gingr_registration::EV_PER_ITER];
     float t = 0.f;
@@ -2174,7 +2461,8 @@ int32_t gingr_registration_get_profile(gingr_registration* g, double* ms, int32_
     ms[4] += el(0, 1);
   }
   if (cpd) {
-    const EstepPlan& p = g->estep.plan;
+    EstepPlan p = g->estep.plan;
+    p.cull = p.cull && !bcpd;
     unsigned long long live[2] = {0, 0};
     if (p.cull) {
       GINGR_CUDA_TRY(ctx, cudaMemcpy(live, g->estep.live.p, sizeof(live), cudaMemcpyDeviceToHost));
@@ -2197,6 +2485,46 @@ int32_t gingr_state_download(gingr_registration* g, gingr_state* state_out, doub
   g->host_mirror_current = true;
   if (alpha_out) g->last_alpha.assign(alpha_out, alpha_out + g->model->r);
   else g->state_valid = false;
+  return GINGR_OK;
+}
+
+int32_t gingr_registration_set_bcpd(gingr_registration* g, double kappa) {
+  if (!g) return gingr_fail(nullptr, GINGR_ERR_ARG, "gingr_registration_set_bcpd: bad argument");
+  if (g->cfg.algorithm != GINGR_ALGO_BCPD) return gingr_fail(g->ctx, GINGR_ERR_ARG, "gingr_registration_set_bcpd: not a BCPD registration");
+  if (!(kappa > 0.0 && kappa < INFINITY)) return gingr_fail(g->ctx, GINGR_ERR_ARG, "gingr_registration_set_bcpd: kappa must be positive and finite");
+  if (kappa != g->bcpd_kappa) {
+    GINGR_CUDA_TRY(g->ctx, cudaSetDevice(g->ctx->device));
+    GINGR_CUDA_TRY(g->ctx, cudaStreamSynchronize(g->ctx->stream));
+    g->bcpd_kappa = kappa;
+    drop_graph(g);   // kappa is an argument of the captured bcpd_state_kernel
+  }
+  return GINGR_OK;
+}
+
+int32_t gingr_bcpd_state_download(gingr_registration* g, double* alpha, double* sigma) {
+  if (!g || (!alpha && !sigma)) return gingr_fail(g ? g->ctx : nullptr, GINGR_ERR_ARG, "gingr_bcpd_state_download: bad argument");
+  gingr_ctx* ctx = g->ctx;
+  if (g->cfg.algorithm != GINGR_ALGO_BCPD) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_bcpd_state_download: not a BCPD registration");
+  const int M = g->model->M;
+  GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  if (alpha) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(alpha, g->bcpd_alpha.p, sizeof(double) * M, cudaMemcpyDeviceToHost, ctx->stream));
+  if (sigma) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(sigma, g->bcpd_sigma.p, sizeof(double) * M, cudaMemcpyDeviceToHost, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  return GINGR_OK;
+}
+
+// Test window on the device digamma of the BCPD state update (not in gingr_cuda.h): out[i] = psi(x[i]).
+GINGR_API int32_t gingr_debug_digamma(gingr_ctx* ctx, int32_t n, const double* x, double* out) {
+  if (!ctx || n < 0 || (n > 0 && (!x || !out))) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_debug_digamma: bad argument");
+  if (n == 0) return GINGR_OK;
+  GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  DevBuf<double> d;
+  GINGR_CUDA_TRY(ctx, d.alloc((size_t)2 * n));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(d.p, x, sizeof(double) * n, cudaMemcpyHostToDevice, ctx->stream));
+  GINGR_LAUNCH(ctx, digamma_kernel, ceil_div(n, 256), 256, 0, ctx->stream, n, d.p, d.p + n);
+  GINGR_LAUNCHED(ctx);
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(out, d.p + n, sizeof(double) * n, cudaMemcpyDeviceToHost, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
   return GINGR_OK;
 }
 

@@ -20,6 +20,7 @@
 #include <functional>
 #include <optional>
 #include <stdexcept>
+#include <type_traits>
 #include <string>
 #include <utility>
 #include <vector>
@@ -174,6 +175,35 @@ struct IcpConfiguration {
   }
 };
 
+// The BCPD configuration (GINGR_ALGO_BCPD in gingr_cuda.h): the CPD fields with their CPD meaning, plus the Dirichlet
+// concentration kappa of the mixing-weight update (BCPD.scala:218)
+struct BcpdConfiguration {
+  int maxIterations = 100;
+  double threshold = 1e-10;
+  bool useLandmarkCorrespondence = true;
+  std::optional<double> initialSigma;
+  double w = 0.0;
+  double lambda = 1.0;
+  double kappa = 1.0;
+  static constexpr const char* name = "BCPD";
+
+  bool converged(const GeneralRegistrationState& last, const GeneralRegistrationState& current, double thr) const {
+    return std::fabs(last.sigma2 - current.sigma2) < thr;
+  }
+  gingr_config toPod() const {
+    CpdConfiguration c;
+    c.maxIterations = maxIterations;
+    c.threshold = threshold;
+    c.useLandmarkCorrespondence = useLandmarkCorrespondence;
+    c.initialSigma = initialSigma;
+    c.w = w;
+    c.lambda = lambda;
+    gingr_config pod = c.toPod();
+    pod.algorithm = GINGR_ALGO_BCPD;
+    return pod;
+  }
+};
+
 // sampling/evaluators/IndependentPointDistanceEvaluator.scala:26-32
 enum class EvaluationMode : int32_t { ModelToTargetEvaluation = GINGR_EVAL_MODEL_TO_TARGET,
                                       TargetToModelEvaluation = GINGR_EVAL_TARGET_TO_MODEL, SymmetricEvaluation = GINGR_EVAL_SYMMETRIC };
@@ -323,7 +353,8 @@ class Target {
   int N_ = 0;
 };
 
-// GingrAlgorithm[State, Config] (api/GingrAlgorithm.scala:65-302) for Config = CpdConfiguration / IcpConfiguration
+// GingrAlgorithm[State, Config] (api/GingrAlgorithm.scala:65-302) for Config = CpdConfiguration / IcpConfiguration /
+// BcpdConfiguration
 template <class Config>
 class GingrAlgorithm {
  public:
@@ -332,6 +363,7 @@ class GingrAlgorithm {
       : ctx_(&ctx), model_(&model), config_(std::move(config)) {
     const gingr_config pod = config_.toPod();
     ctx.check(gingr_registration_create(ctx.handle(), model.handle(), target.handle(), &pod, &h_));
+    if constexpr (std::is_same_v<Config, BcpdConfiguration>) ctx.check(gingr_registration_set_bcpd(h_, config_.kappa));
   }
   ~GingrAlgorithm() { if (h_) gingr_registration_destroy(h_); }
   GingrAlgorithm(const GingrAlgorithm&) = delete;
@@ -449,6 +481,14 @@ class GingrAlgorithm {
     return best;
   }
 
+  // BCPD registrations: (alpha[M], Sigma[M]), the mixing weights and per-vertex posterior variances the next update uses
+  // (throws Error(GINGR_ERR_ARG) for the other configurations)
+  std::pair<std::vector<double>, std::vector<double>> bcpdState() const {
+    std::vector<double> alpha(model_->points()), sigma(model_->points());
+    ctx_->check(gingr_bcpd_state_download(h_, alpha.data(), sigma.data()));
+    return {std::move(alpha), std::move(sigma)};
+  }
+
   gingr_registration* handle() const { return h_; }
 
  private:
@@ -469,5 +509,6 @@ class GingrAlgorithm {
 
 using CpdRegistration = GingrAlgorithm<CpdConfiguration>;  // registration/config/CPD.scala:117-160
 using IcpRegistration = GingrAlgorithm<IcpConfiguration>;  // registration/config/ICP.scala:84-110
+using BcpdRegistration = GingrAlgorithm<BcpdConfiguration>;  // GINGR_ALGO_BCPD (gingr_cuda.h)
 
 }  // namespace gingr

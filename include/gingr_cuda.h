@@ -64,6 +64,17 @@ extern "C" {
 /* which GingrAlgorithm subclass */
 #define GINGR_ALGO_CPD 0 /* registration/config/CPD.scala:117 CpdRegistration */
 #define GINGR_ALGO_ICP 1 /* registration/config/ICP.scala:84 IcpRegistration */
+/* BCPD correspondences (other/algorithms/cpd/BCPD.scala) on GiNGR's hooks -- this project's reading, the reference ships no
+ * BCPD configuration: the BCPD E-step with per-vertex mixing weights alpha and posterior variances Sigma, observations
+ * xhat_m with noise sigma2 lambda / nu_m I3, the GPMM posterior as for CPD, sigma2 = (sXX - 2 sXY + sYY + sigma2 sigma2bar) /
+ * (3 Nhat), alpha_m = exp(psi(kappa + nu_m) - psi(kappa M + Nhat)), Sigma_m = tr(posterior cov_m) / 3.  w, lambda,
+ * initial_sigma, max_iterations, threshold, use_landmark_correspondence as for CPD; kappa: gingr_registration_set_bcpd.
+ * Single GPU, deterministic updates only (the probabilistic / MCMC calls return GINGR_ERR_UNSUPPORTED).
+ * Scale: the outlier term of the E-step is c = w / N as in BCPD.scala (no volume normalisation), against Gaussians of
+ * height (2 pi sigma2)^-3/2.  With w > 0 on data whose sigma2 is large (coordinates of hundreds of units: the initial sigma2
+ * is about the squared extent), c outweighs every Gaussian, Nhat becomes tiny and sigma2 sigma2bar / (3 Nhat) makes sigma2
+ * grow without bound.  Such data want w = 0, or coordinates scaled so that (2 pi sigma2)^-3/2 is well above w / N. */
+#define GINGR_ALGO_BCPD 2
 
 typedef struct gingr_ctx gingr_ctx;
 typedef struct gingr_model gingr_model;               /* scalismo PointDistributionModel on device */
@@ -324,6 +335,13 @@ GINGR_API int32_t gingr_update_batch(gingr_registration** regs, int32_t n, int32
 /* Read back the device-resident state after gingr_update_chain / gingr_update_batch. */
 GINGR_API int32_t gingr_state_download(gingr_registration* reg, gingr_state* state_out, double* alpha_out,
                                        double* fit_out);
+/* BCPD registrations: the Dirichlet concentration kappa of the mixing-weight update (BCPD.scala:218; default 1, > 0). */
+GINGR_API int32_t gingr_registration_set_bcpd(gingr_registration* reg, double kappa);
+/* BCPD registrations: the per-vertex mixing weights alpha[M] and posterior variances sigma[M] the next iteration's E-step
+ * uses.  gingr_registration_create and gingr_initialize_state set alpha = 1 / M and Sigma_m = tr(Phi_m Lambda Phi_m^T) / 3
+ * (the prior variance);
+ * every committed iteration advances them, a ModelFlexibilityError iteration leaves them.  Either pointer may be NULL. */
+GINGR_API int32_t gingr_bcpd_state_download(gingr_registration* reg, double* alpha /*[M]*/, double* sigma /*[M]*/);
 
 /* GingrAlgorithm.computePosterior(current) (GingrAlgorithm.scala:281-302): the correspondences and uncertainties of the
  * registration's configuration (CPD E-step / ICP flavours, landmarks) at `state`, then the posterior model as

@@ -84,6 +84,9 @@ object GingrCudaNative {
   val mcmcStats      = fn("gingr_mcmc_stats", JAVA_INT, ADDRESS, ADDRESS, ADDRESS)
   val mcmcBest       = fn("gingr_mcmc_best", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS)
   val stateDownload  = fn("gingr_state_download", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS)
+  // BCPD registrations (GINGR_ALGO_BCPD): the Dirichlet concentration kappa, and the per-vertex mixing weights / variances
+  val registrationSetBcpd = fn("gingr_registration_set_bcpd", JAVA_INT, ADDRESS, JAVA_DOUBLE)
+  val bcpdStateDownload   = fn("gingr_bcpd_state_download", JAVA_INT, ADDRESS, ADDRESS, ADDRESS)
   val modelNewReference = fn("gingr_model_new_reference", JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, ADDRESS)
   // GPMM construction on the device (api/gpmm/GPMMHelper.scala:99-129) and the way back into scalismo's storage
   val gpmmGaussianMixture = fn("gingr_gpmm_gaussian_mixture", JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, JAVA_INT, JAVA_INT,
