@@ -151,8 +151,9 @@ class Model:
         close in space (fingers, the lips of a jaw) do not.  This project's reading of the kernel: L = D - A, the graph
         Laplacian of the triangle edges with unit weights; Ks = scaling (L + gamma I)^-1, or scaling pinv(L) for gamma = 0;
         K = Ks (x) I3; then approximateGPCholesky with the stopping rule of gaussianMixture.  Needs triangles and at most 6000
-        vertices.  The models are nearly full rank (about 0.97-0.99 of 3M at relativeTolerance 0.01); the registrations take
-        a rank of at most 9472, so above about 3200 vertices pass maxRank.  With gamma = 0 the kernel has rank
+        vertices.  The models are nearly full rank (about 0.97-0.99 of 3M at relativeTolerance 0.01); registrations,
+        posteriors and solves take every rank the builders produce, up to 18 000 (tested up to that rank), so maxRank is
+        only needed to trade accuracy for time.  With gamma = 0 the kernel has rank
         3 (M - #components); at relativeTolerance 0 the factorisation would go on to take noise columns from the
         rounding-level residual of the null space, so a full-rank gamma = 0 model wants a small positive tolerance (1e-12
         suffices).  Raises FloatingPointError when L + gamma I is not numerically positive definite."""

@@ -11,7 +11,7 @@
 //   chol_syrk_kernel    trailing update C -= X X^T on DMMA.8x8x4 (64 x 64 tiles, K = 64)
 // Rows below the square part (right-hand sides stored as extra rows) ride along, which performs the
 // forward substitution L^-1 b inside the factorisation.  The backward substitution L^-T z is a sync-free
-// multi-CTA kernel: one CTA per 64-block, consuming solved blocks as their ready flags appear.
+// multi-CTA kernel: one CTA per 64-block, taken by ticket, consuming solved blocks as their ready flags appear.
 #include <stdlib.h>
 
 #include <algorithm>
@@ -285,9 +285,16 @@ __global__ void __launch_bounds__(128) chol_syrk_kernel(int nrows, int n, int j0
 
 // ---------------------------------------------------------------------------------------------
 // backward substitution  L^T c = z,  one CTA per 64-block, blocks become ready from the last one up.
+// A CTA takes its block from an atomic ticket: ticket t solves block k = nb - 1 - t and waits only for the blocks
+// i > k, which tickets smaller than its own hold.  A ticket is drawn only by a running CTA, so every block waited for
+// belongs to a resident CTA that itself waits only for smaller tickets: the spin waits cannot deadlock whatever the grid
+// size (nb may exceed the SM count) or whatever else occupies the GPU.  The arithmetic depends on the block alone, not
+// on the CTA that solves it.
 // Each CTA first inverts its own diagonal block (off the critical path: it would otherwise spin on the
 // ready flags), accumulates  z_k - sum_{i>k} L_ik^T c_i  as the c_i appear, and finishes with the
 // 64 x 64 product  c_k = D^-T acc.
+// flags: nb + 2 ints (block flags, finished CTAs, ticket), zero on entry; the last CTA out zeroes them again, so a
+// captured graph replays without a memset node.
 // ---------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) chol_backsolve_kernel(int n, const double* __restrict__ L, int ld,
                                                              const double* __restrict__ z, double* __restrict__ c,
@@ -297,9 +304,12 @@ __global__ void __launch_bounds__(256) chol_backsolve_kernel(int n, const double
   __shared__ double sc[NB];
   __shared__ double sacc[4][NB];
   __shared__ double acc[NB];
+  __shared__ int s_ticket;
   const int nb = (n + NB - 1) / NB;
-  const int k = nb - 1 - blockIdx.x;  // first CTAs own the last blocks (solved first)
   const int tid = threadIdx.x;
+  if (tid == 0) s_ticket = atomicAdd((int*)&flags[nb + 1], 1);
+  __syncthreads();
+  const int k = nb - 1 - s_ticket;  // the first tickets own the last blocks (solved first)
   const int k0 = k * NB, kcnt = min(NB, n - k0);
   for (int e = tid; e < NB * NB; e += 256) {
     const int i = e >> 6, j = e & 63;
@@ -358,7 +368,12 @@ __global__ void __launch_bounds__(256) chol_backsolve_kernel(int n, const double
   if (tid < kcnt) c[k0 + tid] = (sacc[0][tid] + sacc[1][tid]) + (sacc[2][tid] + sacc[3][tid]);
   __threadfence();
   __syncthreads();
-  if (tid == 0) flags[k] = 1;
+  if (tid == 0) {
+    flags[k] = 1;
+    if (atomicAdd((int*)&flags[nb], 1) == nb - 1) {   // last CTA out: every flag has been read and every ticket drawn
+      for (int e = 0; e <= nb + 1; ++e) flags[e] = 0;
+    }
+  }
 }
 
 // n <= 64 (one block): plain right-looking back substitution by 64 threads -- the general kernel would spend 50 us
@@ -469,8 +484,6 @@ int32_t chol_backsolve_enqueue(gingr_ctx* ctx, int n, const double* d_L, int ld,
     GINGR_CUDA_TRY(ctx, cudaGetLastError());
     return GINGR_OK;
   }
-  if (nb > ctx->num_sms) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "rank too large for the sync-free back solve");
-  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(d_flags, 0, sizeof(int) * nb, ctx->stream));
   chol_backsolve_kernel<<<nb, 256, 0, ctx->stream>>>(n, d_L, ld, d_z, d_c, d_flags);
   GINGR_LAUNCHED(ctx);
   GINGR_CUDA_TRY(ctx, cudaGetLastError());

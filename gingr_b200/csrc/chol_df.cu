@@ -450,12 +450,18 @@ GINGR_KERNEL((DF_THREADS, 2), chol_small_kernel, int n, int nrows, double* __res
 
 // ---------------------------------------------------------------------------------------------
 // backward substitution  L^T c = z  with the published inverses Z_k = L_kk^-1 of the factorisation above: one CTA per
-// 64-block, blocks become ready from the last one up.  CTA k accumulates  z_k - sum_{i>k} L_ik^T c_i  as the c_i appear
+// 64-block, blocks become ready from the last one up.  A CTA takes its block from an atomic ticket, ticket t solves block
+// k = nb - 1 - t, and it waits only for blocks i > k, which tickets smaller than its own hold.  A ticket is drawn only by
+// a running CTA, so every block waited for belongs to a CTA that is already resident and itself waits only for smaller
+// tickets: the spin waits cannot deadlock whatever the grid size (nb may exceed the SM count) or whatever else occupies
+// the GPU -- the argument of the factorisation above.  The block, not the CTA, fixes the arithmetic, so a block gives the
+// same bits whichever CTA solves it.  CTA k accumulates  z_k - sum_{i>k} L_ik^T c_i  as the c_i appear
 // and finishes with c_k = Z_k^T acc.  Everything the critical step needs is in shared memory BEFORE its flag arrives:
 // Z_k, and the L_ik blocks stream through a two-deep cp.async ring one block ahead of the flags, so between two flags
 // there is one 64 x 64 mat-vec from shared memory, one more with Z_k^T, a fence and the flag (chol.cu's kernel inverted
 // its diagonal block itself and read every L_ik from global memory after the flag: 5.6 us per block, now ~2).
-// flags: nb + 1 ints, zero on entry; the last CTA out zeroes them again.
+// flags: nb + 2 ints (block flags, finished CTAs, ticket), zero on entry; the last CTA out zeroes them again, so a captured
+// graph replays without a memset node.
 // ---------------------------------------------------------------------------------------------
 constexpr int BS_THREADS = 256;
 constexpr size_t BS_SMEM = (size_t)(3 * TB * TB + TB + 4 * TB + TB) * sizeof(double);
@@ -469,9 +475,12 @@ __global__ void __launch_bounds__(BS_THREADS) chol_backsolve_z_kernel(int n, con
   double* sc = bsm + 3 * TB * TB;      // [64] c_i
   double* sacc = sc + TB;              // [4][64] partial sums
   double* acc = sacc + 4 * TB;         // [64]
+  __shared__ int s_ticket;
   const int nb = (n + TB - 1) / TB;
-  const int k = nb - 1 - (int)blockIdx.x;   // first CTAs own the last blocks (solved first)
   const int tid = threadIdx.x, col = tid & 63, part = tid >> 6;
+  if (tid == 0) s_ticket = atomicAdd(&flags[nb + 1], 1);
+  __syncthreads();
+  const int k = nb - 1 - s_ticket;   // the first tickets own the last blocks (solved first)
   const int k0 = k * TB, kcnt = min(TB, n - k0);
   auto load_block = [&](double* dst, int i) {   // rows of block i, columns of block k (k < i: all 64 columns exist)
     const int i0 = i * TB, icnt = min(TB, n - i0);
@@ -526,8 +535,8 @@ __global__ void __launch_bounds__(BS_THREADS) chol_backsolve_z_kernel(int n, con
   __syncthreads();
   if (tid == 0) {
     st_release(&flags[k], 1);
-    if (atomicAdd(&flags[nb], 1) == nb - 1) {   // last CTA out: every flag has been read for the last time
-      for (int e = 0; e <= nb; ++e) flags[e] = 0;
+    if (atomicAdd(&flags[nb], 1) == nb - 1) {   // last CTA out: every flag has been read and every ticket drawn
+      for (int e = 0; e <= nb + 1; ++e) flags[e] = 0;
     }
   }
 }
@@ -542,9 +551,9 @@ int32_t CholWs::alloc(gingr_ctx* ctx, int n, int nrows) {
     GINGR_CUDA_TRY(ctx, cudaMemsetAsync(sync.p, 0, sizeof(int) * ns, ctx->stream));
   }
   GINGR_CUDA_TRY(ctx, linv.alloc((size_t)nb * TB * TB));
-  if (bsync.n < (size_t)nb + 1) {
-    GINGR_CUDA_TRY(ctx, bsync.alloc((size_t)nb + 1));
-    GINGR_CUDA_TRY(ctx, cudaMemsetAsync(bsync.p, 0, sizeof(int) * ((size_t)nb + 1), ctx->stream));
+  if (bsync.n < (size_t)nb + 2) {   // block flags, finished CTAs, ticket
+    GINGR_CUDA_TRY(ctx, bsync.alloc((size_t)nb + 2));
+    GINGR_CUDA_TRY(ctx, cudaMemsetAsync(bsync.p, 0, sizeof(int) * ((size_t)nb + 2), ctx->stream));
   }
   cap_n = std::max(cap_n, n);
   cap_nrows = std::max(cap_nrows, nrows);
@@ -598,8 +607,7 @@ int32_t chol_backsolve_z_enqueue(gingr_ctx* ctx, int n, const double* d_L, int l
     attr_device = ctx->device;
   }
   const int nb = ceil_div(n, TB);
-  if ((size_t)nb + 1 > ws.bsync.n || (size_t)nb * TB * TB > ws.linv.n) return gingr_fail(ctx, GINGR_ERR_ARG, "back solve: workspace too small");
-  if (nb > ctx->num_sms) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "rank too large for the sync-free back solve");
+  if ((size_t)nb + 2 > ws.bsync.n || (size_t)nb * TB * TB > ws.linv.n) return gingr_fail(ctx, GINGR_ERR_ARG, "back solve: workspace too small");
   chol_backsolve_z_kernel<<<nb, BS_THREADS, BS_SMEM, ctx->stream>>>(n, d_L, ld, d_z, d_c, ws.linv.p, ws.bsync.p);
   GINGR_LAUNCHED(ctx);
   GINGR_CUDA_TRY(ctx, cudaGetLastError());

@@ -48,7 +48,8 @@ struct CholWs {
 // ws == nullptr (or GINGR_CHOL_DF=0): the kernel-per-step form of chol.cu; else one persistent data-flow kernel.
 int32_t cholesky_enqueue(gingr_ctx* ctx, int n, int nrows, double* d_A, int ld, int* d_info, CholWs* ws = nullptr);
 int32_t cholesky_df_enqueue(gingr_ctx* ctx, int n, int nrows, double* d_A, int ld, int* d_info, CholWs& ws);
-// c = L^-T z  (sync-free multi-CTA backward substitution).  d_flags: >= ceil(n/64) ints of scratch.
+// c = L^-T z  (sync-free multi-CTA backward substitution, any n).  d_flags: >= ceil(n/64) + 2 ints, zero when first
+// used (the kernel leaves them zero).
 // ws (optional): the workspace the factor was computed with by the data-flow kernel -- the back substitution then uses
 // the published inverses of the diagonal blocks (chol_df.cu); GINGR_CHOL_DF=0 or ws == nullptr: chol.cu's kernel.
 int32_t chol_backsolve_enqueue(gingr_ctx* ctx, int n, const double* d_L, int ld, const double* d_z, double* d_c,

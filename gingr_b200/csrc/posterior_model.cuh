@@ -168,6 +168,7 @@ int32_t gingr_registration_posterior_model(gingr_registration* g, const gingr_st
   GINGR_CUDA_TRY(ctx, c.alloc(rp));
   GINGR_CUDA_TRY(ctx, info.alloc(4));
   GINGR_CUDA_TRY(ctx, flags.alloc((size_t)ceil_div(r, 64) + 8));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(flags.p, 0, sizeof(int) * flags.n, st));
   GINGR_TRY(cws.alloc(ctx, r, 2 * r + 1));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(sys.p, 0, sizeof(double) * (size_t)(2 * r + 8) * rp, st));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(info.p, 0, sizeof(int) * 4, st));

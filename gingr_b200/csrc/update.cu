@@ -1318,10 +1318,11 @@ static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const do
   GINGR_CUDA_TRY(ctx, s.fit_local.alloc((size_t)3 * M));
   GINGR_CUDA_TRY(ctx, s.ds.alloc(DS_COUNT));
   GINGR_CUDA_TRY(ctx, s.is.alloc(IS_COUNT));
-  GINGR_CUDA_TRY(ctx, s.flags.alloc(256));
+  GINGR_CUDA_TRY(ctx, s.flags.alloc((size_t)ceil_div(r, 64) + 2));   // back-solve flags, finished CTAs, ticket
   GINGR_TRY(s.cholws.alloc(ctx, r, r + 1 + xrows));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(s.Mx.p, 0, sizeof(double) * (size_t)(r + 8) * rp, st));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(s.is.p, 0, sizeof(int) * IS_COUNT, st));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(s.flags.p, 0, sizeof(int) * s.flags.n, st));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s.wrow.p, wrow.data(), sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(s.u.p, u.data(), sizeof(double) * 3 * M, cudaMemcpyHostToDevice, st));
   double hds[DS_COUNT];
@@ -1469,6 +1470,7 @@ int32_t gingr_spd_solve(gingr_ctx* ctx, int32_t n, const double* A, int32_t nrhs
   GINGR_CUDA_TRY(ctx, x.alloc(np));
   GINGR_CUDA_TRY(ctx, info.alloc(4));
   GINGR_CUDA_TRY(ctx, flags.alloc((size_t)ceil_div(n, 64) + 8));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(flags.p, 0, sizeof(int) * flags.n, ctx->stream));
   GINGR_TRY(ws.alloc(ctx, n, nrows));
   GINGR_CUDA_TRY(ctx, cudaEventCreate(&ev.e0));
   GINGR_CUDA_TRY(ctx, cudaEventCreate(&ev.e1));
@@ -1641,7 +1643,7 @@ int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, cons
   GINGR_CUDA_TRY(ctx, g->pro_sums.alloc(32));
   GINGR_CUDA_TRY(ctx, g->ds.alloc(DS_COUNT));
   GINGR_CUDA_TRY(ctx, g->is.alloc(IS_COUNT));
-  GINGR_CUDA_TRY(ctx, g->flags.alloc(256));
+  GINGR_CUDA_TRY(ctx, g->flags.alloc((size_t)ceil_div(r, 64) + 2));   // back-solve flags, finished CTAs, ticket
   GINGR_TRY(g->cholws.alloc(ctx, r, r + 1 + xrows));
   GINGR_CUDA_TRY(ctx, g->alpha.alloc((size_t)rp));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->Mx.p, 0, sizeof(double) * (size_t)(r + 8) * rp, ctx->stream));
@@ -1649,6 +1651,7 @@ int32_t gingr_registration_create(gingr_ctx* ctx, const gingr_model* model, cons
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->fit_local.p, 0, sizeof(double) * 3 * Mmax, ctx->stream));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->ds.p, 0, sizeof(double) * DS_COUNT, ctx->stream));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->is.p, 0, sizeof(int) * IS_COUNT, ctx->stream));
+  GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->flags.p, 0, sizeof(int) * g->flags.n, ctx->stream));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(g->is.p + IS_RETRY, &g->retry_counter, sizeof(int), cudaMemcpyHostToDevice, ctx->stream));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->alpha.p, 0, sizeof(double) * rp, ctx->stream));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g->rows_ext.p, 0, sizeof(double) * ((size_t)4 * M + 8), ctx->stream));

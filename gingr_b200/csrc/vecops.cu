@@ -3,7 +3,8 @@
 //   gemv_rows   out[k] = sum_a Phi[k][a] v[a]      instance / posterior mean evaluation at the mesh points:
 //               scalismo `instance(alpha) = ref + mean + basis (sqrt(lambda) * alpha)` (SURVEY.md A1), call sites
 //               GingrAlgorithm.scala:211, :222, :224 and ModelFittingParameters.scala:134.  One warp per row,
-//               two right-hand sides per pass (instance(alpha_old) and instance(alpha_new) share the read).
+//               two right-hand sides per pass (instance(alpha_old) and instance(alpha_new) share the read) while both
+//               fit shared memory (r <= 12 800), one per pass up to r = 25 600.
 //   gemvT       out[a] = s_a sum_k Phi[k][a] u[k]   right-hand side Q^T L^-1 (y - m) of the regression
 //               (SURVEY.md A3).  Thread per column, rows split over CTAs, fixed-order reduction.
 // Both read Phi (8 * 3M * r bytes) exactly once; Phi is row-major [3M][rp] so both are fully coalesced.
@@ -263,6 +264,11 @@ int32_t gemv_rows_enqueue(gingr_ctx* ctx, int rows, int r, int rp, const double*
   if (rows <= 0) return GINGR_OK;
   // one row per warp; four when many chains share the launch (batch.cuh) -- a row's dot product does not depend on it
   const int blocks = std::max(1, std::min(ctx->num_sms * 4, ceil_div(rows, ctx->rec ? 32 : 8)));
+  // two vectors that do not fit shared memory together (r > 12 800) are two one-vector passes: the same per-row sums
+  if (nvec == 2 && (size_t)2 * r * sizeof(double) > 200 * 1024) {
+    GINGR_TRY(gemv_rows_enqueue(ctx, rows, r, rp, d_phi, 1, d_v0, nullptr, d_out0, nullptr, d_scale));
+    return gemv_rows_enqueue(ctx, rows, r, rp, d_phi, 1, d_v1, nullptr, d_out1, nullptr, d_scale);
+  }
   const size_t smem = (size_t)nvec * r * sizeof(double);
   if (smem > 48 * 1024) {
     static bool set1 = false, set2 = false;

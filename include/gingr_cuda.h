@@ -188,8 +188,8 @@ GINGR_API int32_t gingr_gpmm_gaussian_symmetric(gingr_ctx* ctx, int32_t M, const
  *   K = DiagonalKernel(Ks, 3) = Ks (x) I3, then approximateGPCholesky with the stopping rule and outputs of
  *       gingr_gpmm_gaussian_mixture; the mean is zero.
  * Ks is formed densely on the device, so M <= 6000 (GINGR_ERR_UNSUPPORTED above).  Its spectrum decays like 1/k: at
- * rel_tol 0.01 the rank is about 0.97-0.99 of 3M, and the registrations take rank <= 9472 (about M <= 3200 at rel_tol 0.01):
- * larger templates want max_rank.  With gamma = 0 the kernel has rank 3 (M - #components): at rel_tol = 0 the
+ * rel_tol 0.01 the rank is about 0.97-0.99 of 3M.  Registrations, posteriors and solves take any rank the builders
+ * produce, up to 18 000 (3 x 6000 scalar columns); the suite runs them up to that rank.  With gamma = 0 the kernel has rank 3 (M - #components): at rel_tol = 0 the
  * factorisation goes on past that rank and takes up to 3 * #components more columns from the rounding-level residual of
  * the null space, so a full-rank gamma = 0 model wants a small positive rel_tol (1e-12 suffices).  Requires T > 0,
  * indices in [0, M), scaling > 0 and gamma >= 0 finite, rel_tol >= 0, max_rank >= 0 and a single-GPU context.  Returns GINGR_MODEL_FLEXIBILITY with *out = NULL when L + gamma I is not
