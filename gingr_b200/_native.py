@@ -131,6 +131,8 @@ SIGNATURES = {
     "gingr_mcmc_batch": (c_int32, [POINTER(c_void_p), c_int32, c_int32, c_uint64]),
     "gingr_mcmc_stats": (c_int32, [c_void_p, dp, ip]),
     "gingr_mcmc_best": (c_int32, [c_void_p, POINTER(GingrState), dp, dp]),
+    "gingr_mcmc_collect": (c_int32, [c_void_p, c_int32, c_int32, c_int32]),
+    "gingr_mcmc_samples": (c_int32, [POINTER(c_void_p), c_int32, POINTER(c_int64), dp, dp, dp]),
     "gingr_registration_set_profiling": (c_int32, [c_void_p, c_int32]),
     "gingr_registration_get_profile": (c_int32, [c_void_p, dp, ip]),
 }

@@ -827,6 +827,13 @@ class GingrAlgorithm:
         self.ctx.check(self.ctx._lib.gingr_mcmc_best(self.handle, ctypes.byref(st), nat.as_dp(alpha), nat.as_dp(fit)))
         return GeneralRegistrationState.from_pod(st, alpha, fit)
 
+    def collectSamples(self, collection: Optional["SampleCollection"]):
+        """Collect the chain's states on the device by the rule of LogHelper.samplesFromLog (LogHelper.scala:29-43), for
+        the posterior variance maps (sample_statistics).  None switches collection off.  Set it after
+        configureProbabilistic, which discards it; the accumulators restart with every fresh chain."""
+        c = SampleCollection(takeEveryN=0) if collection is None else collection
+        self.ctx.check(self.ctx._lib.gingr_mcmc_collect(self.handle, int(c.burnIn), int(c.takeEveryN), int(c.total)))
+
     def generatorNames(self, settings: "ProbabilisticSettings"):
         """generatedBy of the ten leaves of generatorCombined (GingrAlgorithm.scala:177-190, sampling/Generator.scala:31-83),
         in the order of the device's leaf index (mcmcStats counts[1])."""
@@ -835,7 +842,8 @@ class GingrAlgorithm:
                 [f"Translation{a}-{float(v)!r}" for a, v in zip("XYZ", t)] + [f"RandomShape-{float(v)!r}" for v in sh])
 
     def runProbabilistic(self, initialState: GeneralRegistrationState, settings: "ProbabilisticSettings", seed: int = 0,
-                         iterations: Optional[int] = None, acceptRejectLogger=None, callBackLogger=None) -> GeneralRegistrationState:
+                         iterations: Optional[int] = None, acceptRejectLogger=None, callBackLogger=None,
+                         sampleCollection: Optional["SampleCollection"] = None) -> GeneralRegistrationState:
         """GingrAlgorithm.run with probabilisticSettings (:115-175): maxIterations - 1 MH steps, returns the best sample
         (:160-163) with status MaxIteration unless the chain ended in ModelFlexibilityError.
 
@@ -844,8 +852,12 @@ class GingrAlgorithm:
         the same chain -- same seed, same draws, same decisions -- is advanced one step per call and read back after
         each step, as scalismo's logged iterator does (:126-134).  A rejected proposal is logged with its generator name
         and log values; its scale (the only parameter jsonLogFormat keeps for a rejected sample) is the current
-        state's, which differs from the proposal's only for a rejected informed SimilarityTransforms step."""
+        state's, which differs from the proposal's only for a rejected informed SimilarityTransforms step.
+
+        sampleCollection: collect the chain's states on the device (collectSamples); read them with sample_statistics."""
         self.configureProbabilistic(settings)
+        if sampleCollection is not None:
+            self.collectSamples(sampleCollection)
         logged = acceptRejectLogger is not None or callBackLogger is not None
         # the evaluators depend on the parameters only; evaluated BEFORE initializeState because gingr_evaluate_log_value
         # replaces the device-resident state the chain starts from
@@ -919,6 +931,81 @@ def mcmc_batch(chains: Sequence[GingrAlgorithm], iters: int, seed: int = 0):
     ctx = chains[0].ctx
     arr = (ctypes.c_void_p * len(chains))(*[c.handle for c in chains])
     ctx.check(ctx._lib.gingr_mcmc_batch(arr, len(chains), int(iters), int(seed)))
+
+
+@dataclass(frozen=True)
+class SampleCollection:
+    """Which chain states are collected (LogHelper.samplesFromLog, LogHelper.scala:29-43, with its defaults): state i (0 =
+    the start state, i >= 1 = the state after the i-th MH step) when i >= burnIn, (i - burnIn) % takeEveryN == 0 and
+    i < total, unless state i - 1 ended the chain with a ModelFlexibilityError.  takeEveryN = 0: no collection."""
+    burnIn: int = 0
+    takeEveryN: int = 50
+    total: int = 100
+
+
+@dataclass
+class SampleStatistics:
+    """Per-vertex statistics of collected chain states (gingr_mcmc_samples): count, mean fit [M, 3], covariance [M, 3, 3]
+    (1 / (count - 1) normalisation; NaN below 2 samples), mean of the sample's unit vertex normals [M, 3] (None without
+    model triangles).  The maps of PosteriorHelper (PosteriorHelper.scala:31-79) are closed forms of these."""
+    count: int
+    mean: np.ndarray
+    cov: np.ndarray
+    normal: Optional[np.ndarray]
+
+    def distanceMapTotal(self) -> np.ndarray:
+        """PosteriorHelper.computeDistanceMapFromMeshesTotal (:31-53): the trace of the per-vertex covariance."""
+        return np.trace(self.cov, axis1=1, axis2=2).copy()
+
+    def distanceMapNormal(self, reference=None, triangles=None, sumNormals: bool = True) -> np.ndarray:
+        """PosteriorHelper.computeDistanceMapFromMeshesNormal (:55-79): nu^T cov nu with nu the mean of the sample normals
+        (sumNormals, not renormalised) or the unit vertex normal of the reference mesh (reference points and triangles)."""
+        if sumNormals:
+            if self.normal is None:
+                raise ValueError("no sample normals: the model has no triangles")
+            nu = self.normal
+        else:
+            if reference is None or triangles is None:
+                raise ValueError("sumNormals = False needs the reference points and triangles")
+            from .helper import vertex_normals
+            nu = vertex_normals(reference, triangles)
+        return np.einsum("mi,mij,mj->m", nu, self.cov, nu)
+
+    def merge(self, other: "SampleStatistics") -> "SampleStatistics":
+        """The statistics of both sample sets (Chan et al.'s pairwise update, the formula gingr_mcmc_samples pools chains
+        with), e.g. of chains divided over GPUs or processes (chain_range)."""
+        na, nb = int(self.count), int(other.count)
+        if nb == 0:
+            return self
+        if na == 0:
+            return other
+        n = na + nb
+        zero = np.zeros((self.mean.shape[0], 3, 3))
+        sa = self.cov * float(na - 1) if na > 1 else zero      # one sample: no scatter
+        sb = other.cov * float(nb - 1) if nb > 1 else zero
+        d = other.mean - self.mean
+        mean = self.mean + d * (float(nb) / float(n))
+        scatter = (sa + sb) + d[:, :, None] * d[:, None, :] * (float(na) * float(nb) / float(n))
+        normal = None
+        if self.normal is not None and other.normal is not None:
+            normal = (self.normal * float(na) + other.normal * float(nb)) / float(n)
+        return SampleStatistics(n, mean, scatter / float(n - 1), normal)
+
+
+def sample_statistics(chains: Sequence[GingrAlgorithm]) -> SampleStatistics:
+    """The collected statistics of the chains (collectSamples), pooled on the device in the order of `chains`; the chains
+    share one ctx and one model."""
+    ctx, model = chains[0].ctx, chains[0].model
+    arr = (ctypes.c_void_p * len(chains))(*[c.handle for c in chains])
+    count = ctypes.c_int64()
+    ctx.check(ctx._lib.gingr_mcmc_samples(arr, len(chains), ctypes.byref(count), None, None, None))
+    n = int(count.value)
+    mean = np.empty((model.M, 3))
+    cov = np.full((model.M, 3, 3), np.nan)
+    normal = np.empty((model.M, 3)) if model.T > 0 else None
+    ctx.check(ctx._lib.gingr_mcmc_samples(arr, len(chains), None, nat.as_dp(mean), nat.as_dp(cov) if n >= 2 else None,
+                                          nat.as_dp(normal)))
+    return SampleStatistics(n, mean, cov, normal)
 
 
 @dataclass

@@ -353,6 +353,111 @@ GINGR_KERNEL_NB(mcmc_restore_ints_kernel, const int* __restrict__ flag, int* __r
     for (int k = 0; k < IS_COUNT; ++k) best_is[k] = is[k];
 }
 
+// ---- sample collection: LogHelper.samplesFromLog (LogHelper.scala:29-43) and the moments behind
+// PosteriorHelper.computeDistanceMapFromMeshes* (PosteriorHelper.scala:31-79), accumulated on the device ---------------
+// Per vertex ACC_WORDS doubles: [0, 3) mean fit position, [3, 9) scatter sum (x - mean)(x - mean)^T as xx xy xz yy yz zz,
+// [9, 12) sum of the unit vertex normals of the collected fits; the sample count per vertex beside them.  The products
+// feeding sums are rounded one by one (no FMA contraction), so that tests/test_mcmc_samples_host.py restates them in numpy.
+constexpr int ACC_WORDS = 12;
+__device__ __constant__ const int SCATTER_ROW[6] = {0, 0, 0, 1, 1, 2}, SCATTER_COL[6] = {0, 1, 2, 1, 2, 2};
+
+// vertex_normals_kernel (closest.cu) for one vertex: the normalised mean of the unit normals of the adjacent triangles
+__device__ __forceinline__ void vertex_normal_rn(int i, const double* __restrict__ v, const int32_t* __restrict__ tri,
+                                                 const int32_t* __restrict__ adj_off, const int32_t* __restrict__ adj, double* nrm) {
+  double ax = 0, ay = 0, az = 0;
+  const int b = adj_off[i], e = adj_off[i + 1];
+  for (int k = b; k < e; ++k) {
+    const int t = adj[k];
+    const double* a = v + 3 * tri[3 * t];
+    const double* bb = v + 3 * tri[3 * t + 1];
+    const double* c = v + 3 * tri[3 * t + 2];
+    const double ux = bb[0] - a[0], uy = bb[1] - a[1], uz = bb[2] - a[2];
+    const double wx = c[0] - a[0], wy = c[1] - a[1], wz = c[2] - a[2];
+    double nx = __dsub_rn(__dmul_rn(uy, wz), __dmul_rn(uz, wy));
+    double ny = __dsub_rn(__dmul_rn(uz, wx), __dmul_rn(ux, wz));
+    double nz = __dsub_rn(__dmul_rn(ux, wy), __dmul_rn(uy, wx));
+    const double len = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(nx, nx), __dmul_rn(ny, ny)), __dmul_rn(nz, nz)));
+    nx /= len; ny /= len; nz /= len;
+    ax += nx; ay += ny; az += nz;
+  }
+  const int cnt = e - b;
+  if (cnt > 0) { ax /= cnt; ay /= cnt; az /= cnt; }
+  const double len = sqrt(__dadd_rn(__dadd_rn(__dmul_rn(ax, ax), __dmul_rn(ay, ay)), __dmul_rn(az, az)));
+  nrm[0] = ax / len; nrm[1] = ay / len; nrm[2] = az / len;
+}
+
+// Chain state i = mi[MI_STEP] (0: the primed start state, i >= 1: the state after the i-th MH step, in the working
+// buffers) is collected when i >= burn_in, (i - burn_in) % every == 0, i < total and the state before it (prev_is, null
+// for i = 0) is not a ModelFlexibilityError state.  Every thread decides from values no thread of the launch writes, so a
+// step that collects nothing is one early-exiting launch.  Welford update in FP64; tri = null: no normals (no triangles).
+GINGR_KERNEL((256), mcmc_collect_kernel, int M, const int* __restrict__ mi, const int* __restrict__ prev_is, int burn_in,
+                                         int every, int total, const double* __restrict__ fit, const int32_t* __restrict__ tri,
+                                         const int32_t* __restrict__ adj_off, const int32_t* __restrict__ adj,
+                                         double* __restrict__ acc, long long* __restrict__ cnt) {
+  const int i = mi[MI_STEP];
+  if (i < burn_in || i >= total || (i - burn_in) % every != 0) return;
+  if (prev_is && prev_is[IS_STATUS] == GINGR_STATUS_MODEL_FLEXIBILITY_ERROR) return;
+  const int m = blockIdx.x * blockDim.x + threadIdx.x;
+  if (m >= M) return;
+  const long long n = cnt[m] + 1;
+  cnt[m] = n;
+  double* a = acc + (size_t)ACC_WORDS * m;
+  double d[3], e[3];
+  for (int k = 0; k < 3; ++k) {
+    const double x = fit[3 * (size_t)m + k];
+    d[k] = x - a[k];
+    a[k] = a[k] + d[k] / (double)n;
+    e[k] = x - a[k];
+  }
+  for (int q = 0; q < 6; ++q) a[3 + q] = __dadd_rn(a[3 + q], __dmul_rn(d[SCATTER_ROW[q]], e[SCATTER_COL[q]]));
+  if (tri) {
+    double nrm[3];
+    vertex_normal_rn(m, fit, tri, adj_off, adj, nrm);
+    for (int k = 0; k < 3; ++k) a[9 + k] += nrm[k];
+  }
+}
+
+// gingr_mcmc_samples: the statistics of n chains pooled with Chan et al.'s pairwise formula in the order of the chains,
+// one thread per vertex.  Outputs: mean [3M], covariance S / (n - 1) [9M] row-major, mean of the normals [3M], count.
+__global__ void __launch_bounds__(256) mcmc_samples_pool_kernel(int M, int n, const double* const* __restrict__ accs,
+                                                                const long long* const* __restrict__ cnts,
+                                                                double* __restrict__ mean, double* __restrict__ cov,
+                                                                double* __restrict__ normal, long long* __restrict__ count) {
+  const int m = blockIdx.x * blockDim.x + threadIdx.x;
+  if (m >= M) return;
+  long long na = 0;
+  double mu[3] = {0, 0, 0}, S[6] = {0, 0, 0, 0, 0, 0}, ns[3] = {0, 0, 0};
+  for (int c = 0; c < n; ++c) {
+    const long long nb = cnts[c][m];
+    if (nb == 0) continue;
+    const double* b = accs[c] + (size_t)ACC_WORDS * m;
+    if (na == 0) {
+      for (int k = 0; k < 3; ++k) { mu[k] = b[k]; ns[k] = b[9 + k]; }
+      for (int q = 0; q < 6; ++q) S[q] = b[3 + q];
+      na = nb;
+      continue;
+    }
+    const long long nn = na + nb;
+    const double f = (double)nb / (double)nn, w = __dmul_rn((double)na, (double)nb) / (double)nn;
+    double d[3];
+    for (int k = 0; k < 3; ++k) {
+      d[k] = b[k] - mu[k];
+      mu[k] = __dadd_rn(mu[k], __dmul_rn(d[k], f));
+      ns[k] += b[9 + k];
+    }
+    for (int q = 0; q < 6; ++q) S[q] = __dadd_rn(S[q] + b[3 + q], __dmul_rn(__dmul_rn(d[SCATTER_ROW[q]], d[SCATTER_COL[q]]), w));
+    na = nn;
+  }
+  if (m == 0) count[0] = na;
+  const double dn = (double)na;
+  for (int k = 0; k < 3; ++k) { mean[3 * (size_t)m + k] = na > 0 ? mu[k] : NAN; normal[3 * (size_t)m + k] = ns[k] / dn; }
+  for (int q = 0; q < 6; ++q) {
+    const double c = S[q] / (dn - 1.0);
+    cov[9 * (size_t)m + 3 * SCATTER_ROW[q] + SCATTER_COL[q]] = c;
+    cov[9 * (size_t)m + 3 * SCATTER_COL[q] + SCATTER_ROW[q]] = c;
+  }
+}
+
 }  // namespace gingr
 
 // =================================================================================================
@@ -376,6 +481,10 @@ struct McmcState {
   gingr::ClosestWorkspace ws_m2t, ws_t2m;
   gingr::SpatialGrid fit_tgrid;
   bool use_fit_tgrid = false;
+  // sample collection (gingr_mcmc_collect; every = 0: off): per-vertex moments [M][ACC_WORDS] and counts [M]
+  int col_burn_in = 0, col_every = 0, col_total = 0;
+  DevBuf<double> col_acc;
+  DevBuf<long long> col_cnt;
   bool primed = false;
   GraphExec graph_exec;
   uint64_t graph_seed = 0;
@@ -506,6 +615,29 @@ static int32_t enqueue_to_mesh(gingr_registration* g, double step_length, const 
   return GINGR_OK;
 }
 
+// collection of the chain state in the working buffers (mcmc_collect_kernel); prev_is = null for the start state
+static int32_t enqueue_collect(gingr_registration* g, const int* prev_is) {
+  McmcState* mc = g->mcmc.get();
+  if (mc->col_every <= 0) return GINGR_OK;
+  gingr_ctx* ctx = g->ctx;
+  const gingr_model* m = g->model;
+  const bool normals = m->T > 0;
+  GINGR_LAUNCH(ctx, mcmc_collect_kernel, ceil_div(m->M, 256), 256, 0, ctx->stream, m->M, mc->mi.p, prev_is, mc->col_burn_in,
+               mc->col_every, mc->col_total, g->fit.p, normals ? m->tri.p : nullptr, normals ? m->adj_off.p : nullptr,
+               normals ? m->adj.p : nullptr, mc->col_acc.p, mc->col_cnt.p);
+  GINGR_LAUNCHED(ctx);
+  return GINGR_OK;
+}
+
+static int32_t collect_reset(gingr_registration* g) {
+  McmcState* mc = g->mcmc.get();
+  if (mc->col_every <= 0) return GINGR_OK;
+  const size_t M = (size_t)g->model->M;
+  GINGR_CUDA_TRY(g->ctx, cudaMemsetAsync(mc->col_acc.p, 0, sizeof(double) * ACC_WORDS * M, g->ctx->stream));
+  GINGR_CUDA_TRY(g->ctx, cudaMemsetAsync(mc->col_cnt.p, 0, sizeof(long long) * M, g->ctx->stream));
+  return GINGR_OK;
+}
+
 // posterior-mean coefficients of the state whose factor + z sit in g->Mx
 static int32_t enqueue_posterior_mean_coeffs(gingr_registration* g, double* d_out) {
   const gingr_model* m = g->model;
@@ -534,6 +666,7 @@ static int32_t mcmc_prime(gingr_registration* g) {
   // a new chain: step counter (the Philox stream position) and statistics start at zero
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(mc->md.p, 0, sizeof(double) * MD_COUNT, st));
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(mc->mi.p, 0, sizeof(int) * MI_COUNT, st));
+  GINGR_TRY(collect_reset(g));
   GINGR_TRY(enqueue_posterior_phase(g));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mc->raw_cur.p, g->Mx_raw.p, sizeof(double) * (size_t)(r + 1) * rp, cudaMemcpyDeviceToDevice, st));
   GINGR_TRY(enqueue_posterior_mean_coeffs(g, mc->cm_cur.p));
@@ -545,6 +678,7 @@ static int32_t mcmc_prime(gingr_registration* g) {
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mc->best_is.p, g->is.p, sizeof(int) * IS_COUNT, cudaMemcpyDeviceToDevice, st));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mc->best_alpha.p, g->alpha.p, sizeof(double) * r, cudaMemcpyDeviceToDevice, st));
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mc->best_fit.p, g->fit.p, sizeof(double) * 3 * (size_t)M, cudaMemcpyDeviceToDevice, st));
+  GINGR_TRY(enqueue_collect(g, nullptr));   // chain state 0
   // MD_LP_BEST = lp_cur
   double h[2];
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(h, mc->md.p + MD_LP_CUR, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
@@ -626,6 +760,8 @@ static int32_t enqueue_mcmc_step(gingr_registration* g, uint64_t seed) {
     GINGR_LAUNCH(ctx, multi_copy_kernel, 16, 256, 0, st, sg);
     GINGR_LAUNCHED(ctx);
   }
+  // 9. sample collection of the state the step leaves (only when switched on: the step is otherwise unchanged)
+  GINGR_TRY(enqueue_collect(g, mc->s_is.p));
   GINGR_CUDA_TRY(ctx, cudaGetLastError());
   return GINGR_OK;
 }
@@ -839,6 +975,77 @@ int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t iters, ui
   GINGR_TRY(replay_chain_graphs(ctx, sp, n, iters, [&](int k) { return regs[k]->mcmc->graph_exec.h; }, [](int, cudaStream_t) {}));
   for (int k = 0; k < n; ++k) ctx->launches += (int64_t)iters * regs[k]->mcmc->graph_launches;
   GINGR_CUDA_TRY(ctx, cudaGetLastError());
+  return GINGR_OK;
+}
+
+// Sample collection of the chain (LogHelper.samplesFromLog, LogHelper.scala:29-43): the rule lives with the chain and the
+// accumulators start from zero here and whenever the chain is primed afresh.  take_every_n = 0 switches it off.
+int32_t gingr_mcmc_collect(gingr_registration* g, int32_t burn_in, int32_t take_every_n, int32_t total) {
+  GINGR_TRY(mcmc_check(g, "gingr_mcmc_collect: bad argument"));
+  gingr_ctx* ctx = g->ctx;
+  McmcState* mc = g->mcmc.get();
+  if (burn_in < 0 || take_every_n < 0 || total < 0)
+    return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_collect: burn_in, take_every_n and total must be >= 0");
+  GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
+  mc->col_burn_in = burn_in;
+  mc->col_every = take_every_n;
+  mc->col_total = total;
+  if (take_every_n > 0) {
+    const size_t M = (size_t)g->model->M;
+    GINGR_CUDA_TRY(ctx, mc->col_acc.alloc(ACC_WORDS * M));
+    GINGR_CUDA_TRY(ctx, mc->col_cnt.alloc(M));
+    GINGR_TRY(collect_reset(g));
+  }
+  mc->graph_exec.reset();   // the captured step holds the rule and the accumulators
+  ++g_batch_epoch;          // ... and so do batched plans that name this chain
+  return GINGR_OK;
+}
+
+// The collected statistics of n chains pooled in the order regs[0], regs[1], ... (PosteriorHelper.scala:31-79 reduces
+// them to the distance maps).  Chains share one ctx and one model and have collection on.  Outputs may be null.
+int32_t gingr_mcmc_samples(gingr_registration** regs, int32_t n, int64_t* count, double* mean, double* cov, double* normal) {
+  if (!regs || n <= 0 || !regs[0]) return gingr_fail(nullptr, GINGR_ERR_ARG, "gingr_mcmc_samples: bad argument");
+  gingr_ctx* ctx = regs[0]->ctx;
+  const gingr_model* m = regs[0]->model;
+  std::vector<const double*> accs(n);
+  std::vector<const long long*> cnts(n);
+  for (int k = 0; k < n; ++k) {
+    if (!regs[k] || regs[k]->ctx != ctx || regs[k]->model != m)
+      return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_samples: chains must share one ctx and one model");
+    GINGR_TRY(mcmc_check(regs[k], "gingr_mcmc_samples: bad argument"));
+    const McmcState* mc = regs[k]->mcmc.get();
+    if (mc->col_every <= 0) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_samples: sample collection is off (gingr_mcmc_collect)");
+    accs[k] = mc->col_acc.p;
+    cnts[k] = mc->col_cnt.p;
+  }
+  if (normal && m->T <= 0) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_samples: normals need the model triangles");
+  GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const size_t M = (size_t)m->M;
+  DevBuf<const double*> d_accs;
+  DevBuf<const long long*> d_cnts;
+  DevBuf<double> out;
+  DevBuf<long long> d_count;
+  GINGR_CUDA_TRY(ctx, d_accs.alloc(n));
+  GINGR_CUDA_TRY(ctx, d_cnts.alloc(n));
+  GINGR_CUDA_TRY(ctx, out.alloc(15 * M));
+  GINGR_CUDA_TRY(ctx, d_count.alloc(1));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(d_accs.p, accs.data(), sizeof(const double*) * n, cudaMemcpyHostToDevice, st));
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(d_cnts.p, cnts.data(), sizeof(const long long*) * n, cudaMemcpyHostToDevice, st));
+  mcmc_samples_pool_kernel<<<ceil_div(m->M, 256), 256, 0, st>>>(m->M, n, d_accs.p, d_cnts.p, out.p, out.p + 3 * M, out.p + 12 * M,
+                                                              d_count.p);
+  GINGR_LAUNCHED(ctx);
+  GINGR_CUDA_TRY(ctx, cudaGetLastError());
+  long long h_count = 0;
+  GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(&h_count, d_count.p, sizeof(long long), cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  if (cov && h_count < 2) return gingr_fail(ctx, GINGR_ERR_ARG, "gingr_mcmc_samples: the covariance needs at least 2 samples");
+  if (count) *count = h_count;
+  if (mean) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(mean, out.p, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
+  if (cov) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(cov, out.p + 3 * M, sizeof(double) * 9 * M, cudaMemcpyDeviceToHost, st));
+  if (normal) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(normal, out.p + 12 * M, sizeof(double) * 3 * M, cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
   return GINGR_OK;
 }
 

@@ -234,6 +234,36 @@ struct ProbabilisticSettings {
   }
 };
 
+// LogHelper.samplesFromLog (LogHelper.scala:29-43) with its defaults: chain state i is collected when i >= burnIn,
+// (i - burnIn) % takeEveryN == 0 and i < total (gingr_mcmc_collect); takeEveryN = 0 switches collection off.
+struct SampleCollection {
+  int32_t burnIn = 0;
+  int32_t takeEveryN = 50;
+  int32_t total = 100;
+};
+
+// Per-vertex statistics of the collected states of one or more chains (gingr_mcmc_samples); the maps of
+// PosteriorHelper.scala:31-79 are distanceMapTotal = tr cov and distanceMapNormal = normal^T cov normal.
+struct SampleStatistics {
+  int64_t count = 0;
+  std::vector<double> mean, cov, normal;   // [3M], [9M] row-major 3 x 3 per vertex, [3M] (empty when not requested)
+  std::vector<double> distanceMapTotal() const {
+    std::vector<double> d(mean.size() / 3);
+    for (size_t m = 0; m < d.size(); ++m) d[m] = cov[9 * m] + cov[9 * m + 4] + cov[9 * m + 8];
+    return d;
+  }
+  std::vector<double> distanceMapNormal() const {   // sumNormals = true
+    std::vector<double> d(mean.size() / 3);
+    for (size_t m = 0; m < d.size(); ++m) {
+      double s = 0.0;
+      for (int i = 0; i < 3; ++i)
+        for (int j = 0; j < 3; ++j) s += normal[3 * m + i] * cov[9 * m + 3 * i + j] * normal[3 * m + j];
+      d[m] = s;
+    }
+    return d;
+  }
+};
+
 template <class Config>
 class GingrAlgorithm;
 
@@ -471,6 +501,22 @@ class GingrAlgorithm {
   void mcmcChain(int iters, uint64_t seed) { ctx_->check(gingr_mcmc_chain(h_, iters, seed)); }
   State downloadState() const { return download(&gingr_state_download); }
   State mcmcBest() const { return download(&gingr_mcmc_best); }
+  // collect the chain's states on the device (after configureProbabilistic, which discards the setting)
+  void collectSamples(const SampleCollection& c) { ctx_->check(gingr_mcmc_collect(h_, c.burnIn, c.takeEveryN, c.total)); }
+  // the collected statistics of this chain; cov is left empty below 2 samples, normal when not asked for (withNormals
+  // needs the model triangles)
+  SampleStatistics sampleStatistics(bool withNormals = true) const {
+    gingr_registration* regs[1] = {h_};
+    SampleStatistics s;
+    ctx_->check(gingr_mcmc_samples(regs, 1, &s.count, nullptr, nullptr, nullptr));
+    const size_t M = static_cast<size_t>(model_->points());
+    s.mean.resize(3 * M);
+    if (s.count >= 2) s.cov.resize(9 * M);
+    if (withNormals) s.normal.resize(3 * M);
+    ctx_->check(gingr_mcmc_samples(regs, 1, nullptr, s.mean.data(), s.cov.empty() ? nullptr : s.cov.data(),
+                                   s.normal.empty() ? nullptr : s.normal.data()));
+    return s;
+  }
   // run(...) with probabilisticSettings: maxIterations - 1 steps, the best sample is returned (:160-171)
   State runProbabilistic(const State& initial, const ProbabilisticSettings& settings, uint64_t seed = 0) {
     configureProbabilistic(settings);

@@ -394,6 +394,27 @@ GINGR_API int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t
 GINGR_API int32_t gingr_mcmc_stats(gingr_registration* reg, double* values /*[16]*/, int32_t* counts /*[32]*/);
 /* BestAndCurrentSampleLogger.currentBestSample (GingrAlgorithm.scala:160-163). */
 GINGR_API int32_t gingr_mcmc_best(gingr_registration* reg, gingr_state* state_out, double* alpha_out, double* fit_out);
+/* Sample collection on the device: LogHelper.samplesFromLog (LogHelper.scala:29-43) over the chain's states, reduced to the
+ * per-vertex moments behind PosteriorHelper.computeDistanceMapFromMeshesTotal / ...Normal (PosteriorHelper.scala:31-79).
+ * Chain state i is the start state (i = 0, the state the chain is primed from) or the state after the i-th MH step (the
+ * proposal if accepted, else the previous state).  State i is collected when i >= burn_in, (i - burn_in) % take_every_n
+ * == 0, i < total, and state i - 1 is not a ModelFlexibilityError state (the logged run stops at the first error state,
+ * GingrAlgorithm.scala:150-153).  Per vertex the device keeps the count, the mean fit s (R instance + t), the scatter
+ * sum (x - mean)(x - mean)^T (Welford, FP64, in step order: the statistics do not depend on how the steps are split over
+ * calls) and the sum of the unit vertex normals of the collected fits.  take_every_n = 0 switches collection off (the
+ * default); the MH step then runs exactly as without collection.  Otherwise every MH step costs one more launch.
+ * The settings belong to the chain: gingr_mcmc_configure discards them with the rest of the chain.  The accumulators
+ * start from zero at this call and whenever the chain starts afresh (gingr_initialize_state, gingr_update, ... before the
+ * next gingr_mcmc_chain / gingr_mcmc_batch).  Needs gingr_mcmc_configure first; negative arguments: GINGR_ERR_ARG. */
+GINGR_API int32_t gingr_mcmc_collect(gingr_registration* reg, int32_t burn_in, int32_t take_every_n, int32_t total);
+/* The collected statistics of n chains, pooled with Chan et al.'s pairwise formula in the order regs[0], regs[1], ...
+ * (deterministic; n = 1: the chain's own): count, mean[3M], cov[9M] (row-major 3 x 3 per vertex, scatter / (count - 1)),
+ * normal[3M] (the mean of the sample normals, not renormalised).  distance_map_total = tr cov; distance_map_normal =
+ * normal^T cov normal.  Any output may be NULL.  GINGR_ERR_ARG when the chains do not share one ctx and one model, a
+ * chain has collection off, cov is requested with fewer than 2 samples, or normal is requested on a model without
+ * triangles. */
+GINGR_API int32_t gingr_mcmc_samples(gingr_registration** regs, int32_t n, int64_t* count, double* mean /*[3M]*/,
+                                     double* cov /*[9M]*/, double* normal /*[3M]*/);
 
 /* ---- measurement hooks (new; used by bench.py for the roofline numbers) ------------------------ */
 /* Per-phase device timing with CUDA events recorded on the ctx stream around the kernels of gingr_update /

@@ -83,6 +83,9 @@ object GingrCudaNative {
   val mcmcBatch      = fn("gingr_mcmc_batch", JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_LONG)
   val mcmcStats      = fn("gingr_mcmc_stats", JAVA_INT, ADDRESS, ADDRESS, ADDRESS)
   val mcmcBest       = fn("gingr_mcmc_best", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS)
+  // sample collection (LogHelper.scala:29-43) and the pooled per-vertex moments of the maps (PosteriorHelper.scala:31-79)
+  val mcmcCollect    = fn("gingr_mcmc_collect", JAVA_INT, ADDRESS, JAVA_INT, JAVA_INT, JAVA_INT)
+  val mcmcSamples    = fn("gingr_mcmc_samples", JAVA_INT, ADDRESS, JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS)
   val stateDownload  = fn("gingr_state_download", JAVA_INT, ADDRESS, ADDRESS, ADDRESS, ADDRESS)
   // BCPD registrations (GINGR_ALGO_BCPD): the Dirichlet concentration kappa, and the per-vertex mixing weights / variances
   val registrationSetBcpd = fn("gingr_registration_set_bcpd", JAVA_INT, ADDRESS, JAVA_DOUBLE)
