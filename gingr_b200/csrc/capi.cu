@@ -68,7 +68,6 @@ int32_t gingr_ctx_create(int32_t device, gingr_ctx** out) {
   int prio_lo = 0, prio_hi = 0;
   GINGR_CUDA_TRY(nullptr, cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi));
   GINGR_CUDA_TRY(nullptr, cudaStreamCreateWithPriority(&ctx->stream, cudaStreamNonBlocking, prio_hi));
-  GINGR_CUDA_TRY(nullptr, cudaStreamCreateWithPriority(&ctx->side_stream, cudaStreamNonBlocking, prio_lo));
   GINGR_CUDA_TRY(nullptr, cudaMallocHost((void**)&ctx->h_pinned, ctx->h_pinned_count * sizeof(double)));
   *out = ctx.release();
   return GINGR_OK;
@@ -80,8 +79,6 @@ int32_t gingr_ctx_destroy(gingr_ctx* ctx) {
   cudaStreamSynchronize(ctx->stream);
   gingr::comm_destroy(ctx);
   if (ctx->h_pinned) cudaFreeHost(ctx->h_pinned);
-  for (auto& e : ctx->chol_events) cudaEventDestroy(e);
-  if (ctx->side_stream) cudaStreamDestroy(ctx->side_stream);
   if (ctx->stream) cudaStreamDestroy(ctx->stream);
   delete static_cast<gingr_ctx_full*>(ctx);   // frees the scratch buffers
   return GINGR_OK;

@@ -20,9 +20,7 @@
 //     CTA, so the spin waits cannot deadlock whatever else occupies the GPU.  No launch boundary, no grid-wide barrier.
 //
 // Rows below the square part (right-hand sides stored as extra rows) ride along, which performs the forward
-// substitution L^-1 b inside the factorisation (as chol.cu's kernels did).
-#include <stdlib.h>
-
+// substitution L^-1 b inside the factorisation.
 #include <algorithm>
 
 #include "batch.cuh"
@@ -578,8 +576,7 @@ int32_t cholesky_df_enqueue(gingr_ctx* ctx, int n, int nrows, double* d_A, int l
   if ((size_t)(2 + (size_t)P.nb * P.nbr) > ws.sync.n || (size_t)P.nb * TB * TB > ws.linv.n)
     return gingr_fail(ctx, GINGR_ERR_ARG, "cholesky: workspace too small");
   if ((ld & 1) != 0 || (((uintptr_t)d_A) & 15) != 0) return gingr_fail(ctx, GINGR_ERR_ARG, "cholesky: matrix must be 16-byte aligned with an even pitch");
-  static const int env_small = [] { const char* e = getenv("GINGR_CHOL_SMALL"); return e ? atoi(e) : 1; }();
-  if (P.nb == 1 && env_small) {
+  if (P.nb == 1) {
     static thread_local int attr_small = -1;
     if (attr_small != ctx->device) {
       GINGR_CUDA_TRY(ctx, cudaFuncSetAttribute(chol_small_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMALL_SMEM));

@@ -19,8 +19,6 @@ struct gingr_ctx {
   int device = 0;
   int num_sms = GINGR_NUM_SMS_B200;
   cudaStream_t stream = nullptr;       // all work of the ctx; highest priority
-  cudaStream_t side_stream = nullptr;  // low priority: bulk trailing updates of the Cholesky lookahead (chol.cu)
-  std::vector<cudaEvent_t> chol_events;  // 2 per block step, created on first use
   std::string last_error;
   int64_t launches = 0;
   LaunchRecorder* rec = nullptr;       // while set, batch-aware launches are recorded instead of issued (batch.cuh)

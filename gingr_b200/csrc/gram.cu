@@ -15,13 +15,11 @@
 // rows of Phi in lockstep from the top (every row slab is fetched from HBM once and served to the other
 // tiles from L2), while the remaining n - T CTAs take the bottom slab of every tile, so all SMs finish
 // together for any r.  Each segment accumulates in registers (warp tile 64x32 = 32 DMMA accumulator
-// fragments), operands stream global -> shared with a 3-stage cp.async pipeline ([k][col] tiles of 32 rows,
+// fragments), operands stream global -> shared through a 3-stage pipeline of bulk copies ([k][col] tiles of 32 rows,
 // pitch 132 doubles: conflict-free LDS.64 fragment loads), the row weights are multiplied into the B
 // fragments.  Partial tiles go to a workspace and are summed in fixed
 // order by gram_finish_kernel (deterministic; no atomics), which also applies D, adds I and the landmark
 // blocks (full 3x3 covariances, GeneralRegistrationState.scala:43-62).
-#include <stdlib.h>
-
 #include <algorithm>
 #include <vector>
 
@@ -35,12 +33,6 @@ constexpr int BT = 128;          // output tile edge
 constexpr int BK = 32;           // rows of Phi per pipeline stage
 constexpr int STAGES = 3;
 constexpr int PITCH = BT + 4;    // smem row pitch in doubles (== 4 mod 16 -> conflict-free fragment loads)
-#ifndef GRAM_WARPS_M
-#define GRAM_WARPS_M 2           // warps along the tile rows: 2 -> 8 warps of 64x32, 4 -> 16 warps of 32x32
-#endif
-constexpr int GRAM_THREADS = GRAM_WARPS_M * 4 * 32;
-constexpr int WTM = BT / GRAM_WARPS_M;   // warp tile rows
-constexpr int MI = WTM / 8;              // 8-row DMMA fragments per warp tile
 constexpr size_t GRAM_SMEM = (size_t)STAGES * (2 * BK * PITCH + BK) * sizeof(double);
 
 // segment of work of one CTA: tile (ta >= tb), chunk range [c0, c1), output slot
@@ -48,113 +40,10 @@ struct GramSegment {
   int ta, tb, c0, c1, slot, pad0, pad1, pad2;
 };
 
-// phi: [rows][rp] row-major, wrow: [rows] (may be null = unit weights)
-__global__ void __launch_bounds__(GRAM_THREADS, 1) gram_streamk_kernel(int rows, int rp,
-                                                                       const double* __restrict__ phi,
-                                                                       const double* __restrict__ wrow,
-                                                                       const GramSegment* __restrict__ segs,
-                                                                       const int* __restrict__ seg_begin,
-                                                                       double* __restrict__ partial) {
-  extern __shared__ __align__(16) double smem[];
-  double* sA = smem;                                   // [STAGES][BK][PITCH]
-  double* sB = sA + (size_t)STAGES * BK * PITCH;       // [STAGES][BK][PITCH]
-  double* sW = sB + (size_t)STAGES * BK * PITCH;       // [STAGES][BK]
-
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int wm = warp >> 2, wn = warp & 3;             // GRAM_WARPS_M x 4 warps, warp tile WTM x 32
-  const int g = lane >> 2, t = lane & 3;
-
-  for (int si = seg_begin[blockIdx.x]; si < seg_begin[blockIdx.x + 1]; ++si) {
-    const GramSegment sg = segs[si];
-    const int a0 = sg.ta * BT, b0 = sg.tb * BT;
-    const bool diag = sg.ta == sg.tb;
-    const int nchunks = sg.c1 - sg.c0;
-
-    double acc[MI][4][2];
-#pragma unroll
-    for (int i = 0; i < MI; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) acc[i][j][0] = acc[i][j][1] = 0.0;
-
-    auto issue = [&](int chunk) {
-      const int stage = chunk % STAGES;
-      const int krow0 = (sg.c0 + chunk) * BK;
-      double* dA = sA + (size_t)stage * BK * PITCH;
-      double* dB = sB + (size_t)stage * BK * PITCH;
-      // BK rows x 64 16-byte pieces per operand tile, BK * 64 / 256 per thread
-#pragma unroll
-      for (int q = 0; q < BK * 64 / GRAM_THREADS; ++q) {
-        const int e = tid + q * GRAM_THREADS;
-        const int kr = e >> 6, c2 = (e & 63) * 2;
-        const int krow = krow0 + kr;
-        const bool rok = krow < rows;
-        {
-          const int col = a0 + c2;
-          const bool ok = rok && col < rp;
-          cp_async16(dA + kr * PITCH + c2, ok ? (const void*)(phi + (size_t)krow * rp + col) : (const void*)phi,
-                     ok ? 16 : 0);
-        }
-        if (!diag) {
-          const int col = b0 + c2;
-          const bool ok = rok && col < rp;
-          cp_async16(dB + kr * PITCH + c2, ok ? (const void*)(phi + (size_t)krow * rp + col) : (const void*)phi,
-                     ok ? 16 : 0);
-        }
-      }
-      if (tid < BK) {
-        const int krow = krow0 + tid;
-        const bool ok = krow < rows && wrow != nullptr;
-        cp_async8(sW + stage * BK + tid, ok ? (const void*)(wrow + krow) : (const void*)phi, ok ? 8 : 0);
-      }
-    };
-
-    __syncthreads();  // previous segment's readers are done with the stages
-#pragma unroll
-    for (int p = 0; p < STAGES - 1; ++p) {
-      if (p < nchunks) issue(p);
-      cp_async_commit();
-    }
-    for (int ch = 0; ch < nchunks; ++ch) {
-      cp_async_wait<STAGES - 2>();
-      __syncthreads();
-      if (ch + STAGES - 1 < nchunks) issue(ch + STAGES - 1);
-      cp_async_commit();
-      const int stage = ch % STAGES;
-      const double* tA = sA + (size_t)stage * BK * PITCH + wm * WTM + g;
-      const double* tB = (diag ? sA : sB) + (size_t)stage * BK * PITCH + wn * 32 + g;
-      const double* tW = sW + stage * BK;
-#pragma unroll
-      for (int k4 = 0; k4 < BK / 4; ++k4) {
-        const int kk = k4 * 4 + t;
-        const double wk = wrow ? tW[kk] : 1.0;
-        double af[MI], bf[4];
-#pragma unroll
-        for (int i = 0; i < MI; ++i) af[i] = tA[kk * PITCH + i * 8];
-#pragma unroll
-        for (int j = 0; j < 4; ++j) bf[j] = tB[kk * PITCH + j * 8] * wk;
-#pragma unroll
-        for (int i = 0; i < MI; ++i)
-#pragma unroll
-          for (int j = 0; j < 4; ++j) dmma884(acc[i][j][0], acc[i][j][1], af[i], bf[j]);
-      }
-    }
-    cp_async_wait<0>();
-    // store the partial tile: slot-major [slot][128][128]
-    double* out = partial + (size_t)sg.slot * BT * BT;
-#pragma unroll
-    for (int i = 0; i < MI; ++i)
-#pragma unroll
-      for (int j = 0; j < 4; ++j) {
-        const int row = wm * WTM + i * 8 + g, col = wn * 32 + j * 8 + 2 * t;
-        *reinterpret_cast<double2*>(out + (size_t)row * BT + col) = make_double2(acc[i][j][0], acc[i][j][1]);
-      }
-  }
-}
-
 // ---------------------------------------------------------------------------------------------
-// Warp-specialised variant (default): 8 consumer warps + 1 producer warp, stages handed over through mbarriers
-// instead of a CTA-wide barrier per chunk.  ncu on the barrier version: 6 % of the warp samples sit in `barrier`
-// and 7 % in `short scoreboard` right after it (the whole CTA drains the DMMA pipe every 32 rows); here a consumer
+// Warp-specialised: 8 consumer warps + 1 producer warp, stages handed over through mbarriers instead of a CTA-wide
+// barrier per chunk.  ncu on a barrier-per-chunk form: 6 % of the warp samples sit in `barrier` and 7 % in
+// `short scoreboard` right after it (the whole CTA drains the DMMA pipe every 32 rows); here a consumer
 // warp only waits for "its" stage to be full and the producer refills a stage as soon as the 8 warps released it,
 // also across segment boundaries (the partial-tile store of one segment overlaps the loads of the next).
 //   full[s]   count 32 + transaction bytes: every producer lane arrives (lane 0 with expect_tx) and issues one
@@ -529,8 +418,6 @@ int32_t GramPlan::build(gingr_ctx* ctx, int rows_, int r_, int rp_, int max_cta)
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(d_tile_first.p, tile_first.data(), tile_first.size() * sizeof(int),
                                       cudaMemcpyHostToDevice, ctx->stream));
   GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));  // host vectors go out of scope
-  GINGR_CUDA_TRY(ctx, cudaFuncSetAttribute(gram_streamk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                           (int)GRAM_SMEM));
   GINGR_CUDA_TRY(ctx, cudaFuncSetAttribute(gram_ws_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                            (int)GRAM_WS_SMEM));
   return GINGR_OK;
@@ -538,10 +425,8 @@ int32_t GramPlan::build(gingr_ctx* ctx, int rows_, int r_, int rp_, int max_cta)
 
 // partial tiles of G = Phi^T diag(wrow) Phi  (wrow may be null)
 bool gram_rhs_fusable(const GramPlan& plan) {
-  static const int use_ws = [] { const char* e = getenv("GINGR_GRAM_WS"); return e ? atoi(e) : 1; }();
-  static const int fuse = [] { const char* e = getenv("GINGR_GRAM_RHS"); return e ? atoi(e) : 1; }();
   // the same answer on every rank (a rank without rows just contributes zero partials)
-  return fuse && use_ws && GRAM_WARPS_M == 2 && (plan.rp % BT) != 0;
+  return (plan.rp % BT) != 0;
 }
 
 int32_t gram_partials_enqueue(gingr_ctx* ctx, GramPlan& plan, const double* d_phi, const double* d_wrow,
@@ -549,15 +434,9 @@ int32_t gram_partials_enqueue(gingr_ctx* ctx, GramPlan& plan, const double* d_ph
   if (d_resid && !gram_rhs_fusable(plan)) return gingr_fail(ctx, GINGR_ERR_ARG, "gram: the rhs cannot ride along for this rank");
   if (ev0) cudaEventRecord(ev0, ctx->stream);
   if (plan.rows > 0 && plan.nsegs > 0) {
-    static const int use_ws = [] { const char* e = getenv("GINGR_GRAM_WS"); return e ? atoi(e) : 1; }();
-    if (use_ws && GRAM_WARPS_M == 2)
-      GINGR_LAUNCH(ctx, gram_ws_kernel, plan.ncta, GRAM_WS_THREADS, GRAM_WS_SMEM, ctx->stream, 
-          plan.rows, plan.rp, d_phi, d_wrow, d_resid, plan.r, reinterpret_cast<const GramSegment*>(plan.d_segs.p), plan.d_seg_begin.p,
-          plan.d_partial.p);
-    else
-      gram_streamk_kernel<<<plan.ncta, GRAM_THREADS, GRAM_SMEM, ctx->stream>>>(
-          plan.rows, plan.rp, d_phi, d_wrow, reinterpret_cast<const GramSegment*>(plan.d_segs.p), plan.d_seg_begin.p,
-          plan.d_partial.p);
+    GINGR_LAUNCH(ctx, gram_ws_kernel, plan.ncta, GRAM_WS_THREADS, GRAM_WS_SMEM, ctx->stream,
+        plan.rows, plan.rp, d_phi, d_wrow, d_resid, plan.r, reinterpret_cast<const GramSegment*>(plan.d_segs.p), plan.d_seg_begin.p,
+        plan.d_partial.p);
     GINGR_LAUNCHED(ctx);
     GINGR_CUDA_TRY(ctx, cudaGetLastError());
   } else {

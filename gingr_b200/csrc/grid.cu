@@ -9,9 +9,9 @@
 // surface sampling) -> per-cell counts (integer atomics; the order inside a cell is irrelevant because winners are
 // chosen by (value, index)) -> exclusive scan -> scatter.  Triangles are entered in every cell their bounding box
 // overlaps.
-// Queries: one thread per query, expanding Chebyshev shells of cells around the query's cell until the best value is
-// strictly below the distance to the unvisited region (minus a safety margin); lines march slab by slab along their
-// major axis.
+// Queries: one thread per query (one warp for the closest point on the surface), expanding Chebyshev shells of cells
+// around the query's cell until the best value is strictly below the distance to the unvisited region (minus a safety
+// margin); lines march slab by slab along their major axis.
 // Cells are numbered in nested 4x4x4 blocks (two levels: 64 and 4096 fine cells), so the entries of a coarse cell of
 // edge 4h or 16h are ONE contiguous range of the same arrays: a query that is far from the surface (the normal case in
 // the first ICP iterations) climbs to the coarser levels instead of walking thousands of empty fine cells.  A query
@@ -327,8 +327,8 @@ static int32_t grid_common_head(gingr_ctx* ctx, SpatialGrid& g, int n, VertexArr
   cudaStream_t st = ctx->stream;
   grid_bbox_kernel<<<BB_BLOCKS, 256, 0, st>>>(n, v, g.bbox_part.p);
   GINGR_LAUNCHED(ctx);
-  static const double cell_scale = [] { const char* e = getenv("GINGR_K2_CELL_SCALE"); return e && atof(e) > 0.0 ? atof(e) : 2.0; }();
-  grid_params_kernel<<<1, 32, 0, st>>>(n, g.cap_cells, g.bbox_part.p, g.params.p, cell_scale);
+  grid_params_kernel<<<1, 32, 0, st>>>(n, g.cap_cells, g.bbox_part.p, g.params.p,
+                                       2.0 /*cell scale: sweep in profiles/r04b_ncu_k2_surface.md*/);
   GINGR_LAUNCHED(ctx);
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(g.fill.p, 0, sizeof(int32_t) * ((size_t)g.cap_cells + 1), st));
   return GINGR_OK;
@@ -561,75 +561,9 @@ int32_t grid_nn_enqueue(gingr_ctx* ctx, const SpatialGrid& g, int M, const doubl
 }
 
 // ---------------------------------------------------------------------------------------------
-// closest point on the surface
-// ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128) grid_surface_kernel(int M, const double4* __restrict__ order, const double* __restrict__ q, int T,
-                                                           const GridParams* __restrict__ gp,
-                                                           const int32_t* __restrict__ cell_start,
-                                                           const int32_t* __restrict__ entries,
-                                                           const float4* __restrict__ tri_box,
-                                                           const double* __restrict__ verts /*AoS*/,
-                                                           const int32_t* __restrict__ tri, double* __restrict__ d2,
-                                                           int32_t* __restrict__ tri_out, double* __restrict__ cp) {
-  const int slot = blockIdx.x * 128 + threadIdx.x;
-  if (slot >= M) return;
-  const int i = order ? (int)__double_as_longlong(order[slot].w) : slot;   // spatially sorted queries: coherent warps
-  const double qx = q[3 * i], qy = q[3 * i + 1], qz = q[3 * i + 2];
-  double best = INFINITY, bx = 0, by = 0, bz = 0;
-  int bt = -1;
-  GridParams g;
-  auto consider = [&](int t, int x, int y, int z, int sh) {
-    {
-      // quick reject: the triangle lies inside its (outward rounded) box, so it cannot beat or tie the best when
-      // the box is strictly farther.  De-duplication: a triangle is entered in every cell its box overlaps; it is
-      // evaluated only in the cell that holds the point of its box nearest to the query -- that cell is one of its
-      // cells (same box, same monotone cell function as the build) and is never farther than the triangle itself, so
-      // the ball walk reaches it whenever the triangle can win.
-      const float4 lo = tri_box[2 * t], hi = tri_box[2 * t + 1];
-      const double px = fmin(fmax(qx, (double)lo.x), (double)hi.x), py = fmin(fmax(qy, (double)lo.y), (double)hi.y),
-                   pz = fmin(fmax(qz, (double)lo.z), (double)hi.z);
-      const double ex = qx - px, ey = qy - py, ez = qz - pz;
-      if ((ex * ex + ey * ey + ez * ez) * (1.0 - 1e-12) > best) return;
-      if (sh >= 0 && ((cell_coord(px, g.ox, g.inv_h, g.nx) >> sh) != x || (cell_coord(py, g.oy, g.inv_h, g.ny) >> sh) != y ||
-                      (cell_coord(pz, g.oz, g.inv_h, g.nz) >> sh) != z))
-        return;
-    }
-    GSTAT(5, 1);
-    const double* a = verts + 3 * (size_t)tri[3 * t];
-    const double* b = verts + 3 * (size_t)tri[3 * t + 1];
-    const double* c = verts + 3 * (size_t)tri[3 * t + 2];
-    const double va[3] = {a[0], a[1], a[2]}, vb[3] = {b[0], b[1], b[2]}, vc[3] = {c[0], c[1], c[2]};
-    double cx, cy, cz;
-    closest_on_triangle(qx, qy, qz, va, vb, vc, cx, cy, cz);
-    const double dx = qx - cx, dy = qy - cy, dz = qz - cz;
-    const double d = dx * dx + dy * dy + dz * dz;
-    if (d < best || (d == best && t < bt)) { best = d; bt = t; bx = cx; by = cy; bz = cz; }
-  };
-  if (isfinite(qx) && isfinite(qy) && isfinite(qz)) {
-    g = *gp;
-    bool done = false;
-    if (!g.overflow) {
-      done = grid_search(g, cell_start, qx, qy, qz,
-                         [&](int e0, int e1, int x, int y, int z, int sh) {
-                           for (int e = e0; e < e1; ++e) consider(entries[e], x, y, z, sh);
-                         },
-                         [&]() { return best; }, [&](double& x, double& y, double& z) { x = bx; y = by; z = bz; });
-    }
-    if (!done) {
-      best = INFINITY; bt = -1; bx = by = bz = 0;
-      for (int t = 0; t < T; ++t) consider(t, 0, 0, 0, -1);
-    }
-  }
-  d2[i] = best;
-  if (tri_out) tri_out[i] = bt;
-  cp[3 * i] = bx; cp[3 * i + 1] = by; cp[3 * i + 2] = bz;
-}
-
-
-// ---------------------------------------------------------------------------------------------
 // closest point on the surface, one WARP per query.
-// The thread-per-query kernel above runs with 3-9 of 32 lanes active in its hot loops (profiles/r01s_ncu_grid_surface.md:
-// every lane walks its own cells and takes its own branches of the exact triangle evaluation).  Here the 32 lanes share
+// A thread per query ran with 3-9 of 32 lanes active in its hot loops (profiles/r01s_ncu_grid_surface.md: every lane
+// walks its own cells and takes its own branches of the exact triangle evaluation).  Here the 32 lanes share
 // one query: cells of the seed cube / the refinement block / the ball are examined 32 at a time, the entries of a passing
 // cell are box-tested 32 at a time, the survivors are COMPACTED into a per-warp queue and evaluated exactly 32 at a time.
 // Same candidates' arithmetic, same conservative bounds, winners by (value, lowest triangle index) across lanes: the
@@ -667,7 +601,10 @@ __global__ void __launch_bounds__(WQ_WARPS * 32, WQ_MINB) grid_surface_warp_kern
     int M, const double4* __restrict__ order, const double* __restrict__ q, int T, const GridParams* __restrict__ gp,
     const int32_t* __restrict__ cell_start, const int32_t* __restrict__ entries, const float4* __restrict__ tri_box,
     const double* __restrict__ verts /*AoS*/, const int32_t* __restrict__ tri, double* __restrict__ d2,
-    int32_t* __restrict__ tri_out, double* __restrict__ cp, int descend /*GINGR_K2_DESCEND, A/B measurements*/,
+    int32_t* __restrict__ tri_out, double* __restrict__ cp,
+    int descend /*1: a coarse cell of the ball walk descends to its children; 0: it offers all its entries.  The caller
+                  passes 1; folded in as a constant, it changes the code generation, and the far-query search at 200k
+                  points took 4.94 instead of 4.89 ms (B200, 1000 W power limit)*/,
     const float4* __restrict__ entry_box /*boxes stored with the entries (static grids), may be null*/) {
   __shared__ int s_queue[WQ_WARPS][WQ_CAP];
   const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
@@ -942,27 +879,12 @@ __global__ void __launch_bounds__(WQ_WARPS * 32, WQ_MINB) grid_surface_warp_kern
   }
 }
 
-
-static bool warp_search_wanted() {
-  const char* e = getenv("GINGR_K2_WARP");   // 0: thread-per-query surface search (A/B measurements); default: warp-per-query
-  return !(e && *e && atoi(e) == 0);
-}
-
 int32_t grid_surface_enqueue(gingr_ctx* ctx, const SpatialGrid& g, int M, const double* d_q, const double* d_verts_aos,
                              const int32_t* d_tri, double* d_d2, int32_t* d_tri_out, double* d_cp, const SpatialGrid* order) {
   if (!g.built || !g.triangles) return gingr_fail(ctx, GINGR_ERR_ARG, "grid_surface: triangle grid not built");
-  if (warp_search_wanted()) {
-    static const int descend = [] { const char* e = getenv("GINGR_K2_DESCEND"); return e ? atoi(e) : 1; }();
-    static const int use_entry_boxes = [] { const char* e = getenv("GINGR_K2_ENTRY_BOXES"); return e ? atoi(e) : 1; }();
-    grid_surface_warp_kernel<<<ceil_div(M, WQ_WARPS), WQ_WARPS * 32, 0, ctx->stream>>>(
-        M, order_ptr(order, M), d_q, g.n_items, g.params.p, g.cell_start.p, g.entries.p, g.tri_box.p, d_verts_aos, d_tri, d_d2,
-        d_tri_out, d_cp, descend, (g.entry_boxes && use_entry_boxes) ? g.entry_box.p : nullptr);
-    GINGR_LAUNCHED(ctx);
-    GINGR_CUDA_TRY(ctx, cudaGetLastError());
-    return GINGR_OK;
-  }
-  grid_surface_kernel<<<ceil_div(M, 128), 128, 0, ctx->stream>>>(M, order_ptr(order, M), d_q, g.n_items, g.params.p, g.cell_start.p, g.entries.p,
-                                                                 g.tri_box.p, d_verts_aos, d_tri, d_d2, d_tri_out, d_cp);
+  grid_surface_warp_kernel<<<ceil_div(M, WQ_WARPS), WQ_WARPS * 32, 0, ctx->stream>>>(
+      M, order_ptr(order, M), d_q, g.n_items, g.params.p, g.cell_start.p, g.entries.p, g.tri_box.p, d_verts_aos, d_tri, d_d2,
+      d_tri_out, d_cp, 1, g.entry_boxes ? g.entry_box.p : nullptr);
   GINGR_LAUNCHED(ctx);
   GINGR_CUDA_TRY(ctx, cudaGetLastError());
   return GINGR_OK;

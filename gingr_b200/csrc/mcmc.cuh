@@ -587,7 +587,7 @@ static int32_t enqueue_log_transition(gingr_registration* g, const double* d_raw
   GINGR_LAUNCH(ctx, mcmc_build_system_kernel, ceil_div((r + 1) * rp, 256), 256, 0, st, r, rp, m->S.p, d_raw, 1e-5, v, v + rp, mc->sys.p,
                                                                         mc->mi.p + MI_INFO2);
   GINGR_LAUNCHED(ctx);
-  GINGR_TRY(cholesky_enqueue(ctx, r, r + 1, mc->sys.p, rp, mc->mi.p + MI_INFO2, &g->cholws));
+  GINGR_TRY(cholesky_df_enqueue(ctx, r, r + 1, mc->sys.p, rp, mc->mi.p + MI_INFO2, g->cholws));
   GINGR_TRY(chol_backsolve_enqueue(ctx, r, mc->sys.p, rp, mc->sys.p + (size_t)r * rp, v + 2 * rp, g->flags.p));
   GINGR_TRY(dense_matvec_enqueue(ctx, r, d_raw, rp, v + 2 * rp, v + 3 * rp));
   GINGR_LAUNCH(ctx, mcmc_quadform_kernel, 1, 256, 0, st, r, v + 2 * rp, v + 3 * rp, d_from_is, mc->mi.p + MI_INFO2, d_out);
@@ -939,8 +939,8 @@ static int32_t mcmc_batch_plan_build(gingr_ctx* ctx, gingr_registration** regs, 
 }
 
 // Independent chains batched on one GPU (BASELINE config 5): chain k uses seed + k.  The chains' steps run as one
-// batched kernel sequence (blockIdx.z = chain; GINGR_MCMC_BATCHED=0 or a step that is not batchable: the captured
-// per-chain step graphs replayed round-robin on a pool of streams, as gingr_update_batch does).
+// batched kernel sequence (blockIdx.z = chain; a step that is not batchable: the captured per-chain step graphs
+// replayed round-robin on a pool of streams, as gingr_update_batch does).
 int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t iters, uint64_t seed) {
   if (!regs || n <= 0 || iters < 0) return gingr_fail(nullptr, GINGR_ERR_ARG, "gingr_mcmc_batch: bad argument");
   gingr_ctx* ctx = regs[0] ? regs[0]->ctx : nullptr;
@@ -951,8 +951,7 @@ int32_t gingr_mcmc_batch(gingr_registration** regs, int32_t n, int32_t iters, ui
     regs[k]->host_mirror_current = false;
   }
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  static const int batched = [] { const char* e = getenv("GINGR_MCMC_BATCHED"); return e ? atoi(e) : 1; }();
-  if (batched && n >= 2 && n <= 65535 && graphs_enabled(ctx)) {
+  if (n >= 2 && n <= 65535 && graphs_enabled(ctx)) {
     static thread_local BatchPlan& bp = *new BatchPlan();   // never deleted (BatchPlan)
     if (!batch_plan_current(bp, ctx, regs, n, seed, 2)) {
       const int32_t rc = mcmc_batch_plan_build(ctx, regs, n, seed, bp);

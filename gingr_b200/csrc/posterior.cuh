@@ -32,9 +32,9 @@ size_t gram_packed_doubles(const GramPlan& plan);
 int32_t gram_unpack_enqueue(gingr_ctx* ctx, GramPlan& plan, const double* d_packed, int ld_out, double* d_out,
                             bool rhs_row = false);
 
-// ---- chol.cu -------------------------------------------------------------------------------------
+// ---- chol_df.cu, chol.cu -------------------------------------------------------------------------
 // In-place blocked Cholesky A = L L^T of the leading n x n block (lower triangle, row-major, pitch ld) of a
-// matrix with nrows >= n rows.  The extra rows i >= n are carried through the panel solves, so on return
+// matrix with nrows >= n rows.  The extra rows i >= n are carried through the factorisation, so on return
 // row n + q holds  L^-1 b_q  for the right-hand side b_q that was stored there (forward substitution for free).
 // d_info[0] is set to 1 if a non-positive / non-finite pivot appears (matrix not SPD).
 // Workspace of the data-flow factorisation (chol_df.cu): tile tickets / flags and the inverses of the diagonal blocks.
@@ -45,13 +45,14 @@ struct CholWs {
   int cap_n = 0, cap_nrows = 0;
   int32_t alloc(gingr_ctx* ctx, int n, int nrows);
 };
-// ws == nullptr (or GINGR_CHOL_DF=0): the kernel-per-step form of chol.cu; else one persistent data-flow kernel.
-int32_t cholesky_enqueue(gingr_ctx* ctx, int n, int nrows, double* d_A, int ld, int* d_info, CholWs* ws = nullptr);
+// One persistent data-flow kernel (chol_small_kernel for n <= 64); it publishes the inverses of the diagonal blocks in ws.
 int32_t cholesky_df_enqueue(gingr_ctx* ctx, int n, int nrows, double* d_A, int ld, int* d_info, CholWs& ws);
 // c = L^-T z  (sync-free multi-CTA backward substitution, any n).  d_flags: >= ceil(n/64) + 2 ints, zero when first
 // used (the kernel leaves them zero).
-// ws (optional): the workspace the factor was computed with by the data-flow kernel -- the back substitution then uses
-// the published inverses of the diagonal blocks (chol_df.cu); GINGR_CHOL_DF=0 or ws == nullptr: chol.cu's kernel.
+// ws: the workspace the factor was computed with -- the back substitution then uses the published inverses of the
+// diagonal blocks (chol_df.cu).  ws == nullptr: chol.cu's kernels, which read the factor alone -- for a factor whose
+// inverses in the workspace may belong to another factorisation (the Metropolis-Hastings step; an update phase that does
+// not directly follow the factorisation of its system).
 int32_t chol_backsolve_enqueue(gingr_ctx* ctx, int n, const double* d_L, int ld, const double* d_z, double* d_c,
                                int* d_flags, CholWs* ws = nullptr);
 int32_t chol_backsolve_z_enqueue(gingr_ctx* ctx, int n, const double* d_L, int ld, const double* d_z, double* d_c, CholWs& ws);

@@ -175,7 +175,7 @@ int32_t gingr_registration_posterior_model(gingr_registration* g, const gingr_st
   GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(sys.p, g->Mx_raw.p, sizeof(double) * (size_t)(r + 1) * rp, cudaMemcpyDeviceToDevice, st));
   gingr::posterior_model_rows_kernel<<<dim3(ceil_div(rp, 256), r), 256, 0, st>>>(r, rp, m->sqrt_lambda.p, sys.p + (size_t)(r + 1) * rp);
   GINGR_LAUNCHED(ctx);
-  GINGR_TRY(cholesky_enqueue(ctx, r, 2 * r + 1, sys.p, rp, info.p, &cws));
+  GINGR_TRY(cholesky_df_enqueue(ctx, r, 2 * r + 1, sys.p, rp, info.p, cws));
   GINGR_TRY(chol_backsolve_enqueue(ctx, r, sys.p, rp, sys.p + (size_t)r * rp, c.p, flags.p, &cws));
   GINGR_LAUNCH(ctx, check_finite_kernel, ceil_div(r, 256), 256, 0, st, r, c.p, info.p + 1);
   GINGR_LAUNCHED(ctx);

@@ -1125,7 +1125,7 @@ static int32_t model_build_constants(gingr_ctx* ctx, gingr_model* m) {
   GINGR_TRY(build_regression_system_enqueue(ctx, r, rp, m->S.p, 1e-5, B.p));
   CholWs cws;
   GINGR_TRY(cws.alloc(ctx, r, 2 * r));
-  GINGR_TRY(cholesky_enqueue(ctx, r, 2 * r, B.p, rp, info.p, &cws));
+  GINGR_TRY(cholesky_df_enqueue(ctx, r, 2 * r, B.p, rp, info.p, cws));
   // W0 = Rm Rm^T = Gram of Rm^T
   GINGR_CUDA_TRY(ctx, cudaMemsetAsync(Rt.p, 0, sizeof(double) * r * rp, ctx->stream));
   GINGR_TRY(transpose_enqueue(ctx, r, B.p + (size_t)r * rp, rp, Rt.p, rp));
@@ -1358,7 +1358,7 @@ static int32_t posterior_core(gingr_ctx* ctx, const gingr_model* model, const do
     gingr::posterior_model_rows_kernel<<<dim3(ceil_div(rp, 256), r), 256, 0, st>>>(r, rp, m->sqrt_lambda.p, s.Mx.p + (size_t)(r + 1) * rp);
     GINGR_LAUNCHED(ctx);
   }
-  GINGR_TRY(cholesky_enqueue(ctx, r, r + 1 + xrows, s.Mx.p, rp, s.is.p + IS_INFO, &s.cholws));
+  GINGR_TRY(cholesky_df_enqueue(ctx, r, r + 1 + xrows, s.Mx.p, rp, s.is.p + IS_INFO, s.cholws));
   double* c = s.vec.p;
   GINGR_TRY(chol_backsolve_enqueue(ctx, r, s.Mx.p, rp, rhs, c, s.flags.p, &s.cholws));
   GINGR_LAUNCH(ctx, check_finite_kernel, ceil_div(r, 256), 256, 0, st, r, c, s.is.p + IS_FAIL_POST);
@@ -1484,7 +1484,7 @@ int32_t gingr_spd_solve(gingr_ctx* ctx, int32_t n, const double* A, int32_t nrhs
   for (int it = 0; it < reps; ++it) {
     GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(work.p, in.p, sizeof(double) * (size_t)nrows * np, cudaMemcpyDeviceToDevice, st));
     GINGR_CUDA_TRY(ctx, cudaEventRecord(ev.e0, st));
-    GINGR_TRY(cholesky_enqueue(ctx, n, nrows, work.p, np, info.p, &ws));
+    GINGR_TRY(cholesky_df_enqueue(ctx, n, nrows, work.p, np, info.p, ws));
     if (nrhs > 0) GINGR_TRY(chol_backsolve_enqueue(ctx, n, work.p, np, work.p + (size_t)n * np, x.p, flags.p, &ws));
     GINGR_CUDA_TRY(ctx, cudaEventRecord(ev.e1, st));
     GINGR_CUDA_TRY(ctx, cudaEventSynchronize(ev.e1));
@@ -1923,7 +1923,7 @@ static int32_t enqueue_posterior_phase(gingr_registration* g) {
     GINGR_LAUNCHED(ctx);
   }
   g->rec(8);
-  GINGR_TRY(cholesky_enqueue(ctx, r, r + 1 + xrows, g->Mx.p, rp, g->is.p + IS_INFO, &g->cholws));
+  GINGR_TRY(cholesky_df_enqueue(ctx, r, r + 1 + xrows, g->Mx.p, rp, g->is.p + IS_INFO, g->cholws));
   return GINGR_OK;
 }
 
@@ -2398,9 +2398,8 @@ int32_t gingr_update_batch(gingr_registration** regs, int32_t n, int32_t iters, 
   if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_update_batch: chains are replicas, one ctx per GPU without a communicator");
   GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   // one batched kernel sequence per iteration for all chains (batch.cuh) when every launch of the iteration is batch-aware
-  // (the ICP flavours on the scans; the CPD E-step is not: per-chain graphs), GINGR_UPDATE_BATCHED=0: always per-chain graphs
-  static const int batched = [] { const char* e = getenv("GINGR_UPDATE_BATCHED"); return e ? atoi(e) : 1; }();
-  if (batched && n >= 2 && n <= 65535 && graphs_enabled(ctx)) {
+  // (the ICP flavours on the scans; the CPD E-step is not: per-chain graphs)
+  if (n >= 2 && n <= 65535 && graphs_enabled(ctx)) {
     static thread_local BatchPlan& bp = *new BatchPlan();   // never deleted (BatchPlan)
     const int kind = probabilistic ? 3 : 1;
     if (!batch_plan_current(bp, ctx, regs, n, seed, kind)) {

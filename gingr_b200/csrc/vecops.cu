@@ -313,9 +313,8 @@ int32_t gemvT_enqueue(gingr_ctx* ctx, int rows, int r, int rp, const double* d_p
 
 int32_t dense_matvec_enqueue(gingr_ctx* ctx, int r, const double* d_A, int ld, const double* d_x, double* d_y,
                              int* d_flag_in, int* d_flag_out) {
-  static const int two_warps = [] { const char* e = getenv("GINGR_MATVEC2"); return e ? atoi(e) : 1; }();
   // (short rows -- the rank-50 chains of C5 -- are better off with one warp per row: 856 k against 762 k MH steps/s)
-  if (two_warps && r >= 512 && (ld & 1) == 0 && ((((uintptr_t)d_A) | ((uintptr_t)d_x)) & 15) == 0)
+  if (r >= 512 && (ld & 1) == 0 && ((((uintptr_t)d_A) | ((uintptr_t)d_x)) & 15) == 0)
     GINGR_LAUNCH(ctx, dense_matvec2_kernel, ceil_div(r, 4), 256, 0, ctx->stream, r, d_A, ld, d_x, d_y, d_flag_in, d_flag_out);
   else
     GINGR_LAUNCH(ctx, dense_matvec_kernel, ceil_div(r * 32, 256), 256, 0, ctx->stream, r, d_A, ld, d_x, d_y, d_flag_in, d_flag_out);

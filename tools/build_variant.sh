@@ -12,4 +12,4 @@ nvcc -gencode arch=compute_100a,code=sm_100a -O3 -std=c++17 -lineinfo -Xcompiler
   -c gingr_b200/csrc/$SRC -o gingr_b200/lib/variants/${SRC%.cu}_$NAME.o 2> gingr_b200/lib/variants/${SRC%.cu}_$NAME.log
 OBJS=$(ls gingr_b200/lib/obj/*.o | grep -v "/${SRC%.cu}.o")
 nvcc -gencode arch=compute_100a,code=sm_100a -shared -o gingr_b200/lib/variants/libgingr_cuda_$NAME.so $OBJS gingr_b200/lib/variants/${SRC%.cu}_$NAME.o -ldl
-grep -A2 "estep_colsum\|estep_rowsum\|gram_streamk" gingr_b200/lib/variants/${SRC%.cu}_$NAME.log | grep "Used" | tr '\n' ' '; echo
+grep -A2 "estep_colsum\|estep_rowsum" gingr_b200/lib/variants/${SRC%.cu}_$NAME.log | grep "Used" | tr '\n' ' '; echo

@@ -22,15 +22,5 @@ reg.updateChain(iters)
 ms, it = reg.getProfile()
 st = reg.downloadState()
 assert np.all(np.isfinite(st.fit)) and st.status != api.STATUS_MODEL_FLEXIBILITY_ERROR
-out_t = None
-lib = ctx._lib
-if hasattr(lib, "gingr_debug_chol_timing"):
-    import ctypes
-    buf = (ctypes.c_ulonglong * 8)()
-    lib.gingr_debug_chol_timing(buf, 1)
-    names = ["loads", "chol32 (x2)", "trsm32", "A22 update", "store L", "panel rows", "store panel"]
-    tot = float(sum(buf[:7])) or 1.0
-    out_t = {n: round(100.0 * buf[k] / tot, 1) for k, n in enumerate(names)}
-    out_t["cycles_per_panel_launch"] = tot / max(1, (it + 3) * ((r + 63) // 64) + 2 * ((r + 63) // 64))
-print(json.dumps({"panel_phase_percent": out_t, "rank": r, "iters": it, "cholesky_backsolve_ms": ms[3] / it, "iteration_ms": ms[4] / it,
+print(json.dumps({"rank": r, "iters": it, "cholesky_backsolve_ms": ms[3] / it, "iteration_ms": ms[4] / it,
                   "alpha_checksum": float(np.sum(st.modelParameters.shape)), "sigma2": st.sigma2}))

@@ -1,5 +1,5 @@
 """n independent deterministic CPD registrations (M = N = 200, rank 50) through gingr_update_batch.
-usage: [GINGR_UPDATE_BATCHED=0] python tools/time_cpd_batch.py [n] [iters]"""
+usage: python tools/time_cpd_batch.py [n] [iters]"""
 import json
 import os
 import sys
@@ -28,7 +28,7 @@ t0 = time.perf_counter()
 api.update_batch(chains, iters)
 ctx.synchronize()
 dt = time.perf_counter() - t0
-print(json.dumps({"workload": f"{n} CPD registrations M=N={M} rank={r}", "batched": os.environ.get("GINGR_UPDATE_BATCHED", "1"),
+print(json.dumps({"workload": f"{n} CPD registrations M=N={M} rank={r}",
                   "chain_iterations_per_s": n * iters / dt, "ms_per_iteration_of_all_chains": dt / iters * 1e3,
                   "launches_per_iteration": (ctx.launch_count - l0) / iters,
                   "finite": bool(np.all(np.isfinite(chains[-1].downloadState().fit)))}))

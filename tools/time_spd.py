@@ -1,12 +1,12 @@
 """Cholesky + back substitution alone through gingr_spd_solve (CUDA events inside the library).
-usage: python tools/time_spd.py [n ...]   env GINGR_CUDA_LIB selects a variant build, GINGR_CHOL_DF=0 the kernel-per-step form"""
+usage: python tools/time_spd.py [n ...]   env GINGR_CUDA_LIB selects a variant build"""
 import json, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 from gingr_b200 import api
 ns = [int(a) for a in sys.argv[1:]] or [50, 200, 520, 2000]
 ctx = api.Context(0)
-out = {"lib": os.environ.get("GINGR_CUDA_LIB", "default"), "chol_df": os.environ.get("GINGR_CHOL_DF", "1")}
+out = {"lib": os.environ.get("GINGR_CUDA_LIB", "default")}
 for n in ns:
     rng = np.random.default_rng(n)
     Q = rng.normal(size=(n, n + 8))
