@@ -238,6 +238,65 @@ GINGR_API int32_t gingr_debug_posterior_system(gingr_registration* g, const ging
   return hflags[0] || hflags[1] ? GINGR_MODEL_FLEXIBILITY : GINGR_OK;
 }
 
+// Test window on the iteration's update phase (not in gingr_cuda.h): the posterior phase at the given state, then the update
+// phase as an iteration runs it, with the inputs and results of every stage copied out.  Every output may be null:
+//   L [r x r], z [r]     the factor and the forward-substituted rhs before the update phase (unpadded; upper triangle as stored)
+//   z2 [r]               the rhs row after it: z plus the Philox normals when `probabilistic` is set
+//   vec [6 x r]          c, S c, alpha*, alpha_c, q, alpha_new
+//   inst_a, inst_b, newshape, u [3M]; pro_sums [10]; ds [DS_COUNT] and is [IS_COUNT] of the state block
+//   alpha_out [r], fit [3M]   the committed coefficients and the refreshed fit
+//   S, W0 [r x r]        the model's regression constants
+// kept_factor = 1 takes the back substitution that needs the factor alone (the MH chain's kept factors).  The captured
+// iteration graph and the MH memo are dropped afterwards.
+GINGR_API int32_t gingr_debug_update_phase(gingr_registration* g, const gingr_state* state, const double* alpha,
+                                           int32_t probabilistic, uint64_t seed, int32_t kept_factor, double* L, double* z,
+                                           double* z2, double* vec, double* inst_a, double* inst_b, double* newshape,
+                                           double* u, double* pro_sums, double* ds, int32_t* is, double* alpha_out,
+                                           double* fit, double* S, double* W0) {
+  if (!g || !state || !alpha) return gingr_fail(g ? g->ctx : nullptr, GINGR_ERR_ARG, "gingr_debug_update_phase: bad argument");
+  gingr_ctx* ctx = g->ctx;
+  if (ctx->nranks != 1) return gingr_fail(ctx, GINGR_ERR_UNSUPPORTED, "gingr_debug_update_phase: single-GPU entry point");
+  const gingr_model* m = g->model;
+  const int r = m->r, rp = m->rp, M = m->M;
+  const size_t row = sizeof(double) * r, pitch = sizeof(double) * rp;
+  cudaStream_t st = ctx->stream;
+  GINGR_CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  drop_graph(g);
+  mcmc_invalidate(g);
+  g->state_valid = false;
+  g->host_mirror_current = false;
+  GINGR_TRY(upload_state(g, state, alpha));
+  GINGR_TRY(evaluate_fit(g, DS_SCALE, DS_T, DS_R));
+  GINGR_TRY(enqueue_posterior_phase(g));
+  const double* Mx = g->Mx.p;
+  if (L) GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(L, row, Mx, pitch, row, r, cudaMemcpyDeviceToHost, st));
+  if (z) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(z, Mx + (size_t)r * rp, row, cudaMemcpyDeviceToHost, st));
+  // the fit refresh writes inst_a again: it runs below, after the copies, as the update phase would have run it
+  g->skip_fit_refresh = true;
+  const int32_t rc = enqueue_update_phase(g, probabilistic, seed, /*fresh_factor=*/kept_factor == 0);
+  g->skip_fit_refresh = false;
+  GINGR_TRY(rc);
+  if (z2) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(z2, Mx + (size_t)r * rp, row, cudaMemcpyDeviceToHost, st));
+  if (vec) GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(vec, row, g->vec.p, pitch, row, 6, cudaMemcpyDeviceToHost, st));
+  const size_t pts = sizeof(double) * 3 * M;
+  if (inst_a) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(inst_a, g->inst_a.p, pts, cudaMemcpyDeviceToHost, st));
+  if (inst_b) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(inst_b, g->inst_b.p, pts, cudaMemcpyDeviceToHost, st));
+  if (newshape) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(newshape, g->newshape.p, pts, cudaMemcpyDeviceToHost, st));
+  if (u) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(u, g->u.p, pts, cudaMemcpyDeviceToHost, st));
+  if (pro_sums) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(pro_sums, g->pro_sums.p, sizeof(double) * 10, cudaMemcpyDeviceToHost, st));
+  if (ds) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(ds, g->ds.p, sizeof(double) * DS_COUNT, cudaMemcpyDeviceToHost, st));
+  if (is) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(is, g->is.p, sizeof(int) * IS_COUNT, cudaMemcpyDeviceToHost, st));
+  if (alpha_out) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(alpha_out, g->alpha.p, row, cudaMemcpyDeviceToHost, st));
+  GINGR_TRY(evaluate_fit(g, DS_SCALE, DS_T, DS_R2));
+  if (fit) GINGR_CUDA_TRY(ctx, cudaMemcpyAsync(fit, g->fit.p, pts, cudaMemcpyDeviceToHost, st));
+  if (S) GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(S, row, m->S.p, pitch, row, r, cudaMemcpyDeviceToHost, st));
+  if (W0) GINGR_CUDA_TRY(ctx, cudaMemcpy2DAsync(W0, row, m->W0.p, pitch, row, r, cudaMemcpyDeviceToHost, st));
+  GINGR_CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  drop_graph(g);
+  mcmc_invalidate(g);
+  return GINGR_OK;
+}
+
 int32_t gingr_posterior_model_profile(const gingr_ctx* ctx, double* ms, int32_t* sweeps) {
   if (!ctx || !ms) return gingr_fail(nullptr, GINGR_ERR_ARG, "gingr_posterior_model_profile: bad argument");
   for (int k = 0; k < 5; ++k) ms[k] = ctx->posterior_model_ms[k];

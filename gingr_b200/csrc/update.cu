@@ -728,7 +728,19 @@ __device__ void svd3(const double* Ain, double* U, double* S, double* V) {
       V[3 * k + j] = Vm[3 * k + c];
     }
   }
-  // a zero singular value leaves a zero column in U: complete it to a right-handed orthonormal frame
+  // zero singular values leave zero columns in U: complete it to an orthonormal frame.  Rank 1 (collinear shapes): column
+  // 1 is the normalised cross product of column 0 with the axis least aligned with it (column 0 = e_0 for Sxy = 0)
+  if (S[1] <= 0.0) {
+    if (S[0] <= 0.0) { U[0] = 1.0; U[3] = 0.0; U[6] = 0.0; }
+    const double ax = fabs(U[0]), ay = fabs(U[3]), az = fabs(U[6]);
+    const int e = (ax <= ay && ax <= az) ? 0 : (ay <= az ? 1 : 2);
+    const double w0 = e == 2 ? U[3] : (e == 1 ? -U[6] : 0.0);   // U_0 x e_e
+    const double w1 = e == 0 ? U[6] : (e == 2 ? -U[0] : 0.0);
+    const double w2 = e == 1 ? U[0] : (e == 0 ? -U[3] : 0.0);
+    const double nw = sqrt(w0 * w0 + w1 * w1 + w2 * w2);
+    U[1] = w0 / nw; U[4] = w1 / nw; U[7] = w2 / nw;
+  }
+  // rank <= 2: column 2 completes a right-handed frame
   if (S[2] <= 0.0) {
     U[2] = U[3] * U[7] - U[6] * U[4];
     U[5] = U[6] * U[1] - U[0] * U[7];
@@ -755,7 +767,9 @@ __device__ void procrustes_solve_dev(int M, const double* __restrict__ sums, dou
     const double s2x = sums[0] / M;
     for (int i = 0; i < 9; ++i) Sxy[i] = sums[1 + i] / M;
     svd3(Sxy, U, S, V);
-    const double sign = det3(Sxy) < 0.0 ? -1.0 : 1.0;
+    // Kabsch / Umeyama: R = U diag(1, 1, det U det V) V^T is the proper rotation that maximises tr(R^T Sxy).  The sign
+    // equals sign det Sxy at full rank; for a planar shape (Sxy of rank 2, det Sxy = +-0) only this form is a rotation.
+    const double sign = det3(U) * det3(V) < 0.0 ? -1.0 : 1.0;
     for (int i = 0; i < 3; ++i)
       for (int j = 0; j < 3; ++j)
         Rm[3 * i + j] = U[3 * i] * V[3 * j] + U[3 * i + 1] * V[3 * j + 1] + sign * U[3 * i + 2] * V[3 * j + 2];

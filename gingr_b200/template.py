@@ -32,7 +32,7 @@ def umeyama(X: np.ndarray, Y: np.ndarray, similarity: bool, euler_round_trip: bo
     S = (Yc.T @ Xc) / n
     U, D, Vt = np.linalg.svd(S)
     J = np.eye(3)
-    if np.linalg.det(S) < 0:
+    if np.linalg.det(U) * np.linalg.det(Vt) < 0:   # sign det S at full rank; also a rotation for planar shapes (rank 2)
         J[2, 2] = -1.0
     R = U @ J @ Vt
     s = float(np.trace(np.diag(D) @ J) / var_x) if similarity else 1.0

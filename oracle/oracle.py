@@ -329,8 +329,11 @@ def umeyama(X, Y, similarity):
     sigma2_x = float(np.sum(Xc * Xc) / n)
     Sxy = (Yc.T @ Xc) / n
     U, D, Vt = np.linalg.svd(Sxy)
+    # The reflection sign is det U det V (Kabsch / Umeyama), where the scalismo rule reads sign det Sxy.  The two agree
+    # whenever Sxy has full rank.  At rank 2 (planar shapes) det Sxy is +-0 or rounding noise and the literal rule's result
+    # depends on the SVD's sign conventions: half the time U V^T is a reflection.  det U det V makes it a rotation always.
     S = np.eye(3)
-    if np.linalg.det(Sxy) < 0:
+    if np.linalg.det(U) * np.linalg.det(Vt) < 0:
         S[2, 2] = -1.0
     R = U @ S @ Vt
     c = float(np.trace(np.diag(D) @ S) / sigma2_x) if similarity else 1.0
